@@ -2,6 +2,7 @@
 """bench.py -- event-detection throughput of the sigtk B200 hot path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads-per-step B] [--mode event+pa|event]
+                  [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (pA conversion + event detection, event table out, pA materialised in the
 default `event+pa` mode) over one device-resident batch of B synthetic DNA reads drawn from the 1,000,000-read
@@ -18,6 +19,9 @@ data path; torch.distributed is used for the barrier and the max-over-ranks only
 
 --impl reference times the reference's CPU path on all host threads (one reference call chain per thread over
 disjoint reads) and prints the same line with "impl": "reference".
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as .npy files, so that two builds can be compared
+output for output on the same inputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -480,9 +484,10 @@ def run_ours(args):
     B_step = sum(p["n_reads"] for p in pool) // len(pool)
     torch.cuda.synchronize()
     ev0.record()
+    last = None
     for k in range(args.steps):          # the timed region: K steps launched back to back, no host synchronisation
         p = pool[(args.warmup + k) % pool_n]
-        step(p)
+        last = (p, step(p))
         n_samples += p["n_samples"]
         n_reads += p["n_reads"]
     ev1.record()
@@ -490,6 +495,8 @@ def run_ours(args):
     if dist:
         dist.barrier()
     ms_total = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0 and last is not None:  # before the next run overwrites the result buffers
+        dump_outputs(ctx, *last, pa_mode, args.dump_outputs)
     # per-kernel times: the same K steps once more, the stage events (CUDA events on the launch stream) read after
     # every step. Reading them inside the timed region costs a host synchronisation per step: 1 % of the step with one
     # rank on the box, 8 % with eight (r02: 5.61 ms against 5.18).
@@ -637,6 +644,50 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_SEED = 20261020
+DUMP_BYTES = 56 << 20
+
+
+def dump_outputs(ctx, batch, res, pa_mode: bool, out_dir: str) -> None:
+    """The result of one device-resident step as .npy files: event counts of every read, and for a seeded sample of
+    reads (picked from the read lengths only, so every build picks the same reads) their events and pA. The sample
+    takes at most DUMP_BYTES (a read of L samples has at most L // 3 + 1 events of 16 bytes, and 4 bytes of pA a sample).
+      read_index   float64[k]    the sampled reads (batch order)
+      read_length  float64[k]    their lengths in samples (pa holds them read after read)
+      event_count  float64[n]    events of every read of the batch
+      event_off    float64[k+1]  the sampled reads' events in event_start / event_mean / event_stdv
+      event_start  float64       sample index of each event start
+      event_mean   float32, event_stdv float32
+      pa           float32       (event+pa mode) the sampled reads' pA samples, read after read"""
+    n = batch["n_reads"]
+    off, lens = batch["host_off"], batch["host_len"]
+    ev_off = ctx.d2h(res.ev_off, np.uint64, n + 1).astype(np.int64)
+    picked, budget = [], DUMP_BYTES
+    for r in np.random.default_rng(DUMP_SEED).permutation(n)[:256]:
+        cost = 4 * int(lens[r]) + 16 * (int(lens[r]) // 3 + 1)
+        if cost <= budget:
+            picked.append(int(r))
+            budget -= cost
+    picked = np.sort(np.array(picked, dtype=np.int64))
+    a, b = ev_off[picked], ev_off[picked + 1]
+    part = lambda ptr, dtype, lo, cnt: ctx.d2h(ptr + np.dtype(dtype).itemsize * int(lo), dtype, int(cnt))
+    cat = lambda xs, dtype: np.concatenate(xs) if len(xs) else np.zeros(0, dtype)
+    out = {
+        "read_index": picked.astype(np.float64),
+        "read_length": lens[picked].astype(np.float64),
+        "event_count": np.diff(ev_off).astype(np.float64),
+        "event_off": np.concatenate([[0], np.cumsum(b - a)]).astype(np.float64),
+        "event_start": cat([part(res.ev_start, np.uint32, x, y - x) for x, y in zip(a, b)], np.uint32).astype(np.float64),
+        "event_mean": cat([part(res.ev_mean, np.float32, x, y - x) for x, y in zip(a, b)], np.float32),
+        "event_stdv": cat([part(res.ev_stdv, np.float32, x, y - x) for x, y in zip(a, b)], np.float32),
+    }
+    if pa_mode:
+        out["pa"] = cat([part(res.pa, np.float32, off[r], lens[r]) for r in picked], np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def run_e2e(args, sg, torch, dev, local, batch, want, pa_mode, dist, rna=0, n_reads=None, ceiling=False):
     """K steps of (pinned slot -> H2D -> kernels -> D2H -> host-visible event table), two slots in flight."""
     B = min(n_reads or args.e2e_reads, batch["n_reads"])
@@ -770,6 +821,8 @@ def main():
     ap.add_argument("--chunk-len", type=int, default=0, help="development: samples per detector chunk (0 = automatic)")
     ap.add_argument("--detector-warmup", type=int, default=0, help="development: detector warm-up in samples (0 = default)")
     ap.add_argument("--no-affinity", action="store_true", help="do not pin the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

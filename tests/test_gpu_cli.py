@@ -1,4 +1,4 @@
-"""The drop-in command line (cli/sigtk: C99 host + slow5lib + libsigtk_b200.so) against the stdout of the compiled,
+"""The drop-in command line (cli/sigtk: C99 host + libsigtk_b200.so) against the stdout of the compiled,
 unmodified reference (fixtures in tests/golden/, made by make_golden.py). Byte for byte."""
 import gzip
 import hashlib
@@ -8,6 +8,8 @@ import shutil
 import subprocess
 
 import pytest
+import _refcases
+from _blow5 import npz_reads, write_blow5
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -17,14 +19,14 @@ SHA = json.load(open(os.path.join(G, "sha256.json")))
 
 
 def run(args, **kw):
-    assert os.path.exists(CLI), "cli/sigtk is built by __graft_entry__.build() in the build container"
+    assert os.path.exists(CLI), "cli/sigtk is built by __graft_entry__.build()"
     return subprocess.run([CLI] + args, check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE, **kw)
 
 
 @pytest.fixture(scope="module")
 def sp1(tmp_path_factory):
     d = tmp_path_factory.mktemp("blow5")
-    shutil.copy(os.path.join(G, "sp1_dna.blow5"), d / "sp1_dna.blow5")  # read-id access writes an index beside it
+    shutil.copy(os.path.join(G, "sp1_dna.blow5"), d / "sp1_dna.blow5")  # the tests run on a copy, never on the tree
     return str(d / "sp1_dna.blow5")
 
 
@@ -92,7 +94,6 @@ def test_no_header_version_help_and_errors(sp1):
 def test_ent_equals_the_reference_stdout(sp1, tmp_path):
     """`sigtk ent` (src/ent.c): stdout of the compiled reference on the DNA file, the synthetic RNA file and a BLOW5 of
     reads with wide / wrapped / single-bin histograms (tests/golden/ent_adversarial.npz); its own option set"""
-    import struct
     import numpy as np
     exp = open(os.path.join(G, "ref_sp1_ent.txt"), "rb").read()
     p = run(["ent", sp1])
@@ -106,18 +107,8 @@ def test_ent_equals_the_reference_stdout(sp1, tmp_path):
     assert r.returncode == 1 and r.stderr.startswith(b"Usage: sigtk ent a.blow5\n")
     r = subprocess.run([CLI, "ent", "/nonexistent.blow5"], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
     assert r.returncode == 1 and b"Error in opening file" in r.stderr
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "blow5_write")):
-        return
-    d = np.load(os.path.join(G, "ent_adversarial.npz"))
     path = str(tmp_path / "ent_adv.blow5")
-    w = subprocess.Popen([os.path.join(ROOT, "oracle", "_ref", "blow5_write"), path, "genomic_dna"], stdin=subprocess.PIPE)
-    for r in range(len(d["read_ids"])):
-        raw = d["samples"][int(d["read_off"][r]):int(d["read_off"][r + 1])]
-        rid = str(d["read_ids"][r]).encode()
-        w.stdin.write(struct.pack("<I", len(rid)) + rid + struct.pack("<Qddd", len(raw), float(d["digitisation"][r]),
-                      float(d["offset"][r]), float(d["range"][r])) + raw.tobytes())
-    w.stdin.close()
-    assert w.wait() == 0
+    write_blow5(path, "genomic_dna", npz_reads(np.load(os.path.join(G, "ent_adversarial.npz"))))
     assert run(["ent", path]).stdout == open(os.path.join(G, "ref_ent_adversarial.txt"), "rb").read()
 
 
@@ -125,7 +116,6 @@ def test_ent_equals_the_reference_stdout(sp1, tmp_path):
 def test_jnn_equals_the_reference_stdout(sp1, tmp_path, kind):
     """`sigtk jnn` and `jnn -c` (src/jnn.c): stdout of the compiled reference on the DNA file / the synthetic RNA file
     and on a BLOW5 of reads with stalls (tests/golden/jnn_stalls_*.npz)"""
-    import struct
     import numpy as np
     path, tag = (sp1, "sp1") if kind == "dna" else (RNA, "rna")
     p = run(["jnn", path])
@@ -133,19 +123,8 @@ def test_jnn_equals_the_reference_stdout(sp1, tmp_path, kind):
     assert (b"RNA data detected." if kind == "rna" else b"DNA data detected.") in p.stderr
     assert run(["jnn", "-c", "--batch-samples", "30000", path]).stdout == open(os.path.join(G, f"ref_{tag}_jnn_c.txt"), "rb").read()
     assert run(["jnn", "--cpu-decode", "-n", path]).stdout == open(os.path.join(G, f"ref_{tag}_jnn.txt"), "rb").read().split(b"\n", 1)[1]
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "blow5_write")):
-        return
-    d = np.load(os.path.join(G, f"jnn_stalls_{kind}.npz"))
     path = str(tmp_path / "stalls.blow5")
-    w = subprocess.Popen([os.path.join(ROOT, "oracle", "_ref", "blow5_write"), path, "rna" if kind == "rna" else "genomic_dna"],
-                         stdin=subprocess.PIPE)
-    for r in range(len(d["read_ids"])):
-        raw = d["samples"][int(d["read_off"][r]):int(d["read_off"][r + 1])]
-        rid = str(d["read_ids"][r]).encode()
-        w.stdin.write(struct.pack("<I", len(rid)) + rid + struct.pack("<Qddd", len(raw), float(d["digitisation"][r]),
-                      float(d["offset"][r]), float(d["range"][r])) + raw.tobytes())
-    w.stdin.close()
-    assert w.wait() == 0
+    write_blow5(path, "rna" if kind == "rna" else "genomic_dna", npz_reads(np.load(os.path.join(G, f"jnn_stalls_{kind}.npz"))))
     assert run(["jnn", path]).stdout == open(os.path.join(G, f"ref_jnn_stalls_{kind}.txt"), "rb").read()
     assert run(["jnn", "-c", path]).stdout == open(os.path.join(G, f"ref_jnn_stalls_{kind}_c.txt"), "rb").read()
 
@@ -155,7 +134,6 @@ def test_prefix_equals_the_reference_stdout(sp1, tmp_path, kind):
     """`sigtk prefix` and `prefix --print-stat` (src/cfunc.c:169-234): the reference's own golden test/prefix_dna.exp,
     the stdout of the compiled reference on the DNA file / the synthetic RNA file and on a BLOW5 of reads with adaptor
     and poly-A like stretches (tests/golden/prefix_adaptor_*.npz)"""
-    import struct
     import numpy as np
     path, tag = (sp1, "sp1") if kind == "dna" else (RNA, "rna")
     exp_stat = open(os.path.join(G, f"ref_{tag}_prefix_stat.txt"), "rb").read()
@@ -165,19 +143,8 @@ def test_prefix_equals_the_reference_stdout(sp1, tmp_path, kind):
     if kind == "dna":
         assert run(["prefix", path]).stdout == open(os.path.join(G, "prefix_dna.exp"), "rb").read()
     assert run(["prefix", "--print-stat", "--cpu-decode", "--batch-samples", "60000", "-n", path]).stdout == exp_stat.split(b"\n", 1)[1]
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "blow5_write")):
-        return
-    d = np.load(os.path.join(G, f"prefix_adaptor_{kind}.npz"))
     path = str(tmp_path / "adaptor.blow5")
-    w = subprocess.Popen([os.path.join(ROOT, "oracle", "_ref", "blow5_write"), path, "rna" if kind == "rna" else "genomic_dna"],
-                         stdin=subprocess.PIPE)
-    for r in range(len(d["read_ids"])):
-        raw = d["samples"][int(d["read_off"][r]):int(d["read_off"][r + 1])]
-        rid = str(d["read_ids"][r]).encode()
-        w.stdin.write(struct.pack("<I", len(rid)) + rid + struct.pack("<Qddd", len(raw), float(d["digitisation"][r]),
-                      float(d["offset"][r]), float(d["range"][r])) + raw.tobytes())
-    w.stdin.close()
-    assert w.wait() == 0
+    write_blow5(path, "rna" if kind == "rna" else "genomic_dna", npz_reads(np.load(os.path.join(G, f"prefix_adaptor_{kind}.npz"))))
     assert run(["prefix", path]).stdout == open(os.path.join(G, f"ref_prefix_adaptor_{kind}.txt"), "rb").read()
     assert run(["prefix", "--print-stat", path]).stdout == open(os.path.join(G, f"ref_prefix_adaptor_{kind}_stat.txt"), "rb").read()
 
@@ -193,7 +160,7 @@ def test_two_gpus_same_bytes(sp1):
 
 def test_cpu_decode_flag_gives_the_same_bytes(sp1):
     """sp1_dna.blow5 is zlib + svb-zd: by default the svb-zd streams are decoded on the GPU (svbzd.cu); --cpu-decode
-    keeps slow5_decode on the host threads. Both equal the reference."""
+    decodes them on the host threads (cli/blow5.c). Both equal the reference."""
     exp = open(os.path.join(G, "ref_sp1_event_c.txt"), "rb").read()
     assert run(["event", "-c", "--cpu-decode", sp1]).stdout == exp
     p = run(["event", "-c", sp1], env=dict(os.environ, SIGTK_PROFILE="1"))
@@ -204,41 +171,18 @@ def test_cpu_decode_flag_gives_the_same_bytes(sp1):
     assert run(["stat", "--batch-samples", "30000", sp1]).stdout == open(os.path.join(G, "ref_sp1_stat.txt"), "rb").read()
 
 
-REF_CLI = os.path.join(ROOT, "oracle", "_ref", "sigtk")
-WRITE = os.path.join(ROOT, "oracle", "_ref", "blow5_write")
+REF_OUT = json.load(open(os.path.join(G, "ref_outputs.json")))
 
 
-@pytest.mark.skipif(not (os.path.exists(REF_CLI) and os.path.exists(WRITE)), reason="oracle/_ref not built")
-@pytest.mark.parametrize("kind", ["genomic_dna", "rna"])
+@pytest.mark.parametrize("kind", _refcases.FUZZ_KINDS)
 def test_adversarial_blow5_against_the_reference_binary(tmp_path, kind):
-    """a BLOW5 (zlib + svb-zd) of reads with glitches (pA <= 0), flat stretches, ramps, steps and saturation,
-    written with the reference's slow5lib; stdout of `event`, `event -c`, `stat` and `pa` must equal the stdout of
-    the compiled unmodified reference, byte for byte (reads on which the reference aborts are left out: n < 200,
-    constant chunks)"""
-    import struct
-    import numpy as np
-    from test_gpu_parity import _fuzz_read
-    rng = np.random.default_rng(11 if kind == "rna" else 7)
+    """a BLOW5 (zlib + svb-zd) of reads with glitches (pA <= 0), flat stretches, ramps, steps and saturation
+    (_refcases.fuzz_reads); stdout of `event`, `event -c`, `stat` and `pa` must equal the stdout of the compiled
+    unmodified reference on the same file, byte for byte (sha256 in tests/golden/ref_outputs.json, the `stat`
+    stdout in ref_fuzz_<kind>_stat.txt; made by make_ref_outputs.py)"""
     path = str(tmp_path / "fuzz.blow5")
-    p = subprocess.Popen([WRITE, path, kind], stdin=subprocess.PIPE)
-    k = n_written = 0
-    while n_written < 150:
-        raw, dig, off, rg = _fuzz_read(rng, k)
-        k += 1
-        if len(raw) < 1000:
-            continue
-        # the reference's dead trimming step asserts on chunk-wise constant signals (events.c:242): keep reads whose
-        # first and last 200 samples vary
-        if np.ptp(raw[:200]) < 20 or np.ptp(raw[-200:]) < 20:
-            continue
-        rid = f"fuzz-{k:05d}".encode()
-        p.stdin.write(struct.pack("<I", len(rid)) + rid + struct.pack("<Qddd", len(raw), dig, off, rg) + raw.tobytes())
-        n_written += 1
-    p.stdin.close()
-    assert p.wait() == 0
+    write_blow5(path, kind, _refcases.fuzz_reads(kind))
+    assert run(["stat", path]).stdout == open(os.path.join(G, f"ref_fuzz_{kind}_stat.txt"), "rb").read()
     for args in (["event", "-c"], ["event"], ["stat"], ["pa"]):
-        ref = subprocess.run([REF_CLI] + args + [path], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-        if ref.returncode != 0:
-            pytest.skip("the reference aborted on this input: " + ref.stderr.decode(errors="replace")[-200:])
         ours = run(args + [path])
-        assert ours.stdout == ref.stdout, args
+        assert hashlib.sha256(ours.stdout).hexdigest() == REF_OUT["fuzz"][kind][" ".join(args)], args

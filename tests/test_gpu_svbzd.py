@@ -1,14 +1,17 @@
 """GPU parity of the svb-zd decoder (sigtk_b200/csrc/svbzd.cu) through the C-ABI: samples decoded in HBM from the
 streams slow5lib stores in BLOW5 records must equal the reference's own decode (golden streams written by the
-reference's slow5lib, the oracle, and -- where oracle/_ref is built -- slow5_ptr_depress_solo itself), and the
+reference's slow5lib, streams checked byte for byte against the reference's by their sha256, the oracle), and the
 whole path (streams in -> events / pA / stat out) must equal the path fed with decoded records."""
+import hashlib
+import json
 import os
 
 import numpy as np
 import pytest
 
 import sigtk_b200 as sg
-from _oracle import Oracle, Reference, have_ref
+import _refcases
+from _oracle import Oracle
 from sigtk_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -61,13 +64,15 @@ def test_wraparound(ctx, orc):
     assert np.array_equal(decode_on_gpu(ctx, [stream])[0], raw.astype(np.int64))
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built")
-def test_streams_written_by_reference_slow5lib(ctx):
-    ref = Reference()
-    reads = synth.make_reads(24, mean=30000.0, seed=91)
-    streams = [ref.svbzd_encode(r[0]) for r in reads]
-    for g, r in zip(decode_on_gpu(ctx, streams), reads):
-        assert np.array_equal(g, r[0].astype(np.int64))
+def test_streams_written_by_reference_slow5lib(ctx, orc):
+    """the streams the reference's slow5lib writes for 24 synthetic reads (each made here and checked against the
+    sha256 of the reference's bytes in tests/golden/ref_outputs.json) decode on the GPU to the reads"""
+    raws = _refcases.svbzd_reads()
+    want = json.load(open(os.path.join(G, "ref_outputs.json")))["svbzd_reads"]
+    streams = [orc.svbzd_encode(r) for r in raws]
+    assert [hashlib.sha256(s.tobytes()).hexdigest() for s in streams] == want
+    for g, r in zip(decode_on_gpu(ctx, streams), raws):
+        assert np.array_equal(g, r.astype(np.int64))
 
 
 @pytest.mark.parametrize("rna", [0, 1])

@@ -1,19 +1,28 @@
 """Pins the CPU oracle (oracle/sigtk_oracle.c) to the reference:
    - the reference's own golden file test/event_dna.exp (scripts/test.sh:70-72),
    - stdout of the compiled, unmodified reference (fixtures in tests/golden/, made by make_golden.py),
-   - the compiled reference functions themselves (oracle/_ref) on seeded synthetic reads, when present.
+   - stdout of the compiled reference and the svb-zd streams of its slow5lib on seeded synthetic reads
+     (sha256 in tests/golden/ref_outputs.json, made by make_ref_outputs.py).
 CPU only."""
 import gzip
+import hashlib
+import json
 import os
 
 import numpy as np
 import pytest
 
 import _fmt
-from _oracle import Oracle, Reference, have_ref
+import _refcases
+from _oracle import Oracle
 from sigtk_b200 import synth
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF_OUT = json.load(open(os.path.join(G, "ref_outputs.json")))
+
+
+def _sha(b):
+    return hashlib.sha256(b).hexdigest()
 
 
 @pytest.fixture(scope="module")
@@ -161,20 +170,18 @@ def test_prefix_dna_exp(orc, sp1):
     assert got == open(os.path.join(G, "prefix_dna.exp")).read()
 
 
-def _bits(a):
-    return a.view(np.uint32) if a.dtype == np.float32 else a
-
-
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
-@pytest.mark.parametrize("rna_flag,seed", [(0, 1), (0, 2), (1, 3)])
+@pytest.mark.parametrize("rna_flag,seed", _refcases.ORACLE_CASES)
 def test_oracle_equals_compiled_reference(orc, rna_flag, seed):
-    ref = Reference()
-    for rd in synth.make_reads(8, mean=15000.0, seed=seed, rna=bool(rna_flag)):
-        a, b = orc.events(*rd, rna=rna_flag), ref.events(*rd, rna=rna_flag)
-        for x, y in zip(a, b):
-            assert np.array_equal(_bits(x), _bits(y))
-        assert np.array_equal(_bits(orc.pa(*rd)), _bits(ref.pa(*rd)))
-        assert np.array_equal(_bits(orc.stat(*rd)), _bits(ref.stat(*rd)))
+    """the oracle's events, pA and stat of seeded synthetic reads, printed as the reference prints them, equal the
+    stdout of the compiled reference's `sigtk event`, `pa` and `stat` on a BLOW5 of the same reads"""
+    out = {"event": [_fmt.EVENT_HDR_LONG], "pa": [_fmt.PA_HDR], "stat": [_fmt.STAT_HDR]}
+    for rid, *rd in _refcases.oracle_reads(rna_flag, seed):
+        out["event"].append(_fmt.event_long(rid, *orc.events(*rd, rna=rna_flag)))
+        out["pa"].append(_fmt.pa_line(rid, orc.pa(*rd)))
+        out["stat"].append(_fmt.stat_line(rid, len(rd[0]), orc.stat(*rd)))
+    want = REF_OUT["oracle"][f"{rna_flag}-{seed}"]
+    for mode, parts in out.items():
+        assert _sha("".join(parts).encode()) == want[mode], mode
 
 
 def test_stagewise_consistency(orc):
@@ -239,16 +246,15 @@ def test_svbzd_malformed_rejected(orc, svb_golden):
     assert orc.svbzd_decode(st[:3]) is None                       # no header
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 def test_svbzd_equals_compiled_reference(orc):
-    ref = Reference()
-    rng = np.random.default_rng(5)
-    for n in (0, 1, 2, 3, 4, 5, 31, 32, 33, 1023, 1024, 1025, 4097, 50001):
-        for scale in (3, 200, 40000):
-            raw = np.clip(np.cumsum(rng.integers(-scale, scale + 1, n)), -32768, 32767).astype(np.int16)
-            a, b = orc.svbzd_encode(raw), ref.svbzd_encode(raw)
-            assert np.array_equal(a, b)
-            assert np.array_equal(orc.svbzd_decode(a), raw) and np.array_equal(ref.svbzd_decode(a), raw)
+    """the oracle's svb-zd encoder writes the bytes the reference's slow5lib stores (sha256 of each stream), and
+    decodes them back"""
+    raws = _refcases.svbzd_grid()
+    assert len(raws) == len(REF_OUT["svbzd_grid"])
+    for raw, want in zip(raws, REF_OUT["svbzd_grid"]):
+        a = orc.svbzd_encode(raw)
+        assert _sha(a.tobytes()) == want, len(raw)
+        assert np.array_equal(orc.svbzd_decode(a), raw)
 
 
 def test_synthetic_svbzd_encoder_equals_oracle(orc):
