@@ -6,6 +6,7 @@
 // kernels themselves are serialised (they share one scratch area).
 #include "../../include/sigtk_b200.h"
 
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -17,19 +18,64 @@ using namespace sgpu;
 
 namespace {
 
-struct DevOut {  // device-side outputs of one batch
-    uint64_t* ev_off = nullptr;
-    uint32_t* ev_start = nullptr;
-    float* ev_mean = nullptr;
-    float* ev_stdv = nullptr;
-    float* pa = nullptr;
-    float* stat = nullptr;
-    double* ent = nullptr;  // [max_reads][3], allocated on first use
-    uint32_t* jnn_cnt = nullptr;  // [max_reads], allocated on first use
-    int32_t* jnn_seg = nullptr;   // [2 * jnn_seg_capacity]
-    int32_t* prefix_pos = nullptr;   // [max_reads][4], allocated on first use
-    float* prefix_stat = nullptr;    // [max_reads][6]
+// The per-batch output arrays. OUTS describes each one once; every place that allocates, clears, copies back,
+// returns or frees outputs loops over it. Device and pinned host copies are arrays of N_OUT pointers indexed by Out.
+enum Out { EV_OFF, EV_START, EV_MEAN, EV_STDV, SEQ_ORDER, FIXUPS, STAT, ENT, JNN_CNT, JNN_SEG, PREFIX_POS, PREFIX_STAT,
+           PA, N_OUT };
+
+// what an output's element count is proportional to (times OutSpec::per)
+enum Count : uint8_t {
+    READS, READS_PLUS_1, EVENTS,
+    SAMPLES,    // of the batch's span
+    JNN_SLOTS,  // jnn_seg_capacity(): segment slots of the span's reads (SGPU_JNN_BASE)
 };
+
+constexpr int ANY_WANT = 0x100;  // OutSpec::empty flag: cleared for an empty batch whatever the want
+
+struct OutSpec {
+    size_t field;    // offset of its pointer in sgpu_result_t
+    uint32_t size;   // bytes per element
+    uint32_t want;   // SGPU_WANT_* bit of the product it belongs to
+    Count count;
+    uint32_t per;
+    bool eager;      // allocated at creation (returned by every sgpu_run_device), else on the first run that wants it
+    int empty;       // byte every element holds for a batch of empty records (| ANY_WANT), or -1: left as it is
+};
+
+#define OUTPUT(field, want, count, per, eager, empty) \
+    { offsetof(sgpu_result_t, field), sizeof *sgpu_result_t{}.field, want, count, per, eager, empty }
+constexpr OutSpec OUTS[] = {  // in the order of Out
+    //     field        want              count         per  eager  empty
+    OUTPUT(ev_off,      SGPU_WANT_EVENTS, READS_PLUS_1, 1,   true,  0 | ANY_WANT),
+    OUTPUT(ev_start,    SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
+    OUTPUT(ev_mean,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
+    OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
+    OUTPUT(seq_order,   SGPU_WANT_EVENTS, READS,        1,   true,  0),
+    OUTPUT(fixups,      SGPU_WANT_EVENTS, READS,        1,   true,  0),
+    OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0),
+    OUTPUT(ent,         SGPU_WANT_ENT,    READS,        3,   false, 0),
+    OUTPUT(jnn_cnt,     SGPU_WANT_JNN,    READS,        1,   false, 0),
+    OUTPUT(jnn_seg,     SGPU_WANT_JNN,    JNN_SLOTS,    2,   false, -1),
+    OUTPUT(prefix_pos,  SGPU_WANT_PREFIX, READS,        4,   false, 0xff),  // -1: not longer than the window
+    OUTPUT(prefix_stat, SGPU_WANT_PREFIX, READS,        6,   false, 0),
+    OUTPUT(pa,          SGPU_WANT_PA,     SAMPLES,      1,   false, -1),
+};
+#undef OUTPUT
+static_assert(sizeof OUTS / sizeof OUTS[0] == N_OUT, "one row per output");
+
+// elements of output k for a batch of `reads` reads spanning `samples` samples with `events` events; at the
+// context's (max_reads, max_samples, ev_cap) this is the output's capacity
+uint64_t out_elems(int k, uint64_t reads, uint64_t samples, uint64_t events) {
+    const OutSpec& s = OUTS[k];
+    switch (s.count) {
+        case READS: return s.per * reads;
+        case READS_PLUS_1: return s.per * (reads + 1);
+        case EVENTS: return s.per * events;
+        case SAMPLES: return s.per * samples;
+        case JNN_SLOTS: return s.per * jnn_seg_capacity(samples, (uint32_t)reads);
+    }
+    return 0;
+}
 
 struct Slot {
     // pinned host input
@@ -41,23 +87,8 @@ struct Slot {
     uint32_t* d_read_len = nullptr;
     float* d_offset = nullptr;
     float* d_unit = nullptr;
-    DevOut dout;
-    uint32_t* d_seq = nullptr;
-    uint32_t* d_fix = nullptr;
-    // pinned host output
-    uint64_t* h_ev_off = nullptr;
-    uint32_t* h_ev_start = nullptr;
-    float* h_ev_mean = nullptr;
-    float* h_ev_stdv = nullptr;
-    float* h_pa = nullptr;
-    float* h_stat = nullptr;
-    double* h_ent = nullptr;
-    uint32_t* h_jnn_cnt = nullptr;
-    int32_t* h_jnn_seg = nullptr;
-    int32_t* h_prefix_pos = nullptr;
-    float* h_prefix_stat = nullptr;
-    uint32_t* h_seq = nullptr;
-    uint32_t* h_fix = nullptr;
+    void* dout[N_OUT] = {};  // device outputs
+    void* hout[N_OUT] = {};  // their pinned host copies
     unsigned long long* h_counters = nullptr;  // [4]
     int* h_status = nullptr;
     cudaStream_t stream = nullptr;
@@ -84,9 +115,7 @@ struct sgpu_ctx {
     uint32_t flags = 0;
     uint64_t ev_cap = 0;
     Scratch sc{};
-    DevOut dev_out;              // outputs of the device-resident path
-    uint32_t* dev_seq = nullptr; // seq_order / fixups of the device-resident path
-    uint32_t* dev_fix = nullptr;
+    void* dev_out[N_OUT] = {};   // outputs of the device-resident path
     Slot* slots = nullptr;
     SvbScratch svb{};            // workspace of the svb-zd decoder (allocated on first use)
     float* jnn_mom = nullptr;    // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
@@ -118,38 +147,61 @@ bool cuda_fail(sgpu_ctx* c, cudaError_t e, const char* what, int line) {
         if (cuda_fail(ctx, (call), #call, __LINE__)) return SGPU_E_CUDA; \
     } while (0)
 
+// Allocates *p unless it is set already, and sets it only on success: an allocation that failed part-way through
+// a list is completed by the next call instead of leaving a NULL pointer behind a non-NULL one.
+cudaError_t alloc_once(void** p, size_t bytes, bool pinned) {
+    if (*p) return cudaSuccess;
+    void* q = nullptr;
+    const cudaError_t e = pinned ? cudaHostAlloc(&q, bytes, cudaHostAllocDefault) : cudaMalloc(&q, bytes);
+    if (e == cudaSuccess) *p = q;
+    return e;
+}
 template <typename T>
 cudaError_t dev_alloc(T** p, uint64_t count) {
-    return cudaMalloc(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T));
+    return alloc_once(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T), false);
 }
 template <typename T>
 cudaError_t pin_alloc(T** p, uint64_t count) {
-    return cudaHostAlloc(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T), cudaHostAllocDefault);
+    return alloc_once(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T), true);
 }
 
 uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 
-__global__ void fill_u32_kernel(uint32_t* p, uint32_t n, uint32_t v) {
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = v;
+// allocates (device or pinned) every output of `o` that is eager or belongs to `want` and does not exist yet
+cudaError_t alloc_outputs(const sgpu_ctx* ctx, void** o, uint32_t want, bool pinned) {
+    for (int k = 0; k < N_OUT; k++) {
+        if (!OUTS[k].eager && !(want & OUTS[k].want)) continue;
+        const uint64_t n = out_elems(k, ctx->max_reads, ctx->max_samples, ctx->ev_cap);
+        const cudaError_t e = alloc_once(&o[k], (size_t)n * OUTS[k].size, pinned);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
-__global__ void set_u64_kernel(unsigned long long* p, unsigned long long v) { *p = v; }
-
-int alloc_dev_out(sgpu_ctx* ctx, DevOut& o) {
-    CU(dev_alloc(&o.ev_off, (uint64_t)ctx->max_reads + 1));
-    CU(dev_alloc(&o.ev_start, ctx->ev_cap));
-    CU(dev_alloc(&o.ev_mean, ctx->ev_cap));
-    CU(dev_alloc(&o.ev_stdv, ctx->ev_cap));
-    CU(dev_alloc(&o.stat, (uint64_t)ctx->max_reads * 6));
-    o.pa = nullptr;  // allocated on first use (4 B/sample)
-    return SGPU_OK;
+void free_outputs(void** o, bool pinned) {
+    for (int k = 0; k < N_OUT; k++) {
+        if (pinned) cudaFreeHost(o[k]); else cudaFree(o[k]);
+    }
 }
 
-void free_dev_out(DevOut& o) {
-    cudaFree(o.ev_off); cudaFree(o.ev_start); cudaFree(o.ev_mean); cudaFree(o.ev_stdv);
-    cudaFree(o.pa); cudaFree(o.stat); cudaFree(o.ent); cudaFree(o.jnn_cnt); cudaFree(o.jnn_seg);
-    cudaFree(o.prefix_pos); cudaFree(o.prefix_stat);
-    o = DevOut{};
+// points the fields of *r at the outputs of `want`, and at every eager output when `all_eager`; the others stay NULL
+void fill_result(sgpu_result_t* r, void* const* o, uint32_t want, bool all_eager) {
+    for (int k = 0; k < N_OUT; k++)
+        if ((want & OUTS[k].want) || (all_eager && OUTS[k].eager))
+            memcpy(reinterpret_cast<char*>(r) + OUTS[k].field, &o[k], sizeof(void*));
+}
+
+// queues on the slot's stream the D2H copy of every output of `want` that is sized by the batch's reads and samples,
+// or (by_events) of every one sized by its n_events
+cudaError_t queue_d2h(Slot& sl, uint32_t want, bool by_events, uint64_t n_events) {
+    for (int k = 0; k < N_OUT; k++) {
+        if (!(want & OUTS[k].want) || (OUTS[k].count == EVENTS) != by_events) continue;
+        const uint64_t n = out_elems(k, sl.batch.n_reads, sl.used, n_events);
+        const cudaError_t e = cudaMemcpyAsync(sl.hout[k], sl.dout[k], (size_t)n * OUTS[k].size, cudaMemcpyDeviceToHost,
+                                              sl.stream);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 struct StageMarks {  // records a CUDA event between kernel groups when the context has stage timers
@@ -172,10 +224,8 @@ struct StageMarks {  // records a CUDA event between kernel groups when the cont
     }
 };
 
-// The kernel sequence of one batch. No host synchronisation, no host<->device copies.
 int alloc_svb_scratch(sgpu_ctx* ctx) {
     SvbScratch& w = ctx->svb;
-    if (w.cnt) return SGPU_OK;
     w.max_blocks = svbzd_max_blocks(ctx->max_samples, ctx->max_reads);
     CU(dev_alloc(&w.cnt, ctx->max_reads));
     CU(dev_alloc(&w.base, (uint64_t)ctx->max_reads + 1));
@@ -188,10 +238,12 @@ int alloc_svb_scratch(sgpu_ctx* ctx) {
     return SGPU_OK;
 }
 
-int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevOut& o, uint32_t* d_seq, uint32_t* d_fix,
-                 cudaStream_t st, const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
+// The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies.
+int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cudaStream_t st,
+                 const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
     if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
+    CU(alloc_outputs(ctx, o, want, false));
     CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
     CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
     StageMarks marks(ctx, st);
@@ -199,31 +251,11 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevOut& o, uin
         // nothing but empty records: every per-read output gets its defined value for an empty record (no event,
         // zero statistics / entropies / segments, "record not longer than the window" for prefix) instead of whatever
         // the previous batch left in the buffers
-        const size_t nr = b.n_reads;
-        CU(cudaMemsetAsync(o.ev_off, 0, (nr + 1) * sizeof(uint64_t), st));
-        if (nr && (want & SGPU_WANT_STAT)) CU(cudaMemsetAsync(o.stat, 0, nr * 6 * sizeof(float), st));
-        if (nr && (want & SGPU_WANT_ENT)) {
-            if (!o.ent) CU(dev_alloc(&o.ent, (uint64_t)ctx->max_reads * 3));
-            CU(cudaMemsetAsync(o.ent, 0, nr * 3 * sizeof(double), st));
-        }
-        if (nr && (want & SGPU_WANT_JNN)) {
-            if (!o.jnn_cnt) {
-                CU(dev_alloc(&o.jnn_cnt, ctx->max_reads));
-                CU(dev_alloc(&o.jnn_seg, 2 * jnn_seg_capacity(ctx->max_samples, ctx->max_reads)));
-            }
-            CU(cudaMemsetAsync(o.jnn_cnt, 0, nr * sizeof(uint32_t), st));
-        }
-        if (nr && (want & SGPU_WANT_PREFIX)) {
-            if (!o.prefix_pos) {
-                CU(dev_alloc(&o.prefix_pos, (uint64_t)ctx->max_reads * 4));
-                CU(dev_alloc(&o.prefix_stat, (uint64_t)ctx->max_reads * 6));
-            }
-            CU(cudaMemsetAsync(o.prefix_pos, 0xff, nr * 4 * sizeof(int32_t), st));   // (-1, -1, -1, -1)
-            CU(cudaMemsetAsync(o.prefix_stat, 0, nr * 6 * sizeof(float), st));
-        }
-        if (nr && (want & SGPU_WANT_EVENTS)) {
-            CU(cudaMemsetAsync(d_seq, 0, nr * sizeof(uint32_t), st));
-            CU(cudaMemsetAsync(d_fix, 0, nr * sizeof(uint32_t), st));
+        for (int k = 0; k < N_OUT; k++) {
+            const OutSpec& s = OUTS[k];
+            if (s.empty < 0 || !((want & s.want) || (s.empty & ANY_WANT))) continue;
+            const uint64_t n = out_elems(k, b.n_reads, b.span, 0);
+            if (n) CU(cudaMemsetAsync(o[k], s.empty & 0xff, (size_t)n * s.size, st));
         }
         ctx->last_launches = 0;
         return SGPU_OK;
@@ -231,66 +263,81 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevOut& o, uin
     if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
     const bool events = (want & SGPU_WANT_EVENTS) != 0;
-    if (want & SGPU_WANT_PA) {
-        if (!o.pa) CU(dev_alloc(&o.pa, align_up(ctx->max_samples, SGPU_ALIGN)));
-        // with events on the fast path the pA store is fused into walk_chunks_kernel
-        if (!events || force_generic) marks.done("pa", launch_pa(b, o.pa, ctx->sm_count, st));
-    }
+    float* const pa = (want & SGPU_WANT_PA) ? static_cast<float*>(o[PA]) : nullptr;
+    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER]);
+    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS]);
+    if (pa && (!events || force_generic))  // with events on the fast path the pA store is fused into walk_chunks_kernel
+        marks.done("pa", launch_pa(b, pa, ctx->sm_count, st));
     if (want & SGPU_WANT_STAT) {
-        marks.done("stat_moments", launch_stat_moments(b, o.stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
-        marks.done("stat_median", launch_stat_median(b, o.stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
+        float* const stat = static_cast<float*>(o[STAT]);
+        marks.done("stat_moments", launch_stat_moments(b, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
+        marks.done("stat_median", launch_stat_median(b, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
     }
     if (want & SGPU_WANT_ENT) {
-        if (!o.ent) CU(dev_alloc(&o.ent, (uint64_t)ctx->max_reads * 3));
         if (!ctx->ent_ovf) {
             const uint64_t words = ent_overflow_words(ctx->sm_count);
             CU(dev_alloc(&ctx->ent_ovf, words));
             CU(cudaMemsetAsync(ctx->ent_ovf, 0, (size_t)words * sizeof(uint32_t), st));
         }
-        marks.done("ent", launch_ent(b, ctx->ent_ovf, o.ent, ctx->sm_count, st));
+        marks.done("ent", launch_ent(b, ctx->ent_ovf, static_cast<double*>(o[ENT]), ctx->sm_count, st));
     }
     if (want & SGPU_WANT_JNN) {
-        if (!o.jnn_cnt) {
-            CU(dev_alloc(&o.jnn_cnt, ctx->max_reads));
-            CU(dev_alloc(&o.jnn_seg, 2 * jnn_seg_capacity(ctx->max_samples, ctx->max_reads)));
-        }
-        if (!ctx->jnn_mom) CU(dev_alloc(&ctx->jnn_mom, (uint64_t)ctx->max_reads * 2));
+        CU(dev_alloc(&ctx->jnn_mom, (uint64_t)ctx->max_reads * 2));
         marks.done("jnn_moments", launch_jnn_moments(b, ctx->jnn_mom, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
-        marks.done("jnn_walk", launch_jnn(b, ctx->jnn_mom, o.jnn_cnt, o.jnn_seg, ctx->sm_count, st));
+        marks.done("jnn_walk", launch_jnn(b, ctx->jnn_mom, static_cast<uint32_t*>(o[JNN_CNT]),
+                                          static_cast<int32_t*>(o[JNN_SEG]), ctx->sm_count, st));
     }
-    if (want & SGPU_WANT_PREFIX) {
-        if (!o.prefix_pos) {
-            CU(dev_alloc(&o.prefix_pos, (uint64_t)ctx->max_reads * 4));
-            CU(dev_alloc(&o.prefix_stat, (uint64_t)ctx->max_reads * 6));
-        }
-        marks.done("prefix", launch_prefix(b, ctx->pore_rna004, o.prefix_pos, o.prefix_stat, ctx->sm_count, st));
-    }
+    if (want & SGPU_WANT_PREFIX)
+        marks.done("prefix", launch_prefix(b, ctx->pore_rna004, static_cast<int32_t*>(o[PREFIX_POS]),
+                                           static_cast<float*>(o[PREFIX_STAT]), ctx->sm_count, st));
     if (events) {
         const uint32_t n_tiles = fast_tiles_for(b.span);
         if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
-        int n = launch_init_reads(b, sc, d_seq, d_fix, ctx->sm_count, st);
+        int n = launch_init_reads(b, sc, seq, fix, ctx->sm_count, st);
         if (force_generic) {
             CU(cudaMemsetAsync(sc.bitmap, 0, (size_t)n_tiles * (FAST_TILE / 32) * sizeof(uint32_t), st));
             marks.done("init", n);
         } else {
             marks.done("init", n);
-            marks.done("walk_chunks", launch_walk(b, sc, (want & SGPU_WANT_PA) ? o.pa : nullptr, d_seq, ctx->sm_count, st));
-            marks.done("long_jobs", launch_long_jobs(b, sc, d_seq, ctx->sm_count, st));
-            marks.done("verify_chunks", launch_verify_chunks(b, sc, d_seq, d_fix, ctx->sm_count, st));
+            marks.done("walk_chunks", launch_walk(b, sc, pa, seq, ctx->sm_count, st));
+            marks.done("long_jobs", launch_long_jobs(b, sc, seq, ctx->sm_count, st));
+            marks.done("verify_chunks", launch_verify_chunks(b, sc, seq, fix, ctx->sm_count, st));
         }
-        n = launch_build_seq_list(b, sc, d_seq, force_generic ? 1 : 0, ctx->sm_count, st);
+        n = launch_build_seq_list(b, sc, seq, force_generic ? 1 : 0, ctx->sm_count, st);
         WorkList wl{sc.seq_list, sc.seq_sbase, sc.seq_count};
         n += launch_generic_detect(b, wl, sc, ctx->sm_count, st);
         marks.done("sequential_order_detect", n);
-        marks.done("rank_events", launch_rank_events(b, sc, o.ev_off, ctx->sm_count, st));
-        marks.done("emit_events", launch_fast_emit(b, sc, ctx->ev_cap, o.ev_start, o.ev_mean, o.ev_stdv, d_fix,
-                                                  ctx->sm_count, st));
-        marks.done("sequential_order_emit", launch_generic_emit(b, wl, sc, o.ev_off, ctx->ev_cap, o.ev_start, o.ev_mean,
-                                                                o.ev_stdv, ctx->sm_count, st));
+        uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF]);
+        uint32_t* const ev_start = static_cast<uint32_t*>(o[EV_START]);
+        float* const ev_mean = static_cast<float*>(o[EV_MEAN]);
+        float* const ev_stdv = static_cast<float*>(o[EV_STDV]);
+        marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
+        marks.done("emit_events",
+                   launch_fast_emit(b, sc, ctx->ev_cap, ev_start, ev_mean, ev_stdv, fix, ctx->sm_count, st));
+        marks.done("sequential_order_emit",
+                   launch_generic_emit(b, wl, sc, ev_off, ctx->ev_cap, ev_start, ev_mean, ev_stdv, ctx->sm_count, st));
     }
     CU(cudaGetLastError());
     ctx->last_launches = marks.launches;
     return SGPU_OK;
+}
+
+// The per-read tail of sgpu_slot_add_read / sgpu_slot_add_read_svbzd: records the read of n samples at sl.used as
+// the batch's next read, with the scalars of its pA conversion.
+int64_t append_record(Slot& sl, uint64_t n, double digitisation, double offset, double range) {
+    sgpu_batch_t& b = sl.batch;
+    const uint32_t r = b.n_reads;
+    b.read_off[r] = sl.used;
+    b.read_len[r] = (uint32_t)n;
+    // misc.c:17-19,26: narrow the three doubles to float first, then ONE float division
+    const float range_f = (float)range, dig_f = (float)digitisation, off_f = (float)offset;
+    volatile float unit = range_f / dig_f;
+    b.offset_f[r] = off_f;
+    b.raw_unit_f[r] = unit;
+    sl.used += align_up(n, SGPU_ALIGN);
+    b.n_reads = r + 1;
+    b.read_off[r + 1] = sl.used;
+    return (int64_t)r;
 }
 
 int map_dev_status(int s) {
@@ -337,7 +384,6 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
     if (flags & SGPU_F_NO_HOST_SLOTS) n_slots = 0; else if (n_slots == 0) n_slots = 2;
     sgpu_ctx* ctx = new (std::nothrow) sgpu_ctx();
     if (!ctx) return SGPU_E_NOMEM;
-    int rc = SGPU_OK;
     auto fail = [&](int code) { sgpu_destroy(ctx); return code; };
     {
         int ndev = 0;
@@ -396,8 +442,6 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
     CUC(dev_alloc(&sc.tile_base, (uint64_t)sc.max_tiles + 1));
     CUC(dev_alloc(&sc.wit_min, max_reads));
     CUC(dev_alloc(&sc.wit_max, max_reads));
-    CUC(dev_alloc(&ctx->dev_seq, max_reads));
-    CUC(dev_alloc(&ctx->dev_fix, max_reads));
     CUC(dev_alloc(&sc.seq_list, max_reads));
     CUC(dev_alloc(&sc.seq_sbase, (uint64_t)max_reads + 1));
     CUC(dev_alloc(&sc.seq_count, 1));
@@ -415,8 +459,7 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
     CUC(dev_alloc(&sc.status, 1));
     CUC(dev_alloc(&sc.counters, 4));
     CUC(cudaStreamCreateWithFlags(&ctx->compute, cudaStreamNonBlocking));
-    rc = alloc_dev_out(ctx, ctx->dev_out);
-    if (rc) return fail(rc);
+    CUC(alloc_outputs(ctx, ctx->dev_out, 0, false));
     if (n_slots) {
         ctx->slots = new (std::nothrow) Slot[n_slots];
         if (!ctx->slots) return fail(SGPU_E_NOMEM);
@@ -432,18 +475,9 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
             CUC(dev_alloc(&sl.d_read_len, max_reads));
             CUC(dev_alloc(&sl.d_offset, max_reads));
             CUC(dev_alloc(&sl.d_unit, max_reads));
-            CUC(dev_alloc(&sl.d_seq, max_reads));
-            CUC(dev_alloc(&sl.d_fix, max_reads));
             // every slot gets its own outputs (its D2H overlaps the next slot's kernels)
-            rc = alloc_dev_out(ctx, sl.dout);
-            if (rc) return fail(rc);
-            CUC(pin_alloc(&sl.h_ev_off, (uint64_t)max_reads + 1));
-            CUC(pin_alloc(&sl.h_ev_start, ctx->ev_cap));
-            CUC(pin_alloc(&sl.h_ev_mean, ctx->ev_cap));
-            CUC(pin_alloc(&sl.h_ev_stdv, ctx->ev_cap));
-            CUC(pin_alloc(&sl.h_stat, (uint64_t)max_reads * 6));
-            CUC(pin_alloc(&sl.h_seq, max_reads));
-            CUC(pin_alloc(&sl.h_fix, max_reads));
+            CUC(alloc_outputs(ctx, sl.dout, 0, false));
+            CUC(alloc_outputs(ctx, sl.hout, 0, true));
             CUC(pin_alloc(&sl.h_counters, 4));
             CUC(pin_alloc(&sl.h_status, 1));
             CUC(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
@@ -468,11 +502,11 @@ void sgpu_destroy(sgpu_ctx_t* ctx) {
     cudaFree(sc.wk_begin); cudaFree(sc.wk_end); cudaFree(sc.wk_cnt); cudaFree(sc.wk_ibase);
     cudaFree(sc.jobs); cudaFree(sc.job_count);
     cudaFree(sc.tile_cnt); cudaFree(sc.tile_base); cudaFree(sc.tile_read0);
-    cudaFree(sc.wit_min); cudaFree(sc.wit_max); cudaFree(ctx->dev_seq); cudaFree(ctx->dev_fix);
+    cudaFree(sc.wit_min); cudaFree(sc.wit_max);
     cudaFree(sc.seq_list); cudaFree(sc.seq_sbase); cudaFree(sc.seq_count); cudaFree(sc.cursor);
     cudaFree(sc.scan_status); cudaFree(sc.scan_ticket); cudaFree(sc.status); cudaFree(sc.counters);
     for (int k = 0; k <= sgpu_ctx::MAX_STAGES; k++) if (ctx->stage_ev[k]) cudaEventDestroy(ctx->stage_ev[k]);
-    free_dev_out(ctx->dev_out);
+    free_outputs(ctx->dev_out, false);
     cudaFree(ctx->ent_ovf); cudaFree(ctx->jnn_mom);
     {
         SvbScratch& w = ctx->svb;
@@ -485,11 +519,10 @@ void sgpu_destroy(sgpu_ctx_t* ctx) {
             cudaFreeHost(sl.batch.samples); cudaFreeHost(sl.batch.read_off); cudaFreeHost(sl.batch.read_len);
             cudaFreeHost(sl.batch.offset_f); cudaFreeHost(sl.batch.raw_unit_f);
             cudaFree(sl.d_samples); cudaFree(sl.d_read_off); cudaFree(sl.d_read_len); cudaFree(sl.d_offset);
-            cudaFree(sl.d_unit); cudaFree(sl.d_seq); cudaFree(sl.d_fix);
-            free_dev_out(sl.dout);
-            cudaFreeHost(sl.h_ev_off); cudaFreeHost(sl.h_ev_start); cudaFreeHost(sl.h_ev_mean);
-            cudaFreeHost(sl.h_ev_stdv); cudaFreeHost(sl.h_pa); cudaFreeHost(sl.h_stat); cudaFreeHost(sl.h_ent); cudaFreeHost(sl.h_jnn_cnt); cudaFreeHost(sl.h_jnn_seg); cudaFreeHost(sl.h_prefix_pos); cudaFreeHost(sl.h_prefix_stat); cudaFreeHost(sl.h_seq);
-            cudaFreeHost(sl.h_fix); cudaFreeHost(sl.h_counters); cudaFreeHost(sl.h_status);
+            cudaFree(sl.d_unit);
+            free_outputs(sl.dout, false);
+            free_outputs(sl.hout, true);
+            cudaFreeHost(sl.h_counters); cudaFreeHost(sl.h_status);
             cudaFreeHost(sl.h_comp); cudaFreeHost(sl.h_comp_off); cudaFreeHost(sl.h_comp_len);
             cudaFree(sl.d_comp); cudaFree(sl.d_comp_off); cudaFree(sl.d_comp_len);
             if (sl.stream) cudaStreamDestroy(sl.stream);
@@ -535,19 +568,8 @@ int64_t sgpu_slot_add_read(sgpu_ctx_t* ctx, uint32_t slot, const int16_t* raw, u
     sgpu_batch_t& b = sl.batch;
     if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples) return SGPU_E_FULL;
     sl.mode = 1;
-    const uint32_t r = b.n_reads;
     memcpy(b.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
-    b.read_off[r] = sl.used;
-    b.read_len[r] = (uint32_t)n;
-    // misc.c:17-19,26: narrow the three doubles to float first, then ONE float division
-    const float range_f = (float)range, dig_f = (float)digitisation, off_f = (float)offset;
-    volatile float unit = range_f / dig_f;
-    b.offset_f[r] = off_f;
-    b.raw_unit_f[r] = unit;
-    sl.used += need;
-    b.n_reads = r + 1;
-    b.read_off[r + 1] = sl.used;
-    return (int64_t)r;
+    return append_record(sl, n, digitisation, offset, range);
 }
 
 int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* stream, uint64_t n_bytes,
@@ -566,7 +588,7 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
     sgpu_batch_t& b = sl.batch;
     if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples || sl.comp_used + cneed > ctx->comp_cap)
         return SGPU_E_FULL;
-    if (!sl.h_comp) {
+    if (sl.mode != 2) {  // the batch's first stream: make sure the slot's svb-zd buffers exist
         CU(cudaSetDevice(ctx->device));
         const int rc = alloc_svb_scratch(ctx);
         if (rc) return rc;
@@ -584,16 +606,7 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
     sl.h_comp_len[r] = (uint32_t)n_bytes;
     sl.comp_used += cneed;
     sl.svb_blocks += svbzd_blocks_of(n);
-    b.read_off[r] = sl.used;
-    b.read_len[r] = (uint32_t)n;
-    const float range_f = (float)range, dig_f = (float)digitisation, off_f = (float)offset;  // misc.c:17-19,26
-    volatile float unit = range_f / dig_f;
-    b.offset_f[r] = off_f;
-    b.raw_unit_f[r] = unit;
-    sl.used += need;
-    b.n_reads = r + 1;
-    b.read_off[r + 1] = sl.used;
-    return (int64_t)r;
+    return append_record(sl, n, digitisation, offset, range);
 }
 
 int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
@@ -622,18 +635,8 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     CU(cudaEventRecord(sl.in_ready, st));
     CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
     DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, (int)hb.rna, sl.used};
-    if ((want & SGPU_WANT_PA) && !sl.h_pa) CU(pin_alloc(&sl.h_pa, ctx->max_samples));
-    if ((want & SGPU_WANT_ENT) && !sl.h_ent) CU(pin_alloc(&sl.h_ent, (uint64_t)ctx->max_reads * 3));
-    if ((want & SGPU_WANT_JNN) && !sl.h_jnn_cnt) {
-        CU(pin_alloc(&sl.h_jnn_cnt, ctx->max_reads));
-        CU(pin_alloc(&sl.h_jnn_seg, 2 * jnn_seg_capacity(ctx->max_samples, ctx->max_reads)));
-    }
-    if ((want & SGPU_WANT_PREFIX) && !sl.h_prefix_pos) {
-        CU(pin_alloc(&sl.h_prefix_pos, (uint64_t)ctx->max_reads * 4));
-        CU(pin_alloc(&sl.h_prefix_stat, (uint64_t)ctx->max_reads * 6));
-    }
-    const int rc = run_pipeline(ctx, b, want, sl.dout, sl.d_seq, sl.d_fix, ctx->compute, compressed ? &svb : nullptr,
-                                sl.d_samples);
+    CU(alloc_outputs(ctx, sl.hout, want, true));
+    const int rc = run_pipeline(ctx, b, want, sl.dout, ctx->compute, compressed ? &svb : nullptr, sl.d_samples);
     if (rc) return rc;
     // small results come back right away; the big arrays are sized by n_events in sgpu_wait
     CU(cudaMemcpyAsync(sl.h_counters, ctx->sc.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
@@ -641,26 +644,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     CU(cudaMemcpyAsync(sl.h_status, ctx->sc.status, sizeof(int), cudaMemcpyDeviceToHost, ctx->compute));
     CU(cudaEventRecord(sl.kernels_done, ctx->compute));
     CU(cudaStreamWaitEvent(st, sl.kernels_done, 0));
-    if (want & SGPU_WANT_EVENTS) {
-        CU(cudaMemcpyAsync(sl.h_ev_off, sl.dout.ev_off, ((size_t)nr + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_seq, sl.d_seq, (size_t)nr * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_fix, sl.d_fix, (size_t)nr * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    }
-    if (want & SGPU_WANT_STAT)
-        CU(cudaMemcpyAsync(sl.h_stat, sl.dout.stat, (size_t)nr * 6 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    if (want & SGPU_WANT_ENT)
-        CU(cudaMemcpyAsync(sl.h_ent, sl.dout.ent, (size_t)nr * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (want & SGPU_WANT_JNN) {
-        CU(cudaMemcpyAsync(sl.h_jnn_cnt, sl.dout.jnn_cnt, (size_t)nr * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_jnn_seg, sl.dout.jnn_seg, (size_t)2 * ((sl.used >> 5) + nr + 1) * sizeof(int32_t),
-                           cudaMemcpyDeviceToHost, st));
-    }
-    if (want & SGPU_WANT_PREFIX) {
-        CU(cudaMemcpyAsync(sl.h_prefix_pos, sl.dout.prefix_pos, (size_t)nr * 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_prefix_stat, sl.dout.prefix_stat, (size_t)nr * 6 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    }
-    if (want & SGPU_WANT_PA)
-        CU(cudaMemcpyAsync(sl.h_pa, sl.dout.pa, (size_t)sl.used * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CU(queue_d2h(sl, want, false, 0));
     CU(cudaEventRecord(sl.small_back, st));
     sl.want = want;
     sl.submitted = true;
@@ -679,26 +663,13 @@ int sgpu_wait(sgpu_ctx_t* ctx, uint32_t slot, sgpu_result_t* out) {
     if (dev_rc) return dev_rc;
     const uint32_t nr = sl.batch.n_reads;
     if (sl.want & SGPU_WANT_EVENTS) {
-        const uint64_t ne = nr ? sl.h_ev_off[nr] : 0;
+        const uint64_t ne = nr ? static_cast<const uint64_t*>(sl.hout[EV_OFF])[nr] : 0;
         if (ne > ctx->ev_cap) return SGPU_E_EVCAP;
-        cudaStream_t st = sl.stream;
-        CU(cudaMemcpyAsync(sl.h_ev_start, sl.dout.ev_start, (size_t)ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_ev_mean, sl.dout.ev_mean, (size_t)ne * sizeof(float), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(sl.h_ev_stdv, sl.dout.ev_stdv, (size_t)ne * sizeof(float), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        out->ev_off = sl.h_ev_off;
-        out->ev_start = sl.h_ev_start;
-        out->ev_mean = sl.h_ev_mean;
-        out->ev_stdv = sl.h_ev_stdv;
-        out->seq_order = sl.h_seq;
-        out->fixups = sl.h_fix;
+        CU(queue_d2h(sl, SGPU_WANT_EVENTS, true, ne));
+        CU(cudaStreamSynchronize(sl.stream));
         out->n_events = ne;
     }
-    if (sl.want & SGPU_WANT_STAT) out->stat = sl.h_stat;
-    if (sl.want & SGPU_WANT_PA) out->pa = sl.h_pa;
-    if (sl.want & SGPU_WANT_ENT) out->ent = sl.h_ent;
-    if (sl.want & SGPU_WANT_JNN) { out->jnn_cnt = sl.h_jnn_cnt; out->jnn_seg = sl.h_jnn_seg; }
-    if (sl.want & SGPU_WANT_PREFIX) { out->prefix_pos = sl.h_prefix_pos; out->prefix_stat = sl.h_prefix_stat; }
+    fill_result(out, sl.hout, sl.want, false);
     return SGPU_OK;
 }
 
@@ -708,23 +679,10 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     CU(cudaSetDevice(ctx->device));
     DevBatch b{batch->samples, batch->read_off, batch->read_len, batch->offset_f, batch->raw_unit_f,
                batch->n_reads, (int)batch->rna, batch->span};
-    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, ctx->dev_seq, ctx->dev_fix,
-                                reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     memset(out, 0, sizeof *out);
-    out->ev_off = ctx->dev_out.ev_off;
-    out->ev_start = ctx->dev_out.ev_start;
-    out->ev_mean = ctx->dev_out.ev_mean;
-    out->ev_stdv = ctx->dev_out.ev_stdv;
-    out->pa = (want & SGPU_WANT_PA) ? ctx->dev_out.pa : nullptr;
-    out->stat = ctx->dev_out.stat;
-    out->ent = (want & SGPU_WANT_ENT) ? ctx->dev_out.ent : nullptr;
-    out->jnn_cnt = (want & SGPU_WANT_JNN) ? ctx->dev_out.jnn_cnt : nullptr;
-    out->jnn_seg = (want & SGPU_WANT_JNN) ? ctx->dev_out.jnn_seg : nullptr;
-    out->prefix_pos = (want & SGPU_WANT_PREFIX) ? ctx->dev_out.prefix_pos : nullptr;
-    out->prefix_stat = (want & SGPU_WANT_PREFIX) ? ctx->dev_out.prefix_stat : nullptr;
-    out->seq_order = ctx->dev_seq;
-    out->fixups = ctx->dev_fix;
+    fill_result(out, ctx->dev_out, want, true);
     return SGPU_OK;
 }
 

@@ -92,6 +92,14 @@ __device__ __forceinline__ void det_reset(DetState& d) {
     d.masked_to = 0; d.peak_pos = -1; d.peak_value = FLT_MAX; d.valid = 0;
 }
 
+// grid of a launch: enough blocks of `block` threads for `work` items, at least 1 and at most max_blocks
+static inline int grid_cap(uint64_t work, int block, int max_blocks) {
+    uint64_t g = (work + block - 1) / block;
+    if (g < 1) g = 1;
+    if (g > (uint64_t)max_blocks) g = max_blocks;
+    return (int)g;
+}
+
 // index of the read containing flat position p: largest r with read_off[r] <= p
 __device__ __forceinline__ uint32_t find_read(const uint64_t* __restrict__ off, uint32_t n, uint64_t p) {
     uint32_t lo = 0, hi = n;  // invariant: off[lo] <= p < off[hi] (off[n] = span)

@@ -323,13 +323,6 @@ __global__ void __launch_bounds__(EWARPS * 32, EMIT_MINB) emit_events_kernel(Dev
     }
 }
 
-static inline int grid_cap(uint64_t work, int block, int max_blocks) {
-    uint64_t g = (work + block - 1) / block;
-    if (g < 1) g = 1;
-    if (g > (uint64_t)max_blocks) g = max_blocks;
-    return (int)g;
-}
-
 __global__ void __launch_bounds__(256) sum_fixups_kernel(uint32_t n_reads, const uint32_t* __restrict__ fixups,
                                                          unsigned long long* __restrict__ counters) {
     unsigned long long acc = 0;

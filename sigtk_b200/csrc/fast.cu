@@ -122,13 +122,6 @@ __global__ void __launch_bounds__(256) init_reads_kernel(DevBatch b, uint32_t n_
     }
 }
 
-static inline int grid_cap(uint64_t work, int block, int max_blocks) {
-    uint64_t g = (work + block - 1) / block;
-    if (g < 1) g = 1;
-    if (g > (uint64_t)max_blocks) g = max_blocks;
-    return (int)g;
-}
-
 uint32_t fast_tiles_for(uint64_t span) { return (uint32_t)((span + T - 1) / T); }
 
 int launch_init_reads(const DevBatch& b, Scratch& sc, uint32_t* seq_flag, uint32_t* fixups, int sm_count,

@@ -464,13 +464,6 @@ __global__ void __launch_bounds__(256) pa_kernel(DevBatch b, float* __restrict__
 
 // ---------------------------------------------------------------------------
 // host-side launchers
-static inline int grid_for(uint64_t work, int block, int max_blocks) {
-    uint64_t g = (work + block - 1) / block;
-    if (g < 1) g = 1;
-    if (g > (uint64_t)max_blocks) g = max_blocks;
-    return (int)g;
-}
-
 int launch_generic_detect(const DevBatch& b, const WorkList& wl, Scratch& sc, int sm_count, cudaStream_t st) {
     gen_prefix_kernel<<<sm_count * 8, 128, 0, st>>>(b, wl, sc.Sinc, sc.Qinc);
     gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, wl, sc.Sinc, sc.Qinc, sc.t1, sc.t2);
@@ -495,7 +488,7 @@ int launch_generic_emit(const DevBatch& b, const WorkList& wl, Scratch& sc, cons
 }
 
 int launch_pa(const DevBatch& b, float* pa, int sm_count, cudaStream_t st) {
-    pa_kernel<<<grid_for(((b.span >> 3) + PA_IT - 1) / PA_IT, 256, sm_count * 16), 256, 0, st>>>(b, pa);
+    pa_kernel<<<grid_cap(((b.span >> 3) + PA_IT - 1) / PA_IT, 256, sm_count * 16), 256, 0, st>>>(b, pa);
     return 1;
 }
 

@@ -203,13 +203,6 @@ __global__ void __launch_bounds__(SVB_WARPS * 32) svb_write_kernel(SvbBatch s, c
     }
 }
 
-static inline int grid_cap(uint64_t work, int block, int max_blocks) {
-    uint64_t g = (work + block - 1) / block;
-    if (g < 1) g = 1;
-    if (g > (uint64_t)max_blocks) g = max_blocks;
-    return (int)g;
-}
-
 }  // namespace
 
 uint64_t svbzd_max_blocks(uint64_t max_samples, uint32_t max_reads) { return max_samples / SVB_BLOCK + max_reads + 1; }

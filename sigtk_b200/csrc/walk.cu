@@ -345,13 +345,6 @@ __global__ void __launch_bounds__(256) verify_chunks_kernel(DevBatch b, uint32_t
     }
 }
 
-static inline int grid_cap(uint64_t work, int block, int max_blocks) {
-    uint64_t g = (work + block - 1) / block;
-    if (g < 1) g = 1;
-    if (g > (uint64_t)max_blocks) g = max_blocks;
-    return (int)g;
-}
-
 }  // namespace
 
 // chunk length for a batch: as long as possible (the warm-up is amortised over it) while the batch still yields
