@@ -318,10 +318,13 @@ static float rank_half(const float *x, int n) {
     return v;
 }
 
-/* jnn.c:103-175 (jnnv2) with JNNV2_RNA_R9_ADAPTOR: the band's lower edge over a 2000-sample rolling mean of the
- * clamped signal, runs below it, first run of a plausible length */
-static void adaptor_r9(const int16_t *raw, int64_t n, int64_t *x, int64_t *y) {
-    const int w = 2000, merge = 1500, longest = 200000, shortest = 2000;
+/* jnn.c:103-175 (jnnv2): the band's lower edge (mean - std_scale * stdv) over a 2000-sample rolling mean of the
+ * clamped signal, runs below it, first run of a plausible length. The two adaptor parameter sets of jnn.h:88-102
+ * differ only in std_scale and the shortest run: JNNV2_RNA_R9_ADAPTOR 0.5f / 2000, JNNV2_RNA_RNA004_ADAPTOR 0.7f / 500
+ * (window 2000, merge distance 1500 and longest run 200000 are common). The RNA004 set is restated from jnn.h as
+ * prefix.cu passes it to prefix_walk_kernel; no stored reference output covers it. */
+static void adaptor_jnnv2(const int16_t *raw, int64_t n, float std_scale, int shortest, int64_t *x, int64_t *y) {
+    const int w = 2000, merge = 1500, longest = 200000;
     if (n <= w) { *x = -1; *y = -1; return; }
     const int nt = (int)n - w;
     float *t = (float *)malloc((size_t)nt * sizeof(float));
@@ -336,7 +339,7 @@ static void adaptor_r9(const int16_t *raw, int64_t n, int64_t *x, int64_t *y) {
     }
     #undef CLAMPED
     const float mn = seq_meanf(t, nt), sd = seq_stdvf(t, nt);
-    const float floor_ = mn - sd * 0.5f;
+    const float floor_ = mn - sd * std_scale;
     int below = 0, first = 0, last = 0;
     int64_t n_seg = 0, cap = 64;
     int64_t *sx = (int64_t *)malloc((size_t)cap * 2 * sizeof(int64_t));
@@ -402,11 +405,12 @@ static void polya_r9(const float *pa, int64_t n, float top, float bot, int64_t *
     if (n_seg > 0) { *x = sx0; *y = sy0; }
 }
 
-void orc_adaptor_polya(const int16_t *raw, uint64_t n, double digitisation, double offset, double range, int rna,
-                int64_t *pos4, float *st6) {
+void orc_adaptor_polya_pore(const int16_t *raw, uint64_t n, double digitisation, double offset, double range, int rna,
+                int pore, int64_t *pos4, float *st6) {
     for (int k = 0; k < 6; k++) st6[k] = 0.0f;
     pos4[2] = -1; pos4[3] = -1;
-    adaptor_r9(raw, (int64_t)n, &pos4[0], &pos4[1]);
+    if (pore) adaptor_jnnv2(raw, (int64_t)n, 0.7f, 500, &pos4[0], &pos4[1]);   /* JNNV2_RNA_RNA004_ADAPTOR */
+    else adaptor_jnnv2(raw, (int64_t)n, 0.5f, 2000, &pos4[0], &pos4[1]);       /* JNNV2_RNA_R9_ADAPTOR */
     if (pos4[1] <= 0) return;                                  /* cfunc.c:173 */
     float *pa = (float *)malloc((n ? n : 1) * sizeof(float));
     orc_pa(raw, n, digitisation, offset, range, pa);
@@ -425,6 +429,11 @@ void orc_adaptor_polya(const int16_t *raw, uint64_t n, double digitisation, doub
         }
     }
     free(pa);
+}
+
+void orc_adaptor_polya(const int16_t *raw, uint64_t n, double digitisation, double offset, double range, int rna,
+                int64_t *pos4, float *st6) {
+    orc_adaptor_polya_pore(raw, n, digitisation, offset, range, rna, 0, pos4, st6);
 }
 
 /* Shannon entropy in bits of a table of bin counts taken over `total` symbols; terms are subtracted in

@@ -83,12 +83,15 @@ void orc_ent(const int16_t *raw, uint64_t n, double *out3);
  * (or -(needed) when cap is too small). */
 int64_t orc_jnn(const int16_t *raw, uint64_t n, int rna, uint64_t cap, int64_t *xy);
 
-/* `sigtk prefix` numbers of one record on an R9 pore (prefix_func cfunc.c:169-234; find_adaptor / jnnv2 jnn.c:103-175
- * with JNNV2_RNA_R9_ADAPTOR jnn.h:88-94; find_polya jnn.c:345-370 = jnn_pa + jnn_core with JNNV1_R9_POLYA jnn.h:47-56).
+/* `sigtk prefix` numbers of one record (prefix_func cfunc.c:169-234; find_adaptor / jnnv2 jnn.c:103-175 with
+ * JNNV2_RNA_R9_ADAPTOR (pore 0) or JNNV2_RNA_RNA004_ADAPTOR (pore 1), jnn.h:88-102; find_polya jnn.c:345-370 = jnn_pa +
+ * jnn_core with JNNV1_R9_POLYA jnn.h:47-56). `pore` is what SGPU_PARAM_PORE holds; orc_adaptor_polya is the R9 call
+ * (pore 0) with the argument list it has always had.
  * pos[0..1] = adaptor (x, y) as jnnv2 returns them ((0,0): none found, (-1,-1): record not longer than the window),
  * pos[2..3] = poly-A (x, y) relative to the adaptor end ((-1,-1): none / DNA); st[0..2] = mean, stdv, median of the
- * adaptor's pA, st[3..5] of the poly-A's (valid when the respective y > 0). NOT yet on the GPU: next round's row
- * (SURVEY 8f rank 3, prefix half); kept here, pinned, so that the CUDA path has its checker from the first line. */
+ * adaptor's pA, st[3..5] of the poly-A's (valid when the respective y > 0). */
+void orc_adaptor_polya_pore(const int16_t *raw, uint64_t n, double digitisation, double offset, double range, int rna,
+                int pore, int64_t *pos4, float *st6);
 void orc_adaptor_polya(const int16_t *raw, uint64_t n, double digitisation, double offset, double range, int rna,
                 int64_t *pos4, float *st6);
 

@@ -140,9 +140,9 @@ class Oracle(_EventLib):
         L.orc_ent.restype = None
         L.orc_jnn.argtypes = [_i16p, C.c_uint64, C.c_int, C.c_uint64, C.POINTER(C.c_int64)]
         L.orc_jnn.restype = C.c_int64
-        L.orc_adaptor_polya.argtypes = [_i16p, C.c_uint64, C.c_double, C.c_double, C.c_double, C.c_int,
-                                        C.POINTER(C.c_int64), _f32p]
-        L.orc_adaptor_polya.restype = None
+        L.orc_adaptor_polya_pore.argtypes = [_i16p, C.c_uint64, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
+                                             C.POINTER(C.c_int64), _f32p]
+        L.orc_adaptor_polya_pore.restype = None
         L.orc_prefix.argtypes = [_f32p, C.c_uint64, _f64p, _f64p]
         L.orc_tstat.argtypes = [_f64p, _f64p, C.c_uint64, C.c_uint32, _f32p]
         L.orc_det_init.argtypes = [C.POINTER(Det), C.POINTER(Det)]
@@ -167,13 +167,14 @@ class Oracle(_EventLib):
         assert k >= 0, k
         return xy[:2 * k].reshape(k, 2).copy()
 
-    def adaptor_polya(self, raw, dig, off, rng, rna=0):
-        """`sigtk prefix` numbers on an R9 pore (cfunc.c:169-234): -> (pos int64[4], stat float32[6])"""
+    def adaptor_polya(self, raw, dig, off, rng, rna=0, pore=0):
+        """`sigtk prefix` numbers (cfunc.c:169-234) with the adaptor parameters of an R9 pore (pore=0) or of RNA004
+        (pore=1, SGPU_PARAM_PORE): -> (pos int64[4], stat float32[6])"""
         raw = np.ascontiguousarray(raw, dtype=np.int16)
         pos = np.zeros(4, dtype=np.int64)
         st = np.zeros(6, dtype=np.float32)
-        self.lib.orc_adaptor_polya(_p(raw, _i16p), raw.shape[0], dig, off, rng, int(rna),
-                                   pos.ctypes.data_as(C.POINTER(C.c_int64)), _p(st, _f32p))
+        self.lib.orc_adaptor_polya_pore(_p(raw, _i16p), raw.shape[0], dig, off, rng, int(rna), int(pore),
+                                        pos.ctypes.data_as(C.POINTER(C.c_int64)), _p(st, _f32p))
         return pos, st
 
     def params(self, rna):
