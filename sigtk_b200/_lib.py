@@ -24,7 +24,8 @@ EXPORTS = (
     "sgpu_abi_version", "sgpu_device_count", "sgpu_create", "sgpu_destroy", "sgpu_strerror",
     "sgpu_last_error", "sgpu_slot_batch", "sgpu_slot_reset", "sgpu_slot_add_read", "sgpu_submit",
     "sgpu_wait", "sgpu_run_device", "sgpu_counters", "sgpu_memcpy_d2h", "sgpu_stage_times",
-    "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param",
+    "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
+    "sgpu_run_device_pa",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -56,6 +57,13 @@ class DevBatch(C.Structure):  # sgpu_dev_batch_t
     _fields_ = [
         ("samples", C.c_void_p), ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("offset_f", C.c_void_p),
         ("raw_unit_f", C.c_void_p), ("n_reads", C.c_uint32), ("rna", C.c_uint32), ("span", C.c_uint64),
+    ]
+
+
+class DevPaBatch(C.Structure):  # sgpu_dev_pa_batch_t
+    _fields_ = [
+        ("pa", C.c_void_p), ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("n_reads", C.c_uint32),
+        ("rna", C.c_uint32), ("span", C.c_uint64),
     ]
 
 
@@ -109,6 +117,10 @@ def load() -> C.CDLL:
     lib.sgpu_slot_add_read.restype = C.c_int64
     lib.sgpu_slot_add_read_svbzd.argtypes = [vp, u32, vp, u64, C.c_double, C.c_double, C.c_double]
     lib.sgpu_slot_add_read_svbzd.restype = C.c_int64
+    lib.sgpu_slot_add_read_pa.argtypes = [vp, u32, vp, u64]
+    lib.sgpu_slot_add_read_pa.restype = C.c_int64
+    lib.sgpu_run_device_pa.argtypes = [vp, C.POINTER(DevPaBatch), u32, vp, C.POINTER(Result)]
+    lib.sgpu_run_device_pa.restype = i32
     lib.sgpu_decode_svbzd_device.argtypes = [vp, C.POINTER(SvbDevBatch), vp, vp]
     lib.sgpu_decode_svbzd_device.restype = i32
     lib.sgpu_submit.argtypes = [vp, u32, u32]

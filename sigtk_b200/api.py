@@ -126,6 +126,20 @@ class Context:
                                                     float(rng))
             self._check(int(rc))
 
+    def fill_pa(self, slot: int, signals: Sequence[np.ndarray], rna: int) -> None:
+        """signals: float32 pA arrays, one per record (getevents(n, pa, rna) on the caller's own signal); a slot holds
+        max_samples / 2 of them"""
+        self._check(self._lib.sgpu_slot_reset(self._h, slot, int(rna)))
+        for pa in signals:
+            pa = np.ascontiguousarray(pa, dtype=np.float32)
+            self._check(int(self._lib.sgpu_slot_add_read_pa(self._h, slot, pa.ctypes.data, pa.shape[0])))
+
+    def run_pa(self, signals: Sequence[np.ndarray], rna: int = 0, want: int = WANT_EVENTS, slot: int = 0) -> BatchResult:
+        """fill_pa + submit + wait: the event tables of records given as pA floats"""
+        self.fill_pa(slot, signals, rna)
+        self.submit(slot, want)
+        return self.wait(slot, want)
+
     def run_svbzd(self, reads: Sequence, rna: int = 0, want: int = WANT_EVENTS, slot: int = 0) -> BatchResult:
         self.fill_svbzd(slot, reads, rna)
         self.submit(slot, want)
@@ -194,6 +208,14 @@ class Context:
         self._check(self._lib.sgpu_run_device(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res)))
         return res
 
+    def run_device_pa(self, pa_ptr: int, read_off_ptr: int, read_len_ptr: int, n_reads: int, span: int, rna: int,
+                      want: int = WANT_EVENTS, stream: int = 0) -> _lib.Result:
+        """sgpu_run_device_pa: events of pA floats already in device memory (read_off multiples of ALIGN)"""
+        db = _lib.DevPaBatch(pa_ptr, read_off_ptr, read_len_ptr, n_reads, int(rna), span)
+        res = _lib.Result()
+        self._check(self._lib.sgpu_run_device_pa(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res)))
+        return res
+
     def d2h(self, dev_ptr: int, dtype, count: int) -> np.ndarray:
         """copy `count` items of a device result array (a pointer from run_device) to a new numpy array"""
         out = np.empty(count, dtype=dtype)
@@ -229,6 +251,11 @@ def getevents(ctx: Context, raw: np.ndarray, digitisation: float, offset: float,
               rna: int = 0) -> EventTable:
     """events.c:553-573 for one record (pA conversion is fused, so this takes the raw samples)."""
     return ctx.run([(raw, digitisation, offset, range_)], rna, WANT_EVENTS).events(0)
+
+
+def getevents_pa(ctx: Context, pa: np.ndarray, rna: int = 0) -> EventTable:
+    """events.c:553-573 for one record given as pA floats, exactly as the reference's getevents(n, pa, rna)."""
+    return ctx.run_pa([pa], rna, WANT_EVENTS).events(0)
 
 
 def stat(ctx: Context, raw: np.ndarray, digitisation: float, offset: float, range_: float) -> np.ndarray:

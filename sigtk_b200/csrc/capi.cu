@@ -40,28 +40,37 @@ struct OutSpec {
     uint32_t per;
     bool eager;      // allocated at creation (returned by every sgpu_run_device), else on the first run that wants it
     int empty;       // byte every element holds for a batch of empty records (| ANY_WANT), or -1: left as it is
+    bool pa_in;      // produced by a run on the caller's pA floats (sgpu_run_device_pa, slots of pA records)
 };
 
-#define OUTPUT(field, want, count, per, eager, empty) \
-    { offsetof(sgpu_result_t, field), sizeof *sgpu_result_t{}.field, want, count, per, eager, empty }
+#define OUTPUT(field, want, count, per, eager, empty, pa_in) \
+    { offsetof(sgpu_result_t, field), sizeof *sgpu_result_t{}.field, want, count, per, eager, empty, pa_in }
 constexpr OutSpec OUTS[] = {  // in the order of Out
-    //     field        want              count         per  eager  empty
-    OUTPUT(ev_off,      SGPU_WANT_EVENTS, READS_PLUS_1, 1,   true,  0 | ANY_WANT),
-    OUTPUT(ev_start,    SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
-    OUTPUT(ev_mean,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
-    OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1),
-    OUTPUT(seq_order,   SGPU_WANT_EVENTS, READS,        1,   true,  0),
-    OUTPUT(fixups,      SGPU_WANT_EVENTS, READS,        1,   true,  0),
-    OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0),
-    OUTPUT(ent,         SGPU_WANT_ENT,    READS,        3,   false, 0),
-    OUTPUT(jnn_cnt,     SGPU_WANT_JNN,    READS,        1,   false, 0),
-    OUTPUT(jnn_seg,     SGPU_WANT_JNN,    JNN_SLOTS,    2,   false, -1),
-    OUTPUT(prefix_pos,  SGPU_WANT_PREFIX, READS,        4,   false, 0xff),  // -1: not longer than the window
-    OUTPUT(prefix_stat, SGPU_WANT_PREFIX, READS,        6,   false, 0),
-    OUTPUT(pa,          SGPU_WANT_PA,     SAMPLES,      1,   false, -1),
+    //     field        want              count         per  eager  empty         pa_in
+    OUTPUT(ev_off,      SGPU_WANT_EVENTS, READS_PLUS_1, 1,   true,  0 | ANY_WANT, true),
+    OUTPUT(ev_start,    SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
+    OUTPUT(ev_mean,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
+    OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
+    OUTPUT(seq_order,   SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
+    OUTPUT(fixups,      SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
+    OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0,            false),
+    OUTPUT(ent,         SGPU_WANT_ENT,    READS,        3,   false, 0,            false),
+    OUTPUT(jnn_cnt,     SGPU_WANT_JNN,    READS,        1,   false, 0,            false),
+    OUTPUT(jnn_seg,     SGPU_WANT_JNN,    JNN_SLOTS,    2,   false, -1,           false),
+    OUTPUT(prefix_pos,  SGPU_WANT_PREFIX, READS,        4,   false, 0xff,         false),  // -1: not longer than the window
+    OUTPUT(prefix_stat, SGPU_WANT_PREFIX, READS,        6,   false, 0,            false),
+    OUTPUT(pa,          SGPU_WANT_PA,     SAMPLES,      1,   false, -1,           false),
 };
 #undef OUTPUT
 static_assert(sizeof OUTS / sizeof OUTS[0] == N_OUT, "one row per output");
+
+// the products a run on pA input can compute: those of its outputs (the others are defined on int16 raw samples, and
+// pA is the input itself)
+constexpr uint32_t pa_input_wants(int k = 0) {
+    return k == N_OUT ? 0u : (OUTS[k].pa_in ? OUTS[k].want : 0u) | pa_input_wants(k + 1);
+}
+constexpr bool pa_input_want_ok(uint32_t want) { return want != 0 && (want & ~pa_input_wants()) == 0; }
+static_assert(pa_input_wants() == SGPU_WANT_EVENTS, "a pA run computes the event table only");
 
 // elements of output k for a batch of `reads` reads spanning `samples` samples with `events` events; at the
 // context's (max_reads, max_samples, ev_cap) this is the output's capacity
@@ -96,7 +105,8 @@ struct Slot {
     bool submitted = false;
     uint32_t want = 0;
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
-    int mode = 0;                    // 0: empty, 1: decoded int16 records, 2: svb-zd streams
+    int mode = 0;                    // 0: empty, 1: decoded int16 records, 2: svb-zd streams, 3: pA records (floats
+                                     // in the sample buffers: max_samples / 2 of them)
     uint8_t* h_comp = nullptr;       // pinned, comp_cap bytes
     uint8_t* d_comp = nullptr;       // comp_cap + 16 bytes
     uint64_t* h_comp_off = nullptr; uint64_t* d_comp_off = nullptr;
@@ -121,6 +131,7 @@ struct sgpu_ctx {
     float* jnn_mom = nullptr;    // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
     int pore_rna004 = 0;         // SGPU_PARAM_PORE: jnnv2 parameters of `prefix` (misc.c:74-101 picks them from the header)
     uint32_t* ent_ovf = nullptr; // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
+    PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     uint64_t comp_cap = 0;       // bytes of compressed input a slot can hold
     cudaStream_t compute = nullptr;
     uint64_t last_launches = 0;
@@ -238,6 +249,20 @@ int alloc_svb_scratch(sgpu_ctx* ctx) {
     return SGPU_OK;
 }
 
+// nothing but empty records: every per-read output gets its defined value for an empty record (no event, zero
+// statistics / entropies / segments, "record not longer than the window" for prefix) instead of whatever the previous
+// batch left in the buffers
+int clear_empty_batch(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cudaStream_t st) {
+    for (int k = 0; k < N_OUT; k++) {
+        const OutSpec& s = OUTS[k];
+        if (s.empty < 0 || !((want & s.want) || (s.empty & ANY_WANT))) continue;
+        const uint64_t n = out_elems(k, b.n_reads, b.span, 0);
+        if (n) CU(cudaMemsetAsync(o[k], s.empty & 0xff, (size_t)n * s.size, st));
+    }
+    ctx->last_launches = 0;
+    return SGPU_OK;
+}
+
 // The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies.
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cudaStream_t st,
                  const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
@@ -247,19 +272,7 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cuda
     CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
     CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
     StageMarks marks(ctx, st);
-    if (b.n_reads == 0 || b.span == 0) {
-        // nothing but empty records: every per-read output gets its defined value for an empty record (no event,
-        // zero statistics / entropies / segments, "record not longer than the window" for prefix) instead of whatever
-        // the previous batch left in the buffers
-        for (int k = 0; k < N_OUT; k++) {
-            const OutSpec& s = OUTS[k];
-            if (s.empty < 0 || !((want & s.want) || (s.empty & ANY_WANT))) continue;
-            const uint64_t n = out_elems(k, b.n_reads, b.span, 0);
-            if (n) CU(cudaMemsetAsync(o[k], s.empty & 0xff, (size_t)n * s.size, st));
-        }
-        ctx->last_launches = 0;
-        return SGPU_OK;
-    }
+    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(ctx, b, want, o, st);
     if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
     const bool events = (want & SGPU_WANT_EVENTS) != 0;
@@ -317,6 +330,84 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cuda
         marks.done("sequential_order_emit",
                    launch_generic_emit(b, wl, sc, ev_off, ctx->ev_cap, ev_start, ev_mean, ev_stdv, ctx->sm_count, st));
     }
+    CU(cudaGetLastError());
+    ctx->last_launches = marks.launches;
+    return SGPU_OK;
+}
+
+int alloc_pa_scratch(sgpu_ctx* ctx) {
+    PaScratch& w = ctx->pa;
+    w.max_tiles = pa_tile_capacity(ctx->max_samples, ctx->max_reads);
+    CU(dev_alloc(&w.tile_cnt, ctx->max_reads));
+    CU(dev_alloc(&w.tile_base, (uint64_t)ctx->max_reads + 1));
+    CU(dev_alloc(&w.tS, w.max_tiles));
+    CU(dev_alloc(&w.tQ, w.max_tiles));
+    CU(dev_alloc(&w.tA, w.max_tiles));
+    CU(dev_alloc(&w.tB, w.max_tiles));
+    CU(dev_alloc(&w.tmin, w.max_tiles));
+    CU(dev_alloc(&w.ord_list, ctx->max_reads));
+    CU(dev_alloc(&w.ord_sbase, ctx->max_reads));
+    CU(dev_alloc(&w.ord_count, 1));
+    return SGPU_OK;
+}
+
+// A pA batch keeps its prefix sums and t-statistics at the reads' own offsets, so the sequential-order scratch must
+// hold the whole span. Contexts over 64 Mi samples start with an eighth of that (sgpu_create); the first pA batch that
+// needs more grows it to max_samples for the rest of the context's life (later int16 batches use it too). The old
+// arrays are freed only once the new ones exist (cudaFree waits for the device).
+int grow_seq_scratch(sgpu_ctx* ctx) {
+    Scratch& sc = ctx->sc;
+    const uint64_t n = ctx->max_samples;
+    double *S = nullptr, *Q = nullptr;
+    float *t1 = nullptr, *t2 = nullptr;
+    cudaError_t e = dev_alloc(&S, n);
+    if (e == cudaSuccess) e = dev_alloc(&Q, n);
+    if (e == cudaSuccess) e = dev_alloc(&t1, n);
+    if (e == cudaSuccess) e = dev_alloc(&t2, n);
+    if (e != cudaSuccess) {
+        cudaFree(S); cudaFree(Q); cudaFree(t1); cudaFree(t2);
+        cudaGetLastError();  // (an allocation failure is reported here, not by the next launch check)
+        snprintf(ctx->err, sizeof ctx->err, "growing the sequential-order scratch to %llu samples: %s",
+                 (unsigned long long)n, cudaGetErrorString(e));
+        return SGPU_E_NOMEM;
+    }
+    cudaFree(sc.Sinc); cudaFree(sc.Qinc); cudaFree(sc.t1); cudaFree(sc.t2);
+    sc.Sinc = S; sc.Qinc = Q; sc.t1 = t1; sc.t2 = t2;
+    sc.gen_cap = n;
+    return SGPU_OK;
+}
+
+// The kernel sequence of a batch of pA records (getevents(n, pa, rna), events.c:553-573) into the device outputs `o`:
+// the prefix sums by the witness-checked scan or in the reference's order (pa_input.cu), then the sequential-order
+// kernels for every read. No host synchronisation, no host<->device copies (except when the scratch grows).
+int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t want, void** o, cudaStream_t st) {
+    Scratch& sc = ctx->sc;
+    if (!pa_input_want_ok(want)) return SGPU_E_INVAL;
+    if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
+    if (b.n_reads && b.span && !pa) return SGPU_E_INVAL;
+    CU(alloc_outputs(ctx, o, want, false));
+    int rc = alloc_pa_scratch(ctx);
+    if (!rc && b.span > sc.gen_cap) rc = grow_seq_scratch(ctx);
+    if (rc) return rc;
+    CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
+    CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
+    StageMarks marks(ctx, st);
+    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(ctx, b, want, o, st);
+    const uint32_t n_tiles = fast_tiles_for(b.span);
+    if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
+    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER]);
+    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS]);
+    CU(cudaMemsetAsync(sc.bitmap, 0, (size_t)n_tiles * (FAST_TILE / 32) * sizeof(uint32_t), st));
+    const int force = (ctx->flags & SGPU_F_FORCE_GENERIC) ? 1 : 0;
+    marks.done("pa_prefix", launch_pa_prefix(b, pa, ctx->pa, sc, seq, fix, force, ctx->sm_count, st));
+    const WorkList ordered{ctx->pa.ord_list, ctx->pa.ord_sbase, ctx->pa.ord_count};
+    const WorkList all{sc.seq_list, sc.seq_sbase, sc.seq_count};
+    marks.done("sequential_order_detect", launch_generic_detect_pa(b, pa, ordered, all, sc, fix, ctx->sm_count, st));
+    uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF]);
+    marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
+    marks.done("sequential_order_emit",
+               launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START]),
+                                   static_cast<float*>(o[EV_MEAN]), static_cast<float*>(o[EV_STDV]), ctx->sm_count, st));
     CU(cudaGetLastError());
     ctx->last_launches = marks.launches;
     return SGPU_OK;
@@ -509,6 +600,11 @@ void sgpu_destroy(sgpu_ctx_t* ctx) {
     free_outputs(ctx->dev_out, false);
     cudaFree(ctx->ent_ovf); cudaFree(ctx->jnn_mom);
     {
+        PaScratch& w = ctx->pa;
+        cudaFree(w.tile_cnt); cudaFree(w.tile_base); cudaFree(w.tS); cudaFree(w.tQ); cudaFree(w.tA); cudaFree(w.tB);
+        cudaFree(w.tmin); cudaFree(w.ord_list); cudaFree(w.ord_sbase); cudaFree(w.ord_count);
+    }
+    {
         SvbScratch& w = ctx->svb;
         cudaFree(w.cnt); cudaFree(w.base); cudaFree(w.blk_bytes); cudaFree(w.blk_gpos); cudaFree(w.blk_sum);
         cudaFree(w.blk_vpos); cudaFree(w.lane_sum); cudaFree(w.blk_read);
@@ -561,7 +657,7 @@ int64_t sgpu_slot_add_read(sgpu_ctx_t* ctx, uint32_t slot, const int16_t* raw, u
     if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
-    if (sl.mode == 2) return SGPU_E_STATE;  // a batch holds decoded records or svb-zd streams, not both
+    if (sl.mode >= 2) return SGPU_E_STATE;  // a batch holds decoded records, svb-zd streams or pA records, never a mix
     if (n >= (1ull << 31)) return SGPU_E_TOOBIG;  // the reference itself narrows to int32_t (misc.c:20)
     const uint64_t need = align_up(n, SGPU_ALIGN);
     if (need > ctx->max_samples) return SGPU_E_TOOBIG;
@@ -576,7 +672,7 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
                                  double digitisation, double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || !stream) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || sl.mode == 1) return SGPU_E_STATE;
+    if (sl.submitted || sl.mode == 1 || sl.mode == 3) return SGPU_E_STATE;
     if (n_bytes != 0 && n_bytes < 4) return SGPU_E_STREAM;
     uint32_t count = 0;
     if (n_bytes) memcpy(&count, stream, 4);  // slow5_press.c:1093: the original length leads the stream
@@ -609,17 +705,37 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
     return append_record(sl, n, digitisation, offset, range);
 }
 
+int64_t sgpu_slot_add_read_pa(sgpu_ctx_t* ctx, uint32_t slot, const float* pa, uint64_t n) {
+    if (!ctx || slot >= ctx->n_slots || (!pa && n)) return SGPU_E_INVAL;
+    Slot& sl = ctx->slots[slot];
+    if (sl.submitted || sl.mode == 1 || sl.mode == 2) return SGPU_E_STATE;
+    // the slot's int16 sample buffers (pinned and device) hold the floats: max_samples / 2 of them
+    const uint64_t cap = ctx->max_samples / 2;
+    if (n >= (1ull << 32)) return SGPU_E_TOOBIG;
+    const uint64_t need = align_up(n, SGPU_ALIGN);
+    if (need > cap) return SGPU_E_TOOBIG;
+    sgpu_batch_t& b = sl.batch;
+    if (b.n_reads >= ctx->max_reads || sl.used + need > cap) return SGPU_E_FULL;
+    sl.mode = 3;
+    memcpy(reinterpret_cast<float*>(b.samples) + sl.used, pa, (size_t)n * sizeof(float));
+    return append_record(sl, n, 1.0, 0.0, 1.0);  // (offset_f 0, raw_unit_f 1: the values are pA already)
+}
+
 int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (!ctx || slot >= ctx->n_slots || (want & ~63u) || want == 0) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
+    const bool pa_in = sl.mode == 3;
+    if (pa_in && !pa_input_want_ok(want)) return SGPU_E_INVAL;
     CU(cudaSetDevice(ctx->device));
     const sgpu_batch_t& hb = sl.batch;
     const uint32_t nr = hb.n_reads;
     cudaStream_t st = sl.stream;
     SvbBatch svb{};
     const bool compressed = sl.mode == 2;
-    if (compressed) {
+    if (pa_in) {
+        CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sizeof(float), cudaMemcpyHostToDevice, st));
+    } else if (compressed) {
         CU(cudaMemcpyAsync(sl.d_comp, sl.h_comp, (size_t)sl.comp_used, cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(sl.d_comp_off, sl.h_comp_off, (size_t)nr * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(sl.d_comp_len, sl.h_comp_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
@@ -636,7 +752,10 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
     DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, (int)hb.rna, sl.used};
     CU(alloc_outputs(ctx, sl.hout, want, true));
-    const int rc = run_pipeline(ctx, b, want, sl.dout, ctx->compute, compressed ? &svb : nullptr, sl.d_samples);
+    const int rc = pa_in ? run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr,
+                                                         (int)hb.rna, sl.used},
+                                           reinterpret_cast<const float*>(sl.d_samples), want, sl.dout, ctx->compute)
+                         : run_pipeline(ctx, b, want, sl.dout, ctx->compute, compressed ? &svb : nullptr, sl.d_samples);
     if (rc) return rc;
     // small results come back right away; the big arrays are sized by n_events in sgpu_wait
     CU(cudaMemcpyAsync(sl.h_counters, ctx->sc.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
@@ -683,6 +802,19 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(out, ctx->dev_out, want, true);
+    return SGPU_OK;
+}
+
+int sgpu_run_device_pa(sgpu_ctx_t* ctx, const sgpu_dev_pa_batch_t* batch, uint32_t want, void* stream,
+                       sgpu_result_t* out) {
+    if (!ctx || !batch || !out || !pa_input_want_ok(want)) return SGPU_E_INVAL;
+    CU(cudaSetDevice(ctx->device));
+    const DevBatch b{nullptr, batch->read_off, batch->read_len, nullptr, nullptr, batch->n_reads, (int)batch->rna,
+                     batch->span};
+    const int rc = run_pipeline_pa(ctx, b, batch->pa, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
+    if (rc) return rc;
+    memset(out, 0, sizeof *out);
+    fill_result(out, ctx->dev_out, want, false);
     return SGPU_OK;
 }
 

@@ -12,7 +12,8 @@
 //
 // They serve (a) reads that fail the exact-sum witness or the detector
 // boundary-state check of the fast path (fast.cu), (b) SGPU_F_FORCE_GENERIC,
-// and (c) as the on-device cross-check of the fast path in the tests.  The
+// (c) as the on-device cross-check of the fast path in the tests, and (d) batches of
+// the caller's own pA floats (pa_input.cu: gen_prefix_pa_kernel, gen_detect_pa_kernel).  The
 // work list is built on the device (build_seq_list_kernel), so every kernel
 // here is launched with a fixed grid and returns at once when the list is empty.  They keep S, Q (16 B/sample) and t1, t2 (8 B/sample) in
 // an HBM scratch area, so they are NOT the roofline path.
@@ -22,40 +23,71 @@
 namespace sgpu {
 
 // ---------------------------------------------------------------------------
+// 8 consecutive samples of one read as the reference's floats: int16 raw samples through misc.c:28, or pA floats
+// as the caller gave them (getevents(n, pa, rna) on the caller's own signal: pa_input.cu)
+template <typename T> struct Samples8;
+template <> struct Samples8<int16_t> {
+    using Group = int4;  // 16 bytes
+    static constexpr bool kRaw = true;
+    static __device__ __forceinline__ Group zero() { return make_int4(0, 0, 0, 0); }
+    static __device__ __forceinline__ Group load(const Group* p) { return __ldg(p); }
+};
+struct Float8 { float4 a, b; };
+template <> struct Samples8<float> {
+    using Group = Float8;  // 32 bytes
+    static constexpr bool kRaw = false;
+    static __device__ __forceinline__ Group zero() { return {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)}; }
+    static __device__ __forceinline__ Group load(const Group* p) {
+        const float4* q = reinterpret_cast<const float4*>(p);
+        return {__ldg(q), __ldg(q + 1)};
+    }
+    static __device__ __forceinline__ void to_float(const Group& cur, float (&x)[8]) {
+        x[0] = cur.a.x; x[1] = cur.a.y; x[2] = cur.a.z; x[3] = cur.a.w;
+        x[4] = cur.b.x; x[5] = cur.b.y; x[6] = cur.b.z; x[7] = cur.b.w;
+    }
+};
+
 // compute_sum_sumsq: Sinc[base+i] = S[i+1], Qinc[base+i] = Q[i+1]  (S[0]=Q[0]=0 implied)
-__global__ void __launch_bounds__(128) gen_prefix_kernel(DevBatch b, WorkList wl, double* __restrict__ Sinc,
-                                                         double* __restrict__ Qinc) {
-    // one WARP per read: lane 0 runs the two dependent chains of additions (the order IS the result), 32 samples at
-    // a time into shared memory; all lanes then store the tile coalesced (32 lanes walking 32 reads would issue 64
-    // store wavefronts per sample: measured 130 cycles per sample)
-    __shared__ double sS[4][32], sQ[4][32];
-    const uint32_t n_list = *wl.count;
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+// one WARP per read: lane 0 runs the two dependent chains of additions (the order IS the result), 32 samples at a
+// time into shared memory (sS, sQ: [4][32]); all lanes then store the tile coalesced (32 lanes walking 32 reads would
+// issue 64 store wavefronts per sample: measured 130 cycles per sample)
+template <typename T>
+__device__ __forceinline__ void gen_prefix_reads(const DevBatch& b, const T* samples, const WorkList& wl,
+                                                 double* __restrict__ Sinc, double* __restrict__ Qinc,
+                                                 double (&sS)[4][32], double (&sQ)[4][32], uint32_t n_list,
+                                                 uint32_t tid) {
+    using L = Samples8<T>;
+    const int lane = tid & 31, wib = tid >> 5;
+    const uint32_t warp = (blockIdx.x * blockDim.x + tid) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t j = warp; j < n_list; j += n_warps) {
         const uint32_t r = wl.list[j];
         const uint64_t base = wl.sbase[j];
-        // reads start on 16-byte boundaries and the batch is padded to one: whole groups of 8 samples can be loaded
-        const int4* __restrict__ raw8 = reinterpret_cast<const int4*>(b.samples + b.read_off[r]);
+        // reads start on 8-sample boundaries and the batch is padded to one: whole groups of 8 samples can be loaded
+        const typename L::Group* __restrict__ raw8 = reinterpret_cast<const typename L::Group*>(samples + b.read_off[r]);
         const uint32_t n = b.read_len[r], n8 = (n + 7u) >> 3;
-        const float off = b.offset[r], unit = b.unit[r];
+        float off = 0.0f, unit = 0.0f;
+        if constexpr (L::kRaw) { off = b.offset[r]; unit = b.unit[r]; }
         double s = 0.0, q = 0.0;
-        int4 buf[4];  // the next tile's samples (lane 0)
+        typename L::Group buf[4];  // the next tile's samples (lane 0)
         if (lane == 0) {
 #pragma unroll
-            for (int k = 0; k < 4; k++) buf[k] = (uint32_t)k < n8 ? __ldg(raw8 + k) : make_int4(0, 0, 0, 0);
+            for (int k = 0; k < 4; k++) buf[k] = (uint32_t)k < n8 ? L::load(raw8 + k) : L::zero();
         }
         for (uint32_t t0 = 0; t0 < n; t0 += 32) {
             if (lane == 0) {
                 const uint32_t g0 = t0 >> 3;
 #pragma unroll
                 for (int k = 0; k < 4; k++) {
-                    const int4 cur = buf[k];
-                    buf[k] = g0 + 4 + k < n8 ? __ldg(raw8 + g0 + 4 + k) : make_int4(0, 0, 0, 0);
-                    const int v[4] = {cur.x, cur.y, cur.z, cur.w};
+                    const typename L::Group cur = buf[k];
+                    buf[k] = g0 + 4 + k < n8 ? L::load(raw8 + g0 + 4 + k) : L::zero();
                     // everything that does not depend on the running sums first (conversions pipeline), then the chain
                     float x[8];
-                    walk::cvt8(v, off, unit, x);   // misc.c:28 per sample (float add, float multiply)
+                    if constexpr (L::kRaw) {
+                        const int v[4] = {cur.x, cur.y, cur.z, cur.w};
+                        walk::cvt8(v, off, unit, x);   // misc.c:28 per sample (float add, float multiply)
+                    } else {
+                        L::to_float(cur, x);
+                    }
                     double xd[8], qd[8];
 #pragma unroll
                     for (int m = 0; m < 8; m++) {
@@ -79,6 +111,22 @@ __global__ void __launch_bounds__(128) gen_prefix_kernel(DevBatch b, WorkList wl
             __syncwarp();
         }
     }
+}
+
+__global__ void __launch_bounds__(128) gen_prefix_kernel(DevBatch b, WorkList wl, double* __restrict__ Sinc,
+                                                         double* __restrict__ Qinc) {
+    __shared__ double sS[4][32], sQ[4][32];
+    const uint32_t n_list = *wl.count;
+    gen_prefix_reads<int16_t>(b, b.samples, wl, Sinc, Qinc, sS, sQ, n_list, threadIdx.x);  // (the thread index is read
+                                                                                            // where its bound is known)
+}
+
+// the same on the caller's pA floats: the reads of a pA batch that fail the exact-sum witness (pa_input.cu)
+__global__ void __launch_bounds__(128) gen_prefix_pa_kernel(DevBatch b, const float* __restrict__ pa, WorkList wl,
+                                                            double* __restrict__ Sinc, double* __restrict__ Qinc) {
+    __shared__ double sS[4][32], sQ[4][32];
+    const uint32_t n_list = *wl.count;
+    gen_prefix_reads<float>(b, pa, wl, Sinc, Qinc, sS, sQ, n_list, threadIdx.x);
 }
 
 // ---------------------------------------------------------------------------
@@ -207,11 +255,14 @@ __device__ void detect_read_in_order(const DetParams& p, const float* __restrict
 // detector step of walk_core.cuh; a chunk's state after its warm-up must equal its predecessor's end state
 // (compared through a shuffle; the group's last state is carried to the next group). Peaks are owned by the step
 // that emits them. Any mismatch in the read: lane 0 redoes the read in the reference's own order.
+// PA (t arrays of a caller's pA signal, which may hold NaN): returns the number of mismatched chunks, and a NaN
+// t-statistic anywhere in the read also sends it to the reference's order -- the branch-free step's fminf / fmaxf
+// would take the other operand where the reference's comparisons keep a NaN running value (events.c:393-409).
 constexpr int GD_CHUNK = 1024;
-template <int RNA>
-__device__ void detect_read_chunked(const float* __restrict__ t1, const float* __restrict__ t2, uint64_t base,
-                                    uint64_t foff, uint32_t n, uint32_t W, uint32_t* __restrict__ bitmap, int lane,
-                                    const DetParams& p) {
+template <int RNA, bool PA>
+__device__ uint32_t detect_read_chunked(const float* __restrict__ t1, const float* __restrict__ t2, uint64_t base,
+                                        uint64_t foff, uint32_t n, uint32_t W, uint32_t* __restrict__ bitmap, int lane,
+                                        const DetParams& p) {
     using namespace walk;
     if (lane == 0) {
         clear_read_bits(bitmap, foff, foff + n);
@@ -219,7 +270,8 @@ __device__ void detect_read_chunked(const float* __restrict__ t1, const float* _
     }
     __syncwarp();
     const uint32_t n_chunks = (n + GD_CHUNK - 1) / GD_CHUNK;
-    bool bad = false;
+    bool bad = false, nan = false;
+    uint32_t n_bad = 0;
     Canon carry = {};  // end state of the previous group's last chunk
     auto on_emit = [&](int pos) { const uint64_t f = foff + (uint32_t)pos; atomicOr(&bitmap[f >> 5], 1u << (f & 31)); };
     for (uint32_t c0 = 0; c0 < n_chunks; c0 += 32) {
@@ -231,11 +283,17 @@ __device__ void detect_read_chunked(const float* __restrict__ t1, const float* _
         if (have) {
             uint32_t i = (c == 0) ? 1u : s0 - W;   // position 0 is never stepped (masked_to = 0, events.c:387)
             dual_cold(d, (int)i);
-            for (; i < s0; i++)   // warm-up: nothing is recorded
-                dual_step<RNA>(d, (int)i, __ldg(t1 + base + i), __ldg(t2 + base + i), NoEmit());
+            for (; i < s0; i++) {   // warm-up: nothing is recorded
+                const float c1 = __ldg(t1 + base + i), c2 = __ldg(t2 + base + i);
+                if constexpr (PA) nan |= (c1 != c1) | (c2 != c2);
+                dual_step<RNA>(d, (int)i, c1, c2, NoEmit());
+            }
             begin = dual_canon(d, (int)s0);
-            for (; i < s1; i++)
-                dual_step<RNA>(d, (int)i, __ldg(t1 + base + i), __ldg(t2 + base + i), on_emit);
+            for (; i < s1; i++) {
+                const float c1 = __ldg(t1 + base + i), c2 = __ldg(t2 + base + i);
+                if constexpr (PA) nan |= (c1 != c1) | (c2 != c2);
+                dual_step<RNA>(d, (int)i, c1, c2, on_emit);
+            }
             end = dual_canon(d, (int)s1);
         }
         // chunk c must have reached the state chunk c-1 ended in
@@ -246,20 +304,24 @@ __device__ void detect_read_chunked(const float* __restrict__ t1, const float* _
             if (lane == 0) prev = carry.v[q];
             same = same && (prev == begin.v[q]);
         }
-        if (have && c > 0 && !same) bad = true;
+        if (have && c > 0 && !same) { bad = true; n_bad++; }
         const int last = (int)min(31u, n_chunks - 1u - c0);
 #pragma unroll
         for (int q = 0; q < 5; q++) carry.v[q] = __shfl_sync(0xffffffffu, end.v[q], last);
     }
-    if (__any_sync(0xffffffffu, bad)) {
+    if (__any_sync(0xffffffffu, bad || nan)) {
         __syncwarp();
         if (lane == 0) detect_read_in_order(p, t1, t2, base, foff, n, bitmap);
     }
+    if constexpr (PA) return __reduce_add_sync(0xffffffffu, n_bad);
+    return 0u;
 }
 
-__global__ void __launch_bounds__(128) gen_detect_kernel(DevBatch b, WorkList wl, const float* __restrict__ t1,
-                                                         const float* __restrict__ t2, uint32_t* __restrict__ bitmap,
-                                                         uint32_t W) {
+// PA: fixups[r] = the read's mismatched chunks
+template <bool PA>
+__device__ __forceinline__ void gen_detect_reads(const DevBatch& b, const WorkList& wl, const float* __restrict__ t1,
+                                                 const float* __restrict__ t2, uint32_t* __restrict__ bitmap,
+                                                 uint32_t W, uint32_t* __restrict__ fixups) {
     const uint32_t n_list = *wl.count;
     const DetParams p = det_params(b.rna);
     const int lane = threadIdx.x & 31;
@@ -271,9 +333,22 @@ __global__ void __launch_bounds__(128) gen_detect_kernel(DevBatch b, WorkList wl
         const uint32_t n = b.read_len[r];
         if (n == 0) continue;
         if (n >= (1u << 30)) { if (lane == 0) detect_read_in_order(p, t1, t2, base, foff, n, bitmap); continue; }
-        if (b.rna) detect_read_chunked<1>(t1, t2, base, foff, n, W, bitmap, lane, p);
-        else detect_read_chunked<0>(t1, t2, base, foff, n, W, bitmap, lane, p);
+        const uint32_t n_bad = b.rna ? detect_read_chunked<1, PA>(t1, t2, base, foff, n, W, bitmap, lane, p)
+                                     : detect_read_chunked<0, PA>(t1, t2, base, foff, n, W, bitmap, lane, p);
+        if constexpr (PA) { if (lane == 0) fixups[r] = n_bad; }
     }
+}
+
+__global__ void __launch_bounds__(128) gen_detect_kernel(DevBatch b, WorkList wl, const float* __restrict__ t1,
+                                                         const float* __restrict__ t2, uint32_t* __restrict__ bitmap,
+                                                         uint32_t W) {
+    gen_detect_reads<false>(b, wl, t1, t2, bitmap, W, nullptr);
+}
+
+__global__ void __launch_bounds__(128) gen_detect_pa_kernel(DevBatch b, WorkList wl, const float* __restrict__ t1,
+                                                            const float* __restrict__ t2, uint32_t* __restrict__ bitmap,
+                                                            uint32_t W, uint32_t* __restrict__ fixups) {
+    gen_detect_reads<true>(b, wl, t1, t2, bitmap, W, fixups);
 }
 
 // ---------------------------------------------------------------------------
@@ -468,6 +543,16 @@ int launch_generic_detect(const DevBatch& b, const WorkList& wl, Scratch& sc, in
     gen_prefix_kernel<<<sm_count * 8, 128, 0, st>>>(b, wl, sc.Sinc, sc.Qinc);
     gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, wl, sc.Sinc, sc.Qinc, sc.t1, sc.t2);
     gen_detect_kernel<<<sm_count * 8, 128, 0, st>>>(b, wl, sc.t1, sc.t2, sc.bitmap, b.rna ? 384u : 64u);  // (its own warm-up, longer than the walker's)
+    return 3;
+}
+
+// a pA batch (pa_input.cu): the prefix sums of the reads in `ordered` (those that failed the exact-sum witness) in
+// the reference's order -- the others' were stored by pa_scan_kernel --, then t-statistics and detector for all reads
+int launch_generic_detect_pa(const DevBatch& b, const float* pa, const WorkList& ordered, const WorkList& all,
+                             Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st) {
+    gen_prefix_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, pa, ordered, sc.Sinc, sc.Qinc);
+    gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, all, sc.Sinc, sc.Qinc, sc.t1, sc.t2);
+    gen_detect_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, all, sc.t1, sc.t2, sc.bitmap, b.rna ? 384u : 64u, fixups);
     return 3;
 }
 

@@ -59,6 +59,8 @@ struct Scratch {
 int launch_generic_detect(const DevBatch& b, const WorkList& wl, Scratch& sc, int sm_count, cudaStream_t st);
 int launch_generic_emit(const DevBatch& b, const WorkList& wl, Scratch& sc, const uint64_t* ev_off, uint64_t ev_cap,
                         uint32_t* ev_start, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
+int launch_generic_detect_pa(const DevBatch& b, const float* pa, const WorkList& ordered, const WorkList& all,
+                             Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st);
 int launch_scan_u32(const uint32_t* cnt, uint32_t n, uint64_t* off, uint64_t* total_out, Scratch& sc, cudaStream_t st);
 uint32_t scan_tiles_for(uint32_t n);
 
@@ -80,6 +82,20 @@ int launch_rank_events(const DevBatch& b, Scratch& sc, uint64_t* ev_off, int sm_
 int launch_fast_emit(const DevBatch& b, Scratch& sc, uint64_t ev_cap, uint32_t* ev_start, float* ev_mean,
                      float* ev_stdv, const uint32_t* fixups, int sm_count, cudaStream_t st);
 int launch_pa(const DevBatch& b, float* pa, int sm_count, cudaStream_t st);
+
+// pa_input.cu (event detection on the caller's pA floats: exactness witness and parallel scan of the prefix sums)
+struct PaScratch {                 // allocated on the first pA batch
+    uint32_t* tile_cnt;            // [max_reads] tiles of every read
+    uint64_t* tile_base;           // [max_reads+1] their exclusive scan
+    double* tS; double* tQ;        // [max_tiles] the tiles' sums, then their prefixes within the read
+    double* tA; double* tB;        // [max_tiles] upper bounds of sum |x| and sum fl(x*x)
+    uint2* tmin;                   // [max_tiles] smallest nonzero |x| and fl(x*x) (float bits)
+    uint32_t* ord_list; uint64_t* ord_sbase; uint32_t* ord_count;  // reads summed in the reference's order
+    uint64_t max_tiles;
+};
+uint64_t pa_tile_capacity(uint64_t max_samples, uint32_t max_reads);
+int launch_pa_prefix(const DevBatch& b, const float* pa, PaScratch& w, Scratch& sc, uint32_t* seq_flag,
+                     uint32_t* fixups, int force_all, int sm_count, cudaStream_t st);
 
 // svbzd.cu (svb-zd signal streams -> int16 samples in HBM)
 struct SvbBatch {
