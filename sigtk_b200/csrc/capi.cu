@@ -10,7 +10,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
+#include <utility>
 
 #include "kernels.cuh"
 
@@ -18,8 +20,8 @@ using namespace sgpu;
 
 namespace {
 
-// The per-batch output arrays. OUTS describes each one once; every place that allocates, clears, copies back,
-// returns or frees outputs loops over it. Device and pinned host copies are arrays of N_OUT pointers indexed by Out.
+// The per-batch output arrays. OUTS describes each one once; every place that allocates, clears, copies back or
+// returns outputs loops over it. Device and pinned host copies are arrays of N_OUT byte buffers indexed by Out.
 enum Out { EV_OFF, EV_START, EV_MEAN, EV_STDV, SEQ_ORDER, FIXUPS, STAT, ENT, JNN_CNT, JNN_SEG, PREFIX_POS, PREFIX_STAT,
            PA, N_OUT };
 
@@ -87,19 +89,22 @@ uint64_t out_elems(int k, uint64_t reads, uint64_t samples, uint64_t events) {
 }
 
 struct Slot {
-    // pinned host input
+    // pinned host input: the fields of `batch` (what sgpu_slot_batch hands out) point at the five arrays below it
     sgpu_batch_t batch{};
+    PinBuf<int16_t> samples;
+    PinBuf<uint64_t> read_off;
+    PinBuf<uint32_t> read_len;
+    PinBuf<float> offset_f, raw_unit_f;
     uint64_t used = 0;
     // device input
-    int16_t* d_samples = nullptr;
-    uint64_t* d_read_off = nullptr;
-    uint32_t* d_read_len = nullptr;
-    float* d_offset = nullptr;
-    float* d_unit = nullptr;
-    void* dout[N_OUT] = {};  // device outputs
-    void* hout[N_OUT] = {};  // their pinned host copies
-    unsigned long long* h_counters = nullptr;  // [4]
-    int* h_status = nullptr;
+    DevBuf<int16_t> d_samples;
+    DevBuf<uint64_t> d_read_off;
+    DevBuf<uint32_t> d_read_len;
+    DevBuf<float> d_offset, d_unit;
+    DevBuf<void> dout[N_OUT];  // device outputs
+    PinBuf<void> hout[N_OUT];  // their pinned host copies
+    PinBuf<unsigned long long> h_counters;  // [4]
+    PinBuf<int> h_status;
     cudaStream_t stream = nullptr;
     cudaEvent_t in_ready = nullptr, kernels_done = nullptr, small_back = nullptr;
     bool submitted = false;
@@ -107,11 +112,18 @@ struct Slot {
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     int mode = 0;                    // 0: empty, 1: decoded int16 records, 2: svb-zd streams, 3: pA records (floats
                                      // in the sample buffers: max_samples / 2 of them)
-    uint8_t* h_comp = nullptr;       // pinned, comp_cap bytes
-    uint8_t* d_comp = nullptr;       // comp_cap + 16 bytes
-    uint64_t* h_comp_off = nullptr; uint64_t* d_comp_off = nullptr;
-    uint32_t* h_comp_len = nullptr; uint32_t* d_comp_len = nullptr;
+    PinBuf<uint8_t> h_comp;          // comp_cap bytes
+    DevBuf<uint8_t> d_comp;          // comp_cap + 16 bytes
+    PinBuf<uint64_t> h_comp_off; DevBuf<uint64_t> d_comp_off;
+    PinBuf<uint32_t> h_comp_len; DevBuf<uint32_t> d_comp_len;
     uint64_t comp_used = 0, svb_blocks = 0;
+
+    ~Slot() {
+        if (stream) cudaStreamDestroy(stream);
+        if (in_ready) cudaEventDestroy(in_ready);
+        if (kernels_done) cudaEventDestroy(kernels_done);
+        if (small_back) cudaEventDestroy(small_back);
+    }
 };
 
 }  // namespace
@@ -125,12 +137,12 @@ struct sgpu_ctx {
     uint32_t flags = 0;
     uint64_t ev_cap = 0;
     Scratch sc{};
-    void* dev_out[N_OUT] = {};   // outputs of the device-resident path
-    Slot* slots = nullptr;
+    DevBuf<void> dev_out[N_OUT]; // outputs of the device-resident path
+    std::unique_ptr<Slot[]> slots;
     SvbScratch svb{};            // workspace of the svb-zd decoder (allocated on first use)
-    float* jnn_mom = nullptr;    // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
+    DevBuf<float> jnn_mom;       // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
     int pore_rna004 = 0;         // SGPU_PARAM_PORE: jnnv2 parameters of `prefix` (misc.c:74-101 picks them from the header)
-    uint32_t* ent_ovf = nullptr; // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
+    DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     uint64_t comp_cap = 0;       // bytes of compressed input a slot can hold
     cudaStream_t compute = nullptr;
@@ -143,6 +155,11 @@ struct sgpu_ctx {
     int n_stages = 0;
     cudaStream_t stage_stream = nullptr;
     char err[512] = {0};
+
+    ~sgpu_ctx() {
+        if (compute) cudaStreamDestroy(compute);
+        for (cudaEvent_t e : stage_ev) if (e) cudaEventDestroy(e);
+    }
 };
 
 namespace {
@@ -158,48 +175,28 @@ bool cuda_fail(sgpu_ctx* c, cudaError_t e, const char* what, int line) {
         if (cuda_fail(ctx, (call), #call, __LINE__)) return SGPU_E_CUDA; \
     } while (0)
 
-// Allocates *p unless it is set already, and sets it only on success: an allocation that failed part-way through
-// a list is completed by the next call instead of leaving a NULL pointer behind a non-NULL one.
-cudaError_t alloc_once(void** p, size_t bytes, bool pinned) {
-    if (*p) return cudaSuccess;
-    void* q = nullptr;
-    const cudaError_t e = pinned ? cudaHostAlloc(&q, bytes, cudaHostAllocDefault) : cudaMalloc(&q, bytes);
-    if (e == cudaSuccess) *p = q;
-    return e;
-}
-template <typename T>
-cudaError_t dev_alloc(T** p, uint64_t count) {
-    return alloc_once(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T), false);
-}
-template <typename T>
-cudaError_t pin_alloc(T** p, uint64_t count) {
-    return alloc_once(reinterpret_cast<void**>(p), (size_t)(count ? count : 1) * sizeof(T), true);
-}
-
 uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 
 // allocates (device or pinned) every output of `o` that is eager or belongs to `want` and does not exist yet
-cudaError_t alloc_outputs(const sgpu_ctx* ctx, void** o, uint32_t want, bool pinned) {
+template <bool PINNED>
+cudaError_t alloc_outputs(const sgpu_ctx* ctx, Buf<void, PINNED>* o, uint32_t want) {
     for (int k = 0; k < N_OUT; k++) {
         if (!OUTS[k].eager && !(want & OUTS[k].want)) continue;
         const uint64_t n = out_elems(k, ctx->max_reads, ctx->max_samples, ctx->ev_cap);
-        const cudaError_t e = alloc_once(&o[k], (size_t)n * OUTS[k].size, pinned);
+        const cudaError_t e = o[k].ensure(n * OUTS[k].size);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
 
-void free_outputs(void** o, bool pinned) {
-    for (int k = 0; k < N_OUT; k++) {
-        if (pinned) cudaFreeHost(o[k]); else cudaFree(o[k]);
-    }
-}
-
 // points the fields of *r at the outputs of `want`, and at every eager output when `all_eager`; the others stay NULL
-void fill_result(sgpu_result_t* r, void* const* o, uint32_t want, bool all_eager) {
+template <bool PINNED>
+void fill_result(sgpu_result_t* r, const Buf<void, PINNED>* o, uint32_t want, bool all_eager) {
     for (int k = 0; k < N_OUT; k++)
-        if ((want & OUTS[k].want) || (all_eager && OUTS[k].eager))
-            memcpy(reinterpret_cast<char*>(r) + OUTS[k].field, &o[k], sizeof(void*));
+        if ((want & OUTS[k].want) || (all_eager && OUTS[k].eager)) {
+            void* const p = o[k];
+            memcpy(reinterpret_cast<char*>(r) + OUTS[k].field, &p, sizeof p);
+        }
 }
 
 // queues on the slot's stream the D2H copy of every output of `want` that is sized by the batch's reads and samples,
@@ -238,21 +235,21 @@ struct StageMarks {  // records a CUDA event between kernel groups when the cont
 int alloc_svb_scratch(sgpu_ctx* ctx) {
     SvbScratch& w = ctx->svb;
     w.max_blocks = svbzd_max_blocks(ctx->max_samples, ctx->max_reads);
-    CU(dev_alloc(&w.cnt, ctx->max_reads));
-    CU(dev_alloc(&w.base, (uint64_t)ctx->max_reads + 1));
-    CU(dev_alloc(&w.blk_bytes, w.max_blocks));
-    CU(dev_alloc(&w.blk_gpos, w.max_blocks + 1));
-    CU(dev_alloc(&w.blk_sum, w.max_blocks));
-    CU(dev_alloc(&w.blk_vpos, w.max_blocks + 1));
-    CU(dev_alloc(&w.lane_sum, w.max_blocks * 32));
-    CU(dev_alloc(&w.blk_read, w.max_blocks));
+    CU(w.cnt.ensure(ctx->max_reads));
+    CU(w.base.ensure((uint64_t)ctx->max_reads + 1));
+    CU(w.blk_bytes.ensure(w.max_blocks));
+    CU(w.blk_gpos.ensure(w.max_blocks + 1));
+    CU(w.blk_sum.ensure(w.max_blocks));
+    CU(w.blk_vpos.ensure(w.max_blocks + 1));
+    CU(w.lane_sum.ensure(w.max_blocks * 32));
+    CU(w.blk_read.ensure(w.max_blocks));
     return SGPU_OK;
 }
 
 // nothing but empty records: every per-read output gets its defined value for an empty record (no event, zero
 // statistics / entropies / segments, "record not longer than the window" for prefix) instead of whatever the previous
 // batch left in the buffers
-int clear_empty_batch(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cudaStream_t st) {
+int clear_empty_batch(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st) {
     for (int k = 0; k < N_OUT; k++) {
         const OutSpec& s = OUTS[k];
         if (s.empty < 0 || !((want & s.want) || (s.empty & ANY_WANT))) continue;
@@ -264,11 +261,11 @@ int clear_empty_batch(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o,
 }
 
 // The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies.
-int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cudaStream_t st,
+int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
                  const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
     if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
-    CU(alloc_outputs(ctx, o, want, false));
+    CU(alloc_outputs(ctx, o, want));
     CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
     CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
     StageMarks marks(ctx, st);
@@ -276,33 +273,33 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cuda
     if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
     const bool events = (want & SGPU_WANT_EVENTS) != 0;
-    float* const pa = (want & SGPU_WANT_PA) ? static_cast<float*>(o[PA]) : nullptr;
-    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER]);
-    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS]);
+    float* const pa = (want & SGPU_WANT_PA) ? static_cast<float*>(o[PA].get()) : nullptr;
+    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
+    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS].get());
     if (pa && (!events || force_generic))  // with events on the fast path the pA store is fused into walk_chunks_kernel
         marks.done("pa", launch_pa(b, pa, ctx->sm_count, st));
     if (want & SGPU_WANT_STAT) {
-        float* const stat = static_cast<float*>(o[STAT]);
+        float* const stat = static_cast<float*>(o[STAT].get());
         marks.done("stat_moments", launch_stat_moments(b, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
         marks.done("stat_median", launch_stat_median(b, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
     }
     if (want & SGPU_WANT_ENT) {
         if (!ctx->ent_ovf) {
             const uint64_t words = ent_overflow_words(ctx->sm_count);
-            CU(dev_alloc(&ctx->ent_ovf, words));
+            CU(ctx->ent_ovf.ensure(words));
             CU(cudaMemsetAsync(ctx->ent_ovf, 0, (size_t)words * sizeof(uint32_t), st));
         }
-        marks.done("ent", launch_ent(b, ctx->ent_ovf, static_cast<double*>(o[ENT]), ctx->sm_count, st));
+        marks.done("ent", launch_ent(b, ctx->ent_ovf, static_cast<double*>(o[ENT].get()), ctx->sm_count, st));
     }
     if (want & SGPU_WANT_JNN) {
-        CU(dev_alloc(&ctx->jnn_mom, (uint64_t)ctx->max_reads * 2));
+        CU(ctx->jnn_mom.ensure((uint64_t)ctx->max_reads * 2));
         marks.done("jnn_moments", launch_jnn_moments(b, ctx->jnn_mom, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
-        marks.done("jnn_walk", launch_jnn(b, ctx->jnn_mom, static_cast<uint32_t*>(o[JNN_CNT]),
-                                          static_cast<int32_t*>(o[JNN_SEG]), ctx->sm_count, st));
+        marks.done("jnn_walk", launch_jnn(b, ctx->jnn_mom, static_cast<uint32_t*>(o[JNN_CNT].get()),
+                                          static_cast<int32_t*>(o[JNN_SEG].get()), ctx->sm_count, st));
     }
     if (want & SGPU_WANT_PREFIX)
-        marks.done("prefix", launch_prefix(b, ctx->pore_rna004, static_cast<int32_t*>(o[PREFIX_POS]),
-                                           static_cast<float*>(o[PREFIX_STAT]), ctx->sm_count, st));
+        marks.done("prefix", launch_prefix(b, ctx->pore_rna004, static_cast<int32_t*>(o[PREFIX_POS].get()),
+                                           static_cast<float*>(o[PREFIX_STAT].get()), ctx->sm_count, st));
     if (events) {
         const uint32_t n_tiles = fast_tiles_for(b.span);
         if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
@@ -320,10 +317,10 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cuda
         WorkList wl{sc.seq_list, sc.seq_sbase, sc.seq_count};
         n += launch_generic_detect(b, wl, sc, ctx->sm_count, st);
         marks.done("sequential_order_detect", n);
-        uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF]);
-        uint32_t* const ev_start = static_cast<uint32_t*>(o[EV_START]);
-        float* const ev_mean = static_cast<float*>(o[EV_MEAN]);
-        float* const ev_stdv = static_cast<float*>(o[EV_STDV]);
+        uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF].get());
+        uint32_t* const ev_start = static_cast<uint32_t*>(o[EV_START].get());
+        float* const ev_mean = static_cast<float*>(o[EV_MEAN].get());
+        float* const ev_stdv = static_cast<float*>(o[EV_STDV].get());
         marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
         marks.done("emit_events",
                    launch_fast_emit(b, sc, ctx->ev_cap, ev_start, ev_mean, ev_stdv, fix, ctx->sm_count, st));
@@ -338,41 +335,39 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, void** o, cuda
 int alloc_pa_scratch(sgpu_ctx* ctx) {
     PaScratch& w = ctx->pa;
     w.max_tiles = pa_tile_capacity(ctx->max_samples, ctx->max_reads);
-    CU(dev_alloc(&w.tile_cnt, ctx->max_reads));
-    CU(dev_alloc(&w.tile_base, (uint64_t)ctx->max_reads + 1));
-    CU(dev_alloc(&w.tS, w.max_tiles));
-    CU(dev_alloc(&w.tQ, w.max_tiles));
-    CU(dev_alloc(&w.tA, w.max_tiles));
-    CU(dev_alloc(&w.tB, w.max_tiles));
-    CU(dev_alloc(&w.tmin, w.max_tiles));
-    CU(dev_alloc(&w.ord_list, ctx->max_reads));
-    CU(dev_alloc(&w.ord_sbase, ctx->max_reads));
-    CU(dev_alloc(&w.ord_count, 1));
+    CU(w.tile_cnt.ensure(ctx->max_reads));
+    CU(w.tile_base.ensure((uint64_t)ctx->max_reads + 1));
+    CU(w.tS.ensure(w.max_tiles));
+    CU(w.tQ.ensure(w.max_tiles));
+    CU(w.tA.ensure(w.max_tiles));
+    CU(w.tB.ensure(w.max_tiles));
+    CU(w.tmin.ensure(w.max_tiles));
+    CU(w.ord_list.ensure(ctx->max_reads));
+    CU(w.ord_sbase.ensure(ctx->max_reads));
+    CU(w.ord_count.ensure(1));
     return SGPU_OK;
 }
 
 // A pA batch keeps its prefix sums and t-statistics at the reads' own offsets, so the sequential-order scratch must
 // hold the whole span. Contexts over 64 Mi samples start with an eighth of that (sgpu_create); the first pA batch that
 // needs more grows it to max_samples for the rest of the context's life (later int16 batches use it too). The old
-// arrays are freed only once the new ones exist (cudaFree waits for the device).
+// arrays are freed only once the new ones exist (freeing waits for the device).
 int grow_seq_scratch(sgpu_ctx* ctx) {
     Scratch& sc = ctx->sc;
     const uint64_t n = ctx->max_samples;
-    double *S = nullptr, *Q = nullptr;
-    float *t1 = nullptr, *t2 = nullptr;
-    cudaError_t e = dev_alloc(&S, n);
-    if (e == cudaSuccess) e = dev_alloc(&Q, n);
-    if (e == cudaSuccess) e = dev_alloc(&t1, n);
-    if (e == cudaSuccess) e = dev_alloc(&t2, n);
-    if (e != cudaSuccess) {
-        cudaFree(S); cudaFree(Q); cudaFree(t1); cudaFree(t2);
+    DevBuf<double> S, Q;
+    DevBuf<float> t1, t2;
+    cudaError_t e = S.ensure(n);
+    if (e == cudaSuccess) e = Q.ensure(n);
+    if (e == cudaSuccess) e = t1.ensure(n);
+    if (e == cudaSuccess) e = t2.ensure(n);
+    if (e != cudaSuccess) {  // (the buffers that were allocated free themselves)
         cudaGetLastError();  // (an allocation failure is reported here, not by the next launch check)
         snprintf(ctx->err, sizeof ctx->err, "growing the sequential-order scratch to %llu samples: %s",
                  (unsigned long long)n, cudaGetErrorString(e));
         return SGPU_E_NOMEM;
     }
-    cudaFree(sc.Sinc); cudaFree(sc.Qinc); cudaFree(sc.t1); cudaFree(sc.t2);
-    sc.Sinc = S; sc.Qinc = Q; sc.t1 = t1; sc.t2 = t2;
+    sc.Sinc = std::move(S); sc.Qinc = std::move(Q); sc.t1 = std::move(t1); sc.t2 = std::move(t2);
     sc.gen_cap = n;
     return SGPU_OK;
 }
@@ -380,12 +375,13 @@ int grow_seq_scratch(sgpu_ctx* ctx) {
 // The kernel sequence of a batch of pA records (getevents(n, pa, rna), events.c:553-573) into the device outputs `o`:
 // the prefix sums by the witness-checked scan or in the reference's order (pa_input.cu), then the sequential-order
 // kernels for every read. No host synchronisation, no host<->device copies (except when the scratch grows).
-int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t want, void** o, cudaStream_t st) {
+int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t want, DevBuf<void>* o,
+                    cudaStream_t st) {
     Scratch& sc = ctx->sc;
     if (!pa_input_want_ok(want)) return SGPU_E_INVAL;
     if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
     if (b.n_reads && b.span && !pa) return SGPU_E_INVAL;
-    CU(alloc_outputs(ctx, o, want, false));
+    CU(alloc_outputs(ctx, o, want));
     int rc = alloc_pa_scratch(ctx);
     if (!rc && b.span > sc.gen_cap) rc = grow_seq_scratch(ctx);
     if (rc) return rc;
@@ -395,19 +391,20 @@ int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t 
     if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(ctx, b, want, o, st);
     const uint32_t n_tiles = fast_tiles_for(b.span);
     if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
-    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER]);
-    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS]);
+    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
+    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS].get());
     CU(cudaMemsetAsync(sc.bitmap, 0, (size_t)n_tiles * (FAST_TILE / 32) * sizeof(uint32_t), st));
     const int force = (ctx->flags & SGPU_F_FORCE_GENERIC) ? 1 : 0;
     marks.done("pa_prefix", launch_pa_prefix(b, pa, ctx->pa, sc, seq, fix, force, ctx->sm_count, st));
     const WorkList ordered{ctx->pa.ord_list, ctx->pa.ord_sbase, ctx->pa.ord_count};
     const WorkList all{sc.seq_list, sc.seq_sbase, sc.seq_count};
     marks.done("sequential_order_detect", launch_generic_detect_pa(b, pa, ordered, all, sc, fix, ctx->sm_count, st));
-    uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF]);
+    uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF].get());
     marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
     marks.done("sequential_order_emit",
-               launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START]),
-                                   static_cast<float*>(o[EV_MEAN]), static_cast<float*>(o[EV_STDV]), ctx->sm_count, st));
+               launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START].get()),
+                                   static_cast<float*>(o[EV_MEAN].get()), static_cast<float*>(o[EV_STDV].get()),
+                                   ctx->sm_count, st));
     CU(cudaGetLastError());
     ctx->last_launches = marks.launches;
     return SGPU_OK;
@@ -511,71 +508,71 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
     // (SGPU_F_FULL_SEQ_SCRATCH: a context opened for one huge read must be able to redo that read in order)
     sc.gen_cap = (max_samples <= (64ull << 20) || (flags & (SGPU_F_FORCE_GENERIC | SGPU_F_FULL_SEQ_SCRATCH)))
                      ? max_samples : max_samples / 8;
-    CUC(dev_alloc(&sc.Sinc, sc.gen_cap));
-    CUC(dev_alloc(&sc.Qinc, sc.gen_cap));
-    CUC(dev_alloc(&sc.t1, sc.gen_cap));
-    CUC(dev_alloc(&sc.t2, sc.gen_cap));
+    CUC(sc.Sinc.ensure(sc.gen_cap));
+    CUC(sc.Qinc.ensure(sc.gen_cap));
+    CUC(sc.t1.ensure(sc.gen_cap));
+    CUC(sc.t2.ensure(sc.gen_cap));
     sc.max_tiles = fast_tiles_for(max_samples) + 1;
     sc.bitmap_words = (uint64_t)sc.max_tiles * (FAST_TILE / 32);
-    CUC(dev_alloc(&sc.bitmap, sc.bitmap_words));
+    CUC(sc.bitmap.ensure(sc.bitmap_words));
     sc.wk_slots = walk_state_slots(max_samples, max_reads);
-    CUC(dev_alloc(&sc.wk_begin, sc.wk_slots * 8));
-    CUC(dev_alloc(&sc.wk_end, sc.wk_slots * 8));
-    CUC(dev_alloc(&sc.wk_cnt, max_reads));
-    CUC(dev_alloc(&sc.wk_ibase, (uint64_t)max_reads + 1));
+    CUC(sc.wk_begin.ensure(sc.wk_slots * 8));
+    CUC(sc.wk_end.ensure(sc.wk_slots * 8));
+    CUC(sc.wk_cnt.ensure(max_reads));
+    CUC(sc.wk_ibase.ensure((uint64_t)max_reads + 1));
     sc.job_cap = walk_job_capacity(max_samples);
-    CUC(dev_alloc(&sc.jobs, (uint64_t)sc.job_cap * 4));
-    CUC(dev_alloc(&sc.job_count, 1));
+    CUC(sc.jobs.ensure((uint64_t)sc.job_cap * 4));
+    CUC(sc.job_count.ensure(1));
     sc.tune_chunk_len = 0; sc.tune_warmup = 0; sc.tune_thr_long = 9.0f;  // events.c:46,53: threshold of the long detector
     sc.tune_stat_cta_min = STAT_CTA_MIN_DEFAULT;
-    CUC(dev_alloc(&sc.tile_cnt, sc.max_tiles));
-    CUC(dev_alloc(&sc.tile_read0, sc.max_tiles));
-    CUC(dev_alloc(&sc.tile_base, (uint64_t)sc.max_tiles + 1));
-    CUC(dev_alloc(&sc.wit_min, max_reads));
-    CUC(dev_alloc(&sc.wit_max, max_reads));
-    CUC(dev_alloc(&sc.seq_list, max_reads));
-    CUC(dev_alloc(&sc.seq_sbase, (uint64_t)max_reads + 1));
-    CUC(dev_alloc(&sc.seq_count, 1));
-    CUC(dev_alloc(&sc.cursor, 1));
+    CUC(sc.tile_cnt.ensure(sc.max_tiles));
+    CUC(sc.tile_read0.ensure(sc.max_tiles));
+    CUC(sc.tile_base.ensure((uint64_t)sc.max_tiles + 1));
+    CUC(sc.wit_min.ensure(max_reads));
+    CUC(sc.wit_max.ensure(max_reads));
+    CUC(sc.seq_list.ensure(max_reads));
+    CUC(sc.seq_sbase.ensure((uint64_t)max_reads + 1));
+    CUC(sc.seq_count.ensure(1));
+    CUC(sc.cursor.ensure(1));
     {
         uint64_t most = sc.max_tiles > max_reads ? sc.max_tiles : max_reads;
         const uint64_t svb_blocks = svbzd_max_blocks(max_samples, max_reads);
         if (svb_blocks > most) most = svb_blocks;
-        CUC(dev_alloc(&sc.scan_status, scan_tiles_for((uint32_t)most) + 1));
+        CUC(sc.scan_status.ensure(scan_tiles_for((uint32_t)most) + 1));
     }
     ctx->comp_cap = 2 * max_samples;
     if (flags & SGPU_F_STAGE_TIMERS)
         for (int k = 0; k <= sgpu_ctx::MAX_STAGES; k++) CUC(cudaEventCreate(&ctx->stage_ev[k]));
-    CUC(dev_alloc(&sc.scan_ticket, 1));
-    CUC(dev_alloc(&sc.status, 1));
-    CUC(dev_alloc(&sc.counters, 4));
+    CUC(sc.scan_ticket.ensure(1));
+    CUC(sc.status.ensure(1));
+    CUC(sc.counters.ensure(4));
     CUC(cudaStreamCreateWithFlags(&ctx->compute, cudaStreamNonBlocking));
-    CUC(alloc_outputs(ctx, ctx->dev_out, 0, false));
+    CUC(alloc_outputs(ctx, ctx->dev_out, 0));
     if (n_slots) {
-        ctx->slots = new (std::nothrow) Slot[n_slots];
+        ctx->slots.reset(new (std::nothrow) Slot[n_slots]);
         if (!ctx->slots) return fail(SGPU_E_NOMEM);
         for (uint32_t s = 0; s < n_slots; s++) {
             Slot& sl = ctx->slots[s];
-            CUC(pin_alloc(&sl.batch.samples, max_samples));
-            CUC(pin_alloc(&sl.batch.read_off, (uint64_t)max_reads + 1));
-            CUC(pin_alloc(&sl.batch.read_len, max_reads));
-            CUC(pin_alloc(&sl.batch.offset_f, max_reads));
-            CUC(pin_alloc(&sl.batch.raw_unit_f, max_reads));
-            CUC(dev_alloc(&sl.d_samples, max_samples));
-            CUC(dev_alloc(&sl.d_read_off, (uint64_t)max_reads + 1));
-            CUC(dev_alloc(&sl.d_read_len, max_reads));
-            CUC(dev_alloc(&sl.d_offset, max_reads));
-            CUC(dev_alloc(&sl.d_unit, max_reads));
+            CUC(sl.samples.ensure(max_samples));
+            CUC(sl.read_off.ensure((uint64_t)max_reads + 1));
+            CUC(sl.read_len.ensure(max_reads));
+            CUC(sl.offset_f.ensure(max_reads));
+            CUC(sl.raw_unit_f.ensure(max_reads));
+            CUC(sl.d_samples.ensure(max_samples));
+            CUC(sl.d_read_off.ensure((uint64_t)max_reads + 1));
+            CUC(sl.d_read_len.ensure(max_reads));
+            CUC(sl.d_offset.ensure(max_reads));
+            CUC(sl.d_unit.ensure(max_reads));
             // every slot gets its own outputs (its D2H overlaps the next slot's kernels)
-            CUC(alloc_outputs(ctx, sl.dout, 0, false));
-            CUC(alloc_outputs(ctx, sl.hout, 0, true));
-            CUC(pin_alloc(&sl.h_counters, 4));
-            CUC(pin_alloc(&sl.h_status, 1));
+            CUC(alloc_outputs(ctx, sl.dout, 0));
+            CUC(alloc_outputs(ctx, sl.hout, 0));
+            CUC(sl.h_counters.ensure(4));
+            CUC(sl.h_status.ensure(1));
             CUC(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
             CUC(cudaEventCreateWithFlags(&sl.in_ready, cudaEventDisableTiming));
             CUC(cudaEventCreateWithFlags(&sl.kernels_done, cudaEventDisableTiming));
             CUC(cudaEventCreateWithFlags(&sl.small_back, cudaEventDisableTiming));
-            sl.batch.n_reads = 0;
+            sl.batch = sgpu_batch_t{sl.samples, sl.read_off, sl.read_len, sl.offset_f, sl.raw_unit_f, 0, 0};
             sl.batch.read_off[0] = 0;
         }
     }
@@ -586,49 +583,9 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
 
 void sgpu_destroy(sgpu_ctx_t* ctx) {
     if (!ctx) return;
-    cudaSetDevice(ctx->device);
+    cudaSetDevice(ctx->device);  // its members free its arrays, streams and events on this device (one thread may
+                                 // drive several GPUs)
     cudaDeviceSynchronize();
-    Scratch& sc = ctx->sc;
-    cudaFree(sc.Sinc); cudaFree(sc.Qinc); cudaFree(sc.t1); cudaFree(sc.t2); cudaFree(sc.bitmap);
-    cudaFree(sc.wk_begin); cudaFree(sc.wk_end); cudaFree(sc.wk_cnt); cudaFree(sc.wk_ibase);
-    cudaFree(sc.jobs); cudaFree(sc.job_count);
-    cudaFree(sc.tile_cnt); cudaFree(sc.tile_base); cudaFree(sc.tile_read0);
-    cudaFree(sc.wit_min); cudaFree(sc.wit_max);
-    cudaFree(sc.seq_list); cudaFree(sc.seq_sbase); cudaFree(sc.seq_count); cudaFree(sc.cursor);
-    cudaFree(sc.scan_status); cudaFree(sc.scan_ticket); cudaFree(sc.status); cudaFree(sc.counters);
-    for (int k = 0; k <= sgpu_ctx::MAX_STAGES; k++) if (ctx->stage_ev[k]) cudaEventDestroy(ctx->stage_ev[k]);
-    free_outputs(ctx->dev_out, false);
-    cudaFree(ctx->ent_ovf); cudaFree(ctx->jnn_mom);
-    {
-        PaScratch& w = ctx->pa;
-        cudaFree(w.tile_cnt); cudaFree(w.tile_base); cudaFree(w.tS); cudaFree(w.tQ); cudaFree(w.tA); cudaFree(w.tB);
-        cudaFree(w.tmin); cudaFree(w.ord_list); cudaFree(w.ord_sbase); cudaFree(w.ord_count);
-    }
-    {
-        SvbScratch& w = ctx->svb;
-        cudaFree(w.cnt); cudaFree(w.base); cudaFree(w.blk_bytes); cudaFree(w.blk_gpos); cudaFree(w.blk_sum);
-        cudaFree(w.blk_vpos); cudaFree(w.lane_sum); cudaFree(w.blk_read);
-    }
-    if (ctx->slots) {
-        for (uint32_t s = 0; s < ctx->n_slots; s++) {
-            Slot& sl = ctx->slots[s];
-            cudaFreeHost(sl.batch.samples); cudaFreeHost(sl.batch.read_off); cudaFreeHost(sl.batch.read_len);
-            cudaFreeHost(sl.batch.offset_f); cudaFreeHost(sl.batch.raw_unit_f);
-            cudaFree(sl.d_samples); cudaFree(sl.d_read_off); cudaFree(sl.d_read_len); cudaFree(sl.d_offset);
-            cudaFree(sl.d_unit);
-            free_outputs(sl.dout, false);
-            free_outputs(sl.hout, true);
-            cudaFreeHost(sl.h_counters); cudaFreeHost(sl.h_status);
-            cudaFreeHost(sl.h_comp); cudaFreeHost(sl.h_comp_off); cudaFreeHost(sl.h_comp_len);
-            cudaFree(sl.d_comp); cudaFree(sl.d_comp_off); cudaFree(sl.d_comp_len);
-            if (sl.stream) cudaStreamDestroy(sl.stream);
-            if (sl.in_ready) cudaEventDestroy(sl.in_ready);
-            if (sl.kernels_done) cudaEventDestroy(sl.kernels_done);
-            if (sl.small_back) cudaEventDestroy(sl.small_back);
-        }
-        delete[] ctx->slots;
-    }
-    if (ctx->compute) cudaStreamDestroy(ctx->compute);
     delete ctx;
 }
 
@@ -688,12 +645,12 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
         CU(cudaSetDevice(ctx->device));
         const int rc = alloc_svb_scratch(ctx);
         if (rc) return rc;
-        CU(pin_alloc(&sl.h_comp, ctx->comp_cap));
-        CU(dev_alloc(&sl.d_comp, ctx->comp_cap + 16));
-        CU(pin_alloc(&sl.h_comp_off, ctx->max_reads));
-        CU(dev_alloc(&sl.d_comp_off, ctx->max_reads));
-        CU(pin_alloc(&sl.h_comp_len, ctx->max_reads));
-        CU(dev_alloc(&sl.d_comp_len, ctx->max_reads));
+        CU(sl.h_comp.ensure(ctx->comp_cap));
+        CU(sl.d_comp.ensure(ctx->comp_cap + 16));
+        CU(sl.h_comp_off.ensure(ctx->max_reads));
+        CU(sl.d_comp_off.ensure(ctx->max_reads));
+        CU(sl.h_comp_len.ensure(ctx->max_reads));
+        CU(sl.d_comp_len.ensure(ctx->max_reads));
     }
     sl.mode = 2;
     const uint32_t r = b.n_reads;
@@ -751,10 +708,11 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     CU(cudaEventRecord(sl.in_ready, st));
     CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
     DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, (int)hb.rna, sl.used};
-    CU(alloc_outputs(ctx, sl.hout, want, true));
+    CU(alloc_outputs(ctx, sl.hout, want));
     const int rc = pa_in ? run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr,
                                                          (int)hb.rna, sl.used},
-                                           reinterpret_cast<const float*>(sl.d_samples), want, sl.dout, ctx->compute)
+                                           reinterpret_cast<const float*>(sl.d_samples.get()), want, sl.dout,
+                                           ctx->compute)
                          : run_pipeline(ctx, b, want, sl.dout, ctx->compute, compressed ? &svb : nullptr, sl.d_samples);
     if (rc) return rc;
     // small results come back right away; the big arrays are sized by n_events in sgpu_wait
@@ -782,7 +740,7 @@ int sgpu_wait(sgpu_ctx_t* ctx, uint32_t slot, sgpu_result_t* out) {
     if (dev_rc) return dev_rc;
     const uint32_t nr = sl.batch.n_reads;
     if (sl.want & SGPU_WANT_EVENTS) {
-        const uint64_t ne = nr ? static_cast<const uint64_t*>(sl.hout[EV_OFF])[nr] : 0;
+        const uint64_t ne = nr ? static_cast<const uint64_t*>(sl.hout[EV_OFF].get())[nr] : 0;
         if (ne > ctx->ev_cap) return SGPU_E_EVCAP;
         CU(queue_d2h(sl, SGPU_WANT_EVENTS, true, ne));
         CU(cudaStreamSynchronize(sl.stream));

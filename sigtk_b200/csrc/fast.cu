@@ -144,7 +144,8 @@ int launch_rank_events(const DevBatch& b, Scratch& sc, uint64_t* ev_off, int sm_
     const uint32_t n_tiles = fast_tiles_for(b.span);
     count_tile_bits_kernel<<<grid_cap((uint64_t)n_tiles * 32, 256, sm_count * 8), 256, 0, st>>>(sc.bitmap, n_tiles,
                                                                                                sc.tile_cnt);
-    int n = 1 + launch_scan_u32(sc.tile_cnt, n_tiles, sc.tile_base, reinterpret_cast<uint64_t*>(sc.counters), sc, st);
+    int n = 1 + launch_scan_u32(sc.tile_cnt, n_tiles, sc.tile_base, reinterpret_cast<uint64_t*>(sc.counters.get()), sc,
+                                st);
     read_event_offsets_kernel<<<grid_cap((uint64_t)b.n_reads + 1, 256, sm_count * 8), 256, 0, st>>>(
         b, sc.bitmap, sc.tile_base, n_tiles, ev_off);
     return n + 1;

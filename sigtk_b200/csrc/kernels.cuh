@@ -1,8 +1,51 @@
 // kernels.cuh -- internal interfaces between the kernel translation units and capi.cu
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace sgpu {
+
+// An owning pointer to an array in device memory (or, PINNED, in pinned host memory; T = void: an array of bytes).
+// Its destructor frees the array, so the code that sizes an array is the only place that lists it. It converts to
+// T*, so launchers take its members as plain pointers. Host code only.
+template <typename T, bool PINNED = false>
+class Buf {
+  public:
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    Buf(Buf&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+    Buf& operator=(Buf&& o) noexcept {
+        if (this != &o) { release(); p_ = o.p_; o.p_ = nullptr; }
+        return *this;
+    }
+    ~Buf() { release(); }  // (holding nothing, it makes no CUDA call)
+
+    // Allocates max(count, 1) elements unless it holds some already, and keeps the pointer only on success: an
+    // allocation that failed part-way through a list is completed by the next call instead of leaving a NULL
+    // pointer behind a non-NULL one.
+    cudaError_t ensure(uint64_t count) {
+        if (p_) return cudaSuccess;
+        size_t bytes = (size_t)(count ? count : 1);
+        if constexpr (!std::is_void_v<T>) bytes *= sizeof(T);
+        void* q = nullptr;
+        const cudaError_t e = PINNED ? cudaHostAlloc(&q, bytes, cudaHostAllocDefault) : cudaMalloc(&q, bytes);
+        if (e == cudaSuccess) p_ = static_cast<T*>(q);
+        return e;
+    }
+    T* get() const { return p_; }
+    operator T*() const { return p_; }
+
+  private:
+    void release() {
+        if (!p_) return;
+        if (PINNED) cudaFreeHost(p_); else cudaFree(p_);
+    }
+    T* p_ = nullptr;
+};
+template <typename T> using DevBuf = Buf<T, false>;
+template <typename T> using PinBuf = Buf<T, true>;
 
 // device-side status codes (mapped to SGPU_E_* by capi.cu)
 enum { SGPU_DEV_OK = 0, SGPU_DEV_E_EVCAP = 1, SGPU_DEV_E_SCRATCH = 2, SGPU_DEV_E_STREAM = 3 };
@@ -22,21 +65,21 @@ struct WorkList {
 // Device workspace owned by a context.
 struct Scratch {
     // sequential-order scratch (gen_cap samples)
-    double* Sinc; double* Qinc; float* t1; float* t2;
+    DevBuf<double> Sinc, Qinc; DevBuf<float> t1, t2;
     uint64_t gen_cap;
     // event-start bitmap over the flat sample span: bit p set <=> an event starts at flat sample p
-    uint32_t* bitmap; uint64_t bitmap_words;
+    DevBuf<uint32_t> bitmap; uint64_t bitmap_words;
     // per tile
-    uint32_t* tile_cnt; uint64_t* tile_base;
-    uint32_t* tile_read0;            // first read that can intersect a 2048-sample tile (emit_events_kernel); the
+    DevBuf<uint32_t> tile_cnt; DevBuf<uint64_t> tile_base;
+    DevBuf<uint32_t> tile_read0;     // first read that can intersect a 2048-sample tile (emit_events_kernel); the
                                      // walker sets the top bit of tiles that hold LOW samples (pA <= 0 or barely above)
     // chunk walker (walk.cu)
-    uint32_t* wk_cnt;                // [max_reads] interior chunks per read
-    uint64_t* wk_ibase;              // [max_reads+1] exclusive scan of wk_cnt
-    int* wk_begin; int* wk_end;      // [wk_slots*8] detector state after the warm-up / after the last step of a chunk
+    DevBuf<uint32_t> wk_cnt;         // [max_reads] interior chunks per read
+    DevBuf<uint64_t> wk_ibase;       // [max_reads+1] exclusive scan of wk_cnt
+    DevBuf<int> wk_begin, wk_end;    // [wk_slots*8] detector state after the warm-up / after the last step of a chunk
     uint64_t wk_slots;
-    int* jobs;                       // [job_cap * 4] lives of the long detector to replay: {read, chunk, l_start, end}
-    uint32_t* job_count;             // device scalar
+    DevBuf<int> jobs;                // [job_cap * 4] lives of the long detector to replay: {read, chunk, l_start, end}
+    DevBuf<uint32_t> job_count;      // device scalar
     uint32_t job_cap;
     // development / test parameters (sgpu_set_param): 0 = automatic
     uint32_t tune_chunk_len, tune_warmup;
@@ -44,15 +87,15 @@ struct Scratch {
     uint32_t tune_stat_cta_min;      // reads of at least this many samples get a CTA in the moments kernels (stat.cu)
     uint32_t max_tiles;
     // per read
-    uint32_t* wit_min; uint32_t* wit_max;  // exact-sum witness: min nonzero |pA| / max |pA| bit patterns
-    uint32_t* seq_list;     // compacted list of reads routed to the sequential-order kernels
-    uint64_t* seq_sbase;
-    uint32_t* seq_count;    // device scalar
-    unsigned long long* cursor;  // device scalar: used scratch samples
+    DevBuf<uint32_t> wit_min, wit_max;  // exact-sum witness: min nonzero |pA| / max |pA| bit patterns
+    DevBuf<uint32_t> seq_list;  // compacted list of reads routed to the sequential-order kernels
+    DevBuf<uint64_t> seq_sbase;
+    DevBuf<uint32_t> seq_count; // device scalar
+    DevBuf<unsigned long long> cursor;  // device scalar: used scratch samples
     // scan
-    unsigned long long* scan_status; uint32_t* scan_ticket;
+    DevBuf<unsigned long long> scan_status; DevBuf<uint32_t> scan_ticket;
     // device-side status / counters
-    int* status; unsigned long long* counters;  // [0]=n_events [1]=n_seq [2]=n_fixups
+    DevBuf<int> status; DevBuf<unsigned long long> counters;  // [0]=n_events [1]=n_seq [2]=n_fixups
 };
 
 // generic.cu (sequential-order kernels)
@@ -85,12 +128,13 @@ int launch_pa(const DevBatch& b, float* pa, int sm_count, cudaStream_t st);
 
 // pa_input.cu (event detection on the caller's pA floats: exactness witness and parallel scan of the prefix sums)
 struct PaScratch {                 // allocated on the first pA batch
-    uint32_t* tile_cnt;            // [max_reads] tiles of every read
-    uint64_t* tile_base;           // [max_reads+1] their exclusive scan
-    double* tS; double* tQ;        // [max_tiles] the tiles' sums, then their prefixes within the read
-    double* tA; double* tB;        // [max_tiles] upper bounds of sum |x| and sum fl(x*x)
-    uint2* tmin;                   // [max_tiles] smallest nonzero |x| and fl(x*x) (float bits)
-    uint32_t* ord_list; uint64_t* ord_sbase; uint32_t* ord_count;  // reads summed in the reference's order
+    DevBuf<uint32_t> tile_cnt;     // [max_reads] tiles of every read
+    DevBuf<uint64_t> tile_base;    // [max_reads+1] their exclusive scan
+    DevBuf<double> tS, tQ;         // [max_tiles] the tiles' sums, then their prefixes within the read
+    DevBuf<double> tA, tB;         // [max_tiles] upper bounds of sum |x| and sum fl(x*x)
+    DevBuf<uint2> tmin;            // [max_tiles] smallest nonzero |x| and fl(x*x) (float bits)
+    DevBuf<uint32_t> ord_list;     // reads summed in the reference's order
+    DevBuf<uint64_t> ord_sbase; DevBuf<uint32_t> ord_count;
     uint64_t max_tiles;
 };
 uint64_t pa_tile_capacity(uint64_t max_samples, uint32_t max_reads);
@@ -109,11 +153,11 @@ struct SvbBatch {
     uint64_t n_blocks;         // sum of svbzd_blocks_of(read_len)
 };
 struct SvbScratch {
-    uint32_t* cnt; uint64_t* base;            // [max_reads], [max_reads+1]
-    uint32_t* blk_bytes; uint64_t* blk_gpos;  // [max_blocks], [max_blocks+1]
-    uint32_t* blk_sum; uint64_t* blk_vpos;
-    uint32_t* lane_sum;                       // [max_blocks*32]
-    uint32_t* blk_read;                       // [max_blocks] read of every block
+    DevBuf<uint32_t> cnt; DevBuf<uint64_t> base;            // [max_reads], [max_reads+1]
+    DevBuf<uint32_t> blk_bytes; DevBuf<uint64_t> blk_gpos;  // [max_blocks], [max_blocks+1]
+    DevBuf<uint32_t> blk_sum; DevBuf<uint64_t> blk_vpos;
+    DevBuf<uint32_t> lane_sum;                // [max_blocks*32]
+    DevBuf<uint32_t> blk_read;                // [max_blocks] read of every block
     uint64_t max_blocks;
 };
 uint64_t svbzd_max_blocks(uint64_t max_samples, uint32_t max_reads);

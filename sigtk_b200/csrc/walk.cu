@@ -389,7 +389,7 @@ static WalkParams walk_params(const DevBatch& b, Scratch& sc, float* pa_out, uin
     p.st_begin = sc.wk_begin; p.st_end = sc.wk_end; p.wit_min = sc.wit_min; p.wit_max = sc.wit_max; p.tile_read0 = sc.tile_read0;
     p.edge_blocks = (uint32_t)((2ull * ((b.n_reads + 31u) & ~31u) + WNT - 1) / WNT);   // (first and last chunks: whole warps each)
     p.thr_long = sc.tune_thr_long;
-    p.jobs = reinterpret_cast<int4*>(sc.jobs); p.job_count = sc.job_count; p.job_cap = sc.job_cap; p.seq_flag = seq_flag;
+    p.jobs = reinterpret_cast<int4*>(sc.jobs.get()); p.job_count = sc.job_count; p.job_cap = sc.job_cap; p.seq_flag = seq_flag;
     p.counters = sc.counters;
     return p;
 }
