@@ -222,6 +222,74 @@ typedef struct {
 } sgpu_svb_dev_batch_t;
 int  sgpu_decode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_svb_dev_batch_t *batch, int16_t *samples_out, void *stream);
 
+/* ---- live event detection: signal that arrives in chunks, channel by channel ----------------------------------
+ * For tools that segment signal while the read is still in the pore (adaptive sampling, Read Until): per channel, a
+ * read is opened by a START entry, grows by entries of int16 samples and is closed by an END entry; one entry may carry
+ * START, samples and END together. The context keeps every channel's detector state in HBM between entries.
+ *   - pA of every sample is misc.c:28 with the calibration given at START (offset_f = (float)offset, raw_unit_f =
+ *     (float)range / (float)digitisation, as sgpu_slot_add_read computes them); the DNA or RNA parameters also come
+ *     from START (SGPU_LIVE_RNA, ignored without START). The long threshold follows SGPU_PARAM_THR_LONG.
+ *   - When events are reported: let a read hold n samples after an entry that does not end it. The detector has then
+ *     been stepped, in the reference's order (short, then long; events.c:385-437), over every position i <= n - w2:
+ *     the positions whose t-statistics can no longer change (their right window [i, i+w2) is complete). Every peak
+ *     emitted during those steps closes one event [a, p), and the entry reports those events. END steps the remaining
+ *     positions (their long t-statistic is 0, events.c:328-338) and reports the last event [a, n). A read with no peak
+ *     ends with the single event [0, n); a read of 0 samples reports no event. A peak may be emitted long after its
+ *     position, in a later entry.
+ *   - Exactness: for every read, the events of all its entries taken in order are bit-identical to the event table of
+ *     the whole read (getevents, events.c:553-573, and sgpu_slot_add_read), for any split into chunks.
+ *   - Ordering: live runs of a context update channel state in the order they are submitted (host slots run their
+ *     kernels on one stream of the context). A device-resident live run is ordered by the caller's stream and must not
+ *     overlap a submitted live slot.
+ *   - START on a channel whose read is still open discards that read: its open event is never reported.
+ * A live slot holds live entries only (SGPU_E_STATE when mixed with other records) in its int16 sample buffers, and
+ * computes SGPU_WANT_EVENTS only (sgpu_submit returns SGPU_E_INVAL for any other want). sgpu_wait on a live slot and
+ * sgpu_wait_live on any other slot return SGPU_E_STATE. sgpu_slot_add_live returns the entry's index, SGPU_E_FULL /
+ * SGPU_E_TOOBIG as sgpu_slot_add_read does, SGPU_E_INVAL for channel >= n_channels, unknown flag bits or a second entry
+ * for the channel in the slot, SGPU_E_STATE before sgpu_live_open. sgpu_submit checks the rules that depend on channel
+ * state against a host mirror updated in submission order: samples or END for a channel without an open read give
+ * SGPU_E_STATE, a read that would exceed 2^31 - 1 samples (misc.c:20) SGPU_E_TOOBIG; then nothing is queued and no
+ * channel changes. sgpu_run_device_live reports the same violations as `status` in sgpu_counters, and the offending
+ * entries leave their channels unchanged. The event capacity covers every possible push (SGPU_E_EVCAP cannot occur). */
+#define SGPU_LIVE_START 1u /* begin a new read on the channel: calibration (and SGPU_LIVE_RNA) taken from this entry */
+#define SGPU_LIVE_END   2u /* the read ends after this entry's samples */
+#define SGPU_LIVE_RNA   4u /* with START: the RNA detector parameters (events.c:50-54) */
+
+/* Once per context: a table of n_channels channels in HBM (about 550 bytes each), all without a read.
+ * SGPU_E_STATE the second time. */
+int  sgpu_live_open(sgpu_ctx_t *ctx, uint32_t n_channels);
+/* Append one entry to a live slot (digitisation, offset, range are read with SGPU_LIVE_START only). */
+int64_t sgpu_slot_add_live(sgpu_ctx_t *ctx, uint32_t slot, uint32_t channel, uint32_t flags, const int16_t *raw,
+                           uint64_t n, double digitisation, double offset, double range);
+/* Events of a live run, entry by entry: host pointers (pinned) from sgpu_wait_live, device pointers from
+ * sgpu_run_device_live (n_events 0 there: see sgpu_counters). */
+typedef struct {
+    uint64_t *ev_off;      /* [n_entries+1]: the events of entry e are [ev_off[e], ev_off[e+1]) */
+    uint32_t *ev_start;    /* sample index in the channel's read */
+    uint32_t *ev_len;      /* end - start */
+    float    *ev_mean;
+    float    *ev_stdv;
+    uint64_t  n_events;
+} sgpu_live_result_t;
+/* Blocks until a live slot submitted with SGPU_WANT_EVENTS is done. */
+int  sgpu_wait_live(sgpu_ctx_t *ctx, uint32_t slot, sgpu_live_result_t *out);
+/* Device-resident live entries: entry e is samples[read_off[e] .. +read_len[e]) of channel[e] with flags[e], and the
+ * calibration offset_f[e], raw_unit_f[e] (read with SGPU_LIVE_START only). read_off[e] + read_len[e] <= read_off[e+1],
+ * read_off[n_entries] = span <= max_samples, n_entries <= max_reads. Runs on `stream` without copies or
+ * synchronisation; *out receives device pointers owned by the context (valid until the next run). */
+typedef struct {
+    const int16_t  *samples;
+    const uint64_t *read_off;   /* [n_entries+1] */
+    const uint32_t *read_len;
+    const uint32_t *channel;
+    const uint32_t *flags;
+    const float    *offset_f;
+    const float    *raw_unit_f;
+    uint32_t n_entries;
+    uint64_t span;
+} sgpu_dev_live_batch_t;
+int  sgpu_run_device_live(sgpu_ctx_t *ctx, const sgpu_dev_live_batch_t *batch, void *stream, sgpu_live_result_t *out);
+
 /* Counters of the last completed run (host path: after sgpu_wait; device path:
  * after the caller synchronised the stream). Synchronises the device. */
 typedef struct {
@@ -229,7 +297,8 @@ typedef struct {
     uint64_t n_seq_order_reads;   /* reads routed to the sequential-order kernels */
     uint64_t n_fixups;            /* detector chunks with a boundary-state mismatch */
     uint64_t n_kernel_launches;   /* kernels launched by the last run */
-    int32_t  status;              /* 0 or SGPU_E_EVCAP / SGPU_E_SCRATCH reported by the device */
+    int32_t  status;              /* 0 or SGPU_E_EVCAP / SGPU_E_SCRATCH reported by the device; after a live run also
+                                     SGPU_E_INVAL / SGPU_E_STATE / SGPU_E_TOOBIG for refused entries */
     uint64_t n_long_jobs;         /* stretches of the long peak detector (events.c:414-437) that were replayed with the
                                      reference's own operations because their t-statistic may exceed its threshold */
 } sgpu_counters_t;

@@ -18,10 +18,12 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS, WANT_EVENTS, WANT_PA,
-                   WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, SgpuError)
+from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS, LIVE_END, LIVE_RNA, LIVE_START,
+                   WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, SgpuError)
 
 Read = Tuple[np.ndarray, float, float, float]  # raw int16, digitisation, offset, range
+LiveEntry = Tuple[int, int, np.ndarray, float, float, float]  # channel, LIVE_* flags, raw int16, digitisation, offset,
+                                                              # range (the calibration is read with LIVE_START only)
 
 
 @dataclass
@@ -65,6 +67,16 @@ class BatchResult:
         end[-1] = self.read_len[r]
         length = (end - start).astype(np.float32)
         return EventTable(start, length, self.ev_mean[a:b].copy(), self.ev_stdv[a:b].copy())
+
+
+def live_tables(ev_off, ev_start, ev_len, ev_mean, ev_stdv) -> List[EventTable]:
+    """one EventTable per entry of a live run (start: sample index in the channel's read)"""
+    out = []
+    for e in range(len(ev_off) - 1):
+        a, b = int(ev_off[e]), int(ev_off[e + 1])
+        out.append(EventTable(ev_start[a:b].astype(np.uint64), ev_len[a:b].astype(np.float32), ev_mean[a:b].copy(),
+                              ev_stdv[a:b].copy()))
+    return out
 
 
 def _np_from(ptr: int, dtype, count: int) -> np.ndarray:
@@ -199,6 +211,44 @@ class Context:
         self.fill(slot, reads, rna)
         self.submit(slot, want)
         return self.wait(slot, want)
+
+    # ---- live event detection: signal in chunks, detector state per channel in HBM -----------------------------
+    def live_open(self, n_channels: int) -> None:
+        """sgpu_live_open: the table of n_channels channels (once per context)"""
+        self._check(self._lib.sgpu_live_open(self._h, int(n_channels)))
+
+    def live_fill(self, slot: int, entries: Sequence[LiveEntry]) -> None:
+        self._check(self._lib.sgpu_slot_reset(self._h, slot, 0))
+        for ch, flags, raw, dig, off, rng in entries:
+            raw = np.ascontiguousarray(raw, dtype=np.int16)
+            self._check(int(self._lib.sgpu_slot_add_live(self._h, slot, int(ch), int(flags), raw.ctypes.data,
+                                                         raw.shape[0], float(dig), float(off), float(rng))))
+
+    def live_wait(self, slot: int) -> List[EventTable]:
+        res = _lib.LiveResult()
+        self._check(self._lib.sgpu_wait_live(self._h, slot, C.byref(res)))
+        pb = C.POINTER(_lib.Batch)()
+        self._check(self._lib.sgpu_slot_batch(self._h, slot, C.byref(pb)))
+        n, ne = int(pb.contents.n_reads), int(res.n_events)
+        return live_tables(_np_from(res.ev_off, np.uint64, n + 1), _np_from(res.ev_start, np.uint32, ne),
+                           _np_from(res.ev_len, np.uint32, ne), _np_from(res.ev_mean, np.float32, ne),
+                           _np_from(res.ev_stdv, np.float32, ne))
+
+    def live_push(self, entries: Sequence[LiveEntry], slot: int = 0) -> List[EventTable]:
+        """one push of live entries (at most one per channel): fill + submit + wait; -> the events each entry reports"""
+        self.live_fill(slot, entries)
+        self.submit(slot, WANT_EVENTS)
+        return self.live_wait(slot)
+
+    def run_device_live(self, samples_ptr: int, read_off_ptr: int, read_len_ptr: int, channel_ptr: int, flags_ptr: int,
+                        offset_ptr: int, unit_ptr: int, n_entries: int, span: int, stream: int = 0) -> _lib.LiveResult:
+        """sgpu_run_device_live: live entries already in device memory; -> device pointers of the events (the count
+        is counters()["n_events"] once the stream is done)"""
+        db = _lib.DevLiveBatch(samples_ptr, read_off_ptr, read_len_ptr, channel_ptr, flags_ptr, offset_ptr, unit_ptr,
+                               n_entries, span)
+        res = _lib.LiveResult()
+        self._check(self._lib.sgpu_run_device_live(self._h, C.byref(db), C.c_void_p(stream), C.byref(res)))
+        return res
 
     # ---- device-resident path ---------------------------------------------
     def run_device(self, samples_ptr: int, read_off_ptr: int, read_len_ptr: int, offset_ptr: int, unit_ptr: int,

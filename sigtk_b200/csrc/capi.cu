@@ -111,12 +111,18 @@ struct Slot {
     uint32_t want = 0;
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     int mode = 0;                    // 0: empty, 1: decoded int16 records, 2: svb-zd streams, 3: pA records (floats
-                                     // in the sample buffers: max_samples / 2 of them)
+                                     // in the sample buffers: max_samples / 2 of them), 4: live entries
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
     DevBuf<uint8_t> d_comp;          // comp_cap + 16 bytes
     PinBuf<uint64_t> h_comp_off; DevBuf<uint64_t> d_comp_off;
     PinBuf<uint32_t> h_comp_len; DevBuf<uint32_t> d_comp_len;
     uint64_t comp_used = 0, svb_blocks = 0;
+    // live entries (allocated by sgpu_live_open): channel and flags of every entry, the run's events
+    PinBuf<uint32_t> h_channel, h_flags; DevBuf<uint32_t> d_channel, d_flags;
+    LiveOut<false> live_dout;
+    LiveOut<true> live_hout;
+    std::unique_ptr<uint32_t[]> live_claim;  // [n_channels] live_gen of the batch that holds an entry for the channel
+    uint32_t live_gen = 0;
 
     ~Slot() {
         if (stream) cudaStreamDestroy(stream);
@@ -144,6 +150,11 @@ struct sgpu_ctx {
     int pore_rna004 = 0;         // SGPU_PARAM_PORE: jnnv2 parameters of `prefix` (misc.c:74-101 picks them from the header)
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
+    LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
+    LiveOut<false> live_dev_out; // outputs of sgpu_run_device_live
+    std::unique_ptr<uint32_t[]> live_mirror;  // [n_channels] nopen of every channel after the submitted live slots
+    bool live_mirror_stale = false;           // a device-resident live run changed channels since
+    uint32_t live_gen = 0;
     uint64_t comp_cap = 0;       // bytes of compressed input a slot can hold
     cudaStream_t compute = nullptr;
     uint64_t last_launches = 0;
@@ -410,6 +421,25 @@ int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t 
     return SGPU_OK;
 }
 
+// The kernels of a push of live entries into `o` (live.cu). No host synchronisation, no host<->device copies.
+int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, LiveOut<false>& o, cudaStream_t st) {
+    if (b.n_entries > ctx->max_reads || b.span > ctx->max_samples) return SGPU_E_INVAL;
+    if (b.n_entries && (!b.samples || !b.read_off || !b.read_len || !b.channel || !b.flags || !b.offset || !b.unit))
+        return SGPU_E_INVAL;
+    CU(cudaMemsetAsync(ctx->sc.status, 0, sizeof(int), st));
+    CU(cudaMemsetAsync(ctx->sc.counters, 0, 4 * sizeof(unsigned long long), st));
+    StageMarks marks(ctx, st);
+    if (b.n_entries == 0) {
+        CU(cudaMemsetAsync(o.ev_off, 0, sizeof(uint64_t), st));
+        ctx->last_launches = 0;
+        return SGPU_OK;
+    }
+    marks.done("live", launch_live(b, ctx->live, ctx->sc, o, ctx->sm_count, st));
+    CU(cudaGetLastError());
+    ctx->last_launches = marks.launches;
+    return SGPU_OK;
+}
+
 // The per-read tail of sgpu_slot_add_read / sgpu_slot_add_read_svbzd: records the read of n samples at sl.used as
 // the batch's next read, with the scalars of its pA conversion.
 int64_t append_record(Slot& sl, uint64_t n, double digitisation, double offset, double range) {
@@ -430,9 +460,72 @@ int64_t append_record(Slot& sl, uint64_t n, double digitisation, double offset, 
 
 int map_dev_status(int s) {
     if (s == SGPU_DEV_E_EVCAP) return SGPU_E_EVCAP;
+    if (s == SGPU_DEV_E_INVAL) return SGPU_E_INVAL;
+    if (s == SGPU_DEV_E_STATE) return SGPU_E_STATE;
+    if (s == SGPU_DEV_E_TOOBIG) return SGPU_E_TOOBIG;
     if (s == SGPU_DEV_E_SCRATCH) return SGPU_E_SCRATCH;
     if (s == SGPU_DEV_E_STREAM) return SGPU_E_STREAM;
     return SGPU_OK;
+}
+
+// sgpu_submit of a live slot: the checks against the channel mirror, then copies, kernels (context stream) and the
+// copy of ev_off back, like the other slots
+int submit_live(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
+    if (want != SGPU_WANT_EVENTS) return SGPU_E_INVAL;
+    CU(cudaSetDevice(ctx->device));
+    uint32_t* const mirror = ctx->live_mirror.get();
+    if (ctx->live_mirror_stale) {  // sgpu_run_device_live changed channels: their state is read back once
+        CU(cudaDeviceSynchronize());
+        CU(cudaMemcpy(mirror, ctx->live.nopen, (size_t)ctx->live.n_channels * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        ctx->live_mirror_stale = false;
+    }
+    const sgpu_batch_t& hb = sl.batch;
+    const uint32_t nr = hb.n_reads;
+    // the rules that depend on channel state (entries of one slot have distinct channels); nothing is queued and no
+    // channel changes unless every entry passes
+    for (uint32_t e = 0; e < nr; e++) {
+        const uint32_t f = sl.h_flags[e], no = mirror[sl.h_channel[e]];
+        const bool start = (f & SGPU_LIVE_START) != 0;
+        if (!start && !(no & LIVE_OPEN) && (hb.read_len[e] || (f & SGPU_LIVE_END))) return SGPU_E_STATE;
+        if ((start ? 0ull : (uint64_t)(no & ~LIVE_OPEN)) + hb.read_len[e] > 0x7fffffffull) return SGPU_E_TOOBIG;
+    }
+    cudaStream_t st = sl.stream;
+    CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_read_off, hb.read_off, ((size_t)nr + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_read_len, hb.read_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_offset, hb.offset_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_unit, hb.raw_unit_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_channel, sl.h_channel, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(sl.d_flags, sl.h_flags, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(sl.in_ready, st));
+    CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
+    const LiveBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_channel, sl.d_flags, sl.d_offset, sl.d_unit, nr,
+                      sl.used};
+    const int rc = run_pipeline_live(ctx, b, sl.live_dout, ctx->compute);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(sl.h_counters, ctx->sc.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                       ctx->compute));
+    CU(cudaMemcpyAsync(sl.h_status, ctx->sc.status, sizeof(int), cudaMemcpyDeviceToHost, ctx->compute));
+    CU(cudaEventRecord(sl.kernels_done, ctx->compute));
+    CU(cudaStreamWaitEvent(st, sl.kernels_done, 0));
+    CU(cudaMemcpyAsync(sl.live_hout.ev_off, sl.live_dout.ev_off, ((size_t)nr + 1) * sizeof(uint64_t),
+                       cudaMemcpyDeviceToHost, st));
+    CU(cudaEventRecord(sl.small_back, st));
+    for (uint32_t e = 0; e < nr; e++) {  // the channels as the kernel leaves them
+        const uint32_t c = sl.h_channel[e], f = sl.h_flags[e], no = mirror[c];
+        const bool start = (f & SGPU_LIVE_START) != 0;
+        if (!start && !(no & LIVE_OPEN)) continue;
+        mirror[c] = (f & SGPU_LIVE_END) ? 0u : (uint32_t)((start ? 0u : (no & ~LIVE_OPEN)) + hb.read_len[e]) | LIVE_OPEN;
+    }
+    sl.want = want;
+    sl.submitted = true;
+    return SGPU_OK;
+}
+
+template <bool PINNED>
+void fill_live_result(sgpu_live_result_t* r, const LiveOut<PINNED>& o) {
+    memset(r, 0, sizeof *r);
+    r->ev_off = o.ev_off; r->ev_start = o.ev_start; r->ev_len = o.ev_len; r->ev_mean = o.ev_mean; r->ev_stdv = o.ev_stdv;
 }
 
 }  // namespace
@@ -614,7 +707,8 @@ int64_t sgpu_slot_add_read(sgpu_ctx_t* ctx, uint32_t slot, const int16_t* raw, u
     if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
-    if (sl.mode >= 2) return SGPU_E_STATE;  // a batch holds decoded records, svb-zd streams or pA records, never a mix
+    if (sl.mode >= 2) return SGPU_E_STATE;  // a batch holds decoded records, svb-zd streams, pA records or live entries,
+                                           // never a mix
     if (n >= (1ull << 31)) return SGPU_E_TOOBIG;  // the reference itself narrows to int32_t (misc.c:20)
     const uint64_t need = align_up(n, SGPU_ALIGN);
     if (need > ctx->max_samples) return SGPU_E_TOOBIG;
@@ -629,7 +723,7 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
                                  double digitisation, double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || !stream) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || sl.mode == 1 || sl.mode == 3) return SGPU_E_STATE;
+    if (sl.submitted || sl.mode == 1 || sl.mode == 3 || sl.mode == 4) return SGPU_E_STATE;
     if (n_bytes != 0 && n_bytes < 4) return SGPU_E_STREAM;
     uint32_t count = 0;
     if (n_bytes) memcpy(&count, stream, 4);  // slow5_press.c:1093: the original length leads the stream
@@ -665,7 +759,7 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
 int64_t sgpu_slot_add_read_pa(sgpu_ctx_t* ctx, uint32_t slot, const float* pa, uint64_t n) {
     if (!ctx || slot >= ctx->n_slots || (!pa && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || sl.mode == 1 || sl.mode == 2) return SGPU_E_STATE;
+    if (sl.submitted || sl.mode == 1 || sl.mode == 2 || sl.mode == 4) return SGPU_E_STATE;
     // the slot's int16 sample buffers (pinned and device) hold the floats: max_samples / 2 of them
     const uint64_t cap = ctx->max_samples / 2;
     if (n >= (1ull << 32)) return SGPU_E_TOOBIG;
@@ -682,6 +776,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (!ctx || slot >= ctx->n_slots || (want & ~63u) || want == 0) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
+    if (sl.mode == 4) return submit_live(ctx, sl, want);
     const bool pa_in = sl.mode == 3;
     if (pa_in && !pa_input_want_ok(want)) return SGPU_E_INVAL;
     CU(cudaSetDevice(ctx->device));
@@ -731,7 +826,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
 int sgpu_wait(sgpu_ctx_t* ctx, uint32_t slot, sgpu_result_t* out) {
     if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!sl.submitted) return SGPU_E_STATE;
+    if (!sl.submitted || sl.mode == 4) return SGPU_E_STATE;
     CU(cudaSetDevice(ctx->device));
     sl.submitted = false;
     CU(cudaEventSynchronize(sl.small_back));
@@ -859,6 +954,104 @@ int sgpu_memcpy_d2h(sgpu_ctx_t* ctx, void* dst, const void* src, uint64_t bytes)
     CU(cudaSetDevice(ctx->device));
     CU(cudaDeviceSynchronize());
     if (bytes) CU(cudaMemcpy(dst, src, (size_t)bytes, cudaMemcpyDeviceToHost));
+    return SGPU_OK;
+}
+
+int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
+    if (!ctx || n_channels == 0) return SGPU_E_INVAL;
+    LiveScratch& w = ctx->live;
+    if (w.n_channels) return SGPU_E_STATE;
+    CU(cudaSetDevice(ctx->device));
+    w.ev_cap = live_stage_base(ctx->max_samples, ctx->max_reads);
+    CU(w.chan.ensure(n_channels));
+    CU(w.nopen.ensure(n_channels));
+    CU(w.claim.ensure(n_channels));
+    CU(w.cnt.ensure(ctx->max_reads));
+    CU(w.s_start.ensure(w.ev_cap));
+    CU(w.s_len.ensure(w.ev_cap));
+    CU(w.s_mean.ensure(w.ev_cap));
+    CU(w.s_stdv.ensure(w.ev_cap));
+    CU(cudaMemset(w.nopen, 0, (size_t)n_channels * sizeof(uint32_t)));
+    CU(cudaMemset(w.claim, 0, (size_t)n_channels * sizeof(uint32_t)));
+    ctx->live_mirror.reset(new (std::nothrow) uint32_t[n_channels]());
+    if (!ctx->live_mirror) return SGPU_E_NOMEM;
+    for (uint32_t s = 0; s < ctx->n_slots; s++) {
+        Slot& sl = ctx->slots[s];
+        CU(sl.h_channel.ensure(ctx->max_reads));
+        CU(sl.h_flags.ensure(ctx->max_reads));
+        CU(sl.d_channel.ensure(ctx->max_reads));
+        CU(sl.d_flags.ensure(ctx->max_reads));
+        CU(sl.live_dout.alloc(ctx->max_reads, w.ev_cap));
+        CU(sl.live_hout.alloc(ctx->max_reads, w.ev_cap));
+        sl.live_claim.reset(new (std::nothrow) uint32_t[n_channels]());
+        if (!sl.live_claim) return SGPU_E_NOMEM;
+    }
+    w.n_channels = n_channels;  // (last: an open that failed can be repeated, the arrays it made are kept)
+    return SGPU_OK;
+}
+
+int64_t sgpu_slot_add_live(sgpu_ctx_t* ctx, uint32_t slot, uint32_t channel, uint32_t flags, const int16_t* raw,
+                           uint64_t n, double digitisation, double offset, double range) {
+    if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
+    Slot& sl = ctx->slots[slot];
+    if (sl.submitted || !ctx->live.n_channels || (sl.mode != 0 && sl.mode != 4)) return SGPU_E_STATE;
+    if (channel >= ctx->live.n_channels || (flags & ~LIVE_FLAGS)) return SGPU_E_INVAL;
+    if (n >= (1ull << 31)) return SGPU_E_TOOBIG;
+    const uint64_t need = align_up(n, SGPU_ALIGN);
+    if (need > ctx->max_samples) return SGPU_E_TOOBIG;
+    sgpu_batch_t& b = sl.batch;
+    if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples) return SGPU_E_FULL;
+    if (sl.mode != 4) {  // the slot's first entry: a new generation of its channel marks
+        if (++ctx->live_gen == 0) {
+            for (uint32_t s = 0; s < ctx->n_slots; s++)
+                memset(ctx->slots[s].live_claim.get(), 0, (size_t)ctx->live.n_channels * sizeof(uint32_t));
+            ctx->live_gen = 1;
+        }
+        sl.live_gen = ctx->live_gen;
+    }
+    if (sl.live_claim[channel] == sl.live_gen) return SGPU_E_INVAL;  // one entry per channel and slot
+    sl.live_claim[channel] = sl.live_gen;
+    sl.mode = 4;
+    memcpy(b.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
+    sl.h_channel[b.n_reads] = channel;
+    sl.h_flags[b.n_reads] = flags;
+    return append_record(sl, n, digitisation, offset, range);
+}
+
+int sgpu_wait_live(sgpu_ctx_t* ctx, uint32_t slot, sgpu_live_result_t* out) {
+    if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
+    Slot& sl = ctx->slots[slot];
+    if (!sl.submitted || sl.mode != 4) return SGPU_E_STATE;
+    CU(cudaSetDevice(ctx->device));
+    sl.submitted = false;
+    CU(cudaEventSynchronize(sl.small_back));
+    memset(out, 0, sizeof *out);
+    const int dev_rc = map_dev_status(*sl.h_status);
+    if (dev_rc) return dev_rc;
+    const uint64_t ne = sl.live_hout.ev_off[sl.batch.n_reads];
+    if (ne > ctx->live.ev_cap) return SGPU_E_EVCAP;
+    const size_t b4 = (size_t)ne * 4;
+    CU(cudaMemcpyAsync(sl.live_hout.ev_start, sl.live_dout.ev_start, b4, cudaMemcpyDeviceToHost, sl.stream));
+    CU(cudaMemcpyAsync(sl.live_hout.ev_len, sl.live_dout.ev_len, b4, cudaMemcpyDeviceToHost, sl.stream));
+    CU(cudaMemcpyAsync(sl.live_hout.ev_mean, sl.live_dout.ev_mean, b4, cudaMemcpyDeviceToHost, sl.stream));
+    CU(cudaMemcpyAsync(sl.live_hout.ev_stdv, sl.live_dout.ev_stdv, b4, cudaMemcpyDeviceToHost, sl.stream));
+    CU(cudaStreamSynchronize(sl.stream));
+    fill_live_result(out, sl.live_hout);
+    out->n_events = ne;
+    return SGPU_OK;
+}
+
+int sgpu_run_device_live(sgpu_ctx_t* ctx, const sgpu_dev_live_batch_t* batch, void* stream, sgpu_live_result_t* out) {
+    if (!ctx || !batch || !out) return SGPU_E_INVAL;
+    if (!ctx->live.n_channels) return SGPU_E_STATE;
+    CU(cudaSetDevice(ctx->device));
+    CU(ctx->live_dev_out.alloc(ctx->max_reads, ctx->live.ev_cap));
+    const LiveBatch b{batch->samples, batch->read_off, batch->read_len, batch->channel, batch->flags, batch->offset_f,
+                      batch->raw_unit_f, batch->n_entries, batch->span};
+    const int rc = run_pipeline_live(ctx, b, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
+    if (rc) return rc;
+    ctx->live_mirror_stale = true;
+    fill_live_result(out, ctx->live_dev_out);
     return SGPU_OK;
 }
 

@@ -92,6 +92,39 @@ __device__ __forceinline__ void det_reset(DetState& d) {
     d.masked_to = 0; d.peak_pos = -1; d.peak_value = FLT_MAX; d.valid = 0;
 }
 
+// One step of one detector (events.c:387-437). Returns the emitted peak position or -1.
+// `is_short` selects the masking of the long detector (414-422).
+__device__ __forceinline__ int32_t det_step(DetState& d, DetState* other_long, bool is_short, uint32_t i,
+                                            float cur, float thr, int w, float height) {
+    if (d.masked_to >= i) return -1;
+    if (d.peak_pos < 0) {  // CASE 1
+        if (cur < d.peak_value) {
+            d.peak_value = cur;
+        } else if (__fsub_rn(cur, d.peak_value) > height) {
+            d.peak_value = cur;
+            d.peak_pos = (int32_t)i;
+        }
+        return -1;
+    }
+    // CASE 2
+    if (cur > d.peak_value) { d.peak_value = cur; d.peak_pos = (int32_t)i; }
+    if (is_short && d.peak_value > thr) {
+        other_long->masked_to = (uint32_t)d.peak_pos + (uint32_t)w;
+        other_long->peak_pos = -1;
+        other_long->peak_value = FLT_MAX;
+        other_long->valid = 0;
+    }
+    if (__fsub_rn(d.peak_value, cur) > height && d.peak_value > thr) d.valid = 1;
+    if (d.valid && (i - (uint32_t)d.peak_pos) > (uint32_t)(w / 2)) {
+        const int32_t out = d.peak_pos;
+        d.peak_pos = -1;
+        d.peak_value = cur;
+        d.valid = 0;
+        return out;
+    }
+    return -1;
+}
+
 // grid of a launch: enough blocks of `block` threads for `work` items, at least 1 and at most max_blocks
 static inline int grid_cap(uint64_t work, int block, int max_blocks) {
     uint64_t g = (work + block - 1) / block;

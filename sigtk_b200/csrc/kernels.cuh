@@ -48,7 +48,8 @@ template <typename T> using DevBuf = Buf<T, false>;
 template <typename T> using PinBuf = Buf<T, true>;
 
 // device-side status codes (mapped to SGPU_E_* by capi.cu)
-enum { SGPU_DEV_OK = 0, SGPU_DEV_E_EVCAP = 1, SGPU_DEV_E_SCRATCH = 2, SGPU_DEV_E_STREAM = 3 };
+enum { SGPU_DEV_OK = 0, SGPU_DEV_E_EVCAP = 1, SGPU_DEV_E_SCRATCH = 2, SGPU_DEV_E_STREAM = 3, SGPU_DEV_E_INVAL = 4,
+       SGPU_DEV_E_STATE = 5, SGPU_DEV_E_TOOBIG = 6 };
 
 constexpr int FAST_TILE = 2048;  // samples per tile of the fast path; the event-start bitmap is tiled the same way
 
@@ -163,6 +164,63 @@ struct SvbScratch {
 uint64_t svbzd_max_blocks(uint64_t max_samples, uint32_t max_reads);
 uint32_t svbzd_blocks_of(uint64_t n);
 int launch_svbzd_decode(const SvbBatch& s, SvbScratch& w, Scratch& sc, int16_t* samples, int sm_count, cudaStream_t st);
+
+// live.cu (event detection on signal that arrives in chunks: sgpu_slot_add_live, sgpu_run_device_live)
+constexpr uint32_t LIVE_FLAGS = 7u;        // SGPU_LIVE_START | SGPU_LIVE_END | SGPU_LIVE_RNA
+constexpr uint32_t LIVE_OPEN = 1u << 31;   // LiveScratch::nopen: samples so far | LIVE_OPEN while a read is open
+constexpr int LIVE_TAIL = 28;              // prefix sums a channel carries: 2 * w2 of the RNA parameters
+// What a channel carries from one entry to the next (in HBM; its length and open flag are in LiveScratch::nopen).
+struct LiveChan {
+    double tS[LIVE_TAIL], tQ[LIVE_TAIL];  // S[j], Q[j] for j = n-LIVE_TAIL+1 .. n (0 for j <= 0)
+    double pS[2], pQ[2];                  // at the peak_pos of the short / long detector
+    double aS, aQ;                        // at the open event's start
+    DetState det[2];                      // short, long
+    uint32_t a;                           // the open event's start
+    float offset, unit;                   // the read's calibration (misc.c:17-19,26)
+    uint32_t rna;
+};
+struct LiveBatch {                         // entry e: samples[read_off[e] .. +read_len[e]) of channel[e]
+    const int16_t* samples;
+    const uint64_t* read_off;              // [n_entries+1]
+    const uint32_t* read_len;
+    const uint32_t* channel;
+    const uint32_t* flags;
+    const float* offset;                   // used with SGPU_LIVE_START only
+    const float* unit;
+    uint32_t n_entries;
+    uint64_t span;
+};
+// where entry e (at sample offset `off`) stages its events before compaction. The detector steps at most
+// len + w2 - 1 < len + 14 positions in an entry, and a detector that emits at step i emits next at step
+// i + w/2 + 2 or later (its peak is set at i + 1 at the earliest and must be more than w/2 behind): at most
+// ceil(m/3) + ceil(m/5) events in m steps (DNA; RNA fewer) plus the read's last one, which the stride of
+// 8/15 per sample + 24 per entry covers. Evaluated at (max_samples, max_reads) it is the capacity.
+__host__ __device__ inline uint64_t live_stage_base(uint64_t off, uint64_t e) { return off / 15 * 8 + 24 * e; }
+struct LiveScratch {                       // allocated by sgpu_live_open
+    DevBuf<LiveChan> chan;                 // [n_channels]
+    DevBuf<uint32_t> nopen;                // [n_channels]
+    DevBuf<uint32_t> claim;                // [n_channels] stamp of the last run that had an entry for the channel
+    DevBuf<uint32_t> cnt;                  // [max_reads] events of every entry
+    DevBuf<uint32_t> s_start, s_len;       // [ev_cap] staged events
+    DevBuf<float> s_mean, s_stdv;
+    uint32_t n_channels = 0;
+    uint64_t ev_cap = 0;
+    uint32_t stamp = 0;
+};
+template <bool PINNED> struct LiveOut {    // the events of a live run, entry by entry
+    Buf<uint64_t, PINNED> ev_off;          // [max_reads+1]
+    Buf<uint32_t, PINNED> ev_start, ev_len;
+    Buf<float, PINNED> ev_mean, ev_stdv;   // [ev_cap]
+    cudaError_t alloc(uint64_t max_reads, uint64_t ev_cap) {
+        cudaError_t e = ev_off.ensure(max_reads + 1);
+        if (e == cudaSuccess) e = ev_start.ensure(ev_cap);
+        if (e == cudaSuccess) e = ev_len.ensure(ev_cap);
+        if (e == cudaSuccess) e = ev_mean.ensure(ev_cap);
+        if (e == cudaSuccess) e = ev_stdv.ensure(ev_cap);
+        return e;
+    }
+};
+int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, LiveOut<false>& o, int sm_count, cudaStream_t st);
 
 // stat.cu
 constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;
