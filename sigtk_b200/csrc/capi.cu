@@ -20,10 +20,13 @@ using namespace sgpu;
 
 namespace {
 
-// The per-batch output arrays. OUTS describes each one once; every place that allocates, clears, copies back or
-// returns outputs loops over it. Device and pinned host copies are arrays of N_OUT byte buffers indexed by Out.
+// The output arrays. OUTS describes each per-batch output once, LIVE_OUTS each output of a live run; every place that
+// allocates, clears, copies back or returns outputs loops over one of them. Device and pinned host copies are arrays of
+// byte buffers indexed by Out (or Live).
 enum Out { EV_OFF, EV_START, EV_MEAN, EV_STDV, SEQ_ORDER, FIXUPS, STAT, ENT, JNN_CNT, JNN_SEG, PREFIX_POS, PREFIX_STAT,
            PA, N_OUT };
+enum Live { LIVE_EV_OFF, LIVE_EV_START, LIVE_EV_LEN, LIVE_EV_MEAN, LIVE_EV_STDV, N_LIVE_OUT };
+static_assert(EV_OFF == 0 && LIVE_EV_OFF == 0, "row 0 of both tables: ev_off, which sizes the event outputs");
 
 // what an output's element count is proportional to (times OutSpec::per)
 enum Count : uint8_t {
@@ -35,12 +38,12 @@ enum Count : uint8_t {
 constexpr int ANY_WANT = 0x100;  // OutSpec::empty flag: cleared for an empty batch whatever the want
 
 struct OutSpec {
-    size_t field;    // offset of its pointer in sgpu_result_t
+    size_t field;    // offset of its pointer in sgpu_result_t (LIVE_OUTS: sgpu_live_result_t)
     uint32_t size;   // bytes per element
     uint32_t want;   // SGPU_WANT_* bit of the product it belongs to
     Count count;
     uint32_t per;
-    bool eager;      // allocated at creation (returned by every sgpu_run_device), else on the first run that wants it
+    bool eager;      // allocated up front (returned by every device-resident run), else on the first run that wants it
     int empty;       // byte every element holds for a batch of empty records (| ANY_WANT), or -1: left as it is
     bool pa_in;      // produced by a run on the caller's pA floats (sgpu_run_device_pa, slots of pA records)
 };
@@ -66,6 +69,20 @@ constexpr OutSpec OUTS[] = {  // in the order of Out
 #undef OUTPUT
 static_assert(sizeof OUTS / sizeof OUTS[0] == N_OUT, "one row per output");
 
+// the events of a live run, entry by entry (EVENTS: at the capacity LiveScratch::ev_cap)
+#define LIVE_OUTPUT(field, count, empty) \
+    { offsetof(sgpu_live_result_t, field), sizeof *sgpu_live_result_t{}.field, SGPU_WANT_EVENTS, count, 1, true, empty, \
+      false }
+constexpr OutSpec LIVE_OUTS[] = {  // in the order of Live
+    LIVE_OUTPUT(ev_off,   READS_PLUS_1, 0 | ANY_WANT),
+    LIVE_OUTPUT(ev_start, EVENTS,       -1),
+    LIVE_OUTPUT(ev_len,   EVENTS,       -1),
+    LIVE_OUTPUT(ev_mean,  EVENTS,       -1),
+    LIVE_OUTPUT(ev_stdv,  EVENTS,       -1),
+};
+#undef LIVE_OUTPUT
+static_assert(sizeof LIVE_OUTS / sizeof LIVE_OUTS[0] == N_LIVE_OUT, "one row per output");
+
 // the products a run on pA input can compute: those of its outputs (the others are defined on int16 raw samples, and
 // pA is the input itself)
 constexpr uint32_t pa_input_wants(int k = 0) {
@@ -74,10 +91,9 @@ constexpr uint32_t pa_input_wants(int k = 0) {
 constexpr bool pa_input_want_ok(uint32_t want) { return want != 0 && (want & ~pa_input_wants()) == 0; }
 static_assert(pa_input_wants() == SGPU_WANT_EVENTS, "a pA run computes the event table only");
 
-// elements of output k for a batch of `reads` reads spanning `samples` samples with `events` events; at the
-// context's (max_reads, max_samples, ev_cap) this is the output's capacity
-uint64_t out_elems(int k, uint64_t reads, uint64_t samples, uint64_t events) {
-    const OutSpec& s = OUTS[k];
+// elements of output s for a batch of `reads` reads spanning `samples` samples with `events` events; at the
+// context's (max_reads, max_samples) and the table's event capacity this is the output's capacity
+uint64_t out_elems(const OutSpec& s, uint64_t reads, uint64_t samples, uint64_t events) {
     switch (s.count) {
         case READS: return s.per * reads;
         case READS_PLUS_1: return s.per * (reads + 1);
@@ -86,6 +102,16 @@ uint64_t out_elems(int k, uint64_t reads, uint64_t samples, uint64_t events) {
         case JNN_SLOTS: return s.per * jnn_seg_capacity(samples, (uint32_t)reads);
     }
     return 0;
+}
+
+// What a slot holds between two sgpu_slot_reset: records of one kind, never a mix (NONE: nothing appended yet; it submits
+// as an empty batch of int16 records). allowed_wants() is what each kind can compute.
+enum class Input : uint8_t { NONE, RAW, SVBZD, PA, LIVE };
+
+uint32_t allowed_wants(Input k) {
+    if (k == Input::PA) return pa_input_wants();
+    if (k == Input::LIVE) return SGPU_WANT_EVENTS;
+    return 63u;
 }
 
 struct Slot {
@@ -109,9 +135,8 @@ struct Slot {
     cudaEvent_t in_ready = nullptr, kernels_done = nullptr, small_back = nullptr;
     bool submitted = false;
     uint32_t want = 0;
+    Input kind = Input::NONE;        // (PA: the floats are in the sample buffers, max_samples / 2 of them)
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
-    int mode = 0;                    // 0: empty, 1: decoded int16 records, 2: svb-zd streams, 3: pA records (floats
-                                     // in the sample buffers: max_samples / 2 of them), 4: live entries
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
     DevBuf<uint8_t> d_comp;          // comp_cap + 16 bytes
     PinBuf<uint64_t> h_comp_off; DevBuf<uint64_t> d_comp_off;
@@ -119,8 +144,8 @@ struct Slot {
     uint64_t comp_used = 0, svb_blocks = 0;
     // live entries (allocated by sgpu_live_open): channel and flags of every entry, the run's events
     PinBuf<uint32_t> h_channel, h_flags; DevBuf<uint32_t> d_channel, d_flags;
-    LiveOut<false> live_dout;
-    LiveOut<true> live_hout;
+    DevBuf<void> live_dout[N_LIVE_OUT];
+    PinBuf<void> live_hout[N_LIVE_OUT];
     std::unique_ptr<uint32_t[]> live_claim;  // [n_channels] live_gen of the batch that holds an entry for the channel
     uint32_t live_gen = 0;
 
@@ -151,7 +176,7 @@ struct sgpu_ctx {
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
-    LiveOut<false> live_dev_out; // outputs of sgpu_run_device_live
+    DevBuf<void> live_dev_out[N_LIVE_OUT];    // outputs of sgpu_run_device_live
     std::unique_ptr<uint32_t[]> live_mirror;  // [n_channels] nopen of every channel after the submitted live slots
     bool live_mirror_stale = false;           // a device-resident live run changed channels since
     uint32_t live_gen = 0;
@@ -188,50 +213,59 @@ bool cuda_fail(sgpu_ctx* c, cudaError_t e, const char* what, int line) {
 
 uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 
-// allocates (device or pinned) every output of `o` that is eager or belongs to `want` and does not exist yet
-template <bool PINNED>
-cudaError_t alloc_outputs(const sgpu_ctx* ctx, Buf<void, PINNED>* o, uint32_t want) {
-    for (int k = 0; k < N_OUT; k++) {
-        if (!OUTS[k].eager && !(want & OUTS[k].want)) continue;
-        const uint64_t n = out_elems(k, ctx->max_reads, ctx->max_samples, ctx->ev_cap);
-        const cudaError_t e = o[k].ensure(n * OUTS[k].size);
+// allocates (device or pinned) every output of the table `outs` that is eager or belongs to `want` and does not exist
+// yet, at the context's max_reads, max_samples and the table's event capacity ev_cap
+template <size_t N, bool PINNED>
+cudaError_t alloc_outputs(const OutSpec (&outs)[N], const sgpu_ctx* ctx, uint64_t ev_cap, Buf<void, PINNED>* o,
+                          uint32_t want) {
+    for (size_t k = 0; k < N; k++) {
+        if (!outs[k].eager && !(want & outs[k].want)) continue;
+        const uint64_t n = out_elems(outs[k], ctx->max_reads, ctx->max_samples, ev_cap);
+        const cudaError_t e = o[k].ensure(n * outs[k].size);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
 
 // points the fields of *r at the outputs of `want`, and at every eager output when `all_eager`; the others stay NULL
-template <bool PINNED>
-void fill_result(sgpu_result_t* r, const Buf<void, PINNED>* o, uint32_t want, bool all_eager) {
-    for (int k = 0; k < N_OUT; k++)
-        if ((want & OUTS[k].want) || (all_eager && OUTS[k].eager)) {
+template <size_t N, typename R, bool PINNED>
+void fill_result(const OutSpec (&outs)[N], R* r, const Buf<void, PINNED>* o, uint32_t want, bool all_eager) {
+    for (size_t k = 0; k < N; k++)
+        if ((want & outs[k].want) || (all_eager && outs[k].eager)) {
             void* const p = o[k];
-            memcpy(reinterpret_cast<char*>(r) + OUTS[k].field, &p, sizeof p);
+            memcpy(reinterpret_cast<char*>(r) + outs[k].field, &p, sizeof p);
         }
 }
 
-// queues on the slot's stream the D2H copy of every output of `want` that is sized by the batch's reads and samples,
-// or (by_events) of every one sized by its n_events
-cudaError_t queue_d2h(Slot& sl, uint32_t want, bool by_events, uint64_t n_events) {
-    for (int k = 0; k < N_OUT; k++) {
-        if (!(want & OUTS[k].want) || (OUTS[k].count == EVENTS) != by_events) continue;
-        const uint64_t n = out_elems(k, sl.batch.n_reads, sl.used, n_events);
-        const cudaError_t e = cudaMemcpyAsync(sl.hout[k], sl.dout[k], (size_t)n * OUTS[k].size, cudaMemcpyDeviceToHost,
-                                              sl.stream);
+// queues on the slot's stream the D2H copy (d to h) of every output of `want` that is sized by the batch's reads and
+// samples, or (by_events) of every one sized by its n_events
+template <size_t N>
+cudaError_t queue_d2h(const OutSpec (&outs)[N], const DevBuf<void>* d, PinBuf<void>* h, const Slot& sl, uint32_t want,
+                      bool by_events, uint64_t n_events) {
+    for (size_t k = 0; k < N; k++) {
+        if (!(want & outs[k].want) || (outs[k].count == EVENTS) != by_events) continue;
+        const uint64_t n = out_elems(outs[k], sl.batch.n_reads, sl.used, n_events);
+        const cudaError_t e = cudaMemcpyAsync(h[k], d[k], (size_t)n * outs[k].size, cudaMemcpyDeviceToHost, sl.stream);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
 
-struct StageMarks {  // records a CUDA event between kernel groups when the context has stage timers
+// One run of a pipeline on a stream: start() zeroes the device status and counters, done() records a CUDA event after
+// a kernel group when the context has stage timers, finish() checks the launches and keeps their number.
+struct StageMarks {
     sgpu_ctx* ctx;
     cudaStream_t st;
     bool on;
     uint64_t launches = 0;
-    StageMarks(sgpu_ctx* c, cudaStream_t s) : ctx(c), st(s), on((c->flags & SGPU_F_STAGE_TIMERS) != 0) {
-        c->n_stages = 0;
-        c->stage_stream = s;
-        if (on) cudaEventRecord(c->stage_ev[0], s);
+    StageMarks(sgpu_ctx* c, cudaStream_t s) : ctx(c), st(s), on((c->flags & SGPU_F_STAGE_TIMERS) != 0) {}
+    int start() {
+        CU(cudaMemsetAsync(ctx->sc.status, 0, sizeof(int), st));
+        CU(cudaMemsetAsync(ctx->sc.counters, 0, 4 * sizeof(unsigned long long), st));
+        ctx->n_stages = 0;
+        ctx->stage_stream = st;
+        if (on) cudaEventRecord(ctx->stage_ev[0], st);
+        return SGPU_OK;
     }
     void done(const char* name, int n) {
         launches += (uint64_t)n;
@@ -240,6 +274,11 @@ struct StageMarks {  // records a CUDA event between kernel groups when the cont
         ctx->stage_name[k] = name;
         ctx->stage_launches[k] = (uint32_t)n;
         cudaEventRecord(ctx->stage_ev[k + 1], st);
+    }
+    int finish() {
+        CU(cudaGetLastError());
+        ctx->last_launches = launches;
+        return SGPU_OK;
     }
 };
 
@@ -259,28 +298,33 @@ int alloc_svb_scratch(sgpu_ctx* ctx) {
 
 // nothing but empty records: every per-read output gets its defined value for an empty record (no event, zero
 // statistics / entropies / segments, "record not longer than the window" for prefix) instead of whatever the previous
-// batch left in the buffers
-int clear_empty_batch(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st) {
-    for (int k = 0; k < N_OUT; k++) {
-        const OutSpec& s = OUTS[k];
+// batch left in the buffers; the run launches no kernel
+template <size_t N>
+int clear_empty_batch(const OutSpec (&outs)[N], uint64_t reads, uint64_t span, uint32_t want, DevBuf<void>* o,
+                      StageMarks& run) {
+    sgpu_ctx* const ctx = run.ctx;
+    for (size_t k = 0; k < N; k++) {
+        const OutSpec& s = outs[k];
         if (s.empty < 0 || !((want & s.want) || (s.empty & ANY_WANT))) continue;
-        const uint64_t n = out_elems(k, b.n_reads, b.span, 0);
-        if (n) CU(cudaMemsetAsync(o[k], s.empty & 0xff, (size_t)n * s.size, st));
+        const uint64_t n = out_elems(s, reads, span, 0);
+        if (n) CU(cudaMemsetAsync(o[k], s.empty & 0xff, (size_t)n * s.size, run.st));
     }
-    ctx->last_launches = 0;
-    return SGPU_OK;
+    return run.finish();
+}
+
+bool fits(const sgpu_ctx* ctx, const DevBatch& b) {  // a batch of int16 or pA records the context can hold
+    return b.n_reads <= ctx->max_reads && b.span <= ctx->max_samples && !(b.span & (SGPU_ALIGN - 1));
 }
 
 // The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies.
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
                  const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
-    if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
-    CU(alloc_outputs(ctx, o, want));
-    CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
-    CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
+    if (!fits(ctx, b)) return SGPU_E_INVAL;
+    CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
     StageMarks marks(ctx, st);
-    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(ctx, b, want, o, st);
+    if (const int rc = marks.start()) return rc;
+    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
     if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
     const bool events = (want & SGPU_WANT_EVENTS) != 0;
@@ -338,9 +382,7 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
         marks.done("sequential_order_emit",
                    launch_generic_emit(b, wl, sc, ev_off, ctx->ev_cap, ev_start, ev_mean, ev_stdv, ctx->sm_count, st));
     }
-    CU(cudaGetLastError());
-    ctx->last_launches = marks.launches;
-    return SGPU_OK;
+    return marks.finish();
 }
 
 int alloc_pa_scratch(sgpu_ctx* ctx) {
@@ -389,17 +431,14 @@ int grow_seq_scratch(sgpu_ctx* ctx) {
 int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t want, DevBuf<void>* o,
                     cudaStream_t st) {
     Scratch& sc = ctx->sc;
-    if (!pa_input_want_ok(want)) return SGPU_E_INVAL;
-    if (b.n_reads > ctx->max_reads || b.span > ctx->max_samples || (b.span & (SGPU_ALIGN - 1))) return SGPU_E_INVAL;
-    if (b.n_reads && b.span && !pa) return SGPU_E_INVAL;
-    CU(alloc_outputs(ctx, o, want));
+    if (!fits(ctx, b) || (b.n_reads && b.span && !pa)) return SGPU_E_INVAL;
+    CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
     int rc = alloc_pa_scratch(ctx);
     if (!rc && b.span > sc.gen_cap) rc = grow_seq_scratch(ctx);
     if (rc) return rc;
-    CU(cudaMemsetAsync(sc.status, 0, sizeof(int), st));
-    CU(cudaMemsetAsync(sc.counters, 0, 4 * sizeof(unsigned long long), st));
     StageMarks marks(ctx, st);
-    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(ctx, b, want, o, st);
+    if ((rc = marks.start())) return rc;
+    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
     const uint32_t n_tiles = fast_tiles_for(b.span);
     if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
     uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
@@ -416,31 +455,58 @@ int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t 
                launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START].get()),
                                    static_cast<float*>(o[EV_MEAN].get()), static_cast<float*>(o[EV_STDV].get()),
                                    ctx->sm_count, st));
-    CU(cudaGetLastError());
-    ctx->last_launches = marks.launches;
-    return SGPU_OK;
+    return marks.finish();
 }
 
 // The kernels of a push of live entries into `o` (live.cu). No host synchronisation, no host<->device copies.
-int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, LiveOut<false>& o, cudaStream_t st) {
+int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, DevBuf<void>* o, cudaStream_t st) {
     if (b.n_entries > ctx->max_reads || b.span > ctx->max_samples) return SGPU_E_INVAL;
     if (b.n_entries && (!b.samples || !b.read_off || !b.read_len || !b.channel || !b.flags || !b.offset || !b.unit))
         return SGPU_E_INVAL;
-    CU(cudaMemsetAsync(ctx->sc.status, 0, sizeof(int), st));
-    CU(cudaMemsetAsync(ctx->sc.counters, 0, 4 * sizeof(unsigned long long), st));
     StageMarks marks(ctx, st);
-    if (b.n_entries == 0) {
-        CU(cudaMemsetAsync(o.ev_off, 0, sizeof(uint64_t), st));
-        ctx->last_launches = 0;
-        return SGPU_OK;
+    if (const int rc = marks.start()) return rc;
+    // (entries without samples still open and close channels: only a push of no entry is empty)
+    if (b.n_entries == 0) return clear_empty_batch(LIVE_OUTS, 0, b.span, SGPU_WANT_EVENTS, o, marks);
+    marks.done("live", launch_live(b, ctx->live, ctx->sc, static_cast<uint64_t*>(o[LIVE_EV_OFF].get()),
+                                   static_cast<uint32_t*>(o[LIVE_EV_START].get()),
+                                   static_cast<uint32_t*>(o[LIVE_EV_LEN].get()),
+                                   static_cast<float*>(o[LIVE_EV_MEAN].get()),
+                                   static_cast<float*>(o[LIVE_EV_STDV].get()), ctx->sm_count, st));
+    return marks.finish();
+}
+
+// The kernels of a slot's batch on the context's compute stream, from the slot's device input into its outputs.
+int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
+    const uint32_t nr = sl.batch.n_reads;
+    const int rna = (int)sl.batch.rna;
+    if (sl.kind == Input::LIVE) {
+        const LiveBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_channel, sl.d_flags, sl.d_offset, sl.d_unit,
+                          nr, sl.used};
+        return run_pipeline_live(ctx, b, sl.live_dout, ctx->compute);
     }
-    marks.done("live", launch_live(b, ctx->live, ctx->sc, o, ctx->sm_count, st));
-    CU(cudaGetLastError());
-    ctx->last_launches = marks.launches;
+    CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.hout, want));
+    if (sl.kind == Input::PA)
+        return run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr, rna, sl.used},
+                               reinterpret_cast<const float*>(sl.d_samples.get()), want, sl.dout, ctx->compute);
+    const DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, rna, sl.used};
+    const SvbBatch svb{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
+                       sl.svb_blocks};
+    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.kind == Input::SVBZD ? &svb : nullptr, sl.d_samples);
+}
+
+// a slot that is not submitted takes a record of kind k when it is empty or holds records of kind k
+bool accepts(const Slot& sl, Input k) { return !sl.submitted && (sl.kind == Input::NONE || sl.kind == k); }
+
+// whether a record of n samples fits a slot of `cap` samples: never when n reaches `limit` or the record, padded to
+// SGPU_ALIGN, exceeds cap (SGPU_E_TOOBIG); not now when the slot has no room left for it (SGPU_E_FULL)
+int room_for(const sgpu_ctx* ctx, const Slot& sl, uint64_t n, uint64_t limit, uint64_t cap) {
+    const uint64_t need = align_up(n, SGPU_ALIGN);
+    if (n >= limit || need > cap) return SGPU_E_TOOBIG;
+    if (sl.batch.n_reads >= ctx->max_reads || sl.used + need > cap) return SGPU_E_FULL;
     return SGPU_OK;
 }
 
-// The per-read tail of sgpu_slot_add_read / sgpu_slot_add_read_svbzd: records the read of n samples at sl.used as
+// The per-read tail of every sgpu_slot_add_*: records the read of n samples at sl.used as
 // the batch's next read, with the scalars of its pA conversion.
 int64_t append_record(Slot& sl, uint64_t n, double digitisation, double offset, double range) {
     sgpu_batch_t& b = sl.batch;
@@ -468,64 +534,56 @@ int map_dev_status(int s) {
     return SGPU_OK;
 }
 
-// sgpu_submit of a live slot: the checks against the channel mirror, then copies, kernels (context stream) and the
-// copy of ev_off back, like the other slots
-int submit_live(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
-    if (want != SGPU_WANT_EVENTS) return SGPU_E_INVAL;
-    CU(cudaSetDevice(ctx->device));
+// sgpu_submit of a live slot: the rules that depend on channel state, against the host mirror of the channels
+// (entries of one slot have distinct channels); nothing is queued and no channel changes unless every entry passes
+int check_live_entries(sgpu_ctx* ctx, const Slot& sl) {
     uint32_t* const mirror = ctx->live_mirror.get();
     if (ctx->live_mirror_stale) {  // sgpu_run_device_live changed channels: their state is read back once
         CU(cudaDeviceSynchronize());
         CU(cudaMemcpy(mirror, ctx->live.nopen, (size_t)ctx->live.n_channels * sizeof(uint32_t), cudaMemcpyDeviceToHost));
         ctx->live_mirror_stale = false;
     }
-    const sgpu_batch_t& hb = sl.batch;
-    const uint32_t nr = hb.n_reads;
-    // the rules that depend on channel state (entries of one slot have distinct channels); nothing is queued and no
-    // channel changes unless every entry passes
-    for (uint32_t e = 0; e < nr; e++) {
-        const uint32_t f = sl.h_flags[e], no = mirror[sl.h_channel[e]];
+    for (uint32_t e = 0; e < sl.batch.n_reads; e++) {
+        const uint32_t f = sl.h_flags[e], no = mirror[sl.h_channel[e]], len = sl.batch.read_len[e];
         const bool start = (f & SGPU_LIVE_START) != 0;
-        if (!start && !(no & LIVE_OPEN) && (hb.read_len[e] || (f & SGPU_LIVE_END))) return SGPU_E_STATE;
-        if ((start ? 0ull : (uint64_t)(no & ~LIVE_OPEN)) + hb.read_len[e] > 0x7fffffffull) return SGPU_E_TOOBIG;
+        if (!start && !(no & LIVE_OPEN) && (len || (f & SGPU_LIVE_END))) return SGPU_E_STATE;
+        if ((start ? 0ull : (uint64_t)(no & ~LIVE_OPEN)) + len > 0x7fffffffull) return SGPU_E_TOOBIG;
     }
-    cudaStream_t st = sl.stream;
-    CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_read_off, hb.read_off, ((size_t)nr + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_read_len, hb.read_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_offset, hb.offset_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_unit, hb.raw_unit_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_channel, sl.h_channel, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(sl.d_flags, sl.h_flags, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    CU(cudaEventRecord(sl.in_ready, st));
-    CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
-    const LiveBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_channel, sl.d_flags, sl.d_offset, sl.d_unit, nr,
-                      sl.used};
-    const int rc = run_pipeline_live(ctx, b, sl.live_dout, ctx->compute);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(sl.h_counters, ctx->sc.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
-                       ctx->compute));
-    CU(cudaMemcpyAsync(sl.h_status, ctx->sc.status, sizeof(int), cudaMemcpyDeviceToHost, ctx->compute));
-    CU(cudaEventRecord(sl.kernels_done, ctx->compute));
-    CU(cudaStreamWaitEvent(st, sl.kernels_done, 0));
-    CU(cudaMemcpyAsync(sl.live_hout.ev_off, sl.live_dout.ev_off, ((size_t)nr + 1) * sizeof(uint64_t),
-                       cudaMemcpyDeviceToHost, st));
-    CU(cudaEventRecord(sl.small_back, st));
-    for (uint32_t e = 0; e < nr; e++) {  // the channels as the kernel leaves them
-        const uint32_t c = sl.h_channel[e], f = sl.h_flags[e], no = mirror[c];
-        const bool start = (f & SGPU_LIVE_START) != 0;
-        if (!start && !(no & LIVE_OPEN)) continue;
-        mirror[c] = (f & SGPU_LIVE_END) ? 0u : (uint32_t)((start ? 0u : (no & ~LIVE_OPEN)) + hb.read_len[e]) | LIVE_OPEN;
-    }
-    sl.want = want;
-    sl.submitted = true;
     return SGPU_OK;
 }
 
-template <bool PINNED>
-void fill_live_result(sgpu_live_result_t* r, const LiveOut<PINNED>& o) {
-    memset(r, 0, sizeof *r);
-    r->ev_off = o.ev_off; r->ev_start = o.ev_start; r->ev_len = o.ev_len; r->ev_mean = o.ev_mean; r->ev_stdv = o.ev_stdv;
+// the mirror of the channels as the kernels of a submitted live slot leave them
+void advance_live_mirror(sgpu_ctx* ctx, const Slot& sl) {
+    uint32_t* const mirror = ctx->live_mirror.get();
+    for (uint32_t e = 0; e < sl.batch.n_reads; e++) {
+        const uint32_t c = sl.h_channel[e], f = sl.h_flags[e], no = mirror[c], len = sl.batch.read_len[e];
+        const bool start = (f & SGPU_LIVE_START) != 0;
+        if (!start && !(no & LIVE_OPEN)) continue;
+        mirror[c] = (f & SGPU_LIVE_END) ? 0u : (uint32_t)((start ? 0u : (no & ~LIVE_OPEN)) + len) | LIVE_OPEN;
+    }
+}
+
+// sgpu_wait / sgpu_wait_live: the device status of the submitted slot, then its outputs `outs` (device d, pinned h)
+// sized by the batch's events (at most ev_cap of them) copied back, and *out pointed at the pinned copies
+template <size_t N, typename R>
+int wait_slot(sgpu_ctx* ctx, Slot& sl, const OutSpec (&outs)[N], const DevBuf<void>* d, PinBuf<void>* h,
+              uint64_t ev_cap, R* out) {
+    CU(cudaSetDevice(ctx->device));
+    sl.submitted = false;
+    CU(cudaEventSynchronize(sl.small_back));
+    memset(out, 0, sizeof *out);
+    const int dev_rc = map_dev_status(*sl.h_status);
+    if (dev_rc) return dev_rc;
+    const uint32_t nr = sl.batch.n_reads;
+    if (sl.want & SGPU_WANT_EVENTS) {
+        const uint64_t ne = nr ? static_cast<const uint64_t*>(h[0].get())[nr] : 0;  // (row 0: ev_off)
+        if (ne > ev_cap) return SGPU_E_EVCAP;
+        CU(queue_d2h(outs, d, h, sl, SGPU_WANT_EVENTS, true, ne));
+        CU(cudaStreamSynchronize(sl.stream));
+        out->n_events = ne;
+    }
+    fill_result(outs, out, h, sl.want, false);
+    return SGPU_OK;
 }
 
 }  // namespace
@@ -640,7 +698,7 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
     CUC(sc.status.ensure(1));
     CUC(sc.counters.ensure(4));
     CUC(cudaStreamCreateWithFlags(&ctx->compute, cudaStreamNonBlocking));
-    CUC(alloc_outputs(ctx, ctx->dev_out, 0));
+    CUC(alloc_outputs(OUTS, ctx, ctx->ev_cap, ctx->dev_out, 0));
     if (n_slots) {
         ctx->slots.reset(new (std::nothrow) Slot[n_slots]);
         if (!ctx->slots) return fail(SGPU_E_NOMEM);
@@ -657,8 +715,8 @@ int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max
             CUC(sl.d_offset.ensure(max_reads));
             CUC(sl.d_unit.ensure(max_reads));
             // every slot gets its own outputs (its D2H overlaps the next slot's kernels)
-            CUC(alloc_outputs(ctx, sl.dout, 0));
-            CUC(alloc_outputs(ctx, sl.hout, 0));
+            CUC(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.dout, 0));
+            CUC(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.hout, 0));
             CUC(sl.h_counters.ensure(4));
             CUC(sl.h_status.ensure(1));
             CUC(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
@@ -696,7 +754,7 @@ int sgpu_slot_reset(sgpu_ctx_t* ctx, uint32_t slot, uint32_t rna) {
     sl.batch.rna = rna ? 1u : 0u;
     sl.batch.read_off[0] = 0;
     sl.used = 0;
-    sl.mode = 0;
+    sl.kind = Input::NONE;
     sl.comp_used = 0;
     sl.svb_blocks = 0;
     return SGPU_OK;
@@ -706,16 +764,11 @@ int64_t sgpu_slot_add_read(sgpu_ctx_t* ctx, uint32_t slot, const int16_t* raw, u
                            double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted) return SGPU_E_STATE;
-    if (sl.mode >= 2) return SGPU_E_STATE;  // a batch holds decoded records, svb-zd streams, pA records or live entries,
-                                           // never a mix
-    if (n >= (1ull << 31)) return SGPU_E_TOOBIG;  // the reference itself narrows to int32_t (misc.c:20)
-    const uint64_t need = align_up(n, SGPU_ALIGN);
-    if (need > ctx->max_samples) return SGPU_E_TOOBIG;
-    sgpu_batch_t& b = sl.batch;
-    if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples) return SGPU_E_FULL;
-    sl.mode = 1;
-    memcpy(b.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
+    if (!accepts(sl, Input::RAW)) return SGPU_E_STATE;
+    // (2^31 samples: the reference itself narrows to int32_t, misc.c:20)
+    if (const int rc = room_for(ctx, sl, n, 1ull << 31, ctx->max_samples)) return rc;
+    sl.kind = Input::RAW;
+    memcpy(sl.batch.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
     return append_record(sl, n, digitisation, offset, range);
 }
 
@@ -723,19 +776,17 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
                                  double digitisation, double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || !stream) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || sl.mode == 1 || sl.mode == 3 || sl.mode == 4) return SGPU_E_STATE;
+    if (!accepts(sl, Input::SVBZD)) return SGPU_E_STATE;
     if (n_bytes != 0 && n_bytes < 4) return SGPU_E_STREAM;
     uint32_t count = 0;
     if (n_bytes) memcpy(&count, stream, 4);  // slow5_press.c:1093: the original length leads the stream
     const uint64_t n = count;                // (a record without signal stores no stream at all: n_bytes == 0)
     if (n_bytes && (4u + (n + 3u) / 4u + n > n_bytes || n_bytes > 4u + (n + 3u) / 4u + 4u * n)) return SGPU_E_STREAM;
-    if (n >= (1ull << 31) || n_bytes > 0xffffffffull) return SGPU_E_TOOBIG;
-    const uint64_t need = align_up(n, SGPU_ALIGN), cneed = align_up(n_bytes, 16);
-    if (need > ctx->max_samples || cneed > ctx->comp_cap) return SGPU_E_TOOBIG;
-    sgpu_batch_t& b = sl.batch;
-    if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples || sl.comp_used + cneed > ctx->comp_cap)
-        return SGPU_E_FULL;
-    if (sl.mode != 2) {  // the batch's first stream: make sure the slot's svb-zd buffers exist
+    const uint64_t cneed = align_up(n_bytes, 16);
+    if (n_bytes > 0xffffffffull || cneed > ctx->comp_cap) return SGPU_E_TOOBIG;  // (before the samples' SGPU_E_FULL)
+    if (const int rc = room_for(ctx, sl, n, 1ull << 31, ctx->max_samples)) return rc;
+    if (sl.comp_used + cneed > ctx->comp_cap) return SGPU_E_FULL;
+    if (sl.kind != Input::SVBZD) {  // the batch's first stream: make sure the slot's svb-zd buffers exist
         CU(cudaSetDevice(ctx->device));
         const int rc = alloc_svb_scratch(ctx);
         if (rc) return rc;
@@ -746,8 +797,8 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
         CU(sl.h_comp_len.ensure(ctx->max_reads));
         CU(sl.d_comp_len.ensure(ctx->max_reads));
     }
-    sl.mode = 2;
-    const uint32_t r = b.n_reads;
+    sl.kind = Input::SVBZD;
+    const uint32_t r = sl.batch.n_reads;
     if (n_bytes) memcpy(sl.h_comp + sl.comp_used, stream, (size_t)n_bytes);
     sl.h_comp_off[r] = sl.comp_used;
     sl.h_comp_len[r] = (uint32_t)n_bytes;
@@ -759,16 +810,11 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t* ctx, uint32_t slot, const uint8_t* 
 int64_t sgpu_slot_add_read_pa(sgpu_ctx_t* ctx, uint32_t slot, const float* pa, uint64_t n) {
     if (!ctx || slot >= ctx->n_slots || (!pa && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || sl.mode == 1 || sl.mode == 2 || sl.mode == 4) return SGPU_E_STATE;
+    if (!accepts(sl, Input::PA)) return SGPU_E_STATE;
     // the slot's int16 sample buffers (pinned and device) hold the floats: max_samples / 2 of them
-    const uint64_t cap = ctx->max_samples / 2;
-    if (n >= (1ull << 32)) return SGPU_E_TOOBIG;
-    const uint64_t need = align_up(n, SGPU_ALIGN);
-    if (need > cap) return SGPU_E_TOOBIG;
-    sgpu_batch_t& b = sl.batch;
-    if (b.n_reads >= ctx->max_reads || sl.used + need > cap) return SGPU_E_FULL;
-    sl.mode = 3;
-    memcpy(reinterpret_cast<float*>(b.samples) + sl.used, pa, (size_t)n * sizeof(float));
+    if (const int rc = room_for(ctx, sl, n, 1ull << 32, ctx->max_samples / 2)) return rc;
+    sl.kind = Input::PA;
+    memcpy(reinterpret_cast<float*>(sl.batch.samples) + sl.used, pa, (size_t)n * sizeof(float));
     return append_record(sl, n, 1.0, 0.0, 1.0);  // (offset_f 0, raw_unit_f 1: the values are pA already)
 }
 
@@ -776,48 +822,44 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (!ctx || slot >= ctx->n_slots || (want & ~63u) || want == 0) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
-    if (sl.mode == 4) return submit_live(ctx, sl, want);
-    const bool pa_in = sl.mode == 3;
-    if (pa_in && !pa_input_want_ok(want)) return SGPU_E_INVAL;
+    if (want & ~allowed_wants(sl.kind)) return SGPU_E_INVAL;
     CU(cudaSetDevice(ctx->device));
+    const bool live = sl.kind == Input::LIVE;
+    int rc = live ? check_live_entries(ctx, sl) : SGPU_OK;
+    if (rc) return rc;
     const sgpu_batch_t& hb = sl.batch;
     const uint32_t nr = hb.n_reads;
     cudaStream_t st = sl.stream;
-    SvbBatch svb{};
-    const bool compressed = sl.mode == 2;
-    if (pa_in) {
-        CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sizeof(float), cudaMemcpyHostToDevice, st));
-    } else if (compressed) {
+    if (sl.kind == Input::SVBZD) {
         CU(cudaMemcpyAsync(sl.d_comp, sl.h_comp, (size_t)sl.comp_used, cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(sl.d_comp_off, sl.h_comp_off, (size_t)nr * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(sl.d_comp_len, sl.h_comp_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-        svb = SvbBatch{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
-                       sl.svb_blocks};
     } else {
-        CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+        const size_t sample_size = sl.kind == Input::PA ? sizeof(float) : sizeof(int16_t);
+        CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sample_size, cudaMemcpyHostToDevice, st));
     }
     CU(cudaMemcpyAsync(sl.d_read_off, hb.read_off, ((size_t)nr + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(sl.d_read_len, hb.read_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(sl.d_offset, hb.offset_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(sl.d_unit, hb.raw_unit_f, (size_t)nr * sizeof(float), cudaMemcpyHostToDevice, st));
+    if (live) {
+        CU(cudaMemcpyAsync(sl.d_channel, sl.h_channel, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(sl.d_flags, sl.h_flags, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    }
     CU(cudaEventRecord(sl.in_ready, st));
     CU(cudaStreamWaitEvent(ctx->compute, sl.in_ready, 0));
-    DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, (int)hb.rna, sl.used};
-    CU(alloc_outputs(ctx, sl.hout, want));
-    const int rc = pa_in ? run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr,
-                                                         (int)hb.rna, sl.used},
-                                           reinterpret_cast<const float*>(sl.d_samples.get()), want, sl.dout,
-                                           ctx->compute)
-                         : run_pipeline(ctx, b, want, sl.dout, ctx->compute, compressed ? &svb : nullptr, sl.d_samples);
+    rc = run_slot(ctx, sl, want);
     if (rc) return rc;
-    // small results come back right away; the big arrays are sized by n_events in sgpu_wait
+    // small results come back right away; the big arrays are sized by n_events in sgpu_wait / sgpu_wait_live
     CU(cudaMemcpyAsync(sl.h_counters, ctx->sc.counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
                        ctx->compute));
     CU(cudaMemcpyAsync(sl.h_status, ctx->sc.status, sizeof(int), cudaMemcpyDeviceToHost, ctx->compute));
     CU(cudaEventRecord(sl.kernels_done, ctx->compute));
     CU(cudaStreamWaitEvent(st, sl.kernels_done, 0));
-    CU(queue_d2h(sl, want, false, 0));
+    CU(live ? queue_d2h(LIVE_OUTS, sl.live_dout, sl.live_hout, sl, want, false, 0)
+            : queue_d2h(OUTS, sl.dout, sl.hout, sl, want, false, 0));
     CU(cudaEventRecord(sl.small_back, st));
+    if (live) advance_live_mirror(ctx, sl);
     sl.want = want;
     sl.submitted = true;
     return SGPU_OK;
@@ -826,23 +868,8 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
 int sgpu_wait(sgpu_ctx_t* ctx, uint32_t slot, sgpu_result_t* out) {
     if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!sl.submitted || sl.mode == 4) return SGPU_E_STATE;
-    CU(cudaSetDevice(ctx->device));
-    sl.submitted = false;
-    CU(cudaEventSynchronize(sl.small_back));
-    memset(out, 0, sizeof *out);
-    const int dev_rc = map_dev_status(*sl.h_status);
-    if (dev_rc) return dev_rc;
-    const uint32_t nr = sl.batch.n_reads;
-    if (sl.want & SGPU_WANT_EVENTS) {
-        const uint64_t ne = nr ? static_cast<const uint64_t*>(sl.hout[EV_OFF].get())[nr] : 0;
-        if (ne > ctx->ev_cap) return SGPU_E_EVCAP;
-        CU(queue_d2h(sl, SGPU_WANT_EVENTS, true, ne));
-        CU(cudaStreamSynchronize(sl.stream));
-        out->n_events = ne;
-    }
-    fill_result(out, sl.hout, sl.want, false);
-    return SGPU_OK;
+    if (!sl.submitted || sl.kind == Input::LIVE) return SGPU_E_STATE;
+    return wait_slot(ctx, sl, OUTS, sl.dout, sl.hout, ctx->ev_cap, out);
 }
 
 int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t want, void* stream,
@@ -854,7 +881,7 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     memset(out, 0, sizeof *out);
-    fill_result(out, ctx->dev_out, want, true);
+    fill_result(OUTS, out, ctx->dev_out, want, true);
     return SGPU_OK;
 }
 
@@ -867,7 +894,7 @@ int sgpu_run_device_pa(sgpu_ctx_t* ctx, const sgpu_dev_pa_batch_t* batch, uint32
     const int rc = run_pipeline_pa(ctx, b, batch->pa, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     memset(out, 0, sizeof *out);
-    fill_result(out, ctx->dev_out, want, false);
+    fill_result(OUTS, out, ctx->dev_out, want, false);
     return SGPU_OK;
 }
 
@@ -981,8 +1008,8 @@ int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
         CU(sl.h_flags.ensure(ctx->max_reads));
         CU(sl.d_channel.ensure(ctx->max_reads));
         CU(sl.d_flags.ensure(ctx->max_reads));
-        CU(sl.live_dout.alloc(ctx->max_reads, w.ev_cap));
-        CU(sl.live_hout.alloc(ctx->max_reads, w.ev_cap));
+        CU(alloc_outputs(LIVE_OUTS, ctx, w.ev_cap, sl.live_dout, 0));
+        CU(alloc_outputs(LIVE_OUTS, ctx, w.ev_cap, sl.live_hout, 0));
         sl.live_claim.reset(new (std::nothrow) uint32_t[n_channels]());
         if (!sl.live_claim) return SGPU_E_NOMEM;
     }
@@ -994,14 +1021,10 @@ int64_t sgpu_slot_add_live(sgpu_ctx_t* ctx, uint32_t slot, uint32_t channel, uin
                            uint64_t n, double digitisation, double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (sl.submitted || !ctx->live.n_channels || (sl.mode != 0 && sl.mode != 4)) return SGPU_E_STATE;
+    if (!accepts(sl, Input::LIVE) || !ctx->live.n_channels) return SGPU_E_STATE;
     if (channel >= ctx->live.n_channels || (flags & ~LIVE_FLAGS)) return SGPU_E_INVAL;
-    if (n >= (1ull << 31)) return SGPU_E_TOOBIG;
-    const uint64_t need = align_up(n, SGPU_ALIGN);
-    if (need > ctx->max_samples) return SGPU_E_TOOBIG;
-    sgpu_batch_t& b = sl.batch;
-    if (b.n_reads >= ctx->max_reads || sl.used + need > ctx->max_samples) return SGPU_E_FULL;
-    if (sl.mode != 4) {  // the slot's first entry: a new generation of its channel marks
+    if (const int rc = room_for(ctx, sl, n, 1ull << 31, ctx->max_samples)) return rc;
+    if (sl.kind != Input::LIVE) {  // the slot's first entry: a new generation of its channel marks
         if (++ctx->live_gen == 0) {
             for (uint32_t s = 0; s < ctx->n_slots; s++)
                 memset(ctx->slots[s].live_claim.get(), 0, (size_t)ctx->live.n_channels * sizeof(uint32_t));
@@ -1011,47 +1034,32 @@ int64_t sgpu_slot_add_live(sgpu_ctx_t* ctx, uint32_t slot, uint32_t channel, uin
     }
     if (sl.live_claim[channel] == sl.live_gen) return SGPU_E_INVAL;  // one entry per channel and slot
     sl.live_claim[channel] = sl.live_gen;
-    sl.mode = 4;
-    memcpy(b.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
-    sl.h_channel[b.n_reads] = channel;
-    sl.h_flags[b.n_reads] = flags;
+    sl.kind = Input::LIVE;
+    memcpy(sl.batch.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
+    sl.h_channel[sl.batch.n_reads] = channel;
+    sl.h_flags[sl.batch.n_reads] = flags;
     return append_record(sl, n, digitisation, offset, range);
 }
 
 int sgpu_wait_live(sgpu_ctx_t* ctx, uint32_t slot, sgpu_live_result_t* out) {
     if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!sl.submitted || sl.mode != 4) return SGPU_E_STATE;
-    CU(cudaSetDevice(ctx->device));
-    sl.submitted = false;
-    CU(cudaEventSynchronize(sl.small_back));
-    memset(out, 0, sizeof *out);
-    const int dev_rc = map_dev_status(*sl.h_status);
-    if (dev_rc) return dev_rc;
-    const uint64_t ne = sl.live_hout.ev_off[sl.batch.n_reads];
-    if (ne > ctx->live.ev_cap) return SGPU_E_EVCAP;
-    const size_t b4 = (size_t)ne * 4;
-    CU(cudaMemcpyAsync(sl.live_hout.ev_start, sl.live_dout.ev_start, b4, cudaMemcpyDeviceToHost, sl.stream));
-    CU(cudaMemcpyAsync(sl.live_hout.ev_len, sl.live_dout.ev_len, b4, cudaMemcpyDeviceToHost, sl.stream));
-    CU(cudaMemcpyAsync(sl.live_hout.ev_mean, sl.live_dout.ev_mean, b4, cudaMemcpyDeviceToHost, sl.stream));
-    CU(cudaMemcpyAsync(sl.live_hout.ev_stdv, sl.live_dout.ev_stdv, b4, cudaMemcpyDeviceToHost, sl.stream));
-    CU(cudaStreamSynchronize(sl.stream));
-    fill_live_result(out, sl.live_hout);
-    out->n_events = ne;
-    return SGPU_OK;
+    if (!sl.submitted || sl.kind != Input::LIVE) return SGPU_E_STATE;
+    return wait_slot(ctx, sl, LIVE_OUTS, sl.live_dout, sl.live_hout, ctx->live.ev_cap, out);
 }
 
 int sgpu_run_device_live(sgpu_ctx_t* ctx, const sgpu_dev_live_batch_t* batch, void* stream, sgpu_live_result_t* out) {
     if (!ctx || !batch || !out) return SGPU_E_INVAL;
     if (!ctx->live.n_channels) return SGPU_E_STATE;
     CU(cudaSetDevice(ctx->device));
-    CU(ctx->live_dev_out.alloc(ctx->max_reads, ctx->live.ev_cap));
+    CU(alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, ctx->live_dev_out, 0));
     const LiveBatch b{batch->samples, batch->read_off, batch->read_len, batch->channel, batch->flags, batch->offset_f,
                       batch->raw_unit_f, batch->n_entries, batch->span};
     const int rc = run_pipeline_live(ctx, b, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     ctx->live_mirror_stale = true;
-    fill_live_result(out, ctx->live_dev_out);
+    memset(out, 0, sizeof *out);
+    fill_result(LIVE_OUTS, out, ctx->live_dev_out, SGPU_WANT_EVENTS, false);
     return SGPU_OK;
 }
 

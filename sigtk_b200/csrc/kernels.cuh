@@ -207,20 +207,9 @@ struct LiveScratch {                       // allocated by sgpu_live_open
     uint64_t ev_cap = 0;
     uint32_t stamp = 0;
 };
-template <bool PINNED> struct LiveOut {    // the events of a live run, entry by entry
-    Buf<uint64_t, PINNED> ev_off;          // [max_reads+1]
-    Buf<uint32_t, PINNED> ev_start, ev_len;
-    Buf<float, PINNED> ev_mean, ev_stdv;   // [ev_cap]
-    cudaError_t alloc(uint64_t max_reads, uint64_t ev_cap) {
-        cudaError_t e = ev_off.ensure(max_reads + 1);
-        if (e == cudaSuccess) e = ev_start.ensure(ev_cap);
-        if (e == cudaSuccess) e = ev_len.ensure(ev_cap);
-        if (e == cudaSuccess) e = ev_mean.ensure(ev_cap);
-        if (e == cudaSuccess) e = ev_stdv.ensure(ev_cap);
-        return e;
-    }
-};
-int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, LiveOut<false>& o, int sm_count, cudaStream_t st);
+// the events of entry e go to ev_start, ev_len, ev_mean, ev_stdv [ev_off[e], ev_off[e+1]) (ev_off: [n_entries+1])
+int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start, uint32_t* ev_len,
+                float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
 
 // stat.cu
 constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;

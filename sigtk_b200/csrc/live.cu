@@ -200,14 +200,15 @@ __global__ void __launch_bounds__(256) live_compact_kernel(LiveBatch b, const ui
     }
 }
 
-int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, LiveOut<false>& o, int sm_count, cudaStream_t st) {
+int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start, uint32_t* ev_len,
+                float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st) {
     if (++w.stamp == 0) w.stamp = 1;  // (claim[] starts at 0)
     live_kernel<<<grid_cap(b.n_entries, LIVE_WARPS, sm_count * 8), LIVE_WARPS * 32, 0, st>>>(
         b, w.chan, w.nopen, w.claim, w.n_channels, w.stamp, sc.tune_thr_long, w.cnt, w.s_start, w.s_len, w.s_mean,
         w.s_stdv, w.ev_cap, sc.status);
-    int n = 1 + launch_scan_u32(w.cnt, b.n_entries, o.ev_off, reinterpret_cast<uint64_t*>(sc.counters.get()), sc, st);
+    int n = 1 + launch_scan_u32(w.cnt, b.n_entries, ev_off, reinterpret_cast<uint64_t*>(sc.counters.get()), sc, st);
     live_compact_kernel<<<grid_cap(b.n_entries, 8, sm_count * 8), 256, 0, st>>>(
-        b, w.cnt, o.ev_off, w.s_start, w.s_len, w.s_mean, w.s_stdv, o.ev_start, o.ev_len, o.ev_mean, o.ev_stdv);
+        b, w.cnt, ev_off, w.s_start, w.s_len, w.s_mean, w.s_stdv, ev_start, ev_len, ev_mean, ev_stdv);
     return n + 1;
 }
 
