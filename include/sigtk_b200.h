@@ -224,9 +224,14 @@ int  sgpu_decode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_svb_dev_batch_t *batch
 
 /* ---- live event detection: signal that arrives in chunks, channel by channel ----------------------------------
  * For tools that segment signal while the read is still in the pore (adaptive sampling, Read Until): per channel, a
- * read is opened by a START entry, grows by entries of int16 samples and is closed by an END entry; one entry may carry
+ * read is opened by a START entry, grows by entries of samples and is closed by an END entry; one entry may carry
  * START, samples and END together. The context keeps every channel's detector state in HBM between entries.
- *   - pA of every sample is misc.c:28 with the calibration given at START (offset_f = (float)offset, raw_unit_f =
+ *   - Two forms of entry: int16 samples with a calibration (sgpu_slot_add_live, sgpu_run_device_live), or pA floats
+ *     taken as they are (sgpu_slot_add_live_pa, sgpu_run_device_live_pa: calibrated, filtered, normalised or simulated
+ *     signal). A read keeps the form of the entry that carries its START: an entry without START on a channel whose
+ *     read is open must have that form, whatever its length and flags (an empty entry too), else it is refused with
+ *     SGPU_E_STATE like the other violations below. A START entry of either form discards an open read of either form.
+ *   - pA of every int16 sample is misc.c:28 with the calibration given at START (offset_f = (float)offset, raw_unit_f =
  *     (float)range / (float)digitisation, as sgpu_slot_add_read computes them); the DNA or RNA parameters also come
  *     from START (SGPU_LIVE_RNA, ignored without START). The long threshold follows SGPU_PARAM_THR_LONG.
  *   - When events are reported: let a read hold n samples after an entry that does not end it. The detector has then
@@ -237,19 +242,25 @@ int  sgpu_decode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_svb_dev_batch_t *batch
  *     ends with the single event [0, n); a read of 0 samples reports no event. A peak may be emitted long after its
  *     position, in a later entry.
  *   - Exactness: for every read, the events of all its entries taken in order are bit-identical to the event table of
- *     the whole read (getevents, events.c:553-573, and sgpu_slot_add_read), for any split into chunks.
+ *     the whole read (getevents, events.c:553-573, and sgpu_slot_add_read), for any split into chunks. For a read of
+ *     pA entries this holds for every finite input, against getevents(n, pa, rna) and sgpu_slot_add_read_pa (the
+ *     prefix sums are formed one sample after another in the reference's order, so no exactness witness is needed);
+ *     with NaN or Inf in the input the event boundaries are identical and the NaN statistics are NaN in the same
+ *     places.
  *   - Ordering: live runs of a context update channel state in the order they are submitted (host slots run their
  *     kernels on one stream of the context). A device-resident live run is ordered by the caller's stream and must not
  *     overlap a submitted live slot.
  *   - START on a channel whose read is still open discards that read: its open event is never reported.
- * A live slot holds live entries only (SGPU_E_STATE when mixed with other records) in its int16 sample buffers, and
- * computes SGPU_WANT_EVENTS only (sgpu_submit returns SGPU_E_INVAL for any other want). sgpu_wait on a live slot and
- * sgpu_wait_live on any other slot return SGPU_E_STATE. sgpu_slot_add_live returns the entry's index, SGPU_E_FULL /
- * SGPU_E_TOOBIG as sgpu_slot_add_read does, SGPU_E_INVAL for channel >= n_channels, unknown flag bits or a second entry
- * for the channel in the slot, SGPU_E_STATE before sgpu_live_open. sgpu_submit checks the rules that depend on channel
- * state against a host mirror updated in submission order: samples or END for a channel without an open read give
- * SGPU_E_STATE, a read that would exceed 2^31 - 1 samples (misc.c:20) SGPU_E_TOOBIG; then nothing is queued and no
- * channel changes. sgpu_run_device_live reports the same violations as `status` in sgpu_counters, and the offending
+ * A live slot holds live entries of one form only (SGPU_E_STATE when mixed with other records or with entries of the
+ * other form) in its int16 sample buffers, and computes SGPU_WANT_EVENTS only (sgpu_submit returns SGPU_E_INVAL for any
+ * other want). sgpu_wait on a live slot and sgpu_wait_live on any other slot return SGPU_E_STATE. sgpu_slot_add_live
+ * returns the entry's index, SGPU_E_FULL / SGPU_E_TOOBIG as sgpu_slot_add_read does (sgpu_slot_add_live_pa: as
+ * sgpu_slot_add_read_pa does, max_samples / 2 floats a slot, and never a read of 2^31 samples), SGPU_E_INVAL for
+ * channel >= n_channels, unknown flag bits or a second entry for the channel in the slot, SGPU_E_STATE before
+ * sgpu_live_open. sgpu_submit checks the rules that depend on channel state against a host mirror updated in
+ * submission order: samples or END for a channel without an open read, or an entry that continues a read of the other
+ * form, give SGPU_E_STATE, a read that would exceed 2^31 - 1 samples (misc.c:20) SGPU_E_TOOBIG; then nothing is queued
+ * and no channel changes. sgpu_run_device_live reports the same violations as `status` in sgpu_counters, and the offending
  * entries leave their channels unchanged. The event capacity covers every possible push (SGPU_E_EVCAP cannot occur). */
 #define SGPU_LIVE_START 1u /* begin a new read on the channel: calibration (and SGPU_LIVE_RNA) taken from this entry */
 #define SGPU_LIVE_END   2u /* the read ends after this entry's samples */
@@ -261,6 +272,9 @@ int  sgpu_live_open(sgpu_ctx_t *ctx, uint32_t n_channels);
 /* Append one entry to a live slot (digitisation, offset, range are read with SGPU_LIVE_START only). */
 int64_t sgpu_slot_add_live(sgpu_ctx_t *ctx, uint32_t slot, uint32_t channel, uint32_t flags, const int16_t *raw,
                            uint64_t n, double digitisation, double offset, double range);
+/* Append one live entry given as pA floats (channel, SGPU_LIVE_* flags as for sgpu_slot_add_live; no calibration). */
+int64_t sgpu_slot_add_live_pa(sgpu_ctx_t *ctx, uint32_t slot, uint32_t channel, uint32_t flags, const float *pa,
+                              uint64_t n);
 /* Events of a live run, entry by entry: host pointers (pinned) from sgpu_wait_live, device pointers from
  * sgpu_run_device_live (n_events 0 there: see sgpu_counters). */
 typedef struct {
@@ -289,6 +303,18 @@ typedef struct {
     uint64_t span;
 } sgpu_dev_live_batch_t;
 int  sgpu_run_device_live(sgpu_ctx_t *ctx, const sgpu_dev_live_batch_t *batch, void *stream, sgpu_live_result_t *out);
+/* Device-resident live entries of pA floats: as sgpu_run_device_live, entry e is pa[read_off[e] .. +read_len[e]). */
+typedef struct {
+    const float    *pa;         /* device; entry e is pa[read_off[e] .. +read_len[e]) */
+    const uint64_t *read_off;   /* [n_entries+1] */
+    const uint32_t *read_len;
+    const uint32_t *channel;
+    const uint32_t *flags;
+    uint32_t n_entries;
+    uint64_t span;              /* = read_off[n_entries] <= max_samples */
+} sgpu_dev_live_pa_batch_t;
+int  sgpu_run_device_live_pa(sgpu_ctx_t *ctx, const sgpu_dev_live_pa_batch_t *batch, void *stream,
+                             sgpu_live_result_t *out);
 
 /* Counters of the last completed run (host path: after sgpu_wait; device path:
  * after the caller synchronised the stream). Synchronises the device. */

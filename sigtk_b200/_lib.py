@@ -18,7 +18,7 @@ F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS = 0, 1, 2, 4
 ALIGN = 8
 
 E_FULL, E_TOOBIG = -4, -5
-LIVE_START, LIVE_END, LIVE_RNA = 1, 2, 4  # flags of a live entry (sgpu_slot_add_live)
+LIVE_START, LIVE_END, LIVE_RNA = 1, 2, 4  # flags of a live entry (sgpu_slot_add_live, sgpu_slot_add_live_pa)
 
 # every symbol include/sigtk_b200.h declares
 EXPORTS = (
@@ -27,6 +27,7 @@ EXPORTS = (
     "sgpu_wait", "sgpu_run_device", "sgpu_counters", "sgpu_memcpy_d2h", "sgpu_stage_times",
     "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
     "sgpu_run_device_pa", "sgpu_live_open", "sgpu_slot_add_live", "sgpu_wait_live", "sgpu_run_device_live",
+    "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -87,6 +88,13 @@ class DevLiveBatch(C.Structure):  # sgpu_dev_live_batch_t
         ("samples", C.c_void_p), ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("channel", C.c_void_p),
         ("flags", C.c_void_p), ("offset_f", C.c_void_p), ("raw_unit_f", C.c_void_p), ("n_entries", C.c_uint32),
         ("span", C.c_uint64),
+    ]
+
+
+class DevLivePaBatch(C.Structure):  # sgpu_dev_live_pa_batch_t
+    _fields_ = [
+        ("pa", C.c_void_p), ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("channel", C.c_void_p),
+        ("flags", C.c_void_p), ("n_entries", C.c_uint32), ("span", C.c_uint64),
     ]
 
 
@@ -159,6 +167,10 @@ def load() -> C.CDLL:
     lib.sgpu_wait_live.restype = i32
     lib.sgpu_run_device_live.argtypes = [vp, C.POINTER(DevLiveBatch), vp, C.POINTER(LiveResult)]
     lib.sgpu_run_device_live.restype = i32
+    lib.sgpu_slot_add_live_pa.argtypes = [vp, u32, u32, u32, vp, u64]
+    lib.sgpu_slot_add_live_pa.restype = C.c_int64
+    lib.sgpu_run_device_live_pa.argtypes = [vp, C.POINTER(DevLivePaBatch), vp, C.POINTER(LiveResult)]
+    lib.sgpu_run_device_live_pa.restype = i32
     lib.sgpu_set_param.argtypes = [vp, i32, C.c_double]
     lib.sgpu_set_param.restype = i32
     _lib = lib

@@ -24,6 +24,7 @@ from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_T
 Read = Tuple[np.ndarray, float, float, float]  # raw int16, digitisation, offset, range
 LiveEntry = Tuple[int, int, np.ndarray, float, float, float]  # channel, LIVE_* flags, raw int16, digitisation, offset,
                                                               # range (the calibration is read with LIVE_START only)
+LivePaEntry = Tuple[int, int, np.ndarray]  # channel, LIVE_* flags, pA float32
 
 
 @dataclass
@@ -224,7 +225,16 @@ class Context:
             self._check(int(self._lib.sgpu_slot_add_live(self._h, slot, int(ch), int(flags), raw.ctypes.data,
                                                          raw.shape[0], float(dig), float(off), float(rng))))
 
+    def live_fill_pa(self, slot: int, entries: Sequence[LivePaEntry]) -> None:
+        """live entries given as pA floats (sgpu_slot_add_live_pa); a slot holds max_samples / 2 of them"""
+        self._check(self._lib.sgpu_slot_reset(self._h, slot, 0))
+        for ch, flags, pa in entries:
+            pa = np.ascontiguousarray(pa, dtype=np.float32)
+            self._check(int(self._lib.sgpu_slot_add_live_pa(self._h, slot, int(ch), int(flags), pa.ctypes.data,
+                                                            pa.shape[0])))
+
     def live_wait(self, slot: int) -> List[EventTable]:
+        """the events of a submitted live slot of either form, entry by entry"""
         res = _lib.LiveResult()
         self._check(self._lib.sgpu_wait_live(self._h, slot, C.byref(res)))
         pb = C.POINTER(_lib.Batch)()
@@ -240,6 +250,12 @@ class Context:
         self.submit(slot, WANT_EVENTS)
         return self.live_wait(slot)
 
+    def live_push_pa(self, entries: Sequence[LivePaEntry], slot: int = 0) -> List[EventTable]:
+        """one push of live entries of pA floats (at most one per channel); -> the events each entry reports"""
+        self.live_fill_pa(slot, entries)
+        self.submit(slot, WANT_EVENTS)
+        return self.live_wait(slot)
+
     def run_device_live(self, samples_ptr: int, read_off_ptr: int, read_len_ptr: int, channel_ptr: int, flags_ptr: int,
                         offset_ptr: int, unit_ptr: int, n_entries: int, span: int, stream: int = 0) -> _lib.LiveResult:
         """sgpu_run_device_live: live entries already in device memory; -> device pointers of the events (the count
@@ -248,6 +264,15 @@ class Context:
                                n_entries, span)
         res = _lib.LiveResult()
         self._check(self._lib.sgpu_run_device_live(self._h, C.byref(db), C.c_void_p(stream), C.byref(res)))
+        return res
+
+    def run_device_live_pa(self, pa_ptr: int, read_off_ptr: int, read_len_ptr: int, channel_ptr: int, flags_ptr: int,
+                           n_entries: int, span: int, stream: int = 0) -> _lib.LiveResult:
+        """sgpu_run_device_live_pa: live entries of pA floats already in device memory; -> device pointers of the
+        events, as run_device_live"""
+        db = _lib.DevLivePaBatch(pa_ptr, read_off_ptr, read_len_ptr, channel_ptr, flags_ptr, n_entries, span)
+        res = _lib.LiveResult()
+        self._check(self._lib.sgpu_run_device_live_pa(self._h, C.byref(db), C.c_void_p(stream), C.byref(res)))
         return res
 
     # ---- device-resident path ---------------------------------------------

@@ -105,12 +105,15 @@ uint64_t out_elems(const OutSpec& s, uint64_t reads, uint64_t samples, uint64_t 
 }
 
 // What a slot holds between two sgpu_slot_reset: records of one kind, never a mix (NONE: nothing appended yet; it submits
-// as an empty batch of int16 records). allowed_wants() is what each kind can compute.
-enum class Input : uint8_t { NONE, RAW, SVBZD, PA, LIVE };
+// as an empty batch of int16 records). allowed_wants() is what each kind can compute. LIVE and LIVE_PA are live entries
+// of int16 samples and of pA floats.
+enum class Input : uint8_t { NONE, RAW, SVBZD, PA, LIVE, LIVE_PA };
+
+bool is_live(Input k) { return k == Input::LIVE || k == Input::LIVE_PA; }
 
 uint32_t allowed_wants(Input k) {
     if (k == Input::PA) return pa_input_wants();
-    if (k == Input::LIVE) return SGPU_WANT_EVENTS;
+    if (is_live(k)) return SGPU_WANT_EVENTS;
     return 63u;
 }
 
@@ -135,7 +138,7 @@ struct Slot {
     cudaEvent_t in_ready = nullptr, kernels_done = nullptr, small_back = nullptr;
     bool submitted = false;
     uint32_t want = 0;
-    Input kind = Input::NONE;        // (PA: the floats are in the sample buffers, max_samples / 2 of them)
+    Input kind = Input::NONE;        // (PA, LIVE_PA: the floats are in the sample buffers, max_samples / 2 of them)
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
     DevBuf<uint8_t> d_comp;          // comp_cap + 16 bytes
@@ -178,6 +181,7 @@ struct sgpu_ctx {
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
     DevBuf<void> live_dev_out[N_LIVE_OUT];    // outputs of sgpu_run_device_live
     std::unique_ptr<uint32_t[]> live_mirror;  // [n_channels] nopen of every channel after the submitted live slots
+    std::unique_ptr<uint8_t[]> live_form;     // [n_channels] and the form of its open read (LiveScratch::form)
     bool live_mirror_stale = false;           // a device-resident live run changed channels since
     uint32_t live_gen = 0;
     uint64_t comp_cap = 0;       // bytes of compressed input a slot can hold
@@ -458,20 +462,22 @@ int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t 
     return marks.finish();
 }
 
-// The kernels of a push of live entries into `o` (live.cu). No host synchronisation, no host<->device copies.
-int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, DevBuf<void>* o, cudaStream_t st) {
+// The kernels of a push of live entries into `o` (live.cu; pa: the entries are b.pa floats). No host synchronisation, no
+// host<->device copies.
+int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, bool pa, DevBuf<void>* o, cudaStream_t st) {
     if (b.n_entries > ctx->max_reads || b.span > ctx->max_samples) return SGPU_E_INVAL;
-    if (b.n_entries && (!b.samples || !b.read_off || !b.read_len || !b.channel || !b.flags || !b.offset || !b.unit))
+    if (b.n_entries && (!b.samples || !b.read_off || !b.read_len || !b.channel || !b.flags ||
+                        (!pa && (!b.offset || !b.unit))))
         return SGPU_E_INVAL;
     StageMarks marks(ctx, st);
     if (const int rc = marks.start()) return rc;
     // (entries without samples still open and close channels: only a push of no entry is empty)
     if (b.n_entries == 0) return clear_empty_batch(LIVE_OUTS, 0, b.span, SGPU_WANT_EVENTS, o, marks);
-    marks.done("live", launch_live(b, ctx->live, ctx->sc, static_cast<uint64_t*>(o[LIVE_EV_OFF].get()),
-                                   static_cast<uint32_t*>(o[LIVE_EV_START].get()),
-                                   static_cast<uint32_t*>(o[LIVE_EV_LEN].get()),
-                                   static_cast<float*>(o[LIVE_EV_MEAN].get()),
-                                   static_cast<float*>(o[LIVE_EV_STDV].get()), ctx->sm_count, st));
+    marks.done(pa ? "live_pa" : "live",
+               launch_live(b, pa, ctx->live, ctx->sc, static_cast<uint64_t*>(o[LIVE_EV_OFF].get()),
+                           static_cast<uint32_t*>(o[LIVE_EV_START].get()), static_cast<uint32_t*>(o[LIVE_EV_LEN].get()),
+                           static_cast<float*>(o[LIVE_EV_MEAN].get()), static_cast<float*>(o[LIVE_EV_STDV].get()),
+                           ctx->sm_count, st));
     return marks.finish();
 }
 
@@ -479,10 +485,10 @@ int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, DevBuf<void>* o, cudaSt
 int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
     const uint32_t nr = sl.batch.n_reads;
     const int rna = (int)sl.batch.rna;
-    if (sl.kind == Input::LIVE) {
+    if (is_live(sl.kind)) {  // (LIVE_PA: the union's pa is the same pointer, the floats in the sample buffers)
         const LiveBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_channel, sl.d_flags, sl.d_offset, sl.d_unit,
                           nr, sl.used};
-        return run_pipeline_live(ctx, b, sl.live_dout, ctx->compute);
+        return run_pipeline_live(ctx, b, sl.kind == Input::LIVE_PA, sl.live_dout, ctx->compute);
     }
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.hout, want));
     if (sl.kind == Input::PA)
@@ -524,6 +530,29 @@ int64_t append_record(Slot& sl, uint64_t n, double digitisation, double offset, 
     return (int64_t)r;
 }
 
+// The checks of sgpu_slot_add_live and sgpu_slot_add_live_pa in their order, then the entry's channel and flags: an
+// entry of kind k (LIVE or LIVE_PA) of n samples in a slot that holds `cap` of them. The caller copies the samples.
+int add_live_entry(sgpu_ctx* ctx, Slot& sl, Input k, uint32_t channel, uint32_t flags, uint64_t n, uint64_t cap) {
+    if (!accepts(sl, k) || !ctx->live.n_channels) return SGPU_E_STATE;
+    if (channel >= ctx->live.n_channels || (flags & ~LIVE_FLAGS)) return SGPU_E_INVAL;
+    // (2^31 samples: a read may not reach them, misc.c:20)
+    if (const int rc = room_for(ctx, sl, n, 1ull << 31, cap)) return rc;
+    if (sl.kind != k) {  // the slot's first entry: a new generation of its channel marks
+        if (++ctx->live_gen == 0) {
+            for (uint32_t s = 0; s < ctx->n_slots; s++)
+                memset(ctx->slots[s].live_claim.get(), 0, (size_t)ctx->live.n_channels * sizeof(uint32_t));
+            ctx->live_gen = 1;
+        }
+        sl.live_gen = ctx->live_gen;
+    }
+    if (sl.live_claim[channel] == sl.live_gen) return SGPU_E_INVAL;  // one entry per channel and slot
+    sl.live_claim[channel] = sl.live_gen;
+    sl.kind = k;
+    sl.h_channel[sl.batch.n_reads] = channel;
+    sl.h_flags[sl.batch.n_reads] = flags;
+    return SGPU_OK;
+}
+
 int map_dev_status(int s) {
     if (s == SGPU_DEV_E_EVCAP) return SGPU_E_EVCAP;
     if (s == SGPU_DEV_E_INVAL) return SGPU_E_INVAL;
@@ -534,19 +563,26 @@ int map_dev_status(int s) {
     return SGPU_OK;
 }
 
+uint8_t live_form_of(Input k) { return k == Input::LIVE_PA ? LIVE_FORM_PA : LIVE_FORM_INT16; }
+
 // sgpu_submit of a live slot: the rules that depend on channel state, against the host mirror of the channels
 // (entries of one slot have distinct channels); nothing is queued and no channel changes unless every entry passes
 int check_live_entries(sgpu_ctx* ctx, const Slot& sl) {
     uint32_t* const mirror = ctx->live_mirror.get();
-    if (ctx->live_mirror_stale) {  // sgpu_run_device_live changed channels: their state is read back once
+    uint8_t* const form = ctx->live_form.get();
+    const uint32_t nc = ctx->live.n_channels;
+    if (ctx->live_mirror_stale) {  // a device-resident live run changed channels: their state is read back once
         CU(cudaDeviceSynchronize());
-        CU(cudaMemcpy(mirror, ctx->live.nopen, (size_t)ctx->live.n_channels * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(mirror, ctx->live.nopen, (size_t)nc * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(form, ctx->live.form, (size_t)nc * sizeof(uint8_t), cudaMemcpyDeviceToHost));
         ctx->live_mirror_stale = false;
     }
+    const uint8_t my_form = live_form_of(sl.kind);
     for (uint32_t e = 0; e < sl.batch.n_reads; e++) {
-        const uint32_t f = sl.h_flags[e], no = mirror[sl.h_channel[e]], len = sl.batch.read_len[e];
+        const uint32_t c = sl.h_channel[e], f = sl.h_flags[e], no = mirror[c], len = sl.batch.read_len[e];
         const bool start = (f & SGPU_LIVE_START) != 0;
         if (!start && !(no & LIVE_OPEN) && (len || (f & SGPU_LIVE_END))) return SGPU_E_STATE;
+        if (!start && (no & LIVE_OPEN) && form[c] != my_form) return SGPU_E_STATE;  // a read of the other form
         if ((start ? 0ull : (uint64_t)(no & ~LIVE_OPEN)) + len > 0x7fffffffull) return SGPU_E_TOOBIG;
     }
     return SGPU_OK;
@@ -560,6 +596,7 @@ void advance_live_mirror(sgpu_ctx* ctx, const Slot& sl) {
         const bool start = (f & SGPU_LIVE_START) != 0;
         if (!start && !(no & LIVE_OPEN)) continue;
         mirror[c] = (f & SGPU_LIVE_END) ? 0u : (uint32_t)((start ? 0u : (no & ~LIVE_OPEN)) + len) | LIVE_OPEN;
+        if (start) ctx->live_form[c] = live_form_of(sl.kind);
     }
 }
 
@@ -824,7 +861,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (sl.submitted) return SGPU_E_STATE;
     if (want & ~allowed_wants(sl.kind)) return SGPU_E_INVAL;
     CU(cudaSetDevice(ctx->device));
-    const bool live = sl.kind == Input::LIVE;
+    const bool live = is_live(sl.kind);
     int rc = live ? check_live_entries(ctx, sl) : SGPU_OK;
     if (rc) return rc;
     const sgpu_batch_t& hb = sl.batch;
@@ -835,7 +872,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
         CU(cudaMemcpyAsync(sl.d_comp_off, sl.h_comp_off, (size_t)nr * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(sl.d_comp_len, sl.h_comp_len, (size_t)nr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     } else {
-        const size_t sample_size = sl.kind == Input::PA ? sizeof(float) : sizeof(int16_t);
+        const size_t sample_size = sl.kind == Input::PA || sl.kind == Input::LIVE_PA ? sizeof(float) : sizeof(int16_t);
         CU(cudaMemcpyAsync(sl.d_samples, hb.samples, (size_t)sl.used * sample_size, cudaMemcpyHostToDevice, st));
     }
     CU(cudaMemcpyAsync(sl.d_read_off, hb.read_off, ((size_t)nr + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
@@ -868,7 +905,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
 int sgpu_wait(sgpu_ctx_t* ctx, uint32_t slot, sgpu_result_t* out) {
     if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!sl.submitted || sl.kind == Input::LIVE) return SGPU_E_STATE;
+    if (!sl.submitted || is_live(sl.kind)) return SGPU_E_STATE;
     return wait_slot(ctx, sl, OUTS, sl.dout, sl.hout, ctx->ev_cap, out);
 }
 
@@ -993,6 +1030,7 @@ int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
     CU(w.chan.ensure(n_channels));
     CU(w.nopen.ensure(n_channels));
     CU(w.claim.ensure(n_channels));
+    CU(w.form.ensure(n_channels));
     CU(w.cnt.ensure(ctx->max_reads));
     CU(w.s_start.ensure(w.ev_cap));
     CU(w.s_len.ensure(w.ev_cap));
@@ -1000,8 +1038,10 @@ int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
     CU(w.s_stdv.ensure(w.ev_cap));
     CU(cudaMemset(w.nopen, 0, (size_t)n_channels * sizeof(uint32_t)));
     CU(cudaMemset(w.claim, 0, (size_t)n_channels * sizeof(uint32_t)));
+    CU(cudaMemset(w.form, LIVE_FORM_INT16, (size_t)n_channels * sizeof(uint8_t)));
     ctx->live_mirror.reset(new (std::nothrow) uint32_t[n_channels]());
-    if (!ctx->live_mirror) return SGPU_E_NOMEM;
+    ctx->live_form.reset(new (std::nothrow) uint8_t[n_channels]());
+    if (!ctx->live_mirror || !ctx->live_form) return SGPU_E_NOMEM;
     for (uint32_t s = 0; s < ctx->n_slots; s++) {
         Slot& sl = ctx->slots[s];
         CU(sl.h_channel.ensure(ctx->max_reads));
@@ -1021,30 +1061,25 @@ int64_t sgpu_slot_add_live(sgpu_ctx_t* ctx, uint32_t slot, uint32_t channel, uin
                            uint64_t n, double digitisation, double offset, double range) {
     if (!ctx || slot >= ctx->n_slots || (!raw && n)) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!accepts(sl, Input::LIVE) || !ctx->live.n_channels) return SGPU_E_STATE;
-    if (channel >= ctx->live.n_channels || (flags & ~LIVE_FLAGS)) return SGPU_E_INVAL;
-    if (const int rc = room_for(ctx, sl, n, 1ull << 31, ctx->max_samples)) return rc;
-    if (sl.kind != Input::LIVE) {  // the slot's first entry: a new generation of its channel marks
-        if (++ctx->live_gen == 0) {
-            for (uint32_t s = 0; s < ctx->n_slots; s++)
-                memset(ctx->slots[s].live_claim.get(), 0, (size_t)ctx->live.n_channels * sizeof(uint32_t));
-            ctx->live_gen = 1;
-        }
-        sl.live_gen = ctx->live_gen;
-    }
-    if (sl.live_claim[channel] == sl.live_gen) return SGPU_E_INVAL;  // one entry per channel and slot
-    sl.live_claim[channel] = sl.live_gen;
-    sl.kind = Input::LIVE;
+    if (const int rc = add_live_entry(ctx, sl, Input::LIVE, channel, flags, n, ctx->max_samples)) return rc;
     memcpy(sl.batch.samples + sl.used, raw, (size_t)n * sizeof(int16_t));
-    sl.h_channel[sl.batch.n_reads] = channel;
-    sl.h_flags[sl.batch.n_reads] = flags;
     return append_record(sl, n, digitisation, offset, range);
+}
+
+int64_t sgpu_slot_add_live_pa(sgpu_ctx_t* ctx, uint32_t slot, uint32_t channel, uint32_t flags, const float* pa,
+                              uint64_t n) {
+    if (!ctx || slot >= ctx->n_slots || (!pa && n)) return SGPU_E_INVAL;
+    Slot& sl = ctx->slots[slot];
+    // the slot's int16 sample buffers (pinned and device) hold the floats: max_samples / 2 of them
+    if (const int rc = add_live_entry(ctx, sl, Input::LIVE_PA, channel, flags, n, ctx->max_samples / 2)) return rc;
+    memcpy(reinterpret_cast<float*>(sl.batch.samples) + sl.used, pa, (size_t)n * sizeof(float));
+    return append_record(sl, n, 1.0, 0.0, 1.0);  // (offset_f 0, raw_unit_f 1: the values are pA already)
 }
 
 int sgpu_wait_live(sgpu_ctx_t* ctx, uint32_t slot, sgpu_live_result_t* out) {
     if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
-    if (!sl.submitted || sl.kind != Input::LIVE) return SGPU_E_STATE;
+    if (!sl.submitted || !is_live(sl.kind)) return SGPU_E_STATE;
     return wait_slot(ctx, sl, LIVE_OUTS, sl.live_dout, sl.live_hout, ctx->live.ev_cap, out);
 }
 
@@ -1055,7 +1090,24 @@ int sgpu_run_device_live(sgpu_ctx_t* ctx, const sgpu_dev_live_batch_t* batch, vo
     CU(alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, ctx->live_dev_out, 0));
     const LiveBatch b{batch->samples, batch->read_off, batch->read_len, batch->channel, batch->flags, batch->offset_f,
                       batch->raw_unit_f, batch->n_entries, batch->span};
-    const int rc = run_pipeline_live(ctx, b, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline_live(ctx, b, false, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
+    if (rc) return rc;
+    ctx->live_mirror_stale = true;
+    memset(out, 0, sizeof *out);
+    fill_result(LIVE_OUTS, out, ctx->live_dev_out, SGPU_WANT_EVENTS, false);
+    return SGPU_OK;
+}
+
+int sgpu_run_device_live_pa(sgpu_ctx_t* ctx, const sgpu_dev_live_pa_batch_t* batch, void* stream,
+                            sgpu_live_result_t* out) {
+    if (!ctx || !batch || !out) return SGPU_E_INVAL;
+    if (!ctx->live.n_channels) return SGPU_E_STATE;
+    CU(cudaSetDevice(ctx->device));
+    CU(alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, ctx->live_dev_out, 0));
+    LiveBatch b{nullptr, batch->read_off, batch->read_len, batch->channel, batch->flags, nullptr, nullptr,
+                batch->n_entries, batch->span};
+    b.pa = batch->pa;
+    const int rc = run_pipeline_live(ctx, b, true, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     ctx->live_mirror_stale = true;
     memset(out, 0, sizeof *out);

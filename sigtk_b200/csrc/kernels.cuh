@@ -169,6 +169,8 @@ int launch_svbzd_decode(const SvbBatch& s, SvbScratch& w, Scratch& sc, int16_t* 
 constexpr uint32_t LIVE_FLAGS = 7u;        // SGPU_LIVE_START | SGPU_LIVE_END | SGPU_LIVE_RNA
 constexpr uint32_t LIVE_OPEN = 1u << 31;   // LiveScratch::nopen: samples so far | LIVE_OPEN while a read is open
 constexpr int LIVE_TAIL = 28;              // prefix sums a channel carries: 2 * w2 of the RNA parameters
+// LiveScratch::form: the form of the entry that started a channel's read (sgpu_slot_add_live or sgpu_slot_add_live_pa)
+constexpr uint8_t LIVE_FORM_INT16 = 0, LIVE_FORM_PA = 1;
 // What a channel carries from one entry to the next (in HBM; its length and open flag are in LiveScratch::nopen).
 struct LiveChan {
     double tS[LIVE_TAIL], tQ[LIVE_TAIL];  // S[j], Q[j] for j = n-LIVE_TAIL+1 .. n (0 for j <= 0)
@@ -179,8 +181,11 @@ struct LiveChan {
     float offset, unit;                   // the read's calibration (misc.c:17-19,26)
     uint32_t rna;
 };
-struct LiveBatch {                         // entry e: samples[read_off[e] .. +read_len[e]) of channel[e]
-    const int16_t* samples;
+struct LiveBatch {                         // entry e: samples (or pa)[read_off[e] .. +read_len[e]) of channel[e]
+    union {
+        const int16_t* samples;            // int16 entries, with offset and unit
+        const float* pa;                   // pA entries (launch_live's pa): offset and unit are not read
+    };
     const uint64_t* read_off;              // [n_entries+1]
     const uint32_t* read_len;
     const uint32_t* channel;
@@ -200,6 +205,7 @@ struct LiveScratch {                       // allocated by sgpu_live_open
     DevBuf<LiveChan> chan;                 // [n_channels]
     DevBuf<uint32_t> nopen;                // [n_channels]
     DevBuf<uint32_t> claim;                // [n_channels] stamp of the last run that had an entry for the channel
+    DevBuf<uint8_t> form;                  // [n_channels] LIVE_FORM_* of the open read (written at START)
     DevBuf<uint32_t> cnt;                  // [max_reads] events of every entry
     DevBuf<uint32_t> s_start, s_len;       // [ev_cap] staged events
     DevBuf<float> s_mean, s_stdv;
@@ -207,9 +213,10 @@ struct LiveScratch {                       // allocated by sgpu_live_open
     uint64_t ev_cap = 0;
     uint32_t stamp = 0;
 };
-// the events of entry e go to ev_start, ev_len, ev_mean, ev_stdv [ev_off[e], ev_off[e+1]) (ev_off: [n_entries+1])
-int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start, uint32_t* ev_len,
-                float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
+// the events of entry e go to ev_start, ev_len, ev_mean, ev_stdv [ev_off[e], ev_off[e+1]) (ev_off: [n_entries+1]);
+// pa: the entries are b.pa floats
+int launch_live(const LiveBatch& b, bool pa, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start,
+                uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
 
 // stat.cu
 constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;

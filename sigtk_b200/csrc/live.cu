@@ -8,12 +8,17 @@
 // (events.c:328-338). A peak can be emitted long after its position, so the channel keeps the prefix sums at each
 // detector's peak and at the open event's start. Every emitted peak p closes the event [a, p) (events.c:475-504).
 //
-//   live_kernel          one warp per entry, tiles of LIVE_TILE samples: pA by all lanes, the S/Q chain by lane 0
+//   live_kernel<PA>      one warp per entry, tiles of LIVE_TILE samples: pA by all lanes (misc.c:28 on int16 samples,
+//                        or the caller's floats as they are), the S/Q chain by lane 0
 //                        (the lane-0 chain of gen_prefix_reads), the t-statistics of the positions that became final
 //                        one lane per position (tstat_reference_chain), the detector by lane 0 (det_step), events
 //                        staged at live_stage_base of the entry
 //   scan_counts_kernel   events per entry -> ev_off (launch_scan_u32)
 //   live_compact_kernel  staged events -> the compact event table
+//
+// The S/Q chain is formed one sample after another in the reference's order whatever the input, so pA entries need no
+// exactness witness (pa_input.cu): the floats go through the same chain as the pA of int16 samples. A read keeps the
+// form of the entry that started it (LiveScratch::form); an entry of the other form that continues it is refused.
 #include "../../include/sigtk_b200.h"
 #include "kernels.cuh"
 
@@ -38,11 +43,14 @@ __device__ __forceinline__ float live_tstat(const double* S, const double* Q, in
                                  __dsub_rn(Q[ki + w], q_i), (float)w);
 }
 
+// PA: the entries are the caller's pA floats (b.pa), else int16 samples with the calibration given at START
+template <bool PA>
 __global__ void __launch_bounds__(LIVE_WARPS * 32)
 live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nopen, uint32_t* __restrict__ claim,
             uint32_t n_channels, uint32_t stamp, float thr_long, uint32_t* __restrict__ cnt,
             uint32_t* __restrict__ s_start, uint32_t* __restrict__ s_len, float* __restrict__ s_mean,
-            float* __restrict__ s_stdv, uint64_t ev_cap, int* __restrict__ status) {
+            float* __restrict__ s_stdv, uint64_t ev_cap, int* __restrict__ status, uint8_t* __restrict__ form) {
+    constexpr uint8_t my_form = PA ? LIVE_FORM_PA : LIVE_FORM_INT16;
     __shared__ LiveWarpSmem smem[LIVE_WARPS];
     LiveWarpSmem& sm = smem[threadIdx.x >> 5];
     const int lane = threadIdx.x & 31;
@@ -63,6 +71,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
             else {
                 no = nopen[c];
                 if (!start && !(no & LIVE_OPEN) && (len || end)) code = SGPU_DEV_E_STATE;
+                else if (!start && (no & LIVE_OPEN) && form[c] != my_form) code = SGPU_DEV_E_STATE;  // the other form
                 else if ((start ? 0ull : (uint64_t)(no & ~LIVE_OPEN)) + len > 0x7fffffffull) code = SGPU_DEV_E_TOOBIG;
             }
             if (code) atomicExch(status, code);
@@ -75,7 +84,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
         }
         LiveChan& ch = chan[c];
         const uint32_t rna = start ? ((f & SGPU_LIVE_RNA) ? 1u : 0u) : ch.rna;
-        const float offv = start ? b.offset[e] : ch.offset, unitv = start ? b.unit[e] : ch.unit;
+        const float offv = PA ? 0.0f : (start ? b.offset[e] : ch.offset), unitv = PA ? 1.0f : (start ? b.unit[e] : ch.unit);
         const DetParams p = det_params((int)rna);
         const uint32_t w1 = (uint32_t)p.w1, w2 = (uint32_t)p.w2;
         uint64_t n_cur = start ? 0 : (no & ~LIVE_OPEN);
@@ -111,7 +120,10 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
         uint32_t t0 = 0;
         do {
             const uint32_t m = min((uint32_t)LIVE_TILE, len - t0);
-            for (uint32_t k = lane; k < m; k += 32) sm.pa[k] = pa_of(b.samples[off + t0 + k], offv, unitv);
+            if constexpr (PA)
+                for (uint32_t k = lane; k < m; k += 32) sm.pa[k] = b.pa[off + t0 + k];
+            else
+                for (uint32_t k = lane; k < m; k += 32) sm.pa[k] = pa_of(b.samples[off + t0 + k], offv, unitv);
             __syncwarp();
             if (lane == 0) {  // events.c:293-303: the order of the additions is the result
                 double s = sm.S[LIVE_TAIL - 1], q = sm.Q[LIVE_TAIL - 1];
@@ -171,6 +183,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
                 ch.aS = aS; ch.aQ = aQ; ch.a = a;
                 ch.offset = offv; ch.unit = unitv; ch.rna = rna;
                 nopen[c] = (uint32_t)n_cur | LIVE_OPEN;
+                if (start) form[c] = my_form;
             }
         }
         if (lane == 0) cnt[e] = n_ev;
@@ -200,12 +213,13 @@ __global__ void __launch_bounds__(256) live_compact_kernel(LiveBatch b, const ui
     }
 }
 
-int launch_live(const LiveBatch& b, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start, uint32_t* ev_len,
-                float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st) {
+int launch_live(const LiveBatch& b, bool pa, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start,
+                uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st) {
     if (++w.stamp == 0) w.stamp = 1;  // (claim[] starts at 0)
-    live_kernel<<<grid_cap(b.n_entries, LIVE_WARPS, sm_count * 8), LIVE_WARPS * 32, 0, st>>>(
+    auto* const kernel = pa ? live_kernel<true> : live_kernel<false>;
+    kernel<<<grid_cap(b.n_entries, LIVE_WARPS, sm_count * 8), LIVE_WARPS * 32, 0, st>>>(
         b, w.chan, w.nopen, w.claim, w.n_channels, w.stamp, sc.tune_thr_long, w.cnt, w.s_start, w.s_len, w.s_mean,
-        w.s_stdv, w.ev_cap, sc.status);
+        w.s_stdv, w.ev_cap, sc.status, w.form);
     int n = 1 + launch_scan_u32(w.cnt, b.n_entries, ev_off, reinterpret_cast<uint64_t*>(sc.counters.get()), sc, st);
     live_compact_kernel<<<grid_cap(b.n_entries, 8, sm_count * 8), 256, 0, st>>>(
         b, w.cnt, ev_off, w.s_start, w.s_len, w.s_mean, w.s_stdv, ev_start, ev_len, ev_mean, ev_stdv);
