@@ -233,10 +233,12 @@ int  sgpu_decode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_svb_dev_batch_t *batch
  *     SGPU_E_STATE like the other violations below. A START entry of either form discards an open read of either form.
  *   - pA of every int16 sample is misc.c:28 with the calibration given at START (offset_f = (float)offset, raw_unit_f =
  *     (float)range / (float)digitisation, as sgpu_slot_add_read computes them); the DNA or RNA parameters also come
- *     from START (SGPU_LIVE_RNA, ignored without START). The long threshold follows SGPU_PARAM_THR_LONG.
+ *     from START (SGPU_LIVE_RNA, ignored without START). The long threshold follows SGPU_PARAM_THR_LONG. With a
+ *     detector set (sgpu_set_detector) the read runs the set in force for its START entry instead.
  *   - When events are reported: let a read hold n samples after an entry that does not end it. The detector has then
- *     been stepped, in the reference's order (short, then long; events.c:385-437), over every position i <= n - w2:
- *     the positions whose t-statistics can no longer change (their right window [i, i+w2) is complete). Every peak
+ *     been stepped, in the reference's order (short, then long; events.c:385-437), over every position
+ *     i <= n - max(w1, w2) (n - w2 for the reference's sets): the positions whose t-statistics can no longer change
+ *     (both right windows [i, i+w) are complete). Every peak
  *     emitted during those steps closes one event [a, p), and the entry reports those events. END steps the remaining
  *     positions (their long t-statistic is 0, events.c:328-338) and reports the last event [a, n). A read with no peak
  *     ends with the single event [0, n); a read of 0 samples reports no event. A peak may be emitted long after its
@@ -342,6 +344,38 @@ int  sgpu_counters(sgpu_ctx_t *ctx, sgpu_counters_t *out);
 #define SGPU_PARAM_STAT_CTA_MIN 5 /* stat / jnn moments: reads of at least this many samples are added up by a CTA
                                   (several warps per read), shorter ones by one warp; 0 = every read by a CTA */
 int  sgpu_set_param(sgpu_ctx_t *ctx, int key, double value);
+
+/* ---- the caller's own detector parameters -------------------------------------------------------------------
+ * The reference's detector takes a detector_param (events.c:35-41); getevents uses one of two constant sets chosen by
+ * rna (events.c:43-54: DNA {3, 6, 1.4, 9.0, 0.2}, RNA {7, 14, 2.5, 9.0, 1.0}). sgpu_set_detector makes every event
+ * detection of the context use the caller's set instead, as short_long_peak_detector(..., &set) would:
+ *   - Scope: int16 records, svb-zd streams and pA records, on host slots and in device-resident runs, and live
+ *     entries of both forms. rna and SGPU_LIVE_RNA then no longer choose the event parameters (they still choose those
+ *     of SGPU_WANT_JNN and SGPU_WANT_PREFIX), and SGPU_PARAM_THR_LONG is ignored. The other products of a batch (PA,
+ *     STAT, ENT, JNN, PREFIX) do not depend on it.
+ *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
+ *     different sets); a device-resident run the set in force when it is called; a live read the set in force for its
+ *     START entry, until its END, whatever is set in between (like the form of its START entry).
+ *   - Results: for every finite input the events are bit-identical to the reference's getevents with short_long_peak_
+ *     detector called with the set (the event table of the detector's peaks, events.c:457-504); with NaN or Inf in pA
+ *     input the boundaries are identical and the NaN statistics are NaN in the same places. Batches with a set run on
+ *     the route of pA records whatever their input (seq_order and fixups have the meaning given at
+ *     sgpu_run_device_pa; no long-detector job runs), so a set equal to a reference set gives the default path's events
+ *     bit for bit on another route. The batch event capacity (max_samples / 3 + 2 max_reads + 16) is not proved for
+ *     every set: a batch that exceeds it returns SGPU_E_EVCAP, never a truncated table. Live runs cannot exceed theirs:
+ *     the first live run under a set whose detectors may emit more often than the DNA set's grows the live staging
+ *     and event outputs by a quarter, which allocates and synchronises the device once.
+ *   - Live finality: after an entry that does not end its read (n samples so far), the positions stepped are
+ *     i <= n - max(w_short, w_long) (for the reference sets, w_long > w_short: i <= n - w_long).
+ * NULL restores the reference's sets (chosen by rna). Returns SGPU_E_INVAL, leaving the setting as it was, for a window
+ * outside [2, 14] (a window below 2 has no t-statistic, events.c:328-330; 14 is the reference's largest) or a threshold
+ * or peak_height that is not finite. w_short > w_long is allowed, as in the reference. */
+typedef struct {                  /* detector_param, events.c:35-41 */
+    uint32_t w_short, w_long;     /* window_length1, window_length2 */
+    float    thr_short, thr_long; /* threshold1, threshold2 */
+    float    peak_height;
+} sgpu_detector_t;
+int  sgpu_set_detector(sgpu_ctx_t *ctx, const sgpu_detector_t *p);
 
 /* Device time of every kernel group of the last run, measured with CUDA events on the stream the kernels were
  * launched on (needs SGPU_F_STAGE_TIMERS). Returns the number of entries written, or a negative code. */

@@ -27,7 +27,7 @@ EXPORTS = (
     "sgpu_wait", "sgpu_run_device", "sgpu_counters", "sgpu_memcpy_d2h", "sgpu_stage_times",
     "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
     "sgpu_run_device_pa", "sgpu_live_open", "sgpu_slot_add_live", "sgpu_wait_live", "sgpu_run_device_live",
-    "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa",
+    "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa", "sgpu_set_detector",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -105,6 +105,11 @@ class Counters(C.Structure):  # sgpu_counters_t
     ]
 
 
+class DetectorParams(C.Structure):  # sgpu_detector_t (detector_param, events.c:35-41)
+    _fields_ = [("w_short", C.c_uint32), ("w_long", C.c_uint32), ("thr_short", C.c_float), ("thr_long", C.c_float),
+                ("peak_height", C.c_float)]
+
+
 class StageTime(C.Structure):  # sgpu_stage_time_t
     _fields_ = [("name", C.c_char_p), ("ms", C.c_float), ("launches", C.c_uint32)]
 
@@ -173,5 +178,7 @@ def load() -> C.CDLL:
     lib.sgpu_run_device_live_pa.restype = i32
     lib.sgpu_set_param.argtypes = [vp, i32, C.c_double]
     lib.sgpu_set_param.restype = i32
+    lib.sgpu_set_detector.argtypes = [vp, C.POINTER(DetectorParams)]
+    lib.sgpu_set_detector.restype = i32
     _lib = lib
     return lib

@@ -13,7 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import List, Optional, Sequence, Tuple
+from typing import List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -25,6 +25,16 @@ Read = Tuple[np.ndarray, float, float, float]  # raw int16, digitisation, offset
 LiveEntry = Tuple[int, int, np.ndarray, float, float, float]  # channel, LIVE_* flags, raw int16, digitisation, offset,
                                                               # range (the calibration is read with LIVE_START only)
 LivePaEntry = Tuple[int, int, np.ndarray]  # channel, LIVE_* flags, pA float32
+
+
+class Detector(NamedTuple):
+    """detector_param (events.c:35-41): the reference's DNA set is Detector(3, 6, 1.4, 9.0, 0.2), its RNA set
+    Detector(7, 14, 2.5, 9.0, 1.0)"""
+    w_short: int        # window_length1, in [2, 14]
+    w_long: int         # window_length2, in [2, 14]
+    thr_short: float    # threshold1
+    thr_long: float     # threshold2
+    peak_height: float
 
 
 @dataclass
@@ -310,6 +320,15 @@ class Context:
         return {"n_events": int(c.n_events), "n_seq_order_reads": int(c.n_seq_order_reads),
                 "n_fixups": int(c.n_fixups), "n_kernel_launches": int(c.n_kernel_launches), "status": int(c.status),
                 "n_long_jobs": int(c.n_long_jobs)}
+
+    def set_detector(self, det: Optional[Detector]) -> None:
+        """sgpu_set_detector: every later event detection of the context (batches, device-resident runs, live reads
+        started from now on) uses `det`; None restores the reference's sets, chosen by rna"""
+        if det is None:
+            self._check(self._lib.sgpu_set_detector(self._h, None))
+            return
+        p = _lib.DetectorParams(int(det[0]), int(det[1]), float(det[2]), float(det[3]), float(det[4]))
+        self._check(self._lib.sgpu_set_detector(self._h, C.byref(p)))
 
     def set_param(self, key: int, value: float) -> None:
         """development / test parameters (_lib.PARAM_*): chunk length, detector warm-up, the long detector's threshold"""

@@ -6,6 +6,7 @@
 // kernels themselves are serialised (they share one scratch area).
 #include "../../include/sigtk_b200.h"
 
+#include <cmath>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
@@ -138,6 +139,8 @@ struct Slot {
     cudaEvent_t in_ready = nullptr, kernels_done = nullptr, small_back = nullptr;
     bool submitted = false;
     uint32_t want = 0;
+    const DetParams* det = nullptr;  // the context's detector set at sgpu_submit (&det_set), or nullptr: the reference's
+    DetParams det_set{};
     Input kind = Input::NONE;        // (PA, LIVE_PA: the floats are in the sample buffers, max_samples / 2 of them)
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
@@ -149,6 +152,7 @@ struct Slot {
     PinBuf<uint32_t> h_channel, h_flags; DevBuf<uint32_t> d_channel, d_flags;
     DevBuf<void> live_dout[N_LIVE_OUT];
     PinBuf<void> live_hout[N_LIVE_OUT];
+    uint64_t live_dcap = 0, live_hcap = 0;   // the event capacity they were allocated for
     std::unique_ptr<uint32_t[]> live_claim;  // [n_channels] live_gen of the batch that holds an entry for the channel
     uint32_t live_gen = 0;
 
@@ -176,10 +180,13 @@ struct sgpu_ctx {
     SvbScratch svb{};            // workspace of the svb-zd decoder (allocated on first use)
     DevBuf<float> jnn_mom;       // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
     int pore_rna004 = 0;         // SGPU_PARAM_PORE: jnnv2 parameters of `prefix` (misc.c:74-101 picks them from the header)
+    bool det_on = false;         // sgpu_set_detector: every event detection uses `det` instead of the reference's sets
+    DetParams det{};
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
     DevBuf<void> live_dev_out[N_LIVE_OUT];    // outputs of sgpu_run_device_live
+    uint64_t live_dev_cap = 0;
     std::unique_ptr<uint32_t[]> live_mirror;  // [n_channels] nopen of every channel after the submitted live slots
     std::unique_ptr<uint8_t[]> live_form;     // [n_channels] and the form of its open read (LiveScratch::form)
     bool live_mirror_stale = false;           // a device-resident live run changed channels since
@@ -320,22 +327,103 @@ bool fits(const sgpu_ctx* ctx, const DevBatch& b) {  // a batch of int16 or pA r
     return b.n_reads <= ctx->max_reads && b.span <= ctx->max_samples && !(b.span & (SGPU_ALIGN - 1));
 }
 
-// The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies.
+int alloc_pa_scratch(sgpu_ctx* ctx) {
+    PaScratch& w = ctx->pa;
+    w.max_tiles = pa_tile_capacity(ctx->max_samples, ctx->max_reads);
+    CU(w.tile_cnt.ensure(ctx->max_reads));
+    CU(w.tile_base.ensure((uint64_t)ctx->max_reads + 1));
+    CU(w.tS.ensure(w.max_tiles));
+    CU(w.tQ.ensure(w.max_tiles));
+    CU(w.tA.ensure(w.max_tiles));
+    CU(w.tB.ensure(w.max_tiles));
+    CU(w.tmin.ensure(w.max_tiles));
+    CU(w.ord_list.ensure(ctx->max_reads));
+    CU(w.ord_sbase.ensure(ctx->max_reads));
+    CU(w.ord_count.ensure(1));
+    return SGPU_OK;
+}
+
+// The general route keeps its prefix sums and t-statistics at the reads' own offsets, so the sequential-order scratch
+// must hold the whole span. Contexts over 64 Mi samples start with an eighth of that (sgpu_create); the first batch on
+// the general route (pA records, or a batch with a detector set) that needs more grows it to max_samples for the rest
+// of the context's life (later int16 batches use it too). The old arrays are freed only once the new ones exist
+// (freeing waits for the device).
+int grow_seq_scratch(sgpu_ctx* ctx) {
+    Scratch& sc = ctx->sc;
+    const uint64_t n = ctx->max_samples;
+    DevBuf<double> S, Q;
+    DevBuf<float> t1, t2;
+    cudaError_t e = S.ensure(n);
+    if (e == cudaSuccess) e = Q.ensure(n);
+    if (e == cudaSuccess) e = t1.ensure(n);
+    if (e == cudaSuccess) e = t2.ensure(n);
+    if (e != cudaSuccess) {  // (the buffers that were allocated free themselves)
+        cudaGetLastError();  // (an allocation failure is reported here, not by the next launch check)
+        snprintf(ctx->err, sizeof ctx->err, "growing the sequential-order scratch to %llu samples: %s",
+                 (unsigned long long)n, cudaGetErrorString(e));
+        return SGPU_E_NOMEM;
+    }
+    sc.Sinc = std::move(S); sc.Qinc = std::move(Q); sc.t1 = std::move(t1); sc.t2 = std::move(t2);
+    sc.gen_cap = n;
+    return SGPU_OK;
+}
+
+// The general route's workspace for a batch of `span` samples: the tile arrays of pa_input.cu, and a sequential-order
+// scratch that holds the whole span.
+int prepare_general(sgpu_ctx* ctx, uint64_t span) {
+    int rc = alloc_pa_scratch(ctx);
+    if (!rc && span > ctx->sc.gen_cap) rc = grow_seq_scratch(ctx);
+    return rc;
+}
+
+// The events of a batch on the general route into the device outputs `o`: the prefix sums by the witness-checked scan
+// or in the reference's order (pa_input.cu), then the sequential-order kernels for every read. pa: the caller's
+// floats, or nullptr: b's int16 samples through their calibration; set: the caller's detector set, or nullptr: the
+// reference's chosen by b.rna. (prepare_general first.)
+int general_events(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetParams* set, DevBuf<void>* o,
+                   StageMarks& marks) {
+    Scratch& sc = ctx->sc;
+    const cudaStream_t st = marks.st;
+    const uint32_t n_tiles = fast_tiles_for(b.span);
+    if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
+    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
+    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS].get());
+    CU(cudaMemsetAsync(sc.bitmap, 0, (size_t)n_tiles * (FAST_TILE / 32) * sizeof(uint32_t), st));
+    const int force = (ctx->flags & SGPU_F_FORCE_GENERIC) ? 1 : 0;
+    marks.done("pa_prefix", launch_pa_prefix(b, pa, ctx->pa, sc, seq, fix, force, ctx->sm_count, st));
+    const WorkList ordered{ctx->pa.ord_list, ctx->pa.ord_sbase, ctx->pa.ord_count};
+    const WorkList all{sc.seq_list, sc.seq_sbase, sc.seq_count};
+    marks.done("sequential_order_detect",
+               launch_generic_detect_pa(b, pa, set, ordered, all, sc, fix, ctx->sm_count, st));
+    uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF].get());
+    marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
+    marks.done("sequential_order_emit",
+               launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START].get()),
+                                   static_cast<float*>(o[EV_MEAN].get()), static_cast<float*>(o[EV_STDV].get()),
+                                   ctx->sm_count, st));
+    return SGPU_OK;
+}
+
+// The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies
+// (except when the general route's scratch grows). set: the caller's detector set, whose events take the general
+// route, or nullptr: the reference's sets on the fast path.
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
-                 const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
+                 const DetParams* set, const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
     if (!fits(ctx, b)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
+    const bool events = (want & SGPU_WANT_EVENTS) != 0;
+    if (set && events)
+        if (const int rc = prepare_general(ctx, b.span)) return rc;
     StageMarks marks(ctx, st);
     if (const int rc = marks.start()) return rc;
     if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
     if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
-    const bool events = (want & SGPU_WANT_EVENTS) != 0;
     float* const pa = (want & SGPU_WANT_PA) ? static_cast<float*>(o[PA].get()) : nullptr;
     uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
     uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS].get());
-    if (pa && (!events || force_generic))  // with events on the fast path the pA store is fused into walk_chunks_kernel
+    if (pa && (!events || force_generic || set))  // with events on the fast path the pA store is fused into walk_chunks_kernel
         marks.done("pa", launch_pa(b, pa, ctx->sm_count, st));
     if (want & SGPU_WANT_STAT) {
         float* const stat = static_cast<float*>(o[STAT].get());
@@ -359,7 +447,9 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
     if (want & SGPU_WANT_PREFIX)
         marks.done("prefix", launch_prefix(b, ctx->pore_rna004, static_cast<int32_t*>(o[PREFIX_POS].get()),
                                            static_cast<float*>(o[PREFIX_STAT].get()), ctx->sm_count, st));
-    if (events) {
+    if (events && set) {
+        if (const int rc = general_events(ctx, b, nullptr, set, o, marks)) return rc;
+    } else if (events) {
         const uint32_t n_tiles = fast_tiles_for(b.span);
         if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
         int n = launch_init_reads(b, sc, seq, fix, ctx->sm_count, st);
@@ -389,82 +479,26 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
     return marks.finish();
 }
 
-int alloc_pa_scratch(sgpu_ctx* ctx) {
-    PaScratch& w = ctx->pa;
-    w.max_tiles = pa_tile_capacity(ctx->max_samples, ctx->max_reads);
-    CU(w.tile_cnt.ensure(ctx->max_reads));
-    CU(w.tile_base.ensure((uint64_t)ctx->max_reads + 1));
-    CU(w.tS.ensure(w.max_tiles));
-    CU(w.tQ.ensure(w.max_tiles));
-    CU(w.tA.ensure(w.max_tiles));
-    CU(w.tB.ensure(w.max_tiles));
-    CU(w.tmin.ensure(w.max_tiles));
-    CU(w.ord_list.ensure(ctx->max_reads));
-    CU(w.ord_sbase.ensure(ctx->max_reads));
-    CU(w.ord_count.ensure(1));
-    return SGPU_OK;
-}
-
-// A pA batch keeps its prefix sums and t-statistics at the reads' own offsets, so the sequential-order scratch must
-// hold the whole span. Contexts over 64 Mi samples start with an eighth of that (sgpu_create); the first pA batch that
-// needs more grows it to max_samples for the rest of the context's life (later int16 batches use it too). The old
-// arrays are freed only once the new ones exist (freeing waits for the device).
-int grow_seq_scratch(sgpu_ctx* ctx) {
-    Scratch& sc = ctx->sc;
-    const uint64_t n = ctx->max_samples;
-    DevBuf<double> S, Q;
-    DevBuf<float> t1, t2;
-    cudaError_t e = S.ensure(n);
-    if (e == cudaSuccess) e = Q.ensure(n);
-    if (e == cudaSuccess) e = t1.ensure(n);
-    if (e == cudaSuccess) e = t2.ensure(n);
-    if (e != cudaSuccess) {  // (the buffers that were allocated free themselves)
-        cudaGetLastError();  // (an allocation failure is reported here, not by the next launch check)
-        snprintf(ctx->err, sizeof ctx->err, "growing the sequential-order scratch to %llu samples: %s",
-                 (unsigned long long)n, cudaGetErrorString(e));
-        return SGPU_E_NOMEM;
-    }
-    sc.Sinc = std::move(S); sc.Qinc = std::move(Q); sc.t1 = std::move(t1); sc.t2 = std::move(t2);
-    sc.gen_cap = n;
-    return SGPU_OK;
-}
-
 // The kernel sequence of a batch of pA records (getevents(n, pa, rna), events.c:553-573) into the device outputs `o`:
-// the prefix sums by the witness-checked scan or in the reference's order (pa_input.cu), then the sequential-order
-// kernels for every read. No host synchronisation, no host<->device copies (except when the scratch grows).
-int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, uint32_t want, DevBuf<void>* o,
-                    cudaStream_t st) {
-    Scratch& sc = ctx->sc;
+// the general route (set: the caller's detector set, or nullptr: the reference's chosen by b.rna). No host
+// synchronisation, no host<->device copies (except when the scratch grows).
+int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetParams* set, uint32_t want,
+                    DevBuf<void>* o, cudaStream_t st) {
     if (!fits(ctx, b) || (b.n_reads && b.span && !pa)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
-    int rc = alloc_pa_scratch(ctx);
-    if (!rc && b.span > sc.gen_cap) rc = grow_seq_scratch(ctx);
+    int rc = prepare_general(ctx, b.span);
     if (rc) return rc;
     StageMarks marks(ctx, st);
     if ((rc = marks.start())) return rc;
     if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
-    const uint32_t n_tiles = fast_tiles_for(b.span);
-    if (n_tiles > sc.max_tiles) return SGPU_E_INVAL;
-    uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
-    uint32_t* const fix = static_cast<uint32_t*>(o[FIXUPS].get());
-    CU(cudaMemsetAsync(sc.bitmap, 0, (size_t)n_tiles * (FAST_TILE / 32) * sizeof(uint32_t), st));
-    const int force = (ctx->flags & SGPU_F_FORCE_GENERIC) ? 1 : 0;
-    marks.done("pa_prefix", launch_pa_prefix(b, pa, ctx->pa, sc, seq, fix, force, ctx->sm_count, st));
-    const WorkList ordered{ctx->pa.ord_list, ctx->pa.ord_sbase, ctx->pa.ord_count};
-    const WorkList all{sc.seq_list, sc.seq_sbase, sc.seq_count};
-    marks.done("sequential_order_detect", launch_generic_detect_pa(b, pa, ordered, all, sc, fix, ctx->sm_count, st));
-    uint64_t* const ev_off = static_cast<uint64_t*>(o[EV_OFF].get());
-    marks.done("rank_events", launch_rank_events(b, sc, ev_off, ctx->sm_count, st));
-    marks.done("sequential_order_emit",
-               launch_generic_emit(b, all, sc, ev_off, ctx->ev_cap, static_cast<uint32_t*>(o[EV_START].get()),
-                                   static_cast<float*>(o[EV_MEAN].get()), static_cast<float*>(o[EV_STDV].get()),
-                                   ctx->sm_count, st));
+    if ((rc = general_events(ctx, b, pa, set, o, marks))) return rc;
     return marks.finish();
 }
 
 // The kernels of a push of live entries into `o` (live.cu; pa: the entries are b.pa floats). No host synchronisation, no
 // host<->device copies.
-int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, bool pa, DevBuf<void>* o, cudaStream_t st) {
+int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, bool pa, const DetParams* set, DevBuf<void>* o,
+                      cudaStream_t st) {
     if (b.n_entries > ctx->max_reads || b.span > ctx->max_samples) return SGPU_E_INVAL;
     if (b.n_entries && (!b.samples || !b.read_off || !b.read_len || !b.channel || !b.flags ||
                         (!pa && (!b.offset || !b.unit))))
@@ -474,7 +508,7 @@ int run_pipeline_live(sgpu_ctx* ctx, const LiveBatch& b, bool pa, DevBuf<void>* 
     // (entries without samples still open and close channels: only a push of no entry is empty)
     if (b.n_entries == 0) return clear_empty_batch(LIVE_OUTS, 0, b.span, SGPU_WANT_EVENTS, o, marks);
     marks.done(pa ? "live_pa" : "live",
-               launch_live(b, pa, ctx->live, ctx->sc, static_cast<uint64_t*>(o[LIVE_EV_OFF].get()),
+               launch_live(b, pa, set, ctx->live, ctx->sc, static_cast<uint64_t*>(o[LIVE_EV_OFF].get()),
                            static_cast<uint32_t*>(o[LIVE_EV_START].get()), static_cast<uint32_t*>(o[LIVE_EV_LEN].get()),
                            static_cast<float*>(o[LIVE_EV_MEAN].get()), static_cast<float*>(o[LIVE_EV_STDV].get()),
                            ctx->sm_count, st));
@@ -488,16 +522,17 @@ int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
     if (is_live(sl.kind)) {  // (LIVE_PA: the union's pa is the same pointer, the floats in the sample buffers)
         const LiveBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_channel, sl.d_flags, sl.d_offset, sl.d_unit,
                           nr, sl.used};
-        return run_pipeline_live(ctx, b, sl.kind == Input::LIVE_PA, sl.live_dout, ctx->compute);
+        return run_pipeline_live(ctx, b, sl.kind == Input::LIVE_PA, sl.det, sl.live_dout, ctx->compute);
     }
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.hout, want));
     if (sl.kind == Input::PA)
         return run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr, rna, sl.used},
-                               reinterpret_cast<const float*>(sl.d_samples.get()), want, sl.dout, ctx->compute);
+                               reinterpret_cast<const float*>(sl.d_samples.get()), sl.det, want, sl.dout, ctx->compute);
     const DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, rna, sl.used};
     const SvbBatch svb{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
                        sl.svb_blocks};
-    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.kind == Input::SVBZD ? &svb : nullptr, sl.d_samples);
+    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.kind == Input::SVBZD ? &svb : nullptr,
+                        sl.d_samples);
 }
 
 // a slot that is not submitted takes a record of kind k when it is empty or holds records of kind k
@@ -598,6 +633,43 @@ void advance_live_mirror(sgpu_ctx* ctx, const Slot& sl) {
         mirror[c] = (f & SGPU_LIVE_END) ? 0u : (uint32_t)((start ? 0u : (no & ~LIVE_OPEN)) + len) | LIVE_OPEN;
         if (start) ctx->live_form[c] = live_form_of(sl.kind);
     }
+}
+
+// A detector set whose two detectors may emit more often than the reference's DNA set (8 events per 15 steps) needs
+// the live staging of any set (live_stage_base, dense): a detector emits at most once per w/2 + 2 steps.
+bool live_set_is_dense(const DetParams* set) {
+    if (!set) return false;
+    const int g1 = set->w1 / 2 + 2, g2 = set->w2 / 2 + 2;
+    return 15 * (g1 + g2) > 8 * g1 * g2;
+}
+
+// The first live run under such a set grows the staging to the bound of any set for the rest of the context's life
+// (waiting for the device first: queued runs still use the old arrays); the event outputs follow (fit_live_outputs).
+int fit_live_staging(sgpu_ctx* ctx, const DetParams* set) {
+    LiveScratch& w = ctx->live;
+    if (w.dense || !live_set_is_dense(set)) return SGPU_OK;
+    const uint64_t cap = live_stage_base(ctx->max_samples, ctx->max_reads, true);
+    CU(cudaDeviceSynchronize());
+    DevBuf<uint32_t> st, ln;
+    DevBuf<float> mn, sd;
+    CU(st.ensure(cap));
+    CU(ln.ensure(cap));
+    CU(mn.ensure(cap));
+    CU(sd.ensure(cap));
+    w.s_start = std::move(st); w.s_len = std::move(ln); w.s_mean = std::move(mn); w.s_stdv = std::move(sd);
+    w.ev_cap = cap;
+    w.dense = true;
+    return SGPU_OK;
+}
+
+// (re)allocates the live outputs `o` at the context's live event capacity when they were made for another one
+template <bool PINNED>
+cudaError_t fit_live_outputs(const sgpu_ctx* ctx, Buf<void, PINNED> (&o)[N_LIVE_OUT], uint64_t& cap) {
+    if (cap == ctx->live.ev_cap) return cudaSuccess;
+    for (auto& buf : o) buf = Buf<void, PINNED>();
+    const cudaError_t e = alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, o, 0);
+    if (e == cudaSuccess) cap = ctx->live.ev_cap;
+    return e;
 }
 
 // sgpu_wait / sgpu_wait_live: the device status of the submitted slot, then its outputs `outs` (device d, pinned h)
@@ -864,6 +936,13 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     const bool live = is_live(sl.kind);
     int rc = live ? check_live_entries(ctx, sl) : SGPU_OK;
     if (rc) return rc;
+    sl.det_set = ctx->det;  // the slot runs the set in force now, whatever is set before it is waited for
+    sl.det = ctx->det_on ? &sl.det_set : nullptr;
+    if (live) {
+        if ((rc = fit_live_staging(ctx, sl.det))) return rc;
+        CU(fit_live_outputs(ctx, sl.live_dout, sl.live_dcap));
+        CU(fit_live_outputs(ctx, sl.live_hout, sl.live_hcap));
+    }
     const sgpu_batch_t& hb = sl.batch;
     const uint32_t nr = hb.n_reads;
     cudaStream_t st = sl.stream;
@@ -915,7 +994,8 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     CU(cudaSetDevice(ctx->device));
     DevBatch b{batch->samples, batch->read_off, batch->read_len, batch->offset_f, batch->raw_unit_f,
                batch->n_reads, (int)batch->rna, batch->span};
-    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream),
+                                ctx->det_on ? &ctx->det : nullptr);
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(OUTS, out, ctx->dev_out, want, true);
@@ -928,7 +1008,8 @@ int sgpu_run_device_pa(sgpu_ctx_t* ctx, const sgpu_dev_pa_batch_t* batch, uint32
     CU(cudaSetDevice(ctx->device));
     const DevBatch b{nullptr, batch->read_off, batch->read_len, nullptr, nullptr, batch->n_reads, (int)batch->rna,
                      batch->span};
-    const int rc = run_pipeline_pa(ctx, b, batch->pa, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline_pa(ctx, b, batch->pa, ctx->det_on ? &ctx->det : nullptr, want, ctx->dev_out,
+                                   reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(OUTS, out, ctx->dev_out, want, false);
@@ -996,6 +1077,17 @@ int sgpu_set_param(sgpu_ctx_t* ctx, int key, double value) {
     }
 }
 
+int sgpu_set_detector(sgpu_ctx_t* ctx, const sgpu_detector_t* p) {
+    if (!ctx) return SGPU_E_INVAL;
+    if (!p) { ctx->det_on = false; return SGPU_OK; }
+    const bool windows = p->w_short >= 2 && p->w_short <= 14 && p->w_long >= 2 && p->w_long <= 14;
+    if (!windows || !std::isfinite(p->thr_short) || !std::isfinite(p->thr_long) || !std::isfinite(p->peak_height))
+        return SGPU_E_INVAL;
+    ctx->det = DetParams{(int)p->w_short, (int)p->w_long, p->thr_short, p->thr_long, p->peak_height};
+    ctx->det_on = true;
+    return SGPU_OK;
+}
+
 int sgpu_stage_times(sgpu_ctx_t* ctx, sgpu_stage_time_t* out, uint32_t cap) {
     if (!ctx || (!out && cap)) return SGPU_E_INVAL;
     if (!(ctx->flags & SGPU_F_STAGE_TIMERS)) return SGPU_E_STATE;
@@ -1026,7 +1118,7 @@ int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
     LiveScratch& w = ctx->live;
     if (w.n_channels) return SGPU_E_STATE;
     CU(cudaSetDevice(ctx->device));
-    w.ev_cap = live_stage_base(ctx->max_samples, ctx->max_reads);
+    w.ev_cap = live_stage_base(ctx->max_samples, ctx->max_reads, w.dense);
     CU(w.chan.ensure(n_channels));
     CU(w.nopen.ensure(n_channels));
     CU(w.claim.ensure(n_channels));
@@ -1048,8 +1140,8 @@ int sgpu_live_open(sgpu_ctx_t* ctx, uint32_t n_channels) {
         CU(sl.h_flags.ensure(ctx->max_reads));
         CU(sl.d_channel.ensure(ctx->max_reads));
         CU(sl.d_flags.ensure(ctx->max_reads));
-        CU(alloc_outputs(LIVE_OUTS, ctx, w.ev_cap, sl.live_dout, 0));
-        CU(alloc_outputs(LIVE_OUTS, ctx, w.ev_cap, sl.live_hout, 0));
+        CU(fit_live_outputs(ctx, sl.live_dout, sl.live_dcap));
+        CU(fit_live_outputs(ctx, sl.live_hout, sl.live_hcap));
         sl.live_claim.reset(new (std::nothrow) uint32_t[n_channels]());
         if (!sl.live_claim) return SGPU_E_NOMEM;
     }
@@ -1087,10 +1179,12 @@ int sgpu_run_device_live(sgpu_ctx_t* ctx, const sgpu_dev_live_batch_t* batch, vo
     if (!ctx || !batch || !out) return SGPU_E_INVAL;
     if (!ctx->live.n_channels) return SGPU_E_STATE;
     CU(cudaSetDevice(ctx->device));
-    CU(alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, ctx->live_dev_out, 0));
+    const DetParams* const set = ctx->det_on ? &ctx->det : nullptr;
+    if (const int rc = fit_live_staging(ctx, set)) return rc;
+    CU(fit_live_outputs(ctx, ctx->live_dev_out, ctx->live_dev_cap));
     const LiveBatch b{batch->samples, batch->read_off, batch->read_len, batch->channel, batch->flags, batch->offset_f,
                       batch->raw_unit_f, batch->n_entries, batch->span};
-    const int rc = run_pipeline_live(ctx, b, false, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline_live(ctx, b, false, set, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     ctx->live_mirror_stale = true;
     memset(out, 0, sizeof *out);
@@ -1103,11 +1197,13 @@ int sgpu_run_device_live_pa(sgpu_ctx_t* ctx, const sgpu_dev_live_pa_batch_t* bat
     if (!ctx || !batch || !out) return SGPU_E_INVAL;
     if (!ctx->live.n_channels) return SGPU_E_STATE;
     CU(cudaSetDevice(ctx->device));
-    CU(alloc_outputs(LIVE_OUTS, ctx, ctx->live.ev_cap, ctx->live_dev_out, 0));
+    const DetParams* const set = ctx->det_on ? &ctx->det : nullptr;
+    if (const int rc = fit_live_staging(ctx, set)) return rc;
+    CU(fit_live_outputs(ctx, ctx->live_dev_out, ctx->live_dev_cap));
     LiveBatch b{nullptr, batch->read_off, batch->read_len, batch->channel, batch->flags, nullptr, nullptr,
                 batch->n_entries, batch->span};
     b.pa = batch->pa;
-    const int rc = run_pipeline_live(ctx, b, true, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_pipeline_live(ctx, b, true, set, ctx->live_dev_out, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     ctx->live_mirror_stale = true;
     memset(out, 0, sizeof *out);

@@ -13,7 +13,8 @@
 // They serve (a) reads that fail the exact-sum witness or the detector
 // boundary-state check of the fast path (fast.cu), (b) SGPU_F_FORCE_GENERIC,
 // (c) as the on-device cross-check of the fast path in the tests, and (d) batches of
-// the caller's own pA floats (pa_input.cu: gen_prefix_pa_kernel, gen_detect_pa_kernel).  The
+// the caller's own pA floats (pa_input.cu: gen_prefix_pa_kernel, gen_detect_pa_kernel), and (e) batches with a
+// caller's detector set (sgpu_set_detector: gen_detect_set_kernel, detect_set.cu).  The
 // work list is built on the device (build_seq_list_kernel), so every kernel
 // here is launched with a fixed grid and returns at once when the list is empty.  They keep S, Q (16 B/sample) and t1, t2 (8 B/sample) in
 // an HBM scratch area, so they are NOT the roofline path.
@@ -147,11 +148,11 @@ __device__ __forceinline__ float tstat_at(const double* __restrict__ Sinc, const
     return tstat_reference_chain(sum1, ssq1, sum2, ssq2, (float)w);
 }
 
+// p: the windows of the batch's detector (det_params(b.rna), or the caller's set: sgpu_set_detector)
 __global__ void __launch_bounds__(256) gen_tstat_kernel(DevBatch b, WorkList wl, const double* __restrict__ Sinc,
                                                         const double* __restrict__ Qinc, float* __restrict__ t1,
-                                                        float* __restrict__ t2) {
+                                                        float* __restrict__ t2, DetParams p) {
     const uint32_t n_list = *wl.count;
-    const DetParams p = det_params(b.rna);
     for (uint32_t j = blockIdx.x; j < n_list; j += gridDim.x) {  // one CTA walks one read
         const uint32_t r = wl.list[j];
         const uint64_t base = wl.sbase[j];
@@ -225,7 +226,6 @@ __device__ void detect_read_in_order(const DetParams& p, const float* __restrict
 // PA (t arrays of a caller's pA signal, which may hold NaN): returns the number of mismatched chunks, and a NaN
 // t-statistic anywhere in the read also sends it to the reference's order -- the branch-free step's fminf / fmaxf
 // would take the other operand where the reference's comparisons keep a NaN running value (events.c:393-409).
-constexpr int GD_CHUNK = 1024;
 template <int RNA, bool PA>
 __device__ uint32_t detect_read_chunked(const float* __restrict__ t1, const float* __restrict__ t2, uint64_t base,
                                         uint64_t foff, uint32_t n, uint32_t W, uint32_t* __restrict__ bitmap, int lane,
@@ -508,18 +508,22 @@ __global__ void __launch_bounds__(256) pa_kernel(DevBatch b, float* __restrict__
 // host-side launchers
 int launch_generic_detect(const DevBatch& b, const WorkList& wl, Scratch& sc, int sm_count, cudaStream_t st) {
     gen_prefix_kernel<<<sm_count * 8, 128, 0, st>>>(b, wl, sc.Sinc, sc.Qinc);
-    gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, wl, sc.Sinc, sc.Qinc, sc.t1, sc.t2);
+    gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, wl, sc.Sinc, sc.Qinc, sc.t1, sc.t2, det_params(b.rna));
     gen_detect_kernel<<<sm_count * 8, 128, 0, st>>>(b, wl, sc.t1, sc.t2, sc.bitmap, b.rna ? 384u : 64u);  // (its own warm-up, longer than the walker's)
     return 3;
 }
 
-// a pA batch (pa_input.cu): the prefix sums of the reads in `ordered` (those that failed the exact-sum witness) in
-// the reference's order -- the others' were stored by pa_scan_kernel --, then t-statistics and detector for all reads
-int launch_generic_detect_pa(const DevBatch& b, const float* pa, const WorkList& ordered, const WorkList& all,
-                             Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st) {
-    gen_prefix_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, pa, ordered, sc.Sinc, sc.Qinc);
-    gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, all, sc.Sinc, sc.Qinc, sc.t1, sc.t2);
-    gen_detect_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, all, sc.t1, sc.t2, sc.bitmap, b.rna ? 384u : 64u, fixups);
+// a batch on the general route (pa_input.cu): the prefix sums of the reads in `ordered` (those that failed the
+// exact-sum witness) in the reference's order -- the others' were stored by pa_scan_kernel --, then t-statistics and
+// detector for all reads (pa: the caller's floats, or nullptr: b's int16 samples; set: the caller's detector set, or
+// nullptr: the reference's chosen by b.rna)
+int launch_generic_detect_pa(const DevBatch& b, const float* pa, const DetParams* set, const WorkList& ordered,
+                             const WorkList& all, Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st) {
+    if (pa) gen_prefix_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, pa, ordered, sc.Sinc, sc.Qinc);
+    else    gen_prefix_kernel<<<sm_count * 8, 128, 0, st>>>(b, ordered, sc.Sinc, sc.Qinc);
+    gen_tstat_kernel<<<sm_count * 8, 256, 0, st>>>(b, all, sc.Sinc, sc.Qinc, sc.t1, sc.t2, set ? *set : det_params(b.rna));
+    if (set) launch_detect_set(b, all, sc, fixups, *set, sm_count, st);
+    else     gen_detect_pa_kernel<<<sm_count * 8, 128, 0, st>>>(b, all, sc.t1, sc.t2, sc.bitmap, b.rna ? 384u : 64u, fixups);
     return 3;
 }
 

@@ -100,11 +100,22 @@ struct Scratch {
 };
 
 // generic.cu (sequential-order kernels)
+constexpr int GD_CHUNK = 1024;  // positions per chunk of the warp-chunked detectors
+__device__ void clear_read_bits(uint32_t* __restrict__ bitmap, uint64_t p0, uint64_t p1);
+// the detector of one read in the reference's own order (one thread): events.c:371-443
+__device__ void detect_read_in_order(const DetParams& p, const float* __restrict__ t1, const float* __restrict__ t2,
+                                     uint64_t base, uint64_t foff, uint32_t n, uint32_t* __restrict__ bitmap);
 int launch_generic_detect(const DevBatch& b, const WorkList& wl, Scratch& sc, int sm_count, cudaStream_t st);
 int launch_generic_emit(const DevBatch& b, const WorkList& wl, Scratch& sc, const uint64_t* ev_off, uint64_t ev_cap,
                         uint32_t* ev_start, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
-int launch_generic_detect_pa(const DevBatch& b, const float* pa, const WorkList& ordered, const WorkList& all,
-                             Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st);
+// the general route's ordered prefix sums, t-statistics and detector (pa: the caller's floats, or nullptr: b's int16
+// samples; set: the caller's detector set, or nullptr: the reference's chosen by b.rna)
+int launch_generic_detect_pa(const DevBatch& b, const float* pa, const DetParams* set, const WorkList& ordered,
+                             const WorkList& all, Scratch& sc, uint32_t* fixups, int sm_count, cudaStream_t st);
+// detect_set.cu: the warp-chunked detector of the reads of wl on the t arrays with a caller's set; fixups[r] = the
+// read's mismatched chunks
+int launch_detect_set(const DevBatch& b, const WorkList& wl, Scratch& sc, uint32_t* fixups, const DetParams& set,
+                      int sm_count, cudaStream_t st);
 int launch_scan_u32(const uint32_t* cnt, uint32_t n, uint64_t* off, uint64_t* total_out, Scratch& sc, cudaStream_t st);
 uint32_t scan_tiles_for(uint32_t n);
 
@@ -127,7 +138,8 @@ int launch_fast_emit(const DevBatch& b, Scratch& sc, uint64_t ev_cap, uint32_t* 
                      float* ev_stdv, const uint32_t* fixups, int sm_count, cudaStream_t st);
 int launch_pa(const DevBatch& b, float* pa, int sm_count, cudaStream_t st);
 
-// pa_input.cu (event detection on the caller's pA floats: exactness witness and parallel scan of the prefix sums)
+// pa_input.cu (the general route of event detection -- the caller's pA floats, or any batch with a caller's detector
+// set: exactness witness and parallel scan of the prefix sums)
 struct PaScratch {                 // allocated on the first pA batch
     DevBuf<uint32_t> tile_cnt;     // [max_reads] tiles of every read
     DevBuf<uint64_t> tile_base;    // [max_reads+1] their exclusive scan
@@ -139,6 +151,7 @@ struct PaScratch {                 // allocated on the first pA batch
     uint64_t max_tiles;
 };
 uint64_t pa_tile_capacity(uint64_t max_samples, uint32_t max_reads);
+// pa: the caller's floats, or nullptr: b's int16 samples through their calibration
 int launch_pa_prefix(const DevBatch& b, const float* pa, PaScratch& w, Scratch& sc, uint32_t* seq_flag,
                      uint32_t* fixups, int force_all, int sm_count, cudaStream_t st);
 
@@ -180,6 +193,8 @@ struct LiveChan {
     uint32_t a;                           // the open event's start
     float offset, unit;                   // the read's calibration (misc.c:17-19,26)
     uint32_t rna;
+    uint32_t custom;                      // 1: the read runs the detector set in force at its START (`set`)
+    DetParams set;
 };
 struct LiveBatch {                         // entry e: samples (or pa)[read_off[e] .. +read_len[e]) of channel[e]
     union {
@@ -196,11 +211,15 @@ struct LiveBatch {                         // entry e: samples (or pa)[read_off[
     uint64_t span;
 };
 // where entry e (at sample offset `off`) stages its events before compaction. The detector steps at most
-// len + w2 - 1 < len + 14 positions in an entry, and a detector that emits at step i emits next at step
+// len + max(w1, w2) - 1 < len + 14 positions in an entry, and a detector that emits at step i emits next at step
 // i + w/2 + 2 or later (its peak is set at i + 1 at the earliest and must be more than w/2 behind): at most
 // ceil(m/3) + ceil(m/5) events in m steps (DNA; RNA fewer) plus the read's last one, which the stride of
-// 8/15 per sample + 24 per entry covers. Evaluated at (max_samples, max_reads) it is the capacity.
-__host__ __device__ inline uint64_t live_stage_base(uint64_t off, uint64_t e) { return off / 15 * 8 + 24 * e; }
+// 8/15 per sample + 24 per entry covers. `dense` (LiveScratch::dense): any detector set (w >= 2: gaps of 3 or more
+// for both detectors), ceil(m/3) + ceil(m/3) + 1, covered by 2/3 per sample + 24 per entry. Evaluated at
+// (max_samples, max_reads) it is the capacity.
+__host__ __device__ inline uint64_t live_stage_base(uint64_t off, uint64_t e, bool dense) {
+    return (dense ? off / 3 * 2 : off / 15 * 8) + 24 * e;
+}
 struct LiveScratch {                       // allocated by sgpu_live_open
     DevBuf<LiveChan> chan;                 // [n_channels]
     DevBuf<uint32_t> nopen;                // [n_channels]
@@ -212,11 +231,12 @@ struct LiveScratch {                       // allocated by sgpu_live_open
     uint32_t n_channels = 0;
     uint64_t ev_cap = 0;
     uint32_t stamp = 0;
+    bool dense = false;                    // staged at the bound of any detector set (live_stage_base)
 };
 // the events of entry e go to ev_start, ev_len, ev_mean, ev_stdv [ev_off[e], ev_off[e+1]) (ev_off: [n_entries+1]);
-// pa: the entries are b.pa floats
-int launch_live(const LiveBatch& b, bool pa, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start,
-                uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
+// pa: the entries are b.pa floats; set: the detector set a START entry gives its read, or nullptr: the reference's
+int launch_live(const LiveBatch& b, bool pa, const DetParams* set, LiveScratch& w, Scratch& sc, uint64_t* ev_off,
+                uint32_t* ev_start, uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
 
 // stat.cu
 constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;

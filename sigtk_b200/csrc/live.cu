@@ -19,6 +19,8 @@
 // The S/Q chain is formed one sample after another in the reference's order whatever the input, so pA entries need no
 // exactness witness (pa_input.cu): the floats go through the same chain as the pA of int16 samples. A read keeps the
 // form of the entry that started it (LiveScratch::form); an entry of the other form that continues it is refused.
+// Likewise it keeps the detector set in force for its START entry (sgpu_set_detector; LiveChan::custom, set), and a
+// position is stepped once both of its right windows are complete: i <= n - max(w1, w2).
 #include "../../include/sigtk_b200.h"
 #include "kernels.cuh"
 
@@ -30,7 +32,7 @@ constexpr int LIVE_TILE = 256;   // samples per tile: bounded shared memory for 
 struct LiveWarpSmem {
     double S[LIVE_TAIL + LIVE_TILE], Q[LIVE_TAIL + LIVE_TILE];  // S[jb + k] at k (jb = n - LIVE_TAIL + 1)
     float pa[LIVE_TILE];
-    float t1[LIVE_TILE + 16], t2[LIVE_TILE + 16];                // positions [st, L): at most a tile + w2 - 1
+    float t1[LIVE_TILE + 16], t2[LIVE_TILE + 16];                // positions [st, L): at most a tile + 13
 };
 
 // t-statistic of position i (buffer index ki) with window w once n samples of the read are known: zero unless
@@ -47,9 +49,10 @@ __device__ __forceinline__ float live_tstat(const double* S, const double* Q, in
 template <bool PA>
 __global__ void __launch_bounds__(LIVE_WARPS * 32)
 live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nopen, uint32_t* __restrict__ claim,
-            uint32_t n_channels, uint32_t stamp, float thr_long, uint32_t* __restrict__ cnt,
-            uint32_t* __restrict__ s_start, uint32_t* __restrict__ s_len, float* __restrict__ s_mean,
-            float* __restrict__ s_stdv, uint64_t ev_cap, int* __restrict__ status, uint8_t* __restrict__ form) {
+            uint32_t n_channels, uint32_t stamp, float thr_long, DetParams set, bool use_set, bool dense,
+            uint32_t* __restrict__ cnt, uint32_t* __restrict__ s_start, uint32_t* __restrict__ s_len,
+            float* __restrict__ s_mean, float* __restrict__ s_stdv, uint64_t ev_cap, int* __restrict__ status,
+            uint8_t* __restrict__ form) {
     constexpr uint8_t my_form = PA ? LIVE_FORM_PA : LIVE_FORM_INT16;
     __shared__ LiveWarpSmem smem[LIVE_WARPS];
     LiveWarpSmem& sm = smem[threadIdx.x >> 5];
@@ -85,8 +88,12 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
         LiveChan& ch = chan[c];
         const uint32_t rna = start ? ((f & SGPU_LIVE_RNA) ? 1u : 0u) : ch.rna;
         const float offv = PA ? 0.0f : (start ? b.offset[e] : ch.offset), unitv = PA ? 1.0f : (start ? b.unit[e] : ch.unit);
-        const DetParams p = det_params((int)rna);
-        const uint32_t w1 = (uint32_t)p.w1, w2 = (uint32_t)p.w2;
+        // the read's detector: the caller's set in force at its START, else the reference's for rna with the long
+        // threshold of the push (SGPU_PARAM_THR_LONG)
+        const bool custom = start ? use_set : ch.custom != 0u;
+        const DetParams p = custom ? (start ? set : ch.set) : det_params((int)rna);
+        const float thr2 = custom ? p.thr2 : thr_long;
+        const uint32_t w1 = (uint32_t)p.w1, w2 = (uint32_t)p.w2, wm = max(w1, w2);
         uint64_t n_cur = start ? 0 : (no & ~LIVE_OPEN);
         if (lane < LIVE_TAIL) {  // a new read: S[j] = Q[j] = 0 for every j <= 0
             sm.S[lane] = start ? 0.0 : ch.tS[lane];
@@ -106,7 +113,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
                 aS = ch.aS; aQ = ch.aQ; a = ch.a;
             }
         }
-        const uint64_t sbase = live_stage_base(off, e);
+        const uint64_t sbase = live_stage_base(off, e, dense);
         auto emit = [&](uint32_t pk, double pks, double pkq) {  // peak pk closes the event [a, pk)
             const uint64_t k = sbase + n_ev;
             if (k >= ev_cap) { atomicExch(status, SGPU_DEV_E_EVCAP); return; }  // (cannot happen: live_stage_base)
@@ -116,7 +123,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
             n_ev++;
             a = pk; aS = pks; aQ = pkq;
         };
-        uint64_t st = n_cur + 1 > w2 ? n_cur + 1 - w2 : 0;  // positions [0, st) have been stepped
+        uint64_t st = n_cur + 1 > wm ? n_cur + 1 - wm : 0;  // positions [0, st) have been stepped
         uint32_t t0 = 0;
         do {
             const uint32_t m = min((uint32_t)LIVE_TILE, len - t0);
@@ -137,7 +144,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
             }
             __syncwarp();
             const uint64_t n_new = n_cur + m;
-            uint64_t L = (end && t0 + m == len) ? n_new : (n_new + 1 > w2 ? n_new + 1 - w2 : 0);
+            uint64_t L = (end && t0 + m == len) ? n_new : (n_new + 1 > wm ? n_new + 1 - wm : 0);
             if (L < st) L = st;
             const int64_t jb = (int64_t)n_cur - (LIVE_TAIL - 1);
             for (uint64_t i = st + lane; i < L; i += 32) {
@@ -156,7 +163,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
                     if (ds.peak_pos == (int32_t)pos) { pS0 = si; pQ0 = qi; }
                     if (ps > 0) emit((uint32_t)ps, os, oq);  // peaks[i] > 0 (events.c:481-485)
                     const double ol = pS1, oql = pQ1;
-                    const int32_t pl = det_step(dl, nullptr, false, pos, sm.t2[k], thr_long, p.w2, p.height);
+                    const int32_t pl = det_step(dl, nullptr, false, pos, sm.t2[k], thr2, p.w2, p.height);
                     if (dl.peak_pos == (int32_t)pos) { pS1 = si; pQ1 = qi; }
                     if (pl > 0) emit((uint32_t)pl, ol, oql);
                 }
@@ -182,6 +189,7 @@ live_kernel(LiveBatch b, LiveChan* __restrict__ chan, uint32_t* __restrict__ nop
                 ch.pS[0] = pS0; ch.pQ[0] = pQ0; ch.pS[1] = pS1; ch.pQ[1] = pQ1;
                 ch.aS = aS; ch.aQ = aQ; ch.a = a;
                 ch.offset = offv; ch.unit = unitv; ch.rna = rna;
+                ch.custom = custom ? 1u : 0u; ch.set = p;
                 nopen[c] = (uint32_t)n_cur | LIVE_OPEN;
                 if (start) form[c] = my_form;
             }
@@ -197,13 +205,13 @@ __global__ void __launch_bounds__(256) live_compact_kernel(LiveBatch b, const ui
                                                            const uint32_t* __restrict__ s_start,
                                                            const uint32_t* __restrict__ s_len,
                                                            const float* __restrict__ s_mean,
-                                                           const float* __restrict__ s_stdv, uint32_t* __restrict__ start,
-                                                           uint32_t* __restrict__ len, float* __restrict__ mean,
-                                                           float* __restrict__ stdv) {
+                                                           const float* __restrict__ s_stdv, bool dense,
+                                                           uint32_t* __restrict__ start, uint32_t* __restrict__ len,
+                                                           float* __restrict__ mean, float* __restrict__ stdv) {
     const int lane = threadIdx.x & 31;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t e = warp; e < b.n_entries; e += n_warps) {
-        const uint64_t src = live_stage_base(b.read_off[e], e), dst = ev_off[e];
+        const uint64_t src = live_stage_base(b.read_off[e], e, dense), dst = ev_off[e];
         for (uint32_t k = lane; k < cnt[e]; k += 32) {
             start[dst + k] = s_start[src + k];
             len[dst + k] = s_len[src + k];
@@ -213,16 +221,16 @@ __global__ void __launch_bounds__(256) live_compact_kernel(LiveBatch b, const ui
     }
 }
 
-int launch_live(const LiveBatch& b, bool pa, LiveScratch& w, Scratch& sc, uint64_t* ev_off, uint32_t* ev_start,
-                uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st) {
+int launch_live(const LiveBatch& b, bool pa, const DetParams* set, LiveScratch& w, Scratch& sc, uint64_t* ev_off,
+                uint32_t* ev_start, uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st) {
     if (++w.stamp == 0) w.stamp = 1;  // (claim[] starts at 0)
     auto* const kernel = pa ? live_kernel<true> : live_kernel<false>;
     kernel<<<grid_cap(b.n_entries, LIVE_WARPS, sm_count * 8), LIVE_WARPS * 32, 0, st>>>(
-        b, w.chan, w.nopen, w.claim, w.n_channels, w.stamp, sc.tune_thr_long, w.cnt, w.s_start, w.s_len, w.s_mean,
-        w.s_stdv, w.ev_cap, sc.status, w.form);
+        b, w.chan, w.nopen, w.claim, w.n_channels, w.stamp, sc.tune_thr_long, set ? *set : DetParams{}, set != nullptr,
+        w.dense, w.cnt, w.s_start, w.s_len, w.s_mean, w.s_stdv, w.ev_cap, sc.status, w.form);
     int n = 1 + launch_scan_u32(w.cnt, b.n_entries, ev_off, reinterpret_cast<uint64_t*>(sc.counters.get()), sc, st);
     live_compact_kernel<<<grid_cap(b.n_entries, 8, sm_count * 8), 256, 0, st>>>(
-        b, w.cnt, ev_off, w.s_start, w.s_len, w.s_mean, w.s_stdv, ev_start, ev_len, ev_mean, ev_stdv);
+        b, w.cnt, ev_off, w.s_start, w.s_len, w.s_mean, w.s_stdv, w.dense, ev_start, ev_len, ev_mean, ev_stdv);
     return n + 1;
 }
 

@@ -18,6 +18,12 @@
 // fl(x*x) for Q). If sum |x| < 2^(k+53), every partial sum of any grouping is a multiple of 2^k below 2^(k+53) in
 // magnitude, i.e. a double: no FP64 addition rounds, and the reference's S[i] equals the scan's (DESIGN §3, point 1).
 // A NaN or an infinity makes the bound NaN or infinite and fails the test; so does an fl(x*x) that overflows.
+//
+// Batches of int16 records (and decoded svb-zd streams) whose detector is the caller's set (sgpu_set_detector) take
+// the same route: the tile and scan kernels are templates on the sample type, and an int16 instantiation forms the pA
+// of every sample (misc.c:28) where it loads it, so no pA array is stored.
+#include <type_traits>
+
 #include "kernels.cuh"
 
 namespace sgpu {
@@ -50,6 +56,22 @@ __device__ __forceinline__ double warp_sum_up(double v) {  // rounded upwards: a
 }
 __device__ __forceinline__ uint32_t warp_min(uint32_t v) { return __reduce_min_sync(0xffffffffu, v); }
 
+// the reference's floats of values i .. i+3 of a read (i a multiple of 4; reads start on 8 samples): the caller's pA
+// as it is, or int16 samples through the read's calibration
+__device__ __forceinline__ float4 load4(const float* __restrict__ p, uint64_t i, float, float) {
+    return __ldg(reinterpret_cast<const float4*>(p + i));
+}
+__device__ __forceinline__ float4 load4(const int16_t* __restrict__ p, uint64_t i, float off, float unit) {
+    const uint2 v = __ldg(reinterpret_cast<const uint2*>(p + i));
+    return make_float4(pa_of((int16_t)(uint16_t)v.x, off, unit), pa_of((int16_t)(uint16_t)(v.x >> 16), off, unit),
+                       pa_of((int16_t)(uint16_t)v.y, off, unit), pa_of((int16_t)(uint16_t)(v.y >> 16), off, unit));
+}
+template <typename T>
+__device__ __forceinline__ void calibration(const DevBatch& b, uint32_t r, float& off, float& unit) {
+    off = 0.0f; unit = 0.0f;
+    if constexpr (std::is_same_v<T, int16_t>) { off = b.offset[r]; unit = b.unit[r]; }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) pa_init_kernel(DevBatch b, uint32_t* __restrict__ tile_cnt,
                                                       uint32_t* __restrict__ fixups, uint32_t* __restrict__ all_list,
@@ -66,7 +88,8 @@ __global__ void __launch_bounds__(256) pa_init_kernel(DevBatch b, uint32_t* __re
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(PT_THREADS) pa_tile_kernel(DevBatch b, const float* __restrict__ pa,
+template <typename T>
+__global__ void __launch_bounds__(PT_THREADS) pa_tile_kernel(DevBatch b, const T* __restrict__ pa,
                                                              const uint64_t* __restrict__ tile_base,
                                                              double* __restrict__ tS, double* __restrict__ tQ,
                                                              double* __restrict__ tA, double* __restrict__ tB,
@@ -78,13 +101,15 @@ __global__ void __launch_bounds__(PT_THREADS) pa_tile_kernel(DevBatch b, const f
     for (uint64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
         const uint32_t r = find_read(tile_base, b.n_reads, t);
         const uint32_t i0 = (uint32_t)(t - tile_base[r]) * PT, n = b.read_len[r];
-        const float4* __restrict__ src = reinterpret_cast<const float4*>(pa + b.read_off[r] + i0);
-        // the order of the additions does not matter here (only exact sums are used): coalesced float4 loads
+        const uint64_t src = b.read_off[r] + i0;
+        float off, unit;
+        calibration<T>(b, r, off, unit);
+        // the order of the additions does not matter here (only exact sums are used): coalesced 4-value loads
         float4 v[4];
 #pragma unroll
         for (int k = 0; k < 4; k++) {
-            const uint32_t i = i0 + 4u * (k * PT_THREADS + threadIdx.x);   // reads are padded to 8 samples
-            v[k] = i < n ? __ldg(src + k * PT_THREADS + threadIdx.x) : make_float4(0.f, 0.f, 0.f, 0.f);
+            const uint32_t i = 4u * (k * PT_THREADS + threadIdx.x);   // reads are padded to 8 samples
+            v[k] = i0 + i < n ? load4(pa, src + i, off, unit) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
         double s = 0.0, q = 0.0, a = 0.0, bq = 0.0;
         uint32_t mx = 0xffffffffu, mq = 0xffffffffu;
@@ -192,7 +217,8 @@ __device__ __forceinline__ void cta_scan2(double& s, double& q, double& ts, doub
     __syncthreads();
 }
 
-__global__ void __launch_bounds__(PT_THREADS) pa_scan_kernel(DevBatch b, const float* __restrict__ pa,
+template <typename T>
+__global__ void __launch_bounds__(PT_THREADS) pa_scan_kernel(DevBatch b, const T* __restrict__ pa,
                                                              const uint64_t* __restrict__ tile_base,
                                                              const double* __restrict__ tS, const double* __restrict__ tQ,
                                                              const uint32_t* __restrict__ seq_flag,
@@ -205,15 +231,17 @@ __global__ void __launch_bounds__(PT_THREADS) pa_scan_kernel(DevBatch b, const f
         const uint32_t i0 = (uint32_t)(t - tile_base[r]) * PT, n = b.read_len[r];
         const uint64_t base = b.read_off[r];   // = the read's scratch base
         double cs = tS[t], cq = tQ[t];         // S[i0], Q[i0]
+        float off, unit;
+        calibration<T>(b, r, off, unit);
         // 1,024 samples per round, four consecutive ones per thread; the next round's loads in flight
-        const float4* __restrict__ src = reinterpret_cast<const float4*>(pa + base + i0);
-        float4 nxt = i0 + 4u * threadIdx.x < n ? __ldg(src + threadIdx.x) : make_float4(0.f, 0.f, 0.f, 0.f);
+        const uint64_t src = base + i0 + 4u * threadIdx.x;
+        float4 nxt = i0 + 4u * threadIdx.x < n ? load4(pa, src, off, unit) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 1
         for (int k = 0; k < PT / (4 * PT_THREADS); k++) {
             const uint32_t i = i0 + (uint32_t)(k * 4 * PT_THREADS) + 4u * threadIdx.x;
             const float4 v = nxt;
             const uint32_t ni = i + 4u * PT_THREADS;
-            nxt = (k + 1 < PT / (4 * PT_THREADS) && ni < n) ? __ldg(src + (k + 1) * PT_THREADS + threadIdx.x)
+            nxt = (k + 1 < PT / (4 * PT_THREADS) && ni < n) ? load4(pa, src + (uint64_t)(k + 1) * 4 * PT_THREADS, off, unit)
                                                               : make_float4(0.f, 0.f, 0.f, 0.f);
             const float e[4] = {v.x, v.y, v.z, v.w};
             double ps[4], pq[4], s = 0.0, q = 0.0;
@@ -249,19 +277,26 @@ __global__ void __launch_bounds__(PT_THREADS) pa_scan_kernel(DevBatch b, const f
 // ---------------------------------------------------------------------------------------------------------------
 uint64_t pa_tile_capacity(uint64_t max_samples, uint32_t max_reads) { return max_samples / PT + max_reads + 1; }
 
+template <typename T>
+static void launch_tiles_and_scan(const DevBatch& b, const T* src, PaScratch& w, Scratch& sc, uint32_t* seq_flag,
+                                  int force_all, int sm_count, cudaStream_t st) {
+    const uint64_t tiles = b.span / PT + b.n_reads;   // at least the batch's tiles
+    pa_tile_kernel<T><<<grid_cap(tiles, 1, sm_count * 8), PT_THREADS, 0, st>>>(b, src, w.tile_base, w.tS, w.tQ, w.tA,
+                                                                             w.tB, w.tmin);
+    pa_read_kernel<<<grid_cap((uint64_t)b.n_reads * 32, 128, sm_count * 8), 128, 0, st>>>(
+        b, w.tile_base, w.tS, w.tQ, w.tA, w.tB, w.tmin, force_all, seq_flag, w.ord_list, w.ord_sbase, w.ord_count,
+        sc.counters);
+    pa_scan_kernel<T><<<grid_cap(tiles, 1, sm_count * 8), PT_THREADS, 0, st>>>(b, src, w.tile_base, w.tS, w.tQ,
+                                                                             seq_flag, sc.Sinc, sc.Qinc);
+}
+
 int launch_pa_prefix(const DevBatch& b, const float* pa, PaScratch& w, Scratch& sc, uint32_t* seq_flag,
                      uint32_t* fixups, int force_all, int sm_count, cudaStream_t st) {
     pa_init_kernel<<<grid_cap(b.n_reads, 256, sm_count), 256, 0, st>>>(b, w.tile_cnt, fixups, sc.seq_list, sc.seq_sbase,
                                                                        sc.seq_count, w.ord_count);
     int n = 1 + launch_scan_u32(w.tile_cnt, b.n_reads, w.tile_base, nullptr, sc, st);
-    const uint64_t tiles = b.span / PT + b.n_reads;   // at least the batch's tiles
-    pa_tile_kernel<<<grid_cap(tiles, 1, sm_count * 8), PT_THREADS, 0, st>>>(b, pa, w.tile_base, w.tS, w.tQ, w.tA, w.tB,
-                                                                          w.tmin);
-    pa_read_kernel<<<grid_cap((uint64_t)b.n_reads * 32, 128, sm_count * 8), 128, 0, st>>>(
-        b, w.tile_base, w.tS, w.tQ, w.tA, w.tB, w.tmin, force_all, seq_flag, w.ord_list, w.ord_sbase, w.ord_count,
-        sc.counters);
-    pa_scan_kernel<<<grid_cap(tiles, 1, sm_count * 8), PT_THREADS, 0, st>>>(b, pa, w.tile_base, w.tS, w.tQ, seq_flag,
-                                                                          sc.Sinc, sc.Qinc);
+    if (pa) launch_tiles_and_scan(b, pa, w, sc, seq_flag, force_all, sm_count, st);
+    else    launch_tiles_and_scan(b, b.samples, w, sc, seq_flag, force_all, sm_count, st);
     return n + 4;
 }
 

@@ -46,7 +46,8 @@ def signal(dev, n, seed):
     return (lvl + torch.randint(-20, 21, (n,), device=dev, generator=g)).to(torch.int16)
 
 
-def device_config(dev, channels, per_push, rna, iters, warmup, pa=False):
+def device_config(dev, channels, per_push, rna, iters, warmup, pa=False, det=None):
+    """det: a detector set (sgpu_set_detector) in force for the pushes, or None: the reference's"""
     n = channels * per_push
     unit = np.float32(synth.RANGE) / np.float32(synth.DIGITISATION)
     bufs = [signal(dev, n, 100 + k) for k in range(NBUF)]
@@ -61,6 +62,7 @@ def device_config(dev, channels, per_push, rna, iters, warmup, pa=False):
     units = torch.full((channels,), float(unit), device=dev, dtype=torch.float32)
     with sg.Context(device=0, max_samples=n, max_reads=channels, flags=sg.F_NO_HOST_SLOTS) as c:
         c.live_open(channels)
+        c.set_detector(det)
         stream = torch.cuda.current_stream()
         st = stream.cuda_stream
         if pa:
@@ -89,7 +91,7 @@ def device_config(dev, channels, per_push, rna, iters, warmup, pa=False):
             "events_last_push": cnt["n_events"], "launches_per_push": cnt["n_kernel_launches"]}
 
 
-def host_latency(channels, per_push, iters, warmup, pa=False):
+def host_latency(channels, per_push, iters, warmup, pa=False, det=None):
     raws = np.random.default_rng(7).integers(300, 700, size=(channels, per_push * (warmup + iters))).astype(np.int16)
     unit = np.float32(synth.RANGE) / np.float32(synth.DIGITISATION)
     lib = _lib.load()
@@ -97,6 +99,7 @@ def host_latency(channels, per_push, iters, warmup, pa=False):
     # (a slot holds max_samples / 2 floats)
     with sg.Context(device=0, max_samples=channels * per_push * (2 if pa else 1), max_reads=channels, n_slots=1) as c:
         c.live_open(channels)
+        c.set_detector(det)
         res = _lib.LiveResult()
         for k in range(warmup + iters):
             flags = sg.LIVE_START if k == 0 else 0
