@@ -57,7 +57,8 @@ extern "C" {
 #define SGPU_WANT_STAT     4u /* the six numbers of stat_func, cfunc.c:126-159 */
 #define SGPU_WANT_ENT      8u /* the three entropies of `sigtk ent`, ent.c:108-151 */
 #define SGPU_WANT_JNN     16u /* the segments of `sigtk jnn`: jnn_raw(), jnn.c:269-282 with the parameters of
-                                 jnn_print (jnn.c:305-312: JNNV1_DRNA_R9_PARAM when rna, else JNNV1_CDNA_R9_PARAM) */
+                                 jnn_print (jnn.c:305-312: JNNV1_DRNA_R9_PARAM when rna, else JNNV1_CDNA_R9_PARAM),
+                                 or the caller's set (sgpu_set_jnn) */
 
 #define SGPU_WANT_PREFIX  32u /* `sigtk prefix` (prefix_func, cfunc.c:169-234): find_adaptor (jnnv2, jnn.c:99-188), the
                                  adaptor's pA statistics, find_polya (jnn.c:352-374) when rna, its statistics */
@@ -121,7 +122,8 @@ typedef struct {
     float    *prefix_stat; /* [n_reads][6]: meanf, stdvf, medianf of the adaptor's pA (valid when its y > 0), then of the
                               poly-A's (valid when its y > 0): cfunc.c:178-180, 202-204. Bit-exact. */
 } sgpu_result_t;
-/* first segment slot of read r (a read of n samples has at most n/38 + 1 segments, jnn.c:232) */
+/* first segment slot of read r (a read of n samples has at most n/32 + 1 segments for every set sgpu_set_jnn
+ * accepts; n/38 + 1 for the reference's, jnn.c:232) */
 #define SGPU_JNN_BASE(read_off_r, r) (((uint64_t)(read_off_r) >> 5) + (uint64_t)(r))
 
 /* ---- lifecycle ----------------------------------------------------------- */
@@ -351,7 +353,8 @@ int  sgpu_set_param(sgpu_ctx_t *ctx, int key, double value);
  * detection of the context use the caller's set instead, as short_long_peak_detector(..., &set) would:
  *   - Scope: int16 records, svb-zd streams and pA records, on host slots and in device-resident runs, and live
  *     entries of both forms. rna and SGPU_LIVE_RNA then no longer choose the event parameters (they still choose those
- *     of SGPU_WANT_JNN and SGPU_WANT_PREFIX), and SGPU_PARAM_THR_LONG is ignored. The other products of a batch (PA,
+ *     of SGPU_WANT_PREFIX, and those of SGPU_WANT_JNN unless a jnn set is in force: sgpu_set_jnn), and
+ *     SGPU_PARAM_THR_LONG is ignored. The other products of a batch (PA,
  *     STAT, ENT, JNN, PREFIX) do not depend on it.
  *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
  *     different sets); a device-resident run the set in force when it is called; a live read the set in force for its
@@ -376,6 +379,39 @@ typedef struct {                  /* detector_param, events.c:35-41 */
     float    peak_height;
 } sgpu_detector_t;
 int  sgpu_set_detector(sgpu_ctx_t *ctx, const sgpu_detector_t *p);
+
+/* ---- the caller's own jnn parameters ---------------------------------------------------------------------------
+ * jnn_raw takes a jnn_param_t (jnn.h:24-45); jnn_print uses one of two constant sets chosen by rna (jnn.c:305-312:
+ * JNNV1_CDNA_R9_PARAM {150, 0.25, 5, 50, 50, 0.75}, JNNV1_DRNA_R9_PARAM {1000, 1.0, 5, 50, 50, 0.75}, in the field
+ * order below). Their windows are in samples, tuned for R9.4.1 sample rates. sgpu_set_jnn makes SGPU_WANT_JNN use
+ * the caller's set instead, as jnn_raw(raw, n, set, &n_seg) would:
+ *   - Scope: int16 records and svb-zd streams, on host slots and in device-resident runs (pA records and live entries
+ *     do not compute SGPU_WANT_JNN). rna then no longer chooses the jnn parameters; it still chooses the event
+ *     parameters (unless a detector set is in force) and those of SGPU_WANT_PREFIX. The other products of a batch
+ *     (EVENTS, PA, STAT, ENT, PREFIX) do not depend on it.
+ *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
+ *     different sets); a device-resident run the set in force when it is called.
+ *   - Results: bit-identical to the reference's jnn_raw with the set (the band mean -/+ fl(stdv * std_scale) of the
+ *     clamped signal, the counter machine of jnn.c:176-266 with its corrector). The reference keeps w = corrector +
+ *     in-band samples so far in an int; here it cannot overflow (a corrector near 2^31 with a read near 2^31 samples).
+ *     A set with error <= 6 and error < corrector runs the parallel automaton of the reference's sets (the corrector
+ *     provably never acts there); every other set runs the counter machine sample by sample (slower).
+ *   - Accepted sets: error >= 0, corrector >= 0 (so w >= 1 wherever the reference computes c % w), stall_len and
+ *     std_scale finite, (float)window > 31 and (float)window * stall_len > 31 (formed in float). The last rule keeps
+ *     two things true for every accepted set: (a) a counted stretch is at least 32 samples long, so a read of n samples
+ *     has at most n/32 + 1 segments and SGPU_JNN_BASE holds (no capacity error can occur); (b) at most one counted
+ *     stretch closes per 32-sample word. Windows of 31 samples or fewer are refused. Any other set returns
+ *     SGPU_E_INVAL and leaves the setting as it was. seg_dist may be any value.
+ * NULL restores the reference's sets (chosen by rna). */
+typedef struct {              /* jnn_param_t, jnn.h:24-45 */
+    int32_t window;           /* stretch length (samples) that counts as a segment */
+    float   stall_len;        /* the first segment needs window * stall_len samples only */
+    int32_t error;            /* tolerated outliers in a stretch */
+    int32_t seg_dist;         /* merge distance: a segment starting closer than this to the previous end extends it */
+    int32_t corrector;        /* initial value of the corrector w */
+    float   std_scale;        /* band: mean -/+ std_scale * stdv */
+} sgpu_jnn_t;
+int  sgpu_set_jnn(sgpu_ctx_t *ctx, const sgpu_jnn_t *p);
 
 /* Device time of every kernel group of the last run, measured with CUDA events on the stream the kernels were
  * launched on (needs SGPU_F_STAGE_TIMERS). Returns the number of entries written, or a negative code. */

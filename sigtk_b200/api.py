@@ -37,6 +37,20 @@ class Detector(NamedTuple):
     peak_height: float
 
 
+class Jnn(NamedTuple):
+    """jnn_param_t (jnn.h:24-45): the reference's sets are Jnn.CDNA_R9 and Jnn.DRNA_R9 (jnn_print picks one by rna)"""
+    window: int         # stretch length in samples that counts as a segment; > 31
+    stall_len: float    # the first segment needs window * stall_len samples only; window * stall_len > 31
+    error: int          # tolerated outliers in a stretch, >= 0
+    seg_dist: int       # merge distance
+    corrector: int      # initial value of the corrector, >= 0
+    std_scale: float    # band: mean -/+ std_scale * stdv of the clamped signal
+
+
+Jnn.CDNA_R9 = Jnn(150, 0.25, 5, 50, 50, 0.75)   # JNNV1_CDNA_R9_PARAM
+Jnn.DRNA_R9 = Jnn(1000, 1.0, 5, 50, 50, 0.75)   # JNNV1_DRNA_R9_PARAM
+
+
 @dataclass
 class EventTable:
     """event_table of one read (src/sigtk.h:65-70) as arrays."""
@@ -329,6 +343,15 @@ class Context:
             return
         p = _lib.DetectorParams(int(det[0]), int(det[1]), float(det[2]), float(det[3]), float(det[4]))
         self._check(self._lib.sgpu_set_detector(self._h, C.byref(p)))
+
+    def set_jnn(self, jnn: Optional[Jnn]) -> None:
+        """sgpu_set_jnn: WANT_JNN of every later batch (host slots from their submit, device-resident runs) uses `jnn`;
+        None restores the reference's sets, chosen by rna"""
+        if jnn is None:
+            self._check(self._lib.sgpu_set_jnn(self._h, None))
+            return
+        p = _lib.JnnParams(int(jnn[0]), float(jnn[1]), int(jnn[2]), int(jnn[3]), int(jnn[4]), float(jnn[5]))
+        self._check(self._lib.sgpu_set_jnn(self._h, C.byref(p)))
 
     def set_param(self, key: int, value: float) -> None:
         """development / test parameters (_lib.PARAM_*): chunk length, detector warm-up, the long detector's threshold"""

@@ -141,6 +141,8 @@ struct Slot {
     uint32_t want = 0;
     const DetParams* det = nullptr;  // the context's detector set at sgpu_submit (&det_set), or nullptr: the reference's
     DetParams det_set{};
+    const JnnParams* jnn = nullptr;  // the context's jnn set at sgpu_submit (&jnn_set), or nullptr: jnn_print's by rna
+    JnnParams jnn_set{};
     Input kind = Input::NONE;        // (PA, LIVE_PA: the floats are in the sample buffers, max_samples / 2 of them)
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
@@ -182,6 +184,8 @@ struct sgpu_ctx {
     int pore_rna004 = 0;         // SGPU_PARAM_PORE: jnnv2 parameters of `prefix` (misc.c:74-101 picks them from the header)
     bool det_on = false;         // sgpu_set_detector: every event detection uses `det` instead of the reference's sets
     DetParams det{};
+    bool jnn_on = false;         // sgpu_set_jnn: SGPU_WANT_JNN uses `jnn` instead of jnn_print's sets
+    JnnParams jnn{};
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
@@ -406,9 +410,10 @@ int general_events(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetP
 
 // The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies
 // (except when the general route's scratch grows). set: the caller's detector set, whose events take the general
-// route, or nullptr: the reference's sets on the fast path.
+// route, or nullptr: the reference's sets on the fast path. jnn: the caller's jnn set, or nullptr: jnn_print's (b.rna).
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
-                 const DetParams* set, const SvbBatch* svb = nullptr, int16_t* svb_out = nullptr) {
+                 const DetParams* set, const JnnParams* jnn, const SvbBatch* svb = nullptr,
+                 int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
     if (!fits(ctx, b)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
@@ -441,7 +446,8 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
     if (want & SGPU_WANT_JNN) {
         CU(ctx->jnn_mom.ensure((uint64_t)ctx->max_reads * 2));
         marks.done("jnn_moments", launch_jnn_moments(b, ctx->jnn_mom, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
-        marks.done("jnn_walk", launch_jnn(b, ctx->jnn_mom, static_cast<uint32_t*>(o[JNN_CNT].get()),
+        marks.done("jnn_walk", launch_jnn(b, jnn ? *jnn : jnn_params(b.rna), ctx->jnn_mom,
+                                          static_cast<uint32_t*>(o[JNN_CNT].get()),
                                           static_cast<int32_t*>(o[JNN_SEG].get()), ctx->sm_count, st));
     }
     if (want & SGPU_WANT_PREFIX)
@@ -531,8 +537,8 @@ int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
     const DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, rna, sl.used};
     const SvbBatch svb{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
                        sl.svb_blocks};
-    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.kind == Input::SVBZD ? &svb : nullptr,
-                        sl.d_samples);
+    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.jnn,
+                        sl.kind == Input::SVBZD ? &svb : nullptr, sl.d_samples);
 }
 
 // a slot that is not submitted takes a record of kind k when it is empty or holds records of kind k
@@ -938,6 +944,8 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (rc) return rc;
     sl.det_set = ctx->det;  // the slot runs the set in force now, whatever is set before it is waited for
     sl.det = ctx->det_on ? &sl.det_set : nullptr;
+    sl.jnn_set = ctx->jnn;  // and the jnn set in force now
+    sl.jnn = ctx->jnn_on ? &sl.jnn_set : nullptr;
     if (live) {
         if ((rc = fit_live_staging(ctx, sl.det))) return rc;
         CU(fit_live_outputs(ctx, sl.live_dout, sl.live_dcap));
@@ -995,7 +1003,7 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     DevBatch b{batch->samples, batch->read_off, batch->read_len, batch->offset_f, batch->raw_unit_f,
                batch->n_reads, (int)batch->rna, batch->span};
     const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream),
-                                ctx->det_on ? &ctx->det : nullptr);
+                                ctx->det_on ? &ctx->det : nullptr, ctx->jnn_on ? &ctx->jnn : nullptr);
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(OUTS, out, ctx->dev_out, want, true);
@@ -1085,6 +1093,20 @@ int sgpu_set_detector(sgpu_ctx_t* ctx, const sgpu_detector_t* p) {
         return SGPU_E_INVAL;
     ctx->det = DetParams{(int)p->w_short, (int)p->w_long, p->thr_short, p->thr_long, p->peak_height};
     ctx->det_on = true;
+    return SGPU_OK;
+}
+
+int sgpu_set_jnn(sgpu_ctx_t* ctx, const sgpu_jnn_t* p) {
+    if (!ctx) return SGPU_E_INVAL;
+    if (!p) { ctx->jnn_on = false; return SGPU_OK; }
+    // window and first_min (jnn.c:232, formed as jnn_walk_kernel forms it) above 31: every counted stretch has at
+    // least 32 samples (the segment slots of SGPU_JNN_BASE suffice; at most one candidate closes per word)
+    const float first_min = (float)p->window * p->stall_len;
+    if (p->error < 0 || p->corrector < 0 || !std::isfinite(p->stall_len) || !std::isfinite(p->std_scale) ||
+        !((float)p->window > 31.0f) || !(first_min > 31.0f))
+        return SGPU_E_INVAL;
+    ctx->jnn = JnnParams{p->window, p->stall_len, p->error, p->seg_dist, p->corrector, p->std_scale};
+    ctx->jnn_on = true;
     return SGPU_OK;
 }
 

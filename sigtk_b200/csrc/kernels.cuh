@@ -245,8 +245,24 @@ int launch_stat_median(const DevBatch& b, float* stat6, uint32_t cta_min, int sm
 int launch_jnn_moments(const DevBatch& b, float* moments2, uint32_t cta_min, int sm_count, cudaStream_t st);
 
 // jnn.cu (`sigtk jnn`: band from the clamped signal's mean / stdv, counter machine per read -> (start, end) pairs)
+struct JnnParams {  // jnn_param_t, jnn.h:24-45 (sgpu_jnn_t)
+    int window;
+    float stall_len;
+    int error, seg_dist, corrector;
+    float std_scale;
+};
+// the parameters jnn_print picks (jnn.c:305-312)
+__host__ __device__ inline JnnParams jnn_params(int rna) {
+    JnnParams p;
+    p.std_scale = 0.75f; p.corrector = 50; p.seg_dist = 50; p.error = 5;
+    if (rna) { p.window = 1000; p.stall_len = 1.0f; }   // JNNV1_DRNA_R9_PARAM
+    else     { p.window = 150;  p.stall_len = 0.25f; }  // JNNV1_CDNA_R9_PARAM
+    return p;
+}
 uint64_t jnn_seg_capacity(uint64_t max_samples, uint32_t max_reads);
-int launch_jnn(const DevBatch& b, const float* moments, uint32_t* seg_cnt, int32_t* seg, int sm_count, cudaStream_t st);
+// p: the parameters (jnn_params(b.rna), or the caller's set; every set sgpu_set_jnn accepts)
+int launch_jnn(const DevBatch& b, const JnnParams& p, const float* moments, uint32_t* seg_cnt, int32_t* seg,
+               int sm_count, cudaStream_t st);
 
 
 // prefix.cu (`sigtk prefix`: adaptor by jnnv2 on the rolling mean, poly-A by jnn_core on pA, statistics of both)
