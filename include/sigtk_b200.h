@@ -61,7 +61,8 @@ extern "C" {
                                  or the caller's set (sgpu_set_jnn) */
 
 #define SGPU_WANT_PREFIX  32u /* `sigtk prefix` (prefix_func, cfunc.c:169-234): find_adaptor (jnnv2, jnn.c:99-188), the
-                                 adaptor's pA statistics, find_polya (jnn.c:352-374) when rna, its statistics */
+                                 adaptor's pA statistics, find_polya (jnn.c:352-374) when rna, its statistics; with
+                                 the reference's sets or the caller's (sgpu_set_prefix) */
 
 /* ---- context flags ------------------------------------------------------ */
 #define SGPU_F_DEFAULT       0u
@@ -342,7 +343,8 @@ int  sgpu_counters(sgpu_ctx_t *ctx, sgpu_counters_t *out);
 #define SGPU_PARAM_THR_LONG  3 /* threshold of the long detector */
 #define SGPU_PARAM_PORE      4 /* 0: R9 (JNNV2_RNA_R9_ADAPTOR), 1: RNA004 (JNNV2_RNA_RNA004_ADAPTOR), jnn.h:88-102: the
                                   host picks it from the BLOW5 header like pore_detect (misc.c:74-101); used by
-                                  SGPU_WANT_PREFIX only (not a test parameter) */
+                                  SGPU_WANT_PREFIX only, and not while a prefix set is in
+                                  force: sgpu_set_prefix (not a test parameter) */
 #define SGPU_PARAM_STAT_CTA_MIN 5 /* stat / jnn moments: reads of at least this many samples are added up by a CTA
                                   (several warps per read), shorter ones by one warp; 0 = every read by a CTA */
 int  sgpu_set_param(sgpu_ctx_t *ctx, int key, double value);
@@ -353,7 +355,8 @@ int  sgpu_set_param(sgpu_ctx_t *ctx, int key, double value);
  * detection of the context use the caller's set instead, as short_long_peak_detector(..., &set) would:
  *   - Scope: int16 records, svb-zd streams and pA records, on host slots and in device-resident runs, and live
  *     entries of both forms. rna and SGPU_LIVE_RNA then no longer choose the event parameters (they still choose those
- *     of SGPU_WANT_PREFIX, and those of SGPU_WANT_JNN unless a jnn set is in force: sgpu_set_jnn), and
+ *     of SGPU_WANT_JNN and SGPU_WANT_PREFIX unless a jnn or prefix set is in force: sgpu_set_jnn,
+ *     sgpu_set_prefix), and
  *     SGPU_PARAM_THR_LONG is ignored. The other products of a batch (PA,
  *     STAT, ENT, JNN, PREFIX) do not depend on it.
  *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
@@ -387,7 +390,8 @@ int  sgpu_set_detector(sgpu_ctx_t *ctx, const sgpu_detector_t *p);
  * the caller's set instead, as jnn_raw(raw, n, set, &n_seg) would:
  *   - Scope: int16 records and svb-zd streams, on host slots and in device-resident runs (pA records and live entries
  *     do not compute SGPU_WANT_JNN). rna then no longer chooses the jnn parameters; it still chooses the event
- *     parameters (unless a detector set is in force) and those of SGPU_WANT_PREFIX. The other products of a batch
+ *     parameters (unless a detector set is in force) and those of SGPU_WANT_PREFIX (unless a prefix set is
+ *     in force). The other products of a batch
  *     (EVENTS, PA, STAT, ENT, PREFIX) do not depend on it.
  *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
  *     different sets); a device-resident run the set in force when it is called.
@@ -412,6 +416,54 @@ typedef struct {              /* jnn_param_t, jnn.h:24-45 */
     float   std_scale;        /* band: mean -/+ std_scale * stdv */
 } sgpu_jnn_t;
 int  sgpu_set_jnn(sgpu_ctx_t *ctx, const sgpu_jnn_t *p);
+
+/* ---- the caller's own prefix parameters -----------------------------------------------------------------------
+ * prefix_func (cfunc.c:169-234) finds the adaptor with jnnv2 and one of two constant sets (jnn.h:88-102, chosen by
+ * SGPU_PARAM_PORE: JNNV2_RNA_R9_ADAPTOR {2000, 0.5, 1500, 2000, 200000}, JNNV2_RNA_RNA004_ADAPTOR {2000, 0.7, 1500,
+ * 500, 200000}, in the field order of sgpu_adaptor_t) and the poly-A behind it with jnn_core and JNNV1_R9_POLYA
+ * (jnn.h:47-56: {250, 1.0, 30, 200, 50} in the field order of sgpu_polya_t). Their windows are in samples, tuned for
+ * R9.4.1 direct RNA at 3 kHz. sgpu_set_prefix makes SGPU_WANT_PREFIX use the caller's sets instead, as prefix_func
+ * would with jnnv2(set.adaptor) and jnn_core(set.polya):
+ *   - Scope: int16 records and svb-zd streams, on host slots and in device-resident runs (pA records and live entries
+ *     do not compute SGPU_WANT_PREFIX). SGPU_PARAM_PORE then no longer chooses the adaptor set. rna still decides
+ *     whether a poly-A is searched at all (the reference searches RNA only). The other products of a batch (EVENTS,
+ *     PA, STAT, ENT, JNN) do not depend on it.
+ *   - When it takes effect: a host slot runs the set in force at its sgpu_submit (two slots in flight may carry
+ *     different sets); a device-resident run the set in force when it is called.
+ *   - Results: positions and all six statistics bit-identical to the reference's prefix_func with the sets: the
+ *     rolling mean over adaptor.window samples, positions mapped by + window/2 - 1 (integer division), a read taken
+ *     only when longer than the window; the poly-A band (adaptor mean + 30) -/+ 20 as in cfunc.c:189-190 (not a field).
+ *     The reference keeps the poly-A corrector w = corrector + in-band samples so far in an int; here it cannot
+ *     overflow. A poly-A set with error < corrector (the reference's among them) runs the parallel form, where the
+ *     corrector provably never acts; every other set steps the reference's counters sample by sample (slower).
+ *     A set with lo_thresh <= 0 admits runs of one rolling position, which jnnv2 reports with y <= x (it resets its
+ *     `last` to 0): the statistics of such a stretch of no samples are the float loops' (-0, or NaN for y == x, whose
+ *     bits may differ from the reference's) and its median is 0, where the reference's medianf is undefined.
+ *   - Accepted sets (any other returns SGPU_E_INVAL and leaves the setting as it was):
+ *       2 <= adaptor.window: a run at rolling position 0 then maps to sample window/2 - 1 >= 0, inside the read;
+ *       adaptor.window <= 13981: then 1200 * window <= 2^24, so the reference's FLOAT running window sum
+ *         (jnn.c:20-50) holds an exact integer at every step, which the kernel's integer window sums rely on;
+ *       adaptor.std_scale and polya.stall_len finite;
+ *       polya.error >= 0 and polya.corrector >= 0: then w >= 1 wherever the reference computes c % w.
+ *     Every other value is accepted: negative seg_dist, lo_thresh > hi_thresh (no run is plausible),
+ *     polya.window <= 0, polya.error = INT32_MAX.
+ * NULL restores the reference's sets (the adaptor's chosen by SGPU_PARAM_PORE). */
+typedef struct {          /* jnnv2's parameters (JNNV2_RNA_R9_ADAPTOR / _RNA004_ADAPTOR, jnn.h:88-102) */
+    int32_t window;       /* rolling-mean window: 2000 */
+    float   std_scale;    /* floor = mean - std_scale * stdv of the rolling means: 0.5 (R9), 0.7 (RNA004) */
+    int32_t seg_dist;     /* runs that start closer than this to the previous run's end are merged: 1500 */
+    int32_t lo_thresh;    /* shortest plausible run: 2000 (R9), 500 (RNA004) */
+    int32_t hi_thresh;    /* longest plausible run: 200000 */
+} sgpu_adaptor_t;
+typedef struct {          /* jnn_core's parameters as find_polya uses them (JNNV1_R9_POLYA, jnn.h:47-56) */
+    int32_t window;       /* 250 */
+    float   stall_len;    /* 1.0: the first segment needs fl((float)window * stall_len) samples only */
+    int32_t error;        /* 30 tolerated outliers */
+    int32_t seg_dist;     /* 200 */
+    int32_t corrector;    /* 50 */
+} sgpu_polya_t;
+typedef struct { sgpu_adaptor_t adaptor; sgpu_polya_t polya; } sgpu_prefix_t;
+int  sgpu_set_prefix(sgpu_ctx_t *ctx, const sgpu_prefix_t *p);
 
 /* Device time of every kernel group of the last run, measured with CUDA events on the stream the kernels were
  * launched on (needs SGPU_F_STAGE_TIMERS). Returns the number of entries written, or a negative code. */

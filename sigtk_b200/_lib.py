@@ -27,7 +27,7 @@ EXPORTS = (
     "sgpu_wait", "sgpu_run_device", "sgpu_counters", "sgpu_memcpy_d2h", "sgpu_stage_times",
     "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
     "sgpu_run_device_pa", "sgpu_live_open", "sgpu_slot_add_live", "sgpu_wait_live", "sgpu_run_device_live",
-    "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa", "sgpu_set_detector", "sgpu_set_jnn",
+    "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa", "sgpu_set_detector", "sgpu_set_jnn", "sgpu_set_prefix",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -115,6 +115,20 @@ class JnnParams(C.Structure):  # sgpu_jnn_t (jnn_param_t, jnn.h:24-45)
                 ("corrector", C.c_int32), ("std_scale", C.c_float)]
 
 
+class AdaptorParams(C.Structure):  # sgpu_adaptor_t (jnnv2's parameters, jnn.h:88-102)
+    _fields_ = [("window", C.c_int32), ("std_scale", C.c_float), ("seg_dist", C.c_int32), ("lo_thresh", C.c_int32),
+                ("hi_thresh", C.c_int32)]
+
+
+class PolyaParams(C.Structure):  # sgpu_polya_t (jnn_core's parameters as find_polya uses them, jnn.h:47-56)
+    _fields_ = [("window", C.c_int32), ("stall_len", C.c_float), ("error", C.c_int32), ("seg_dist", C.c_int32),
+                ("corrector", C.c_int32)]
+
+
+class PrefixParams(C.Structure):  # sgpu_prefix_t
+    _fields_ = [("adaptor", AdaptorParams), ("polya", PolyaParams)]
+
+
 class StageTime(C.Structure):  # sgpu_stage_time_t
     _fields_ = [("name", C.c_char_p), ("ms", C.c_float), ("launches", C.c_uint32)]
 
@@ -187,5 +201,7 @@ def load() -> C.CDLL:
     lib.sgpu_set_detector.restype = i32
     lib.sgpu_set_jnn.argtypes = [vp, C.POINTER(JnnParams)]
     lib.sgpu_set_jnn.restype = i32
+    lib.sgpu_set_prefix.argtypes = [vp, C.POINTER(PrefixParams)]
+    lib.sgpu_set_prefix.restype = i32
     _lib = lib
     return lib

@@ -51,6 +51,38 @@ Jnn.CDNA_R9 = Jnn(150, 0.25, 5, 50, 50, 0.75)   # JNNV1_CDNA_R9_PARAM
 Jnn.DRNA_R9 = Jnn(1000, 1.0, 5, 50, 50, 0.75)   # JNNV1_DRNA_R9_PARAM
 
 
+class Adaptor(NamedTuple):
+    """jnnv2's parameters (jnn.h:88-102): the reference's sets are Adaptor.RNA_R9 and Adaptor.RNA004"""
+    window: int         # rolling-mean window in samples, 2 .. 13981
+    std_scale: float    # floor = mean - std_scale * stdv of the rolling means
+    seg_dist: int       # runs that start closer than this to the previous run's end are merged
+    lo_thresh: int      # shortest plausible run
+    hi_thresh: int      # longest plausible run
+
+
+Adaptor.RNA_R9 = Adaptor(2000, 0.5, 1500, 2000, 200000)   # JNNV2_RNA_R9_ADAPTOR
+Adaptor.RNA004 = Adaptor(2000, 0.7, 1500, 500, 200000)    # JNNV2_RNA_RNA004_ADAPTOR
+
+
+class Polya(NamedTuple):
+    """jnn_core's parameters as find_polya uses them (jnn.h:47-56; its band comes from the adaptor's mean): the
+    reference's set is Polya.R9"""
+    window: int         # stretch length in samples that counts as a segment
+    stall_len: float    # the first segment needs window * stall_len samples only
+    error: int          # tolerated outliers in a stretch, >= 0
+    seg_dist: int       # merge distance
+    corrector: int      # initial value of the corrector, >= 0
+
+
+Polya.R9 = Polya(250, 1.0, 30, 200, 50)   # JNNV1_R9_POLYA
+
+
+class Prefix(NamedTuple):
+    """the sets of `sigtk prefix` (sgpu_set_prefix): Prefix(Adaptor.RNA_R9, Polya.R9) is prefix_func's for an R9 pore"""
+    adaptor: Adaptor
+    polya: Polya
+
+
 @dataclass
 class EventTable:
     """event_table of one read (src/sigtk.h:65-70) as arrays."""
@@ -352,6 +384,17 @@ class Context:
             return
         p = _lib.JnnParams(int(jnn[0]), float(jnn[1]), int(jnn[2]), int(jnn[3]), int(jnn[4]), float(jnn[5]))
         self._check(self._lib.sgpu_set_jnn(self._h, C.byref(p)))
+
+    def set_prefix(self, prefix: Optional[Prefix]) -> None:
+        """sgpu_set_prefix: WANT_PREFIX of every later batch (host slots from their submit, device-resident runs) uses
+        `prefix`; None restores the reference's sets, the adaptor's chosen by PARAM_PORE"""
+        if prefix is None:
+            self._check(self._lib.sgpu_set_prefix(self._h, None))
+            return
+        a, y = prefix[0], prefix[1]
+        p = _lib.PrefixParams(_lib.AdaptorParams(int(a[0]), float(a[1]), int(a[2]), int(a[3]), int(a[4])),
+                              _lib.PolyaParams(int(y[0]), float(y[1]), int(y[2]), int(y[3]), int(y[4])))
+        self._check(self._lib.sgpu_set_prefix(self._h, C.byref(p)))
 
     def set_param(self, key: int, value: float) -> None:
         """development / test parameters (_lib.PARAM_*): chunk length, detector warm-up, the long detector's threshold"""

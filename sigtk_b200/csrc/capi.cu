@@ -143,6 +143,8 @@ struct Slot {
     DetParams det_set{};
     const JnnParams* jnn = nullptr;  // the context's jnn set at sgpu_submit (&jnn_set), or nullptr: jnn_print's by rna
     JnnParams jnn_set{};
+    const PrefixParams* prefix = nullptr;  // the context's prefix set at sgpu_submit (&prefix_set), or nullptr: the
+    PrefixParams prefix_set{};             // reference's, the adaptor's chosen by SGPU_PARAM_PORE
     Input kind = Input::NONE;        // (PA, LIVE_PA: the floats are in the sample buffers, max_samples / 2 of them)
     // svb-zd input (allocated on first use): the batch's compressed streams, decoded in HBM by svbzd.cu
     PinBuf<uint8_t> h_comp;          // comp_cap bytes
@@ -186,6 +188,8 @@ struct sgpu_ctx {
     DetParams det{};
     bool jnn_on = false;         // sgpu_set_jnn: SGPU_WANT_JNN uses `jnn` instead of jnn_print's sets
     JnnParams jnn{};
+    bool prefix_on = false;      // sgpu_set_prefix: SGPU_WANT_PREFIX uses `prefix` instead of prefix_func's sets
+    PrefixParams prefix{};
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
@@ -412,7 +416,7 @@ int general_events(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetP
 // (except when the general route's scratch grows). set: the caller's detector set, whose events take the general
 // route, or nullptr: the reference's sets on the fast path. jnn: the caller's jnn set, or nullptr: jnn_print's (b.rna).
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
-                 const DetParams* set, const JnnParams* jnn, const SvbBatch* svb = nullptr,
+                 const DetParams* set, const JnnParams* jnn, const PrefixParams* prefix, const SvbBatch* svb = nullptr,
                  int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
     if (!fits(ctx, b)) return SGPU_E_INVAL;
@@ -451,7 +455,8 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
                                           static_cast<int32_t*>(o[JNN_SEG].get()), ctx->sm_count, st));
     }
     if (want & SGPU_WANT_PREFIX)
-        marks.done("prefix", launch_prefix(b, ctx->pore_rna004, static_cast<int32_t*>(o[PREFIX_POS].get()),
+        marks.done("prefix", launch_prefix(b, prefix ? *prefix : prefix_params(ctx->pore_rna004),
+                                           static_cast<int32_t*>(o[PREFIX_POS].get()),
                                            static_cast<float*>(o[PREFIX_STAT].get()), ctx->sm_count, st));
     if (events && set) {
         if (const int rc = general_events(ctx, b, nullptr, set, o, marks)) return rc;
@@ -537,7 +542,7 @@ int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
     const DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, rna, sl.used};
     const SvbBatch svb{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
                        sl.svb_blocks};
-    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.jnn,
+    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.jnn, sl.prefix,
                         sl.kind == Input::SVBZD ? &svb : nullptr, sl.d_samples);
 }
 
@@ -946,6 +951,8 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     sl.det = ctx->det_on ? &sl.det_set : nullptr;
     sl.jnn_set = ctx->jnn;  // and the jnn set in force now
     sl.jnn = ctx->jnn_on ? &sl.jnn_set : nullptr;
+    sl.prefix_set = ctx->prefix;  // and the prefix set in force now
+    sl.prefix = ctx->prefix_on ? &sl.prefix_set : nullptr;
     if (live) {
         if ((rc = fit_live_staging(ctx, sl.det))) return rc;
         CU(fit_live_outputs(ctx, sl.live_dout, sl.live_dcap));
@@ -1003,7 +1010,8 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     DevBatch b{batch->samples, batch->read_off, batch->read_len, batch->offset_f, batch->raw_unit_f,
                batch->n_reads, (int)batch->rna, batch->span};
     const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream),
-                                ctx->det_on ? &ctx->det : nullptr, ctx->jnn_on ? &ctx->jnn : nullptr);
+                                ctx->det_on ? &ctx->det : nullptr, ctx->jnn_on ? &ctx->jnn : nullptr,
+                                ctx->prefix_on ? &ctx->prefix : nullptr);
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(OUTS, out, ctx->dev_out, want, true);
@@ -1107,6 +1115,23 @@ int sgpu_set_jnn(sgpu_ctx_t* ctx, const sgpu_jnn_t* p) {
         return SGPU_E_INVAL;
     ctx->jnn = JnnParams{p->window, p->stall_len, p->error, p->seg_dist, p->corrector, p->std_scale};
     ctx->jnn_on = true;
+    return SGPU_OK;
+}
+
+int sgpu_set_prefix(sgpu_ctx_t* ctx, const sgpu_prefix_t* p) {
+    if (!ctx) return SGPU_E_INVAL;
+    if (!p) { ctx->prefix_on = false; return SGPU_OK; }
+    const sgpu_adaptor_t& a = p->adaptor;
+    const sgpu_polya_t& y = p->polya;
+    // window >= 2: a run at rolling position 0 maps to sample window/2 - 1 >= 0; window <= 13981: 1200 * window <= 2^24,
+    // so the reference's float window sum is an exact integer at every step (the kernel's integer sums). error >= 0
+    // and corrector >= 0: w >= 1 wherever the reference takes c % w
+    if (a.window < 2 || a.window > 13981 || !std::isfinite(a.std_scale) || y.error < 0 || y.corrector < 0 ||
+        !std::isfinite(y.stall_len))
+        return SGPU_E_INVAL;
+    ctx->prefix = PrefixParams{a.window, a.std_scale, a.seg_dist, a.lo_thresh, a.hi_thresh,
+                               y.window, y.stall_len, y.error, y.seg_dist, y.corrector};
+    ctx->prefix_on = true;
     return SGPU_OK;
 }
 

@@ -266,7 +266,25 @@ int launch_jnn(const DevBatch& b, const JnnParams& p, const float* moments, uint
 
 
 // prefix.cu (`sigtk prefix`: adaptor by jnnv2 on the rolling mean, poly-A by jnn_core on pA, statistics of both)
-int launch_prefix(const DevBatch& b, int rna004, int32_t* pos4, float* st6, int sm_count, cudaStream_t st);
+struct PrefixParams {  // sgpu_prefix_t: jnnv2's adaptor set (jnn.h:88-102), then jnn_core's poly-A set (jnn.h:47-56)
+    int a_window;
+    float a_std_scale;
+    int a_seg_dist, a_lo, a_hi;
+    int p_window;
+    float p_stall_len;
+    int p_error, p_seg_dist, p_corrector;
+};
+// the sets prefix_func uses (cfunc.c:169-234): JNNV2_RNA_R9_ADAPTOR, or JNNV2_RNA_RNA004_ADAPTOR when SGPU_PARAM_PORE
+// says RNA004, and JNNV1_R9_POLYA
+__host__ __device__ inline PrefixParams prefix_params(int rna004) {
+    PrefixParams p;
+    p.a_window = 2000; p.a_std_scale = rna004 ? 0.7f : 0.5f; p.a_seg_dist = 1500; p.a_lo = rna004 ? 500 : 2000;
+    p.a_hi = 200000;
+    p.p_window = 250; p.p_stall_len = 1.0f; p.p_error = 30; p.p_seg_dist = 200; p.p_corrector = 50;
+    return p;
+}
+// p: prefix_params(SGPU_PARAM_PORE), or the caller's set (every set sgpu_set_prefix accepts)
+int launch_prefix(const DevBatch& b, const PrefixParams& p, int32_t* pos4, float* st6, int sm_count, cudaStream_t st);
 
 // ent.cu (`sigtk ent`: entropies of the raw samples, their zig-zag deltas and the deltas' byte planes)
 uint64_t ent_overflow_words(int sm_count);
