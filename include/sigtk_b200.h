@@ -63,6 +63,10 @@ extern "C" {
 #define SGPU_WANT_PREFIX  32u /* `sigtk prefix` (prefix_func, cfunc.c:169-234): find_adaptor (jnnv2, jnn.c:99-188), the
                                  adaptor's pA statistics, find_polya (jnn.c:352-374) when rna, its statistics; with
                                  the reference's sets or the caller's (sgpu_set_prefix) */
+#define SGPU_WANT_SVBZD   64u /* each read's raw signal as slow5lib stores it with SLOW5_COMPRESS_SVB_ZD
+                                 (ptr_compress_svb_zd, slow5_press.c; streamvbyte_encode.c, streamvbyte_zigzag.c):
+                                 host slots of int16 records or svb-zd streams only, read with sgpu_slot_svbzd; the
+                                 device-resident form is sgpu_encode_svbzd_device (sgpu_run_device refuses this bit) */
 
 /* ---- context flags ------------------------------------------------------ */
 #define SGPU_F_DEFAULT       0u
@@ -185,7 +189,8 @@ typedef struct {
 /* Runs the kernels on `stream` (a cudaStream_t passed as void*, NULL = the
  * legacy default stream) without any host<->device copies or synchronisation.
  * *out receives DEVICE pointers owned by the context (valid until the next
- * run on this context). */
+ * run on this context). SGPU_WANT_SVBZD is refused (SGPU_E_INVAL): sgpu_result_t
+ * cannot carry the streams; sgpu_encode_svbzd_device computes them. */
 int  sgpu_run_device(sgpu_ctx_t *ctx, const sgpu_dev_batch_t *batch, uint32_t want,
                      void *stream, sgpu_result_t *out);
 
@@ -224,6 +229,38 @@ typedef struct {
     uint64_t n_blocks;
 } sgpu_svb_dev_batch_t;
 int  sgpu_decode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_svb_dev_batch_t *batch, int16_t *samples_out, void *stream);
+
+/* ---- svb-zd encode: int16 samples in HBM -> the streams slow5lib stores ----------------------------------------
+ * What ptr_compress_svb_zd (slow5lib/src/slow5_press.c; streamvbyte_encode.c, streamvbyte_zigzag.c) writes for a
+ * record's raw signal with SLOW5_COMPRESS_SVB_ZD, byte for byte: uint32 count | ceil(count/4) key bytes | data bytes,
+ * value i = zigzag(raw[i] - raw[i-1]) in 32-bit arithmetic, raw[-1] = 0, in the fewest little-endian bytes (1 to 3 for
+ * int16 samples). An empty read gives the 4-byte header. Each stream starts on a 16-byte boundary and is followed by
+ * zeros up to the next one; the buffer extends at least 8 bytes past n_bytes. So the result feeds sgpu_decode_svbzd_device
+ * (bytes, n_bytes = comp_off[n_reads], comp_off, comp_len) unchanged, and each stream sgpu_slot_add_read_svbzd.
+ *   - Host slots: SGPU_WANT_SVBZD in sgpu_submit, on slots of int16 records, of svb-zd streams (whose decoded samples
+ *     are encoded again: slow5lib's streams come back as they were, any other valid stream in this canonical form) or
+ *     empty slots, with any other bit; slots of pA records or live entries refuse it (SGPU_E_INVAL). comp_off and
+ *     comp_len come back with the small results, sgpu_wait copies exactly n_bytes bytes. sgpu_slot_svbzd then hands
+ *     out the slot's pinned copies (host pointers, n_bytes set), valid until the slot is reset or submitted again;
+ *     before that wait, or for a slot submitted without the bit, it returns SGPU_E_STATE.
+ *   - Device-resident: sgpu_encode_svbzd_device encodes the caller's batch (offset_f, raw_unit_f and rna are not
+ *     read) on `stream` without copies or synchronisation; *out receives DEVICE pointers owned by the context, valid
+ *     until the next encode run, n_bytes 0 (comp_off[n_reads] on the device holds it).
+ *   - Limit: comp_len is a uint32_t, so a read must satisfy SGPU_SVBZD_MAX_BYTES(n) <= 2^32 - 1, i.e. n <=
+ *     1,321,528,397 samples. sgpu_submit with the bit refuses a batch holding a longer read, and
+ *     sgpu_encode_svbzd_device a batch whose span is longer (it knows only the span), with SGPU_E_TOOBIG. A context
+ *     whose max_samples is at most that never meets the case.
+ *   - Buffers: allocated on the first run that wants them, at most 3.25 * max_samples + 20 * max_reads + 16 bytes
+ *     (pinned: per slot). */
+#define SGPU_SVBZD_MAX_BYTES(n) (4u + ((uint64_t)(n) + 3u) / 4u + 3u * (uint64_t)(n)) /* longest stream of n int16 samples */
+typedef struct {
+    uint8_t  *bytes;     /* stream r = bytes[comp_off[r] .. comp_off[r] + comp_len[r]); zero bytes up to the next 16-byte boundary */
+    uint64_t *comp_off;  /* [n_reads + 1], multiples of 16; comp_off[n_reads] = aligned end of the last stream */
+    uint32_t *comp_len;  /* [n_reads] */
+    uint64_t  n_bytes;   /* = comp_off[n_reads] (host result; 0 from the device path) */
+} sgpu_svb_result_t;
+int  sgpu_slot_svbzd(sgpu_ctx_t *ctx, uint32_t slot, sgpu_svb_result_t *out);
+int  sgpu_encode_svbzd_device(sgpu_ctx_t *ctx, const sgpu_dev_batch_t *batch, void *stream, sgpu_svb_result_t *out);
 
 /* ---- live event detection: signal that arrives in chunks, channel by channel ----------------------------------
  * For tools that segment signal while the read is still in the pore (adaptive sampling, Read Until): per channel, a

@@ -13,7 +13,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsigtk_b200.so")
 
-WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX = 1, 2, 4, 8, 16, 32
+WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, WANT_SVBZD = 1, 2, 4, 8, 16, 32, 64
 F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS = 0, 1, 2, 4
 ALIGN = 8
 
@@ -28,6 +28,7 @@ EXPORTS = (
     "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
     "sgpu_run_device_pa", "sgpu_live_open", "sgpu_slot_add_live", "sgpu_wait_live", "sgpu_run_device_live",
     "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa", "sgpu_set_detector", "sgpu_set_jnn", "sgpu_set_prefix",
+    "sgpu_slot_svbzd", "sgpu_encode_svbzd_device",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -74,6 +75,10 @@ class SvbDevBatch(C.Structure):  # sgpu_svb_dev_batch_t
         ("bytes", C.c_void_p), ("n_bytes", C.c_uint64), ("comp_off", C.c_void_p), ("comp_len", C.c_void_p),
         ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("n_reads", C.c_uint32), ("n_blocks", C.c_uint64),
     ]
+
+
+class SvbResult(C.Structure):  # sgpu_svb_result_t
+    _fields_ = [("bytes", C.c_void_p), ("comp_off", C.c_void_p), ("comp_len", C.c_void_p), ("n_bytes", C.c_uint64)]
 
 
 class LiveResult(C.Structure):  # sgpu_live_result_t
@@ -203,5 +208,9 @@ def load() -> C.CDLL:
     lib.sgpu_set_jnn.restype = i32
     lib.sgpu_set_prefix.argtypes = [vp, C.POINTER(PrefixParams)]
     lib.sgpu_set_prefix.restype = i32
+    lib.sgpu_slot_svbzd.argtypes = [vp, u32, C.POINTER(SvbResult)]
+    lib.sgpu_slot_svbzd.restype = i32
+    lib.sgpu_encode_svbzd_device.argtypes = [vp, C.POINTER(DevBatch), vp, C.POINTER(SvbResult)]
+    lib.sgpu_encode_svbzd_device.restype = i32
     _lib = lib
     return lib

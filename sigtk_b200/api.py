@@ -19,7 +19,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS, LIVE_END, LIVE_RNA, LIVE_START,
-                   WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, SgpuError)
+                   WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, WANT_SVBZD, SgpuError)
 
 Read = Tuple[np.ndarray, float, float, float]  # raw int16, digitisation, offset, range
 LiveEntry = Tuple[int, int, np.ndarray, float, float, float]  # channel, LIVE_* flags, raw int16, digitisation, offset,
@@ -112,6 +112,7 @@ class BatchResult:
     prefix_stat: Optional[np.ndarray] = None  # [n_reads][6] float32: mean, stdv, median of both stretches' pA
     seq_order: Optional[np.ndarray] = None
     fixups: Optional[np.ndarray] = None
+    svbzd: Optional[List[np.ndarray]] = None  # per read uint8: the svb-zd stream slow5lib stores (WANT_SVBZD)
 
     def events(self, r: int) -> EventTable:
         a, b = int(self.ev_off[r]), int(self.ev_off[r + 1])
@@ -261,6 +262,13 @@ class Context:
             span = int(read_off[n]) if n else 0
             flat = _np_from(res.pa, np.float32, span)
             out.pa = [flat[int(read_off[r]): int(read_off[r]) + int(read_len[r])].copy() for r in range(n)]
+        if want & WANT_SVBZD:
+            sv = _lib.SvbResult()
+            self._check(self._lib.sgpu_slot_svbzd(self._h, slot, C.byref(sv)))
+            off = _np_from(sv.comp_off, np.uint64, n + 1)
+            ln = _np_from(sv.comp_len, np.uint32, n)
+            flat = _np_from(sv.bytes, np.uint8, int(sv.n_bytes))
+            out.svbzd = [flat[int(off[r]): int(off[r]) + int(ln[r])].copy() for r in range(n)]
         return out
 
     def run(self, reads: Sequence[Read], rna: int = 0, want: int = WANT_EVENTS, slot: int = 0) -> BatchResult:
@@ -347,6 +355,16 @@ class Context:
         self._check(self._lib.sgpu_run_device_pa(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res)))
         return res
 
+    def encode_svbzd_device(self, samples_ptr: int, read_off_ptr: int, read_len_ptr: int, n_reads: int, span: int,
+                            stream: int = 0) -> _lib.SvbResult:
+        """sgpu_encode_svbzd_device: the svb-zd streams of int16 reads already in device memory (read_off multiples of
+        ALIGN); -> device pointers (bytes, comp_off, comp_len), valid until the next encode run; the total is
+        comp_off[n_reads]"""
+        db = _lib.DevBatch(samples_ptr, read_off_ptr, read_len_ptr, None, None, n_reads, 0, span)
+        res = _lib.SvbResult()
+        self._check(self._lib.sgpu_encode_svbzd_device(self._h, C.byref(db), C.c_void_p(stream), C.byref(res)))
+        return res
+
     def d2h(self, dev_ptr: int, dtype, count: int) -> np.ndarray:
         """copy `count` items of a device result array (a pointer from run_device) to a new numpy array"""
         out = np.empty(count, dtype=dtype)
@@ -426,6 +444,11 @@ def stat(ctx: Context, raw: np.ndarray, digitisation: float, offset: float, rang
 def ent(ctx: Context, raw: np.ndarray) -> np.ndarray:
     """raw_ent, delta_ent, byte_ent of one record as `sigtk ent` prints them (ent.c:108-151)."""
     return ctx.run([(raw, 8192.0, 0.0, 1.0)], 0, WANT_ENT).ent[0]
+
+
+def svbzd_encode(ctx: Context, raw: np.ndarray) -> np.ndarray:
+    """The svb-zd stream slow5lib stores for one record's raw signal (ptr_compress_svb_zd), encoded on the GPU."""
+    return ctx.run([(raw, 8192.0, 0.0, 1.0)], 0, WANT_SVBZD).svbzd[0]
 
 
 def jnn_raw(ctx: Context, raw: np.ndarray, rna: int = 0) -> np.ndarray:

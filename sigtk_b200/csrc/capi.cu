@@ -21,17 +21,20 @@ using namespace sgpu;
 
 namespace {
 
-// The output arrays. OUTS describes each per-batch output once, LIVE_OUTS each output of a live run; every place that
-// allocates, clears, copies back or returns outputs loops over one of them. Device and pinned host copies are arrays of
-// byte buffers indexed by Out (or Live).
+// The output arrays. OUTS describes each per-batch output once, LIVE_OUTS each output of a live run, SVB_OUTS each
+// output of the svb-zd encoder; every place that allocates, clears, copies back or returns outputs loops over one of
+// them. Device and pinned host copies are arrays of byte buffers indexed by Out (or Live, Svb).
 enum Out { EV_OFF, EV_START, EV_MEAN, EV_STDV, SEQ_ORDER, FIXUPS, STAT, ENT, JNN_CNT, JNN_SEG, PREFIX_POS, PREFIX_STAT,
            PA, N_OUT };
 enum Live { LIVE_EV_OFF, LIVE_EV_START, LIVE_EV_LEN, LIVE_EV_MEAN, LIVE_EV_STDV, N_LIVE_OUT };
-static_assert(EV_OFF == 0 && LIVE_EV_OFF == 0, "row 0 of both tables: ev_off, which sizes the event outputs");
+enum Svb { SVB_COMP_OFF, SVB_COMP_LEN, SVB_BYTES, N_SVB_OUT };
+static_assert(EV_OFF == 0 && LIVE_EV_OFF == 0 && SVB_COMP_OFF == 0,
+              "row 0 of every table: ev_off or comp_off, whose entry [n_reads] sizes the outputs counted by TOTAL");
 
 // what an output's element count is proportional to (times OutSpec::per)
 enum Count : uint8_t {
-    READS, READS_PLUS_1, EVENTS,
+    READS, READS_PLUS_1,
+    TOTAL,      // the batch's events (OUTS, LIVE_OUTS) or stream bytes (SVB_OUTS), at capacity the table's capacity
     SAMPLES,    // of the batch's span
     JNN_SLOTS,  // jnn_seg_capacity(): segment slots of the span's reads (SGPU_JNN_BASE)
 };
@@ -39,7 +42,7 @@ enum Count : uint8_t {
 constexpr int ANY_WANT = 0x100;  // OutSpec::empty flag: cleared for an empty batch whatever the want
 
 struct OutSpec {
-    size_t field;    // offset of its pointer in sgpu_result_t (LIVE_OUTS: sgpu_live_result_t)
+    size_t field;    // offset of its pointer in sgpu_result_t (LIVE_OUTS: sgpu_live_result_t, SVB_OUTS: sgpu_svb_result_t)
     uint32_t size;   // bytes per element
     uint32_t want;   // SGPU_WANT_* bit of the product it belongs to
     Count count;
@@ -54,9 +57,9 @@ struct OutSpec {
 constexpr OutSpec OUTS[] = {  // in the order of Out
     //     field        want              count         per  eager  empty         pa_in
     OUTPUT(ev_off,      SGPU_WANT_EVENTS, READS_PLUS_1, 1,   true,  0 | ANY_WANT, true),
-    OUTPUT(ev_start,    SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
-    OUTPUT(ev_mean,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
-    OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, EVENTS,       1,   true,  -1,           true),
+    OUTPUT(ev_start,    SGPU_WANT_EVENTS, TOTAL,        1,   true,  -1,           true),
+    OUTPUT(ev_mean,     SGPU_WANT_EVENTS, TOTAL,        1,   true,  -1,           true),
+    OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, TOTAL,        1,   true,  -1,           true),
     OUTPUT(seq_order,   SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
     OUTPUT(fixups,      SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
     OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0,            false),
@@ -70,19 +73,30 @@ constexpr OutSpec OUTS[] = {  // in the order of Out
 #undef OUTPUT
 static_assert(sizeof OUTS / sizeof OUTS[0] == N_OUT, "one row per output");
 
-// the events of a live run, entry by entry (EVENTS: at the capacity LiveScratch::ev_cap)
+// the events of a live run, entry by entry (TOTAL: at the capacity LiveScratch::ev_cap)
 #define LIVE_OUTPUT(field, count, empty) \
     { offsetof(sgpu_live_result_t, field), sizeof *sgpu_live_result_t{}.field, SGPU_WANT_EVENTS, count, 1, true, empty, \
       false }
 constexpr OutSpec LIVE_OUTS[] = {  // in the order of Live
     LIVE_OUTPUT(ev_off,   READS_PLUS_1, 0 | ANY_WANT),
-    LIVE_OUTPUT(ev_start, EVENTS,       -1),
-    LIVE_OUTPUT(ev_len,   EVENTS,       -1),
-    LIVE_OUTPUT(ev_mean,  EVENTS,       -1),
-    LIVE_OUTPUT(ev_stdv,  EVENTS,       -1),
+    LIVE_OUTPUT(ev_start, TOTAL,        -1),
+    LIVE_OUTPUT(ev_len,   TOTAL,        -1),
+    LIVE_OUTPUT(ev_mean,  TOTAL,        -1),
+    LIVE_OUTPUT(ev_stdv,  TOTAL,        -1),
 };
 #undef LIVE_OUTPUT
 static_assert(sizeof LIVE_OUTS / sizeof LIVE_OUTS[0] == N_LIVE_OUT, "one row per output");
+
+// the svb-zd streams of a batch (TOTAL: at the capacity svbzd_encode_capacity)
+#define SVB_OUTPUT(field, count) \
+    { offsetof(sgpu_svb_result_t, field), sizeof *sgpu_svb_result_t{}.field, SGPU_WANT_SVBZD, count, 1, false, -1, false }
+constexpr OutSpec SVB_OUTS[] = {  // in the order of Svb
+    SVB_OUTPUT(comp_off, READS_PLUS_1),
+    SVB_OUTPUT(comp_len, READS),
+    SVB_OUTPUT(bytes,    TOTAL),
+};
+#undef SVB_OUTPUT
+static_assert(sizeof SVB_OUTS / sizeof SVB_OUTS[0] == N_SVB_OUT, "one row per output");
 
 // the products a run on pA input can compute: those of its outputs (the others are defined on int16 raw samples, and
 // pA is the input itself)
@@ -98,7 +112,7 @@ uint64_t out_elems(const OutSpec& s, uint64_t reads, uint64_t samples, uint64_t 
     switch (s.count) {
         case READS: return s.per * reads;
         case READS_PLUS_1: return s.per * (reads + 1);
-        case EVENTS: return s.per * events;
+        case TOTAL: return s.per * events;
         case SAMPLES: return s.per * samples;
         case JNN_SLOTS: return s.per * jnn_seg_capacity(samples, (uint32_t)reads);
     }
@@ -115,7 +129,7 @@ bool is_live(Input k) { return k == Input::LIVE || k == Input::LIVE_PA; }
 uint32_t allowed_wants(Input k) {
     if (k == Input::PA) return pa_input_wants();
     if (is_live(k)) return SGPU_WANT_EVENTS;
-    return 63u;
+    return 127u;
 }
 
 struct Slot {
@@ -133,6 +147,10 @@ struct Slot {
     DevBuf<float> d_offset, d_unit;
     DevBuf<void> dout[N_OUT];  // device outputs
     PinBuf<void> hout[N_OUT];  // their pinned host copies
+    DevBuf<void> svb_dout[N_SVB_OUT];  // the svb-zd streams of SGPU_WANT_SVBZD
+    PinBuf<void> svb_hout[N_SVB_OUT];
+    bool svb_ready = false;            // svb_hout holds the streams of the last sgpu_wait (n_bytes of them)
+    uint64_t svb_bytes = 0;
     PinBuf<unsigned long long> h_counters;  // [4]
     PinBuf<int> h_status;
     cudaStream_t stream = nullptr;
@@ -180,6 +198,7 @@ struct sgpu_ctx {
     uint64_t ev_cap = 0;
     Scratch sc{};
     DevBuf<void> dev_out[N_OUT]; // outputs of the device-resident path
+    DevBuf<void> svb_dev_out[N_SVB_OUT];  // and of sgpu_encode_svbzd_device
     std::unique_ptr<Slot[]> slots;
     SvbScratch svb{};            // workspace of the svb-zd decoder (allocated on first use)
     DevBuf<float> jnn_mom;       // [max_reads][2] mean / stdv of the clamped signal (allocated on first use)
@@ -257,13 +276,13 @@ void fill_result(const OutSpec (&outs)[N], R* r, const Buf<void, PINNED>* o, uin
 }
 
 // queues on the slot's stream the D2H copy (d to h) of every output of `want` that is sized by the batch's reads and
-// samples, or (by_events) of every one sized by its n_events
+// samples, or (by_total) of every one sized by its total (n_events, or the stream bytes)
 template <size_t N>
 cudaError_t queue_d2h(const OutSpec (&outs)[N], const DevBuf<void>* d, PinBuf<void>* h, const Slot& sl, uint32_t want,
-                      bool by_events, uint64_t n_events) {
+                      bool by_total, uint64_t total) {
     for (size_t k = 0; k < N; k++) {
-        if (!(want & outs[k].want) || (outs[k].count == EVENTS) != by_events) continue;
-        const uint64_t n = out_elems(outs[k], sl.batch.n_reads, sl.used, n_events);
+        if (!(want & outs[k].want) || (outs[k].count == TOTAL) != by_total) continue;
+        const uint64_t n = out_elems(outs[k], sl.batch.n_reads, sl.used, total);
         const cudaError_t e = cudaMemcpyAsync(h[k], d[k], (size_t)n * outs[k].size, cudaMemcpyDeviceToHost, sl.stream);
         if (e != cudaSuccess) return e;
     }
@@ -412,10 +431,25 @@ int general_events(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetP
     return SGPU_OK;
 }
 
-// The kernel sequence of one batch into the device outputs `o`. No host synchronisation, no host<->device copies
-// (except when the general route's scratch grows). set: the caller's detector set, whose events take the general
-// route, or nullptr: the reference's sets on the fast path. jnn: the caller's jnn set, or nullptr: jnn_print's (b.rna).
-int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, cudaStream_t st,
+// whether every stream of a read of n samples fits comp_len's uint32_t: n <= 1,321,528,397
+bool svbzd_stream_fits(uint64_t n) { return SGPU_SVBZD_MAX_BYTES(n) <= 0xffffffffull; }
+
+// The svb-zd streams of b's int16 samples into the outputs `o` of SVB_OUTS (allocated on the first run that wants them).
+int encode_svbzd(sgpu_ctx* ctx, const DevBatch& b, DevBuf<void>* o, StageMarks& marks) {
+    CU(alloc_outputs(SVB_OUTS, ctx, svbzd_encode_capacity(ctx->max_samples, ctx->max_reads), o, SGPU_WANT_SVBZD));
+    if (const int rc = alloc_svb_scratch(ctx)) return rc;
+    marks.done("svbzd_encode", launch_svbzd_encode(b, static_cast<uint8_t*>(o[SVB_BYTES].get()),
+                                                   static_cast<uint64_t*>(o[SVB_COMP_OFF].get()),
+                                                   static_cast<uint32_t*>(o[SVB_COMP_LEN].get()), ctx->svb, ctx->sc,
+                                                   ctx->sm_count, marks.st));
+    return SGPU_OK;
+}
+
+// The kernel sequence of one batch into the device outputs `o` (and the svb-zd streams into `enc`). No host
+// synchronisation, no host<->device copies (except when the general route's scratch grows). set: the caller's detector
+// set, whose events take the general route, or nullptr: the reference's sets on the fast path. jnn: the caller's jnn
+// set, or nullptr: jnn_print's (b.rna).
+int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, DevBuf<void>* enc, cudaStream_t st,
                  const DetParams* set, const JnnParams* jnn, const PrefixParams* prefix, const SvbBatch* svb = nullptr,
                  int16_t* svb_out = nullptr) {
     Scratch& sc = ctx->sc;
@@ -426,8 +460,11 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
         if (const int rc = prepare_general(ctx, b.span)) return rc;
     StageMarks marks(ctx, st);
     if (const int rc = marks.start()) return rc;
-    if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
-    if (svb) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
+    const bool empty = b.n_reads == 0 || b.span == 0;
+    if (svb && !empty) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
+    if (want & SGPU_WANT_SVBZD)  // (also for empty records: each has its 4-byte stream)
+        if (const int rc = encode_svbzd(ctx, b, enc, marks)) return rc;
+    if (empty) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
     const bool force_generic = (ctx->flags & SGPU_F_FORCE_GENERIC) != 0;
     float* const pa = (want & SGPU_WANT_PA) ? static_cast<float*>(o[PA].get()) : nullptr;
     uint32_t* const seq = static_cast<uint32_t*>(o[SEQ_ORDER].get());
@@ -536,13 +573,14 @@ int run_slot(sgpu_ctx* ctx, Slot& sl, uint32_t want) {
         return run_pipeline_live(ctx, b, sl.kind == Input::LIVE_PA, sl.det, sl.live_dout, ctx->compute);
     }
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, sl.hout, want));
+    CU(alloc_outputs(SVB_OUTS, ctx, svbzd_encode_capacity(ctx->max_samples, ctx->max_reads), sl.svb_hout, want));
     if (sl.kind == Input::PA)
         return run_pipeline_pa(ctx, DevBatch{nullptr, sl.d_read_off, sl.d_read_len, nullptr, nullptr, nr, rna, sl.used},
                                reinterpret_cast<const float*>(sl.d_samples.get()), sl.det, want, sl.dout, ctx->compute);
     const DevBatch b{sl.d_samples, sl.d_read_off, sl.d_read_len, sl.d_offset, sl.d_unit, nr, rna, sl.used};
     const SvbBatch svb{sl.d_comp, sl.comp_used, sl.d_comp_off, sl.d_comp_len, sl.d_read_off, sl.d_read_len, nr,
                        sl.svb_blocks};
-    return run_pipeline(ctx, b, want, sl.dout, ctx->compute, sl.det, sl.jnn, sl.prefix,
+    return run_pipeline(ctx, b, want, sl.dout, sl.svb_dout, ctx->compute, sl.det, sl.jnn, sl.prefix,
                         sl.kind == Input::SVBZD ? &svb : nullptr, sl.d_samples);
 }
 
@@ -684,7 +722,8 @@ cudaError_t fit_live_outputs(const sgpu_ctx* ctx, Buf<void, PINNED> (&o)[N_LIVE_
 }
 
 // sgpu_wait / sgpu_wait_live: the device status of the submitted slot, then its outputs `outs` (device d, pinned h)
-// sized by the batch's events (at most ev_cap of them) copied back, and *out pointed at the pinned copies
+// sized by the batch's events (at most ev_cap of them) and its svb-zd streams copied back, and *out pointed at the
+// pinned copies
 template <size_t N, typename R>
 int wait_slot(sgpu_ctx* ctx, Slot& sl, const OutSpec (&outs)[N], const DevBuf<void>* d, PinBuf<void>* h,
               uint64_t ev_cap, R* out) {
@@ -701,6 +740,13 @@ int wait_slot(sgpu_ctx* ctx, Slot& sl, const OutSpec (&outs)[N], const DevBuf<vo
         CU(queue_d2h(outs, d, h, sl, SGPU_WANT_EVENTS, true, ne));
         CU(cudaStreamSynchronize(sl.stream));
         out->n_events = ne;
+    }
+    if (sl.want & SGPU_WANT_SVBZD) {  // (never on a live slot)
+        const uint64_t nb = static_cast<const uint64_t*>(sl.svb_hout[SVB_COMP_OFF].get())[nr];
+        CU(queue_d2h(SVB_OUTS, sl.svb_dout, sl.svb_hout, sl, SGPU_WANT_SVBZD, true, nb));
+        CU(cudaStreamSynchronize(sl.stream));
+        sl.svb_bytes = nb;
+        sl.svb_ready = true;
     }
     fill_result(outs, out, h, sl.want, false);
     return SGPU_OK;
@@ -877,6 +923,7 @@ int sgpu_slot_reset(sgpu_ctx_t* ctx, uint32_t slot, uint32_t rna) {
     sl.kind = Input::NONE;
     sl.comp_used = 0;
     sl.svb_blocks = 0;
+    sl.svb_ready = false;
     return SGPU_OK;
 }
 
@@ -939,10 +986,13 @@ int64_t sgpu_slot_add_read_pa(sgpu_ctx_t* ctx, uint32_t slot, const float* pa, u
 }
 
 int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
-    if (!ctx || slot >= ctx->n_slots || (want & ~63u) || want == 0) return SGPU_E_INVAL;
+    if (!ctx || slot >= ctx->n_slots || (want & ~127u) || want == 0) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
     if (want & ~allowed_wants(sl.kind)) return SGPU_E_INVAL;
+    if ((want & SGPU_WANT_SVBZD) && !svbzd_stream_fits(ctx->max_samples))  // (only such a context holds such a read)
+        for (uint32_t r = 0; r < sl.batch.n_reads; r++)
+            if (!svbzd_stream_fits(sl.batch.read_len[r])) return SGPU_E_TOOBIG;
     CU(cudaSetDevice(ctx->device));
     const bool live = is_live(sl.kind);
     int rc = live ? check_live_entries(ctx, sl) : SGPU_OK;
@@ -958,6 +1008,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
         CU(fit_live_outputs(ctx, sl.live_dout, sl.live_dcap));
         CU(fit_live_outputs(ctx, sl.live_hout, sl.live_hcap));
     }
+    sl.svb_ready = false;
     const sgpu_batch_t& hb = sl.batch;
     const uint32_t nr = hb.n_reads;
     cudaStream_t st = sl.stream;
@@ -989,6 +1040,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     CU(cudaStreamWaitEvent(st, sl.kernels_done, 0));
     CU(live ? queue_d2h(LIVE_OUTS, sl.live_dout, sl.live_hout, sl, want, false, 0)
             : queue_d2h(OUTS, sl.dout, sl.hout, sl, want, false, 0));
+    CU(queue_d2h(SVB_OUTS, sl.svb_dout, sl.svb_hout, sl, want, false, 0));  // (comp_off sizes the bytes in sgpu_wait)
     CU(cudaEventRecord(sl.small_back, st));
     if (live) advance_live_mirror(ctx, sl);
     sl.want = want;
@@ -1009,7 +1061,7 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
     CU(cudaSetDevice(ctx->device));
     DevBatch b{batch->samples, batch->read_off, batch->read_len, batch->offset_f, batch->raw_unit_f,
                batch->n_reads, (int)batch->rna, batch->span};
-    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, reinterpret_cast<cudaStream_t>(stream),
+    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, nullptr, reinterpret_cast<cudaStream_t>(stream),
                                 ctx->det_on ? &ctx->det : nullptr, ctx->jnn_on ? &ctx->jnn : nullptr,
                                 ctx->prefix_on ? &ctx->prefix : nullptr);
     if (rc) return rc;
@@ -1045,6 +1097,32 @@ int sgpu_decode_svbzd_device(sgpu_ctx_t* ctx, const sgpu_svb_dev_batch_t* batch,
                batch->n_reads, batch->n_blocks};
     ctx->last_launches = (uint64_t)launch_svbzd_decode(s, ctx->svb, ctx->sc, samples_out, ctx->sm_count, st);
     CU(cudaGetLastError());
+    return SGPU_OK;
+}
+
+int sgpu_slot_svbzd(sgpu_ctx_t* ctx, uint32_t slot, sgpu_svb_result_t* out) {
+    if (!ctx || slot >= ctx->n_slots || !out) return SGPU_E_INVAL;
+    const Slot& sl = ctx->slots[slot];
+    if (!sl.svb_ready) return SGPU_E_STATE;
+    memset(out, 0, sizeof *out);
+    fill_result(SVB_OUTS, out, sl.svb_hout, SGPU_WANT_SVBZD, false);
+    out->n_bytes = sl.svb_bytes;
+    return SGPU_OK;
+}
+
+int sgpu_encode_svbzd_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, void* stream, sgpu_svb_result_t* out) {
+    if (!ctx || !batch || !out) return SGPU_E_INVAL;
+    const DevBatch b{batch->samples, batch->read_off, batch->read_len, nullptr, nullptr, batch->n_reads, 0, batch->span};
+    if (!fits(ctx, b)) return SGPU_E_INVAL;
+    if (!svbzd_stream_fits(b.span)) return SGPU_E_TOOBIG;  // (the host does not know the reads' lengths)
+    CU(cudaSetDevice(ctx->device));
+    StageMarks marks(ctx, reinterpret_cast<cudaStream_t>(stream));
+    int rc = marks.start();
+    if (!rc) rc = encode_svbzd(ctx, b, ctx->svb_dev_out, marks);
+    if (!rc) rc = marks.finish();
+    if (rc) return rc;
+    memset(out, 0, sizeof *out);
+    fill_result(SVB_OUTS, out, ctx->svb_dev_out, SGPU_WANT_SVBZD, false);
     return SGPU_OK;
 }
 

@@ -177,6 +177,13 @@ struct SvbScratch {
 uint64_t svbzd_max_blocks(uint64_t max_samples, uint32_t max_reads);
 uint32_t svbzd_blocks_of(uint64_t n);
 int launch_svbzd_decode(const SvbBatch& s, SvbScratch& w, Scratch& sc, int16_t* samples, int sm_count, cudaStream_t st);
+// svbzd.cu encoder (int16 samples -> svb-zd streams in HBM): bytes of the streams of a batch of at most (max_samples,
+// max_reads), 8 bytes of slack included
+uint64_t svbzd_encode_capacity(uint64_t max_samples, uint32_t max_reads);
+// stream r at bytes[comp_off[r] ..], comp_len[r] bytes, zeros up to the next 16-byte boundary; comp_off: [n_reads+1].
+// Every read must satisfy SGPU_SVBZD_MAX_BYTES(read_len) <= 2^32 - 1. Uses w's cnt, base, blk_bytes, blk_gpos, blk_read.
+int launch_svbzd_encode(const DevBatch& b, uint8_t* bytes, uint64_t* comp_off, uint32_t* comp_len, SvbScratch& w,
+                        Scratch& sc, int sm_count, cudaStream_t st);
 
 // live.cu (event detection on signal that arrives in chunks: sgpu_slot_add_live, sgpu_run_device_live)
 constexpr uint32_t LIVE_FLAGS = 7u;        // SGPU_LIVE_START | SGPU_LIVE_END | SGPU_LIVE_RNA
