@@ -213,6 +213,60 @@ typedef struct {
 int  sgpu_run_device_pa(sgpu_ctx_t *ctx, const sgpu_dev_pa_batch_t *batch, uint32_t want, void *stream,
                         sgpu_result_t *out);
 
+/* ---- reads at any sample offset (device-resident) ------------------------------------------------------------
+ * sgpu_run_device and sgpu_run_device_pa need every read_off[r] to be a multiple of SGPU_ALIGN. These two take reads
+ * that start anywhere: trimmed reads (read_off + the adaptor's or the stall's end, computed on the device), packed
+ * arrays without padding (a torch tensor or slice of one, another reader's buffer), overlapping windows.
+ *   - Staging: a gather kernel (its stage in sgpu_stage_times: "stage_reads", counted in n_kernel_launches) copies the
+ *     reads into a staged layout of the context, back to back at
+ *       stage_off[r] = sum over q < r of align_up(staged length of q, SGPU_ALIGN),
+ *     padding with zeros; the existing kernels then run on it unchanged, in the same run on `stream`, without copies
+ *     or host synchronisation. *stage_off receives that DEVICE array of n_reads + 1 entries (stage_off[n_reads]: the
+ *     staged total, at most span), owned by the context and valid until its next run.
+ *   - Results: bit for bit what sgpu_run_device (sgpu_run_device_pa) returns for an aligned copy of the reads in the
+ *     staged layout with the same span (read_off = stage_off, read_off[n_reads] = span), for every want it accepts,
+ *     with the detector, jnn and prefix sets in force, SGPU_PARAM_* and SGPU_F_FORCE_GENERIC. So `pa` of read r is at
+ *     out->pa + stage_off[r] and its jnn segments start at SGPU_JNN_BASE(stage_off[r], r); the other outputs are per
+ *     read or per event. (fixups and seq_order depend on the span, which sets the walker's chunk length.)
+ *   - Host refusals (SGPU_E_INVAL, nothing queued): n_reads > max_reads, span > max_samples or not a multiple of
+ *     SGPU_ALIGN; a NULL pointer the run needs (samples may be NULL when n_samples is 0; offset_f / raw_unit_f are
+ *     needed for EVENTS, PA, STAT and PREFIX); samples not aligned to its element; SGPU_WANT_SVBZD; for the pA entry
+ *     any want but SGPU_WANT_EVENTS.
+ *   - Device refusals: the run never reads outside samples[0 .. n_samples) (no load touches a 16-byte word holding
+ *     none of those elements) and never faults. A read with read_off[r] + read_len[r] > n_samples is staged as an
+ *     empty record and `status` in sgpu_counters reports SGPU_E_INVAL; reads whose staged end would pass span are
+ *     staged as empty records (stage_off clamped to span) and `status` reports SGPU_E_TOOBIG; SGPU_E_INVAL when both
+ *     happen. A refused read stages no samples, so the other reads' results stay exact.
+ *   - Buffers: the first run of either entry allocates, once, the staged offsets and lengths (24 * max_reads + 16
+ *     bytes), and the staged samples: 2 * max_samples bytes of int16 for sgpu_run_device_at, 4 * max_samples bytes of
+ *     floats for sgpu_run_device_pa_at. A context that never calls them allocates nothing for them. */
+typedef struct {
+    const int16_t  *samples;    /* device; any 2-byte-aligned address (a tensor slice is fine) */
+    uint64_t        n_samples;  /* samples[0 .. n_samples) may be read, nothing past it */
+    const uint64_t *read_off;   /* device [n_reads]: ANY sample index; reads may overlap */
+    const uint32_t *read_len;   /* device [n_reads]: read_off[r] + read_len[r] <= n_samples */
+    const float    *offset_f;   /* device [n_reads] */
+    const float    *raw_unit_f; /* device [n_reads] */
+    uint32_t n_reads;
+    uint32_t rna;
+    uint64_t span;              /* host-known bound: >= sum of align_up(read_len[r], SGPU_ALIGN), <= max_samples, a
+                                   multiple of SGPU_ALIGN (e.g. align_up(total samples + 7 * n_reads, SGPU_ALIGN)) */
+} sgpu_dev_reads_t;
+int  sgpu_run_device_at(sgpu_ctx_t *ctx, const sgpu_dev_reads_t *batch, uint32_t want, void *stream,
+                        sgpu_result_t *out, const uint64_t **stage_off);
+/* pA floats at any 4-byte-aligned address and any offset; want must be SGPU_WANT_EVENTS, as in sgpu_run_device_pa */
+typedef struct {
+    const float    *pa;         /* device; any 4-byte-aligned address */
+    uint64_t        n_samples;  /* pa[0 .. n_samples) may be read, nothing past it */
+    const uint64_t *read_off;   /* device [n_reads]: ANY sample index; reads may overlap */
+    const uint32_t *read_len;   /* device [n_reads] */
+    uint32_t n_reads;
+    uint32_t rna;
+    uint64_t span;              /* as in sgpu_dev_reads_t */
+} sgpu_dev_pa_reads_t;
+int  sgpu_run_device_pa_at(sgpu_ctx_t *ctx, const sgpu_dev_pa_reads_t *batch, uint32_t want, void *stream,
+                           sgpu_result_t *out, const uint64_t **stage_off);
+
 /* Device-resident svb-zd decode (benchmarks / callers that hold the compressed records in HBM). All pointers are
  * DEVICE pointers; `bytes` holds the streams back to back, each starting on a 16-byte boundary, and its
  * allocation extends at least 8 bytes past n_bytes. n_blocks = sum over reads of ceil(read_len / 1024).
@@ -366,7 +420,9 @@ typedef struct {
     uint64_t n_fixups;            /* detector chunks with a boundary-state mismatch */
     uint64_t n_kernel_launches;   /* kernels launched by the last run */
     int32_t  status;              /* 0 or SGPU_E_EVCAP / SGPU_E_SCRATCH reported by the device; after a live run also
-                                     SGPU_E_INVAL / SGPU_E_STATE / SGPU_E_TOOBIG for refused entries */
+                                     SGPU_E_INVAL / SGPU_E_STATE / SGPU_E_TOOBIG for refused entries, after
+                                     sgpu_run_device_at / sgpu_run_device_pa_at SGPU_E_INVAL / SGPU_E_TOOBIG for
+                                     refused reads */
     uint64_t n_long_jobs;         /* stretches of the long peak detector (events.c:414-437) that were replayed with the
                                      reference's own operations because their t-statistic may exceed its threshold */
 } sgpu_counters_t;

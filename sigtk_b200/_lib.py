@@ -28,7 +28,7 @@ EXPORTS = (
     "sgpu_slot_add_read_svbzd", "sgpu_decode_svbzd_device", "sgpu_set_param", "sgpu_slot_add_read_pa",
     "sgpu_run_device_pa", "sgpu_live_open", "sgpu_slot_add_live", "sgpu_wait_live", "sgpu_run_device_live",
     "sgpu_slot_add_live_pa", "sgpu_run_device_live_pa", "sgpu_set_detector", "sgpu_set_jnn", "sgpu_set_prefix",
-    "sgpu_slot_svbzd", "sgpu_encode_svbzd_device",
+    "sgpu_slot_svbzd", "sgpu_encode_svbzd_device", "sgpu_run_device_at", "sgpu_run_device_pa_at",
 )
 PARAM_CHUNK_LEN, PARAM_WARMUP, PARAM_THR_LONG, PARAM_PORE, PARAM_STAT_CTA_MIN = 1, 2, 3, 4, 5  # sgpu_set_param keys (development / test parameters)
 
@@ -67,6 +67,21 @@ class DevPaBatch(C.Structure):  # sgpu_dev_pa_batch_t
     _fields_ = [
         ("pa", C.c_void_p), ("read_off", C.c_void_p), ("read_len", C.c_void_p), ("n_reads", C.c_uint32),
         ("rna", C.c_uint32), ("span", C.c_uint64),
+    ]
+
+
+class DevReads(C.Structure):  # sgpu_dev_reads_t: int16 reads at any sample offset
+    _fields_ = [
+        ("samples", C.c_void_p), ("n_samples", C.c_uint64), ("read_off", C.c_void_p), ("read_len", C.c_void_p),
+        ("offset_f", C.c_void_p), ("raw_unit_f", C.c_void_p), ("n_reads", C.c_uint32), ("rna", C.c_uint32),
+        ("span", C.c_uint64),
+    ]
+
+
+class DevPaReads(C.Structure):  # sgpu_dev_pa_reads_t: pA reads at any sample offset
+    _fields_ = [
+        ("pa", C.c_void_p), ("n_samples", C.c_uint64), ("read_off", C.c_void_p), ("read_len", C.c_void_p),
+        ("n_reads", C.c_uint32), ("rna", C.c_uint32), ("span", C.c_uint64),
     ]
 
 
@@ -174,6 +189,10 @@ def load() -> C.CDLL:
     lib.sgpu_slot_add_read_pa.restype = C.c_int64
     lib.sgpu_run_device_pa.argtypes = [vp, C.POINTER(DevPaBatch), u32, vp, C.POINTER(Result)]
     lib.sgpu_run_device_pa.restype = i32
+    lib.sgpu_run_device_at.argtypes = [vp, C.POINTER(DevReads), u32, vp, C.POINTER(Result), C.POINTER(vp)]
+    lib.sgpu_run_device_at.restype = i32
+    lib.sgpu_run_device_pa_at.argtypes = [vp, C.POINTER(DevPaReads), u32, vp, C.POINTER(Result), C.POINTER(vp)]
+    lib.sgpu_run_device_pa_at.restype = i32
     lib.sgpu_decode_svbzd_device.argtypes = [vp, C.POINTER(SvbDevBatch), vp, vp]
     lib.sgpu_decode_svbzd_device.restype = i32
     lib.sgpu_submit.argtypes = [vp, u32, u32]

@@ -355,6 +355,30 @@ class Context:
         self._check(self._lib.sgpu_run_device_pa(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res)))
         return res
 
+    def run_device_at(self, samples_ptr: int, n_samples: int, read_off_ptr: int, read_len_ptr: int, offset_ptr: int,
+                      unit_ptr: int, n_reads: int, span: int, rna: int, want: int,
+                      stream: int = 0) -> Tuple[_lib.Result, int]:
+        """sgpu_run_device_at: int16 reads at ANY sample offset of samples[0 .. n_samples) (a packed tensor, trimmed
+        reads, overlapping windows), staged by the library into its aligned layout; span: a bound on the staged total
+        (>= sum of align_up(read_len, ALIGN), a multiple of ALIGN). -> (device result as run_device, device pointer of
+        stage_off: n_reads + 1 uint64, pa of read r at pa + stage_off[r], jnn segments at SGPU_JNN_BASE(stage_off[r], r))"""
+        db = _lib.DevReads(samples_ptr, n_samples, read_off_ptr, read_len_ptr, offset_ptr, unit_ptr, n_reads, int(rna),
+                           span)
+        res, off = _lib.Result(), C.c_void_p()
+        self._check(self._lib.sgpu_run_device_at(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res),
+                                                 C.byref(off)))
+        return res, int(off.value or 0)
+
+    def run_device_pa_at(self, pa_ptr: int, n_samples: int, read_off_ptr: int, read_len_ptr: int, n_reads: int,
+                         span: int, rna: int, want: int = WANT_EVENTS, stream: int = 0) -> Tuple[_lib.Result, int]:
+        """sgpu_run_device_pa_at: events of pA reads at ANY offset of pa[0 .. n_samples); -> (device result as
+        run_device_pa, device pointer of stage_off)"""
+        db = _lib.DevPaReads(pa_ptr, n_samples, read_off_ptr, read_len_ptr, n_reads, int(rna), span)
+        res, off = _lib.Result(), C.c_void_p()
+        self._check(self._lib.sgpu_run_device_pa_at(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res),
+                                                    C.byref(off)))
+        return res, int(off.value or 0)
+
     def encode_svbzd_device(self, samples_ptr: int, read_off_ptr: int, read_len_ptr: int, n_reads: int, span: int,
                             stream: int = 0) -> _lib.SvbResult:
         """sgpu_encode_svbzd_device: the svb-zd streams of int16 reads already in device memory (read_off multiples of

@@ -212,6 +212,7 @@ struct sgpu_ctx {
     DevBuf<uint32_t> ent_ovf;    // overflow histograms of ent_kernel (allocated on first use, kept all-zero)
     PaScratch pa{};              // workspace of the pA-input path (allocated on first use)
     LiveScratch live{};          // channel table and workspace of live runs (sgpu_live_open)
+    StageScratch stage{};        // staged layout of reads at any offset (allocated on first use, stage.cu)
     DevBuf<void> live_dev_out[N_LIVE_OUT];    // outputs of sgpu_run_device_live
     uint64_t live_dev_cap = 0;
     std::unique_ptr<uint32_t[]> live_mirror;  // [n_channels] nopen of every channel after the submitted live slots
@@ -370,6 +371,27 @@ int alloc_pa_scratch(sgpu_ctx* ctx) {
     return SGPU_OK;
 }
 
+// The staged layout of sgpu_run_device_at (f32: of sgpu_run_device_pa_at), allocated on the first run that needs it.
+int alloc_stage(sgpu_ctx* ctx, bool f32) {
+    StageScratch& w = ctx->stage;
+    CU(f32 ? w.f32.ensure(ctx->max_samples) : w.i16.ensure(ctx->max_samples));
+    CU(w.off.ensure((uint64_t)ctx->max_reads + 1));
+    CU(w.len.ensure(ctx->max_reads));
+    CU(w.grp.ensure(ctx->max_reads));
+    CU(w.goff.ensure((uint64_t)ctx->max_reads + 1));
+    return SGPU_OK;
+}
+
+// The host checks of both entries for reads at any offset: the batch fits the context, the pointers the run needs
+// are there (`calibration`: false when the want reads offset_f / raw_unit_f and one is NULL), the samples are aligned
+// to their element of `elem` bytes.
+bool reads_at_ok(const sgpu_ctx* ctx, const void* samples, uint64_t n_samples, const void* read_off,
+                 const void* read_len, bool calibration, size_t elem, uint32_t n_reads, uint64_t span) {
+    if (n_reads > ctx->max_reads || span > ctx->max_samples || (span & (SGPU_ALIGN - 1))) return false;
+    if (reinterpret_cast<uintptr_t>(samples) % elem) return false;
+    return n_reads == 0 || (read_off && read_len && calibration && (samples || n_samples == 0));
+}
+
 // The general route keeps its prefix sums and t-statistics at the reads' own offsets, so the sequential-order scratch
 // must hold the whole span. Contexts over 64 Mi samples start with an eighth of that (sgpu_create); the first batch on
 // the general route (pA records, or a batch with a detector set) that needs more grows it to max_samples for the rest
@@ -448,10 +470,11 @@ int encode_svbzd(sgpu_ctx* ctx, const DevBatch& b, DevBuf<void>* o, StageMarks& 
 // The kernel sequence of one batch into the device outputs `o` (and the svb-zd streams into `enc`). No host
 // synchronisation, no host<->device copies (except when the general route's scratch grows). set: the caller's detector
 // set, whose events take the general route, or nullptr: the reference's sets on the fast path. jnn: the caller's jnn
-// set, or nullptr: jnn_print's (b.rna).
+// set, or nullptr: jnn_print's (b.rna). at: the caller's reads at any offset, which the run first stages into b's
+// arrays (ctx->stage), or nullptr.
 int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* o, DevBuf<void>* enc, cudaStream_t st,
                  const DetParams* set, const JnnParams* jnn, const PrefixParams* prefix, const SvbBatch* svb = nullptr,
-                 int16_t* svb_out = nullptr) {
+                 int16_t* svb_out = nullptr, const StageSrc* at = nullptr) {
     Scratch& sc = ctx->sc;
     if (!fits(ctx, b)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
@@ -460,6 +483,7 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
         if (const int rc = prepare_general(ctx, b.span)) return rc;
     StageMarks marks(ctx, st);
     if (const int rc = marks.start()) return rc;
+    if (at) marks.done("stage_reads", launch_stage_reads(*at, false, ctx->stage, sc, ctx->sm_count, st));
     const bool empty = b.n_reads == 0 || b.span == 0;
     if (svb && !empty) marks.done("svbzd_decode", launch_svbzd_decode(*svb, ctx->svb, ctx->sc, svb_out, ctx->sm_count, st));
     if (want & SGPU_WANT_SVBZD)  // (also for empty records: each has its 4-byte stream)
@@ -529,15 +553,16 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
 
 // The kernel sequence of a batch of pA records (getevents(n, pa, rna), events.c:553-573) into the device outputs `o`:
 // the general route (set: the caller's detector set, or nullptr: the reference's chosen by b.rna). No host
-// synchronisation, no host<->device copies (except when the scratch grows).
+// synchronisation, no host<->device copies (except when the scratch grows). at: as for run_pipeline.
 int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetParams* set, uint32_t want,
-                    DevBuf<void>* o, cudaStream_t st) {
+                    DevBuf<void>* o, cudaStream_t st, const StageSrc* at = nullptr) {
     if (!fits(ctx, b) || (b.n_reads && b.span && !pa)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
     int rc = prepare_general(ctx, b.span);
     if (rc) return rc;
     StageMarks marks(ctx, st);
     if ((rc = marks.start())) return rc;
+    if (at) marks.done("stage_reads", launch_stage_reads(*at, true, ctx->stage, ctx->sc, ctx->sm_count, st));
     if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
     if ((rc = general_events(ctx, b, pa, set, o, marks))) return rc;
     return marks.finish();
@@ -1081,6 +1106,50 @@ int sgpu_run_device_pa(sgpu_ctx_t* ctx, const sgpu_dev_pa_batch_t* batch, uint32
     if (rc) return rc;
     memset(out, 0, sizeof *out);
     fill_result(OUTS, out, ctx->dev_out, want, false);
+    return SGPU_OK;
+}
+
+int sgpu_run_device_at(sgpu_ctx_t* ctx, const sgpu_dev_reads_t* batch, uint32_t want, void* stream, sgpu_result_t* out,
+                       const uint64_t** stage_off) {
+    if (!ctx || !batch || !out || !stage_off || (want & ~63u) || want == 0) return SGPU_E_INVAL;
+    const bool calibration = (batch->offset_f && batch->raw_unit_f) ||
+                             !(want & (SGPU_WANT_EVENTS | SGPU_WANT_PA | SGPU_WANT_STAT | SGPU_WANT_PREFIX));
+    if (!reads_at_ok(ctx, batch->samples, batch->n_samples, batch->read_off, batch->read_len, calibration,
+                     sizeof(int16_t), batch->n_reads, batch->span))
+        return SGPU_E_INVAL;
+    CU(cudaSetDevice(ctx->device));
+    if (const int rc = alloc_stage(ctx, false)) return rc;
+    StageScratch& w = ctx->stage;
+    const StageSrc at{batch->samples, batch->n_samples, batch->read_off, batch->read_len, batch->n_reads, batch->span};
+    const DevBatch b{w.i16, w.off, w.len, batch->offset_f, batch->raw_unit_f, batch->n_reads, (int)batch->rna,
+                     batch->span};
+    const int rc = run_pipeline(ctx, b, want, ctx->dev_out, nullptr, reinterpret_cast<cudaStream_t>(stream),
+                                ctx->det_on ? &ctx->det : nullptr, ctx->jnn_on ? &ctx->jnn : nullptr,
+                                ctx->prefix_on ? &ctx->prefix : nullptr, nullptr, nullptr, &at);
+    if (rc) return rc;
+    memset(out, 0, sizeof *out);
+    fill_result(OUTS, out, ctx->dev_out, want, true);
+    *stage_off = w.off;
+    return SGPU_OK;
+}
+
+int sgpu_run_device_pa_at(sgpu_ctx_t* ctx, const sgpu_dev_pa_reads_t* batch, uint32_t want, void* stream,
+                          sgpu_result_t* out, const uint64_t** stage_off) {
+    if (!ctx || !batch || !out || !stage_off || !pa_input_want_ok(want)) return SGPU_E_INVAL;
+    if (!reads_at_ok(ctx, batch->pa, batch->n_samples, batch->read_off, batch->read_len, true, sizeof(float),
+                     batch->n_reads, batch->span))
+        return SGPU_E_INVAL;
+    CU(cudaSetDevice(ctx->device));
+    if (const int rc = alloc_stage(ctx, true)) return rc;
+    StageScratch& w = ctx->stage;
+    const StageSrc at{batch->pa, batch->n_samples, batch->read_off, batch->read_len, batch->n_reads, batch->span};
+    const DevBatch b{nullptr, w.off, w.len, nullptr, nullptr, batch->n_reads, (int)batch->rna, batch->span};
+    const int rc = run_pipeline_pa(ctx, b, w.f32, ctx->det_on ? &ctx->det : nullptr, want, ctx->dev_out,
+                                   reinterpret_cast<cudaStream_t>(stream), &at);
+    if (rc) return rc;
+    memset(out, 0, sizeof *out);
+    fill_result(OUTS, out, ctx->dev_out, want, false);
+    *stage_off = w.off;
     return SGPU_OK;
 }
 

@@ -245,6 +245,26 @@ struct LiveScratch {                       // allocated by sgpu_live_open
 int launch_live(const LiveBatch& b, bool pa, const DetParams* set, LiveScratch& w, Scratch& sc, uint64_t* ev_off,
                 uint32_t* ev_start, uint32_t* ev_len, float* ev_mean, float* ev_stdv, int sm_count, cudaStream_t st);
 
+// stage.cu (reads at any sample offset: sgpu_run_device_at, sgpu_run_device_pa_at)
+struct StageSrc {                          // read r is src[read_off[r] .. read_off[r] + read_len[r]) (reads may overlap)
+    const void* src;                       // int16_t or float elements, at any address aligned to the element
+    uint64_t n_elems;                      // src[0 .. n_elems) may be read, nothing past it
+    const uint64_t* read_off;              // [n_reads] any element index
+    const uint32_t* read_len;              // [n_reads]
+    uint32_t n_reads;
+    uint64_t span;                         // the staged batch's span (a multiple of 8, at most max_samples)
+};
+struct StageScratch {                      // allocated on the first run that stages reads
+    DevBuf<int16_t> i16;                   // [max_samples] staged int16 samples (sgpu_run_device_at)
+    DevBuf<float> f32;                     // [max_samples] staged pA floats (sgpu_run_device_pa_at)
+    DevBuf<uint64_t> off;                  // [max_reads+1] staged offsets (the caller's *stage_off)
+    DevBuf<uint32_t> len;                  // [max_reads] staged lengths: read_len, 0 for a refused read
+    DevBuf<uint32_t> grp;                  // [max_reads] 8-sample groups of every read
+    DevBuf<uint64_t> goff;                 // [max_reads+1] their exclusive scan
+};
+// stages s into w.off / w.len and w.f32 (f32) or w.i16; refused reads become empty records and set sc.status
+int launch_stage_reads(const StageSrc& s, bool f32, StageScratch& w, Scratch& sc, int sm_count, cudaStream_t st);
+
 // stat.cu
 constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;
 int launch_stat_moments(const DevBatch& b, float* stat6, uint32_t cta_min, int sm_count, cudaStream_t st);
