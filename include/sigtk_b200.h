@@ -75,6 +75,8 @@ extern "C" {
 #define SGPU_F_STAGE_TIMERS  4u /* record CUDA events between the kernel groups of a run (sgpu_stage_times) */
 #define SGPU_F_FULL_SEQ_SCRATCH 8u /* size the sequential-order scratch for the whole batch (a context opened for one
                                       huge read: the reference handles any read < 2^31 samples, misc.c:20) */
+#define SGPU_F_PA_STAT      16u /* pA records (host slots, sgpu_run_device_pa, sgpu_run_device_pa_at) also compute
+                                   SGPU_WANT_STAT: see SGPU_PA_STAT. Without it they compute SGPU_WANT_EVENTS only. */
 
 typedef struct sgpu_ctx sgpu_ctx_t;
 
@@ -108,7 +110,9 @@ typedef struct {
     float    *ev_mean;     /* [n_events] */
     float    *ev_stdv;     /* [n_events] */
     float    *pa;          /* same layout as samples; NULL unless SGPU_WANT_PA */
-    float    *stat;        /* [n_reads][6]: raw_mean, pa_mean, raw_std, pa_std, raw_median, pa_median */
+    float    *stat;        /* [n_reads][6]: raw_mean, pa_mean, raw_std, pa_std, raw_median, pa_median. For pA records
+                              (SGPU_F_PA_STAT, SGPU_PA_STAT below) columns 1, 3, 5 are meanf, stdvf, medianf of
+                              the floats and columns 0, 2, 4 a quiet NaN: there is no raw signal. */
     uint32_t *seq_order;   /* [n_reads] 1 if the read went through the sequential-order kernels
                               (exact-sum witness failed, or forced); such reads are still bit-exact */
     uint32_t *fixups;      /* [n_reads] number of detector chunks whose warm-up state did not match (the read is then redone
@@ -162,7 +166,8 @@ int64_t sgpu_slot_add_read_svbzd(sgpu_ctx_t *ctx, uint32_t slot, const uint8_t *
 /* Append one record given as pA floats: getevents(n, pa, rna) (events.c:553-573) on the caller's own signal
  * (calibrated, normalised, simulated or filtered), where the other entry points take int16 raw samples. Such a slot
  * holds pA records only (SGPU_E_STATE when mixed with decoded records or svb-zd streams) and computes
- * SGPU_WANT_EVENTS only (sgpu_submit returns SGPU_E_INVAL for any other bit). The floats are kept in the slot's
+ * SGPU_WANT_EVENTS; in a context opened with SGPU_F_PA_STAT also SGPU_WANT_STAT, alone or with EVENTS (see
+ * SGPU_PA_STAT below). sgpu_submit returns SGPU_E_INVAL for any other bit. The floats are kept in the slot's
  * sample buffers: a slot holds max_samples / 2 pA samples, every read padded to SGPU_ALIGN of them (SGPU_E_FULL when
  * the next read does not fit, SGPU_E_TOOBIG when align_up(n, SGPU_ALIGN) > max_samples / 2). Results are bit-identical
  * to the reference's for every finite input; with NaN or Inf in the input the event boundaries are identical and the
@@ -196,12 +201,30 @@ int  sgpu_run_device(sgpu_ctx_t *ctx, const sgpu_dev_batch_t *batch, uint32_t wa
 
 /* Device-resident event detection on the caller's pA floats (see sgpu_slot_add_read_pa): read r occupies
  * pa[read_off[r] .. read_off[r]+read_len[r]), every read_off[r] a multiple of SGPU_ALIGN -- the layout of the `pa`
- * output, so the pA of an int16 run can be fed straight back in. span <= max_samples. want must be SGPU_WANT_EVENTS.
- * Runs on `stream` without copies or synchronisation, like sgpu_run_device; *out receives the event table, seq_order
- * (1: the read's prefix sums were formed in the reference's order because a parallel scan could round) and fixups
- * (detector chunks whose warm-up state did not match), the other pointers NULL. The first batch whose span exceeds the
- * context's sequential-order scratch (an eighth of max_samples above 64 Mi samples) grows it to max_samples, which
- * allocates and synchronises the device once. */
+ * output, so the pA of an int16 run can be fed straight back in. span <= max_samples. want is SGPU_WANT_EVENTS;
+ * with SGPU_F_PA_STAT it may also be SGPU_WANT_STAT or both (SGPU_E_INVAL otherwise). Runs on `stream` without copies or synchronisation, like
+ * sgpu_run_device; *out receives, for EVENTS, the event table, seq_order (1: the read's prefix sums were formed in the
+ * reference's order because a parallel scan could round) and fixups (detector chunks whose warm-up state did not
+ * match); for STAT, `stat`; the other pointers NULL. The first EVENTS batch whose span exceeds the context's
+ * sequential-order scratch (an eighth of max_samples above 64 Mi samples) grows it to max_samples, which allocates and
+ * synchronises the device once; a STAT-only run neither prepares nor grows that scratch and runs no event kernel.
+ *
+ * SGPU_PA_STAT -- the statistics of pA records (host slots, sgpu_run_device_pa, sgpu_run_device_pa_at) in a context
+ * opened with SGPU_F_PA_STAT (a context without it refuses SGPU_WANT_STAT on pA records, as before): stat_func's
+ * float functions (cfunc.c:126-159, stat.h:17-24, 36-44, 56-64) on the caller's floats. Per read, stat[r][1] =
+ * meanf(pa, n), stat[r][3] = stdvf(pa, n), stat[r][5] = medianf(pa, n), the element of rank n/2 (ks_ksmall,
+ * ksort.h:233-259); stat[r][0], [2], [4] hold a quiet NaN.
+ *   - For finite input the mean and stdv are bit-identical to the reference's sequential float loops, subnormals
+ *     included (nothing is flushed to zero). The median is bit-identical, except that when the element of rank n/2 is
+ *     a zero and the read holds zeros of both signs, -0 is taken to come before +0 (the reference's quick-select may
+ *     return either).
+ *   - With NaN or Inf in the input the mean and stdv are NaN or Inf where the reference's are. A read holding a NaN
+ *     gets a NaN median: the reference's quick-select answer then depends on where the NaNs sit, so this is a
+ *     deliberate difference, as the NaN rule of the event table is.
+ *   - An empty record gives what an int16 record gives: mean and stdv 0/0 (NaN), median 0; in a batch of nothing but
+ *     empty records every column is 0, as for int16 records.
+ *   - The detector set, SGPU_F_FORCE_GENERIC and rna do not change them; SGPU_PARAM_STAT_CTA_MIN picks the warp or
+ *     CTA role as for int16 records. Stages "stat_pa_moments" (1 launch) and "stat_pa_median" (2 launches). */
 typedef struct {
     const float    *pa;         /* device */
     const uint64_t *read_off;   /* device [n_reads+1] */
@@ -231,7 +254,7 @@ int  sgpu_run_device_pa(sgpu_ctx_t *ctx, const sgpu_dev_pa_batch_t *batch, uint3
  *   - Host refusals (SGPU_E_INVAL, nothing queued): n_reads > max_reads, span > max_samples or not a multiple of
  *     SGPU_ALIGN; a NULL pointer the run needs (samples may be NULL when n_samples is 0; offset_f / raw_unit_f are
  *     needed for EVENTS, PA, STAT and PREFIX); samples not aligned to its element; SGPU_WANT_SVBZD; for the pA entry
- *     any want but SGPU_WANT_EVENTS.
+ *     any want but SGPU_WANT_EVENTS (and SGPU_WANT_STAT with SGPU_F_PA_STAT).
  *   - Device refusals: the run never reads outside samples[0 .. n_samples) (no load touches a 16-byte word holding
  *     none of those elements) and never faults. A read with read_off[r] + read_len[r] > n_samples is staged as an
  *     empty record and `status` in sgpu_counters reports SGPU_E_INVAL; reads whose staged end would pass span are
@@ -254,7 +277,8 @@ typedef struct {
 } sgpu_dev_reads_t;
 int  sgpu_run_device_at(sgpu_ctx_t *ctx, const sgpu_dev_reads_t *batch, uint32_t want, void *stream,
                         sgpu_result_t *out, const uint64_t **stage_off);
-/* pA floats at any 4-byte-aligned address and any offset; want must be SGPU_WANT_EVENTS, as in sgpu_run_device_pa */
+/* pA floats at any 4-byte-aligned address and any offset; want as in sgpu_run_device_pa (SGPU_WANT_EVENTS;
+ * SGPU_WANT_STAT too with SGPU_F_PA_STAT) */
 typedef struct {
     const float    *pa;         /* device; any 4-byte-aligned address */
     uint64_t        n_samples;  /* pa[0 .. n_samples) may be read, nothing past it */

@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(_HERE, "libsigtk_b200.so")
 
 WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, WANT_SVBZD = 1, 2, 4, 8, 16, 32, 64
 F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS = 0, 1, 2, 4
+F_PA_STAT = 16  # pA records also compute WANT_STAT
 ALIGN = 8
 
 E_FULL, E_TOOBIG = -4, -5

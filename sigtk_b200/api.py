@@ -18,7 +18,7 @@ from typing import List, NamedTuple, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_STAGE_TIMERS, LIVE_END, LIVE_RNA, LIVE_START,
+from ._lib import (ALIGN, F_DEFAULT, F_FORCE_GENERIC, F_NO_HOST_SLOTS, F_PA_STAT, F_STAGE_TIMERS, LIVE_END, LIVE_RNA, LIVE_START,
                    WANT_EVENTS, WANT_PA, WANT_STAT, WANT_ENT, WANT_JNN, WANT_PREFIX, WANT_SVBZD, SgpuError)
 
 Read = Tuple[np.ndarray, float, float, float]  # raw int16, digitisation, offset, range
@@ -205,7 +205,8 @@ class Context:
             self._check(int(self._lib.sgpu_slot_add_read_pa(self._h, slot, pa.ctypes.data, pa.shape[0])))
 
     def run_pa(self, signals: Sequence[np.ndarray], rna: int = 0, want: int = WANT_EVENTS, slot: int = 0) -> BatchResult:
-        """fill_pa + submit + wait: the event tables of records given as pA floats"""
+        """fill_pa + submit + wait: the event tables (WANT_EVENTS) and, in a context opened with F_PA_STAT,
+        statistics (WANT_STAT) of records given as pA floats"""
         self.fill_pa(slot, signals, rna)
         self.submit(slot, want)
         return self.wait(slot, want)
@@ -349,7 +350,8 @@ class Context:
 
     def run_device_pa(self, pa_ptr: int, read_off_ptr: int, read_len_ptr: int, n_reads: int, span: int, rna: int,
                       want: int = WANT_EVENTS, stream: int = 0) -> _lib.Result:
-        """sgpu_run_device_pa: events of pA floats already in device memory (read_off multiples of ALIGN)"""
+        """sgpu_run_device_pa: events and / or statistics of pA floats already in device memory (read_off multiples of
+        ALIGN)"""
         db = _lib.DevPaBatch(pa_ptr, read_off_ptr, read_len_ptr, n_reads, int(rna), span)
         res = _lib.Result()
         self._check(self._lib.sgpu_run_device_pa(self._h, C.byref(db), want, C.c_void_p(stream), C.byref(res)))
@@ -371,7 +373,7 @@ class Context:
 
     def run_device_pa_at(self, pa_ptr: int, n_samples: int, read_off_ptr: int, read_len_ptr: int, n_reads: int,
                          span: int, rna: int, want: int = WANT_EVENTS, stream: int = 0) -> Tuple[_lib.Result, int]:
-        """sgpu_run_device_pa_at: events of pA reads at ANY offset of pa[0 .. n_samples); -> (device result as
+        """sgpu_run_device_pa_at: events and / or statistics of pA reads at ANY offset of pa[0 .. n_samples); -> (device result as
         run_device_pa, device pointer of stage_off)"""
         db = _lib.DevPaReads(pa_ptr, n_samples, read_off_ptr, read_len_ptr, n_reads, int(rna), span)
         res, off = _lib.Result(), C.c_void_p()
@@ -463,6 +465,12 @@ def getevents_pa(ctx: Context, pa: np.ndarray, rna: int = 0) -> EventTable:
 def stat(ctx: Context, raw: np.ndarray, digitisation: float, offset: float, range_: float) -> np.ndarray:
     """The six numbers of stat_func (cfunc.c:126-159) for one record."""
     return ctx.run([(raw, digitisation, offset, range_)], 0, WANT_STAT).stat[0]
+
+
+def stat_pa(ctx: Context, pa: np.ndarray) -> np.ndarray:
+    """meanf, stdvf, medianf (stat.h:17-64) of one record given as pA floats: float32[3]. ctx: opened with
+    F_PA_STAT."""
+    return ctx.run_pa([pa], 0, WANT_STAT).stat[0, [1, 3, 5]]
 
 
 def ent(ctx: Context, raw: np.ndarray) -> np.ndarray:

@@ -62,7 +62,7 @@ constexpr OutSpec OUTS[] = {  // in the order of Out
     OUTPUT(ev_stdv,     SGPU_WANT_EVENTS, TOTAL,        1,   true,  -1,           true),
     OUTPUT(seq_order,   SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
     OUTPUT(fixups,      SGPU_WANT_EVENTS, READS,        1,   true,  0,            true),
-    OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0,            false),
+    OUTPUT(stat,        SGPU_WANT_STAT,   READS,        6,   true,  0,            true),   // pA: columns 1, 3, 5
     OUTPUT(ent,         SGPU_WANT_ENT,    READS,        3,   false, 0,            false),
     OUTPUT(jnn_cnt,     SGPU_WANT_JNN,    READS,        1,   false, 0,            false),
     OUTPUT(jnn_seg,     SGPU_WANT_JNN,    JNN_SLOTS,    2,   false, -1,           false),
@@ -98,13 +98,19 @@ constexpr OutSpec SVB_OUTS[] = {  // in the order of Svb
 #undef SVB_OUTPUT
 static_assert(sizeof SVB_OUTS / sizeof SVB_OUTS[0] == N_SVB_OUT, "one row per output");
 
-// the products a run on pA input can compute: those of its outputs (the others are defined on int16 raw samples, and
-// pA is the input itself)
+// the products a run on pA input can compute: those of its outputs (ent, jnn and prefix are defined on int16 raw
+// samples, and pA is the input itself)
 constexpr uint32_t pa_input_wants(int k = 0) {
     return k == N_OUT ? 0u : (OUTS[k].pa_in ? OUTS[k].want : 0u) | pa_input_wants(k + 1);
 }
-constexpr bool pa_input_want_ok(uint32_t want) { return want != 0 && (want & ~pa_input_wants()) == 0; }
-static_assert(pa_input_wants() == SGPU_WANT_EVENTS, "a pA run computes the event table only");
+static_assert(pa_input_wants() == (SGPU_WANT_EVENTS | SGPU_WANT_STAT),
+              "a pA run computes the event table and meanf / stdvf / medianf of the records");
+// what a context with `flags` lets a pA run compute: the statistics only when it was opened with SGPU_F_PA_STAT
+// (a context without the flag keeps refusing SGPU_WANT_STAT on pA records, as it always did)
+constexpr uint32_t pa_wants(uint32_t flags) {
+    return (flags & SGPU_F_PA_STAT) ? pa_input_wants() : (pa_input_wants() & ~SGPU_WANT_STAT);
+}
+constexpr bool pa_input_want_ok(uint32_t want, uint32_t flags) { return want != 0 && (want & ~pa_wants(flags)) == 0; }
 
 // elements of output s for a batch of `reads` reads spanning `samples` samples with `events` events; at the
 // context's (max_reads, max_samples) and the table's event capacity this is the output's capacity
@@ -126,8 +132,8 @@ enum class Input : uint8_t { NONE, RAW, SVBZD, PA, LIVE, LIVE_PA };
 
 bool is_live(Input k) { return k == Input::LIVE || k == Input::LIVE_PA; }
 
-uint32_t allowed_wants(Input k) {
-    if (k == Input::PA) return pa_input_wants();
+uint32_t allowed_wants(Input k, uint32_t flags) {
+    if (k == Input::PA) return pa_wants(flags);
     if (is_live(k)) return SGPU_WANT_EVENTS;
     return 127u;
 }
@@ -551,20 +557,27 @@ int run_pipeline(sgpu_ctx* ctx, const DevBatch& b, uint32_t want, DevBuf<void>* 
     return marks.finish();
 }
 
-// The kernel sequence of a batch of pA records (getevents(n, pa, rna), events.c:553-573) into the device outputs `o`:
-// the general route (set: the caller's detector set, or nullptr: the reference's chosen by b.rna). No host
-// synchronisation, no host<->device copies (except when the scratch grows). at: as for run_pipeline.
+// The kernel sequence of a batch of pA records into the device outputs `o`: the event table (getevents(n, pa, rna),
+// events.c:553-573) on the general route (set: the caller's detector set, or nullptr: the reference's chosen by b.rna),
+// and meanf / stdvf / medianf of every record (stat.cu). No host synchronisation, no host<->device copies (except when
+// the general route's scratch grows, which a run without events neither prepares nor grows). at: as for run_pipeline.
 int run_pipeline_pa(sgpu_ctx* ctx, const DevBatch& b, const float* pa, const DetParams* set, uint32_t want,
                     DevBuf<void>* o, cudaStream_t st, const StageSrc* at = nullptr) {
     if (!fits(ctx, b) || (b.n_reads && b.span && !pa)) return SGPU_E_INVAL;
     CU(alloc_outputs(OUTS, ctx, ctx->ev_cap, o, want));
-    int rc = prepare_general(ctx, b.span);
+    const bool events = (want & SGPU_WANT_EVENTS) != 0;
+    int rc = events ? prepare_general(ctx, b.span) : SGPU_OK;
     if (rc) return rc;
     StageMarks marks(ctx, st);
     if ((rc = marks.start())) return rc;
     if (at) marks.done("stage_reads", launch_stage_reads(*at, true, ctx->stage, ctx->sc, ctx->sm_count, st));
     if (b.n_reads == 0 || b.span == 0) return clear_empty_batch(OUTS, b.n_reads, b.span, want, o, marks);
-    if ((rc = general_events(ctx, b, pa, set, o, marks))) return rc;
+    if (want & SGPU_WANT_STAT) {
+        float* const stat = static_cast<float*>(o[STAT].get());
+        marks.done("stat_pa_moments", launch_stat_pa_moments(b, pa, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
+        marks.done("stat_pa_median", launch_stat_pa_median(b, pa, stat, ctx->sc.tune_stat_cta_min, ctx->sm_count, st));
+    }
+    if (events && (rc = general_events(ctx, b, pa, set, o, marks))) return rc;
     return marks.finish();
 }
 
@@ -809,7 +822,7 @@ const char* sgpu_last_error(const sgpu_ctx_t* ctx) { return ctx ? ctx->err : "no
 
 int sgpu_create(sgpu_ctx_t** out, int device, uint64_t max_samples, uint32_t max_reads, uint32_t n_slots,
                 uint32_t flags) {
-    if (!out || max_samples == 0 || max_reads == 0 || (flags & ~15u)) return SGPU_E_INVAL;
+    if (!out || max_samples == 0 || max_reads == 0 || (flags & ~31u)) return SGPU_E_INVAL;
     *out = nullptr;
     if (flags & SGPU_F_NO_HOST_SLOTS) n_slots = 0; else if (n_slots == 0) n_slots = 2;
     sgpu_ctx* ctx = new (std::nothrow) sgpu_ctx();
@@ -1014,7 +1027,7 @@ int sgpu_submit(sgpu_ctx_t* ctx, uint32_t slot, uint32_t want) {
     if (!ctx || slot >= ctx->n_slots || (want & ~127u) || want == 0) return SGPU_E_INVAL;
     Slot& sl = ctx->slots[slot];
     if (sl.submitted) return SGPU_E_STATE;
-    if (want & ~allowed_wants(sl.kind)) return SGPU_E_INVAL;
+    if (want & ~allowed_wants(sl.kind, ctx->flags)) return SGPU_E_INVAL;
     if ((want & SGPU_WANT_SVBZD) && !svbzd_stream_fits(ctx->max_samples))  // (only such a context holds such a read)
         for (uint32_t r = 0; r < sl.batch.n_reads; r++)
             if (!svbzd_stream_fits(sl.batch.read_len[r])) return SGPU_E_TOOBIG;
@@ -1097,7 +1110,7 @@ int sgpu_run_device(sgpu_ctx_t* ctx, const sgpu_dev_batch_t* batch, uint32_t wan
 
 int sgpu_run_device_pa(sgpu_ctx_t* ctx, const sgpu_dev_pa_batch_t* batch, uint32_t want, void* stream,
                        sgpu_result_t* out) {
-    if (!ctx || !batch || !out || !pa_input_want_ok(want)) return SGPU_E_INVAL;
+    if (!ctx || !batch || !out || !pa_input_want_ok(want, ctx->flags)) return SGPU_E_INVAL;
     CU(cudaSetDevice(ctx->device));
     const DevBatch b{nullptr, batch->read_off, batch->read_len, nullptr, nullptr, batch->n_reads, (int)batch->rna,
                      batch->span};
@@ -1135,7 +1148,7 @@ int sgpu_run_device_at(sgpu_ctx_t* ctx, const sgpu_dev_reads_t* batch, uint32_t 
 
 int sgpu_run_device_pa_at(sgpu_ctx_t* ctx, const sgpu_dev_pa_reads_t* batch, uint32_t want, void* stream,
                           sgpu_result_t* out, const uint64_t** stage_off) {
-    if (!ctx || !batch || !out || !stage_off || !pa_input_want_ok(want)) return SGPU_E_INVAL;
+    if (!ctx || !batch || !out || !stage_off || !pa_input_want_ok(want, ctx->flags)) return SGPU_E_INVAL;
     if (!reads_at_ok(ctx, batch->pa, batch->n_samples, batch->read_off, batch->read_len, true, sizeof(float),
                      batch->n_reads, batch->span))
         return SGPU_E_INVAL;

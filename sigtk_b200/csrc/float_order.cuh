@@ -116,6 +116,141 @@ __device__ __forceinline__ bool summarise_superblock(const float* __restrict__ A
 }
 
 
+// ---- signed values: the first pass over the caller's pA floats ---------------------------------------------------------
+// Values of either sign, accumulators of either sign. fl(s + v) = -fl(-s - v), so an accumulator s < 0 is worked as -s
+// with every value negated (the scale carries the sign). Inside the binade of |s| the step is the same integer
+// recurrence as above, S <- RNE(S + x) with x = v * scale, now with x of either sign, and it still depends on nothing
+// but the parity of S -- as long as every exact S + x lies in [2^23, 2^24]. A run can no longer be checked by where it
+// ends (S goes down as well as up), so a summary also carries the lowest (lo) and highest (hi) point of the path
+// relative to its start. The run is added up by the hardware from the middle of the binade, P = 1.5 * 2^23 (even) and
+// P + 1 (odd): while every rounded point of that path lies strictly inside (2^23, 2^24) each exact sum lay in
+// [2^23, 2^24) (rounding is monotone and both ends are floats), where float rounding is the integer recurrence. The
+// path from the real S follows it shifted by S - P; it is exact while S + lo >= 2^23 + 1 and S + hi <= 2^24 - 1
+// (every exact sum then lies within 1/2 of such a point, inside the binade). The path from P can reach 2^22 either
+// way, so only a tile that moves the accumulator by more than a quarter of its magnitude, or that meets a NaN or an
+// infinity, cannot be summarised; a run that would leave the binade of S (zero, a power of two) is added value by value.
+constexpr int SGN_FAR = 1 << 28;    // lo of a run without a point (the identity); larger than any summarised path
+
+struct SgnSum { int inc[2], lo[2], hi[2]; };  // [parity of the incoming S]: increment, lowest and highest point
+
+__device__ __forceinline__ SgnSum sgn_identity() { return SgnSum{{0, 0}, {SGN_FAR, SGN_FAR}, {-SGN_FAR, -SGN_FAR}}; }
+
+// one lane, one tile of 32 values; scale = +-2^(23-e) (the sign of the accumulator); false when it cannot be summarised
+__device__ __forceinline__ bool tile_summary_signed(const float* __restrict__ row, float scale, SgnSum& u) {
+    constexpr float P = 12582912.0f;                  // 1.5 * 2^23
+    float acc0 = P, acc1 = P + 1.0f;
+    float lo0 = 16777216.0f, lo1 = 16777216.0f, hi0 = 8388608.0f, hi1 = 8388608.0f;
+#pragma unroll 8
+    for (int k = 0; k < 32; k++) {
+        const float x = __fmul_rn(row[k], scale);     // exact, or below 2^-126: too small to move S either way
+        acc0 = __fadd_rn(acc0, x);
+        acc1 = __fadd_rn(acc1, x);
+        lo0 = fminf(lo0, acc0); hi0 = fmaxf(hi0, acc0);
+        lo1 = fminf(lo1, acc1); hi1 = fmaxf(hi1, acc1);
+    }
+    // (a NaN stays NaN to the end and fails the first two tests; an infinity fails the bounds)
+    const bool ok = acc0 > 8388608.0f && acc1 > 8388608.0f && lo0 > 8388608.0f && lo1 > 8388608.0f &&
+                    hi0 < 16777216.0f && hi1 < 16777216.0f;
+    if (!ok) { u = sgn_identity(); return false; }
+    u.inc[0] = (int)acc0 - 12582912; u.lo[0] = (int)lo0 - 12582912; u.hi[0] = (int)hi0 - 12582912;
+    u.inc[1] = (int)acc1 - 12582913; u.lo[1] = (int)lo1 - 12582913; u.hi[1] = (int)hi1 - 12582913;
+    return true;
+}
+
+// b after a: the run of a, then the run of b from the parity a leaves
+__device__ __forceinline__ SgnSum sgn_then(const SgnSum& a, const SgnSum& b) {
+    SgnSum c;
+#pragma unroll
+    for (int p = 0; p < 2; p++) {
+        const int d = a.inc[p], q = (p ^ d) & 1;
+        c.inc[p] = d + b.inc[q];
+        c.lo[p] = min(a.lo[p], d + b.lo[q]);
+        c.hi[p] = max(a.hi[p], d + b.hi[q]);
+    }
+    return c;
+}
+
+// whether the run u keeps the path from S strictly inside the binade
+__device__ __forceinline__ bool sgn_fits(const SgnSum& u, uint32_t S) {
+    const int p = (int)(S & 1u);
+    return (int)S + u.lo[p] >= 0x800001 && (int)S + u.hi[p] <= 0xffffff;
+}
+
+__device__ __forceinline__ void compose_signed(SgnSum& u, int lane) {   // inclusive scan over the lanes
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        SgnSum a;
+#pragma unroll
+        for (int p = 0; p < 2; p++) {
+            a.inc[p] = __shfl_up_sync(0xffffffffu, u.inc[p], d);
+            a.lo[p] = __shfl_up_sync(0xffffffffu, u.lo[p], d);
+            a.hi[p] = __shfl_up_sync(0xffffffffu, u.hi[p], d);
+        }
+        if (lane >= d) u = sgn_then(a, u);
+    }
+}
+
+__device__ __forceinline__ bool summable_signed(float s) { return summable(fabsf(s)); }
+
+// the scale of the binade of s, negative for s < 0
+__device__ __forceinline__ float signed_scale(float s) {
+    const uint32_t sb = __float_as_uint(s);
+    const int e = (int)((sb >> 23) & 0xffu) - 127;
+    return __uint_as_float(((uint32_t)(127 + 23 - e) << 23) | (sb & 0x80000000u));
+}
+
+// chain_superblock for addends of either sign
+__device__ __forceinline__ float chain_superblock_signed(const float* __restrict__ A, int ntiles, float s, int lane,
+                                                        bool first) {
+    int tile = 0;
+    while (tile < ntiles) {  // (uniform across the warp)
+        int fail = tile;
+        if (!first && summable_signed(s)) {
+            const uint32_t sb = __float_as_uint(s);
+            uint32_t S = (sb & 0x7fffffu) | 0x800000u;
+            SgnSum u = sgn_identity();  // lanes outside [tile, ntiles) are the identity
+            bool ok = true;
+            if (lane >= tile && lane < ntiles) ok = tile_summary_signed(A + lane * SB_STRIDE, signed_scale(s), u);
+            compose_signed(u, lane);
+            const uint32_t S_after = S + (uint32_t)u.inc[S & 1u];
+            const uint32_t bad = __ballot_sync(0xffffffffu, !ok || !sgn_fits(u, S));
+            fail = bad ? __ffs(bad) - 1 : ntiles;
+            if (fail > tile) S = __shfl_sync(0xffffffffu, S_after, fail - 1);
+            s = __uint_as_float((sb & 0xff800000u) | (S & 0x7fffffu));
+            __syncwarp();
+        }
+        if (fail < ntiles) {
+            if (lane == 0) {
+                const float* row = A + fail * SB_STRIDE;
+#pragma unroll
+                for (int k = 0; k < 32; k++) s = __fadd_rn(s, row[k]);
+            }
+            s = __shfl_sync(0xffffffffu, s, 0);
+            tile = fail + 1;
+        } else {
+            tile = ntiles;
+        }
+    }
+    return s;
+}
+
+// summarise_superblock for addends of either sign (summable_signed(s) holds); the caller checks sgn_fits
+__device__ __forceinline__ bool summarise_superblock_signed(const float* __restrict__ A, int ntiles, float s, int lane,
+                                                            SgnSum& U) {
+    SgnSum u = sgn_identity();
+    bool ok = true;
+    if (lane < ntiles) ok = tile_summary_signed(A + lane * SB_STRIDE, signed_scale(s), u);
+    compose_signed(u, lane);
+#pragma unroll
+    for (int p = 0; p < 2; p++) {
+        U.inc[p] = __shfl_sync(0xffffffffu, u.inc[p], 31);
+        U.lo[p] = __shfl_sync(0xffffffffu, u.lo[p], 31);
+        U.hi[p] = __shfl_sync(0xffffffffu, u.hi[p], 31);
+    }
+    return __ballot_sync(0xffffffffu, !ok) == 0u;
+}
+
+
 constexpr int MED_BINS = 4096;
 // element of rank `rank` (0-based, ascending) of the int16 samples raw[0..n); all threads of the CTA (256 or more) call it.
 // ALIGNED: raw is 16-byte aligned (a read's first sample: 128-bit loads); otherwise any sub-range of a read.

@@ -270,6 +270,12 @@ constexpr uint32_t STAT_CTA_MIN_DEFAULT = 131072u;
 int launch_stat_moments(const DevBatch& b, float* stat6, uint32_t cta_min, int sm_count, cudaStream_t st);
 int launch_stat_median(const DevBatch& b, float* stat6, uint32_t cta_min, int sm_count, cudaStream_t st);
 int launch_jnn_moments(const DevBatch& b, float* moments2, uint32_t cta_min, int sm_count, cudaStream_t st);
+// meanf / stdvf (columns 1, 3) and medianf (column 5) of the caller's pA floats (b's read_off / read_len, the records
+// in pa); columns 0, 2 and 4 get a quiet NaN
+int launch_stat_pa_moments(const DevBatch& b, const float* pa, float* stat6, uint32_t cta_min, int sm_count,
+                           cudaStream_t st);
+int launch_stat_pa_median(const DevBatch& b, const float* pa, float* stat6, uint32_t cta_min, int sm_count,
+                          cudaStream_t st);
 
 // jnn.cu (`sigtk jnn`: band from the clamped signal's mean / stdv, counter machine per read -> (start, end) pairs)
 struct JnnParams {  // jnn_param_t, jnn.h:24-45 (sgpu_jnn_t)

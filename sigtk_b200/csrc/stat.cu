@@ -315,6 +315,328 @@ int launch_stat_median(const DevBatch& b, float* stat6, uint32_t cta_min, int sm
     return 2;
 }
 
+// ---- the statistics of the caller's pA floats: meanf, stdvf, medianf of every record ----------------------------------
+// The same two roles as stat_moments_kernel with one channel; a superblock of 1024 floats is 8 128-bit words per lane
+// (lane L holds the words q*32 + L: floats q*128 + 4L .. +3). The first pass adds values of either sign
+// (chain_superblock_signed / summarise_superblock_signed), the second the squared deviations, which are not negative.
+
+// the addends of one superblock (floats t0 .. t0+1023 of the read) into the warp's shared rows; +0 past the read's end,
+// whatever the padding holds
+template <int PASS>
+__device__ __forceinline__ void fill_pa_addends(const uint4 (&cur)[8], int t0, int n, int lane, float mean,
+                                                float* __restrict__ add) {
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        const uint32_t wd[4] = {cur[q].x, cur[q].y, cur[q].z, cur[q].w};
+#pragma unroll
+        for (int h = 0; h < 4; h++) {
+            const int j = q * 128 + lane * 4 + h;
+            float a = 0.0f;
+            if (t0 + j < n) {
+                a = __uint_as_float(wd[h]);
+                if (PASS) {
+                    const float d = __fsub_rn(a, mean);
+                    a = __fmul_rn(d, d);
+                }
+            }
+            add[(j >> 5) * SB_STRIDE + (j & 31)] = a;
+        }
+    }
+}
+
+__device__ __forceinline__ void load_pa_superblock(const uint4* __restrict__ src, int t, int n_words, int lane,
+                                                   uint4 (&q)[8]) {
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        const int w = (t >> 2) + k * 32 + lane;
+        q[k] = w < n_words ? __ldg(src + w) : make_uint4(0, 0, 0, 0);
+    }
+}
+
+__device__ __forceinline__ void store_pa_moment(float* __restrict__ out, uint32_t r, int pass, float acc, float nf,
+                                                float& mean, bool writer) {
+    if (pass == 0) {
+        mean = __fdiv_rn(acc, nf);
+        if (writer) out[(size_t)r * 6 + 1] = mean;
+    } else if (writer) {
+        out[(size_t)r * 6 + 3] = __fsqrt_rn(__fdiv_rn(acc, nf));
+    }
+}
+
+__device__ __forceinline__ void pa_moments_by_warp(const DevBatch& b, const float* __restrict__ pa,
+                                                   float* __restrict__ out, uint32_t cta_min, float* __restrict__ add,
+                                                   uint32_t warp, uint32_t n_warps, int lane) {
+    for (uint32_t r = warp; r < b.n_reads; r += n_warps) {
+        if (b.read_len[r] >= cta_min) continue;  // the CTA role's
+        const uint4* __restrict__ src = reinterpret_cast<const uint4*>(pa + b.read_off[r]);
+        const int n = (int)b.read_len[r];
+        const int n_words = (n + 3) >> 2;
+        const float nf = (float)n;
+        float mean = 0.0f;
+        uint4 cur[8], nxt[8];
+        load_pa_superblock(src, 0, n_words, lane, cur);
+        for (int pass = 0; pass < 2; pass++) {
+            float acc = 0.0f;
+            for (int t0 = 0; t0 < n; t0 += SB) {
+                __syncwarp();  // the previous superblock's readers are done
+                load_pa_superblock(src, t0 + SB < n ? t0 + SB : 0, n_words, lane, nxt);
+                if (pass) fill_pa_addends<1>(cur, t0, n, lane, mean, add);
+                else fill_pa_addends<0>(cur, t0, n, lane, mean, add);
+#pragma unroll
+                for (int q = 0; q < 8; q++) cur[q] = nxt[q];
+                __syncwarp();
+                const int ntiles = (min(SB, n - t0) + 31) >> 5;
+                acc = pass ? chain_superblock(add, ntiles, acc, lane, t0 == 0)
+                           : chain_superblock_signed(add, ntiles, acc, lane, t0 == 0);
+            }
+            store_pa_moment(out, r, pass, acc, nf, mean, lane == 0);
+        }
+    }
+}
+
+// as moments_by_cta: CW consecutive superblocks per round, summarised in the binade the accumulator has, composed in
+// order by every thread; the first that cannot be composed is added up by its own warp
+__device__ __forceinline__ void pa_moments_by_cta(const DevBatch& b, const float* __restrict__ pa,
+                                                  float* __restrict__ out, uint32_t cta_min, float* __restrict__ add,
+                                                  uint32_t cta, uint32_t n_ctas, int lane, int warp) {
+    __shared__ SgnSum sum_s[2][CW];                  // [round parity][warp]: first pass
+    __shared__ uint32_t sum_u[2][CW][2];             // second pass: [parity of the incoming mantissa]
+    __shared__ uint32_t sum_ok[2][CW];
+    __shared__ float s_bcast;
+    for (uint32_t r = cta; r < b.n_reads; r += n_ctas) {
+        if (b.read_len[r] < cta_min) continue;       // (the same for every thread of the CTA)
+        const uint4* __restrict__ src = reinterpret_cast<const uint4*>(pa + b.read_off[r]);
+        const int n = (int)b.read_len[r];
+        const int n_words = (n + 3) >> 2;
+        const float nf = (float)n;
+        float mean = 0.0f;
+        uint4 cur[8], nxt[8];
+        load_pa_superblock(src, warp * SB, n_words, lane, cur);
+        int rp = 0;
+        __syncthreads();                             // the previous read's last summaries have been read
+        for (int pass = 0; pass < 2; pass++) {
+            float acc = 0.0f;                        // (every thread holds the same value)
+            for (int round0 = 0; round0 < n; round0 += CW * SB, rp ^= 1) {
+                const int t0 = round0 + warp * SB;
+                const int ntiles = t0 < n ? (min(SB, n - t0) + 31) >> 5 : 0;
+                const int active = min(CW, (n - round0 + SB - 1) / SB);
+                load_pa_superblock(src, (round0 + CW * SB < n ? round0 + CW * SB : 0) + warp * SB, n_words, lane, nxt);
+                __syncwarp();                        // this warp's readers of the previous round's addends are done
+                if (ntiles) {
+                    if (pass) fill_pa_addends<1>(cur, t0, n, lane, mean, add);
+                    else fill_pa_addends<0>(cur, t0, n, lane, mean, add);
+                }
+#pragma unroll
+                for (int q = 0; q < 8; q++) cur[q] = nxt[q];
+                __syncwarp();
+                int start = 0;                       // first superblock of the round not yet added
+                while (start < active) {
+                    const bool binade = (pass ? summable(acc) : summable_signed(acc)) && !(round0 == 0 && start == 0);
+                    if (binade && warp >= start && warp < active) {
+                        bool ok;
+                        if (pass) {
+                            uint32_t U0, U1;
+                            ok = summarise_superblock(add, ntiles, acc, lane, U0, U1);
+                            if (lane == 0) { sum_u[rp][warp][0] = U0; sum_u[rp][warp][1] = U1; }
+                        } else {
+                            SgnSum U;
+                            ok = summarise_superblock_signed(add, ntiles, acc, lane, U);
+                            if (lane == 0) sum_s[rp][warp] = U;
+                        }
+                        if (lane == 0) sum_ok[rp][warp] = ok ? 1u : 0u;
+                    }
+                    __syncthreads();
+                    int fail = start;
+                    if (binade) {
+                        const uint32_t sb = __float_as_uint(acc);
+                        uint32_t S = (sb & 0x7fffffu) | 0x800000u;
+                        bool go = true;
+                        for (int w = start; w < active && go; w++) {
+                            uint32_t inc;
+                            if (pass) {
+                                inc = sum_u[rp][w][S & 1u];
+                                go = sum_ok[rp][w] && inc < 0x1000000u && S + inc < 0x1000000u;
+                            } else {
+                                const SgnSum& u = sum_s[rp][w];
+                                inc = (uint32_t)u.inc[S & 1u];
+                                go = sum_ok[rp][w] && sgn_fits(u, S);
+                            }
+                            if (go) { S += inc; fail = w + 1; }
+                        }
+                        acc = __uint_as_float((sb & 0xff800000u) | (S & 0x7fffffu));
+                    }
+                    if (fail < active) {             // this superblock by its own warp, from the accumulator it meets
+                        if (warp == fail) {
+                            const bool first = round0 == 0 && fail == 0;
+                            const float s = pass ? chain_superblock(add, ntiles, acc, lane, first)
+                                                 : chain_superblock_signed(add, ntiles, acc, lane, first);
+                            if (lane == 0) s_bcast = s;
+                        }
+                        __syncthreads();
+                        acc = s_bcast;
+                        start = fail + 1;
+                    } else {
+                        start = active;
+                    }
+                }
+            }
+            store_pa_moment(out, r, pass, acc, nf, mean, threadIdx.x == 0);
+        }
+    }
+}
+
+__global__ void __launch_bounds__(CW * 32, 2) stat_pa_moments_kernel(DevBatch b, const float* __restrict__ pa,
+                                                                     float* __restrict__ out, uint32_t cta_min,
+                                                                     uint32_t cta_blocks) {
+    __shared__ float pa_add[CW][32 * SB_STRIDE];     // every warp's addends of one superblock
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (blockIdx.x < cta_blocks)
+        pa_moments_by_cta(b, pa, out, cta_min, pa_add[warp], blockIdx.x, cta_blocks, lane, warp);
+    else
+        pa_moments_by_warp(b, pa, out, cta_min, pa_add[warp], (blockIdx.x - cta_blocks) * CW + warp,
+                           (gridDim.x - cta_blocks) * CW, lane);
+}
+
+// Median of float records: a radix select over the order-preserving 32-bit key (-0 before +0, NaN outside +-inf), in
+// three levels of 12, 12 and 8 bits; each level counts, among the read's values whose key starts with the bins chosen
+// so far, the next bits into a shared-memory histogram. Only the read's n values are counted, never its padding.
+__device__ __forceinline__ uint32_t f32_key(uint32_t bits) {
+    return bits ^ ((bits & 0x80000000u) ? 0xffffffffu : 0x80000000u);
+}
+
+// the bin of hist[0 .. MED_BINS) that holds `rank` (0-based; fewer than the histogram's count): sh[0] = the bin,
+// sh[1] = the rank within it. All threads of the CTA (256 or more) call it.
+__device__ void rank_bin(const uint32_t* hist, uint32_t rank, uint32_t* part, uint32_t* sh) {
+    if (threadIdx.x < 256) {   // 256 threads x 16 bins
+        uint32_t sum = 0;
+        for (int k = 0; k < MED_BINS / 256; k++) sum += hist[threadIdx.x * (MED_BINS / 256) + k];
+        part[threadIdx.x] = sum;
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        const int lane = threadIdx.x;
+        uint32_t mine = 0;
+#pragma unroll
+        for (int k = 0; k < 8; k++) mine += part[lane * 8 + k];
+        uint32_t incl = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += t;
+        }
+        const uint32_t owner = __ballot_sync(0xffffffffu, incl > rank);
+        if (lane == __ffs(owner) - 1) {
+            uint32_t seen = incl - mine, g = (uint32_t)lane * 8u;
+            for (;; g++) {
+                if (seen + part[g] > rank) break;
+                seen += part[g];
+            }
+            uint32_t k = g * (MED_BINS / 256);
+            for (;; k++) {
+                if (seen + hist[k] > rank) break;
+                seen += hist[k];
+            }
+            sh[0] = k;
+            sh[1] = rank - seen;
+        }
+    }
+    __syncthreads();
+}
+
+// one level: the keys with key >> MATCH == prefix (MATCH = 32: every key) into hist[(key >> BIN) & MASK]; returns
+// whether this thread met a NaN. Four 128-bit loads in flight per thread.
+template <int MATCH, int BIN, uint32_t MASK>
+__device__ __forceinline__ bool count_keys(const uint4* __restrict__ src, uint32_t n, uint32_t prefix, uint32_t* hist) {
+    const uint32_t n_words = (n + 3u) >> 2;
+    bool nan = false;
+    for (uint32_t w0 = threadIdx.x; w0 < n_words; w0 += 4u * blockDim.x) {
+        uint4 q[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const uint32_t w = w0 + (uint32_t)k * blockDim.x;
+            q[k] = w < n_words ? __ldg(src + w) : make_uint4(0, 0, 0, 0);
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const uint32_t w = w0 + (uint32_t)k * blockDim.x;
+            const uint32_t wd[4] = {q[k].x, q[k].y, q[k].z, q[k].w};
+#pragma unroll
+            for (int h = 0; h < 4; h++) {
+                if (w >= n_words || w * 4u + (uint32_t)h >= n) continue;
+                const uint32_t key = f32_key(wd[h]);
+                if (MATCH == 32) nan |= (wd[h] & 0x7fffffffu) > 0x7f800000u;
+                if (MATCH == 32 || (key >> (MATCH & 31)) == prefix) atomicAdd(&hist[(key >> BIN) & MASK], 1u);
+            }
+        }
+    }
+    return nan;
+}
+
+// the element of rank `rank` of x[0 .. n) (16-byte aligned), NaN when the read holds a NaN
+__device__ float select_rank_f32(const float* __restrict__ x, uint32_t n, uint32_t rank, uint32_t* hist,
+                                 uint32_t* part, uint32_t* sh) {
+    const uint4* __restrict__ src = reinterpret_cast<const uint4*>(x);
+    for (int k = threadIdx.x; k < MED_BINS; k += blockDim.x) hist[k] = 0;
+    __syncthreads();
+    if (__syncthreads_or(count_keys<32, 20, 0xfffu>(src, n, 0u, hist))) return __uint_as_float(0x7fc00000u);
+    rank_bin(hist, rank, part, sh);
+    const uint32_t b1 = sh[0], r1 = sh[1];
+    for (int k = threadIdx.x; k < MED_BINS; k += blockDim.x) hist[k] = 0;
+    __syncthreads();
+    count_keys<20, 8, 0xfffu>(src, n, b1, hist);
+    __syncthreads();
+    rank_bin(hist, r1, part, sh);
+    const uint32_t p2 = (b1 << 12) | sh[0], r2 = sh[1];
+    for (int k = threadIdx.x; k < MED_BINS; k += blockDim.x) hist[k] = 0;
+    __syncthreads();
+    count_keys<8, 0, 0xffu>(src, n, p2, hist);
+    __syncthreads();
+    rank_bin(hist, r2, part, sh);
+    const uint32_t key = (p2 << 8) | sh[0];
+    __syncthreads();                                 // sh and hist are free again
+    return __uint_as_float(key ^ ((key & 0x80000000u) ? 0x80000000u : 0xffffffffu));
+}
+
+// reads of lo <= n < hi floats, one CTA of NT threads each; also the raw columns (NaN: there is no raw signal)
+template <int NT>
+__global__ void __launch_bounds__(NT) stat_pa_median_kernel(DevBatch b, const float* __restrict__ pa,
+                                                            float* __restrict__ out, uint32_t lo, uint32_t hi) {
+    __shared__ uint32_t hist[MED_BINS];
+    __shared__ uint32_t part[256];
+    __shared__ uint32_t sh[4];
+    for (uint32_t r = blockIdx.x; r < b.n_reads; r += gridDim.x) {
+        const uint32_t n = b.read_len[r];
+        if (n < lo || n >= hi) continue;
+        // ks_ksmall(n, copy, n/2), stat.h:56-64; an empty record: 0, as for int16 records
+        const float med = n ? select_rank_f32(pa + b.read_off[r], n, (uint32_t)((int)n / 2), hist, part, sh) : 0.0f;
+        if (threadIdx.x == 0) {
+            float* o = out + (size_t)r * 6;
+            const float nan = __uint_as_float(0x7fc00000u);
+            o[0] = nan; o[2] = nan; o[4] = nan;
+            o[5] = med;
+        }
+    }
+}
+
+int launch_stat_pa_moments(const DevBatch& b, const float* pa, float* stat6, uint32_t cta_min, int sm_count,
+                           cudaStream_t st) {
+    if (b.n_reads == 0) return 0;
+    uint32_t g2 = b.n_reads < (uint32_t)sm_count * 2u ? b.n_reads : (uint32_t)sm_count * 2u;
+    uint32_t g1 = (b.n_reads + CW - 1) / CW;         // one warp per read
+    if (g1 > (uint32_t)sm_count * 8u) g1 = (uint32_t)sm_count * 8u;
+    stat_pa_moments_kernel<<<g2 + g1, CW * 32, 0, st>>>(b, pa, stat6, cta_min, g2);
+    return 1;
+}
+
+int launch_stat_pa_median(const DevBatch& b, const float* pa, float* stat6, uint32_t cta_min, int sm_count,
+                          cudaStream_t st) {
+    if (b.n_reads == 0) return 0;
+    int g = (int)b.n_reads;
+    stat_pa_median_kernel<1024><<<g > sm_count * 2 ? sm_count * 2 : g, 1024, 0, st>>>(b, pa, stat6, cta_min, 0xffffffffu);
+    stat_pa_median_kernel<256><<<g > sm_count * 8 ? sm_count * 8 : g, 256, 0, st>>>(b, pa, stat6, 0u, cta_min);
+    return 2;
+}
+
 // mean and standard deviation (float, in the reference's summation order) of the samples clamped to [0, 1200]:
 // what jnn_core derives its band from (jnn.c:58-75, 181-185). moments2 = [n_reads][2].
 int launch_jnn_moments(const DevBatch& b, float* moments2, uint32_t cta_min, int sm_count, cudaStream_t st) {
